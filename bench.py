@@ -1,6 +1,6 @@
 """Headline benchmark: 640x640 tiles/s end to end (preproc + YOLOv8m + decode/filter + NMS + georef).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One step = one pass of the hot path over one batch of 64 synthetic 640x640 uint8 tiles
 (BASELINE.json configs[1]: "YOLOv8 tokyo, synthetic 640x640 tile batch 64 bf16 on 1xB200"),
@@ -159,6 +159,38 @@ def _geo_params(n: int) -> np.ndarray:
         lat0 = 52.2 + 0.0005 * (i // 8)
         p[i, :6] = (lon0, lon0 + 0.00094, lat0, lat0 + 0.000575, 864.0, 640.0)   # a 64 m tile
     return p
+
+
+NPOOL = 4
+
+
+def input_batches(rank: int):
+    """The NPOOL distinct uint8 host batches [BATCH, SIZE, SIZE, 3] the headline steps rotate through (step i reads batch
+    i % NPOOL); seeded, so the same rank gets the same tiles in every run."""
+    import torch
+    from aerial_image_recognition_b200 import synth
+    base = synth.make_tiles(16, SIZE, seed=1000 + rank)
+    out = []
+    for b in range(NPOOL):
+        idx = (np.arange(BATCH) * 7 + b * 3) % 16
+        h = torch.from_numpy(base[idx]).clone()
+        if b % 2:
+            h = torch.flip(h, dims=[2]).contiguous()
+        out.append(h)
+    return out
+
+
+def dump_outputs(out_dir: str, geo, counts) -> None:
+    """Writes one step's result as a caller of Engine.infer + Engine.georef receives it: one ``<field>.npy`` per
+    ``GEODET_DTYPE`` field over the valid records of every tile (tile by tile, in the engine's order), and ``counts.npy``
+    (records per tile).  float32 fields stay float32, the rest become float64; at most BATCH x MAX_DET records (< 1 MB)."""
+    from aerial_image_recognition_b200.engine import geodets_to_numpy
+    os.makedirs(out_dir, exist_ok=True)
+    recs = np.concatenate(geodets_to_numpy(geo, counts))
+    for name in recs.dtype.names:
+        a = recs[name]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float32 if a.dtype == np.float32 else np.float64))
+    np.save(os.path.join(out_dir, "counts.npy"), counts.cpu().numpy().astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------------------------
@@ -502,6 +534,8 @@ def main():
     ap.add_argument("--mosaic-size", type=int, default=40000)
     ap.add_argument("--precision", default="bf16", choices=["bf16", "fp16", "fp16x2"],
                     help="storage format of activations/weights; bf16 is the configuration BASELINE.json names")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the georeferenced detections of the last one (rank 0) as DIR/<field>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -521,7 +555,6 @@ def main():
 
     import torch
     import torch.distributed as dist
-    from aerial_image_recognition_b200 import synth
     from aerial_image_recognition_b200.engine import Engine
 
     if not torch.cuda.is_available():
@@ -535,15 +568,7 @@ def main():
 
     # inputs: NPOOL distinct batches (> L2 in total: 4 x 78.6 MB u8, and every step streams ~6 GB of
     # activations through a 126 MB L2), rotated step by step
-    NPOOL = 4
-    base = synth.make_tiles(16, SIZE, seed=1000 + rank)
-    host_pool = []
-    for b in range(NPOOL):
-        idx = (np.arange(BATCH) * 7 + b * 3) % 16
-        h = torch.from_numpy(base[idx]).clone()
-        if b % 2:
-            h = torch.flip(h, dims=[2]).contiguous()
-        host_pool.append(h.pin_memory())
+    host_pool = [h.pin_memory() for h in input_batches(rank)]
     dev_pool = [h.to(dev) for h in host_pool]
     params_host = torch.from_numpy(_geo_params(BATCH)).pin_memory()
     params_dev = params_host.to(dev)
@@ -609,6 +634,8 @@ def main():
     ms = sorted(runs)[1]
     clocks = sampler.stop() if rank == 0 else None
     n_det = int(counts.sum().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, geo, counts)
 
     def _value_again(tag):              # diagnostic (B2D_BENCH_DEBUG=1): the same K-step loop again, to stderr
         if os.environ.get("B2D_BENCH_DEBUG"):

@@ -735,6 +735,35 @@ def test_full_batch_determinism_and_batch_invariance():
     eng.close()
 
 
+def test_bench_dump_outputs_are_the_last_timed_step(tmp_path):
+    # bench.py --dump-outputs DIR: the records its timed path (Engine.infer + Engine.georef) returned in the last of --steps
+    # steps; the same inputs through a fresh engine in this process give them bit for bit, so dumps of two builds compare
+    import json
+    import subprocess
+    import sys
+    import bench
+    from aerial_image_recognition_b200.engine import GEODET_DTYPE, geodets_to_numpy
+    steps = 3
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "1", "--legs", "",
+                        "--no-cpu-baseline", "--dump-outputs", str(tmp_path)], stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True)
+    assert r.returncode == 0, r.stderr[-3000:]
+    line = json.loads(r.stdout.strip().splitlines()[-1])
+    assert line["steps"] == steps
+    assert sorted(p.name for p in tmp_path.iterdir()) == sorted([f"{n}.npy" for n in GEODET_DTYPE.names] + ["counts.npy"])
+    got = {p.stem: np.load(p) for p in tmp_path.iterdir()}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values()) and sum(a.nbytes for a in got.values()) <= 64 << 20
+    assert got["counts"].sum() == line["config"]["detections_last_step"] > 0
+    eng = _engine("yolov8m", max_batch=bench.BATCH, seed=0)
+    tiles = bench.input_batches(0)[(steps - 1) % bench.NPOOL].cuda()
+    dets, counts = eng.infer(tiles, "identity", False, bench.CONF, False, bench.IOU, 0, bench.MAX_DET)
+    geo = eng.georef(dets, counts, torch.from_numpy(bench._geo_params(bench.BATCH)).cuda(), "bounds")
+    ref = np.concatenate(geodets_to_numpy(geo, counts))
+    eng.close()
+    assert np.array_equal(got["counts"], counts.cpu().numpy())
+    for name in GEODET_DTYPE.names:
+        assert np.array_equal(got[name], ref[name]), name
+
+
 # ---- SURVEY 8f-1: the model arrives as an .onnx path, as in the reference ---------------------------------------
 def test_detector_built_from_onnx_file_equals_detector_built_from_tensors(tmp_path):
     """``SimpleDetector(model_path)`` / ``GPUHandler(model_path)`` with a real file at the path
