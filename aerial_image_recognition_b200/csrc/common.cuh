@@ -40,20 +40,22 @@ int b2d_func_smem_optin(const void* func, int bytes);
 // ---------------------------------------------------------------------------------------
 // tcgen05 implicit-GEMM convolution (conv_tc.cu)
 // ---------------------------------------------------------------------------------------
-struct EpiChunk {         // one 128/64/32-byte wide column chunk of an output row (epilogue staging + TMA store)
-    uint16_t col0, cols;  // first accumulator column, number of columns
-    uint16_t span, map;   // bytes per row in the staging slab (= swizzle span), index into tmO / tmR
-    uint32_t off;         // byte offset of the chunk's 32-row slab inside a warp's staging region
+// which kernel runs a planned convolution (conv_tc.cu)
+enum ConvKind : int {
+    CONV_GENERIC,     // one TMA box per (tap, chunk); CTA-pair form when ConvTcParams::pair
+    CONV_HALO,        // 3x3 stride 1 on 8-pixel-wide tiles, one halo box per chunk; CTA-pair form when ConvTcParams::pair
+    CONV_DEPTHWISE,   // depthwise 3x3: halo + diagonal weight blocks
+    CONV_STEM,        // the 4-channel network input through TMA: space-to-depth (stride 2) or pixel pairs (stride 1)
+    CONV_DWPW,        // fused depthwise 3x3 + pointwise 1x1
+    CONV_S2HALO,      // 3x3 stride 2 with one K chunk, one halo box per phase map
 };
-constexpr int kMaxEpiChunks = 6;
 
 struct __align__(64) ConvTcParams {
     CUtensorMap tmA[4];   // generic: [0] stride-1 map or [py*2+px] the four stride-2 phase maps; halo: [0] the halo box map
     CUtensorMap tmB;      // packed weights [cout_pad][taps*cin_pad], K contiguous
     CUtensorMap tmO[3];   // output slice, one warp quarter's sub-box, chunk width 128 / 64 / 32 bytes
     CUtensorMap tmR[3];   // residual slice, same boxes
-    EpiChunk epi[kMaxEpiChunks];
-    int epi_nchunks, has_res;
+    int has_res;
     int stg_bufs;         // 1 or 2 staging buffers (each mt tiles x 128 rows x n_tile columns)
     uint32_t stg_off, bar_off;   // smem offsets (from the 1 KiB aligned base) of the staging region / barrier block
     const float* bias;    // [cout_pad]
@@ -68,7 +70,7 @@ struct __align__(64) ConvTcParams {
     uint32_t rcp_nn, rcp_tx, rcp_ty;   // ceil(2^32 / d) for the tile decode (0 when d == 1)
     int act, out_f32;
     int stages;
-    int kind;             // 0 generic (shifted boxes), 1 halo (3x3 s1, bw == 8), 2 stem (im2col gather), 3 depthwise (halo + diagonal blocks), 4 stride-2 stem through TMA, 5 fused depthwise 3x3 + pointwise 1x1
+    ConvKind kind;
     int pair;             // 1: CTA-pair kernel (cta_group::2, M = 256 across two SMs)
     int mt;               // M tiles per round (share B stages, one accumulator stage, one epilogue pass)
     int halo_w;           // bw + 2
@@ -78,8 +80,6 @@ struct __align__(64) ConvTcParams {
     uint32_t a_tx_bytes, b_tx_bytes; // TMA bytes of one A box / one B box
     uint32_t tmem_cols;
     uint32_t idesc;
-    int in_h, in_w;       // input spatial size (stem)
-    const void* src_raw;  // stem: NHWC4 bf16 input
     const void* w_raw;    // stem: packed weights [n_tile][64] bf16
     int f16;              // 16-bit activation / weight format: 0 bf16, 1 fp16 (B2D_PREC_FP16, B2D_PREC_FP16X2)
     int epi_parts;        // epilogue warps per TMEM lane quarter: 2 (warps 4-11) or 3 (warps 4-15), each taking every epi_parts-th 16-column unit
@@ -91,8 +91,6 @@ struct __align__(64) ConvTcParams {
     int dw_act;           // ... SiLU after the depthwise stage
     int rev;              // 1: this op walks its M tiles in descending order (set per op by the engine)
     int rev_last;         // per launch: index of the last M tile when walking backwards, else -1
-    int epi_path;         // epilogue code path (see epilogue_loop; B2D_EPI_PATH, default 2)
-    int exp;              // timing-ablation flags (trace builds only)
     long long* trace;     // debug only (B2D_TRACE=1): per-role clock64 stamps of CTA 0, else nullptr
 };
 

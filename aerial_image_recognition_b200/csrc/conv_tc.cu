@@ -18,8 +18,9 @@
 //       halo     3x3 stride-1 convs on 8-pixel-wide tiles: the (bw+2) x (bh+2) halo of a chunk is
 //                fetched once and the nine taps are nine MMAs over it, the A descriptor starting at
 //                halo row kh*bn*(bw+2) + kw with (bw+2) rows between 8-row groups.  A traffic /6.
-//       stem     the 4-channel network input (8 B per pixel is below TMA's 16 B minimum): gather
-//                warps build the im2col tile (k = tap*4 + c) themselves; weights stay resident.
+//       stem     the 4-channel network input (8 B per pixel): one un-swizzled box per tile, read as
+//                the no-swizzle K-major layout (space-to-depth for stride 2, pixel pairs for stride 1,
+//                see conv_tc_stem2_kernel); weights stay resident.
 //   * weights are pre-packed [Cout][kh][kw][Cin_pad] (K contiguous), fetched by 2-D TMA loads.
 //   * operands are K-major SWIZZLE_128B; a short last chunk is zero-filled by TMA and its unused
 //     K=16 sub-steps are skipped.
@@ -29,11 +30,11 @@
 //     Concat / Split never run as ops, partial tiles and padded channels are clipped by TMA.
 //
 // Kernel shape: persistent, one CTA per SM.  Warps: 0 TMA producer | 1 MMA issuer | 2 TMEM
-// allocator | 3 idle | 4-11 epilogue (warp % 4 = TMEM lane quarter, two warps per quarter) |
-// 12-15 im2col gather (stem only).  Control loops run warp-uniformly and elect one lane around the
-// asynchronous instructions.  Pipelines: smem ring (full/empty mbarriers) TMA -> MMA; two TMEM
-// accumulator stages (tmem_full/tmem_empty) MMA -> epilogue; one or two staging slabs epilogue ->
-// TMA store.
+// allocator | 3 store | 4-11 or 4-15 epilogue (warp % 4 = TMEM lane quarter, two or three warps per
+// quarter; the fused depthwise + pointwise kernel: 4-7 epilogue, 8-15 depthwise).  Control loops run
+// warp-uniformly and elect one lane around the asynchronous instructions.  Pipelines: smem ring
+// (full/empty mbarriers) TMA -> MMA; two TMEM accumulator stages (tmem_full/tmem_empty) MMA ->
+// epilogue; one or two staging slabs epilogue -> TMA store.
 #include "common.cuh"
 
 #include <cudaTypedefs.h>
@@ -44,10 +45,8 @@
 namespace {
 
 constexpr int kThreads = 512;         // 4 control warps + up to 12 epilogue warps (ConvTcParams::epi_parts per TMEM lane quarter)
-constexpr int kStemThreads = 512;     // 4 control warps + 8 epilogue warps + 4 gather warps
 constexpr int kTileM = 128;
 constexpr int kMaxStages = 9;         // 9: a 3x3 layer with one K chunk keeps all nine weight taps resident (b_res)
-constexpr int kMaxMt = 4;
 
 // ---- PTX wrappers -----------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -271,17 +270,6 @@ __device__ __forceinline__ int pair_tile(const ConvTcParams& p, int rd, int rank
     return min(2 * mp + rank, total_tiles / nn - 1) * nn + nt;
 }
 
-// Ablation flags for timing experiments (trace builds only; results are wrong when set): p.exp bit 0 = the MMA warp
-// does not wait for operand barriers, bit 1 = the epilogue skips TMEM loads / math / stores, bit 2 = the producer
-// issues no TMA loads (arrives on the barriers instead).
-#ifdef B2D_ENABLE_TRACE
-#define B2D_EXP(p, bit) (((p).exp >> (bit)) & 1)
-#define B2D_EXPW(p) ((p).exp)
-#else
-#define B2D_EXP(p, bit) 0
-#define B2D_EXPW(p) 0
-#endif
-
 // Debug trace (build with -DB2D_ENABLE_TRACE, run with B2D_TRACE=1): CTA 0 records clock64() at role
 // events of its first kTraceTiles rounds.  Compiled out of product builds.
 constexpr int kTraceTiles = 24, kTraceEvents = 4, kTraceRoles = 4;   // roles: 0 producer, 1 MMA, 2 epilogue warp 4, 3 = warp 4's cycles per round in: TMEM-load waits, slab / residual waits, epi_unit, fence + hand-off
@@ -384,14 +372,7 @@ __device__ __forceinline__ uint64_t join2(uint32_t hi, uint32_t lo) {           
     return pk2(__fadd_rn(a.x, b.x), __fadd_rn(a.y, b.y));
 }
 template <int RES, int F32, int NC>
-__device__ __forceinline__ void epi_store(uint64_t (&v)[8], uint32_t base, int exp, int f16) {
-    if (exp & 64) {             // ablation: no staging stores (keep the values alive)
-        uint64_t acc = 0;
-#pragma unroll
-        for (int i = 0; i < NC / 2; ++i) acc ^= v[i];
-        if (acc == 0x123456789ull) sts_b64x2(base, acc, acc);
-        return;
-    }
+__device__ __forceinline__ void epi_store(uint64_t (&v)[8], uint32_t base, int f16) {
     if (F32 == 2) {             // split fp16: per 8 columns one 16-byte piece of high parts, then one of low parts
 #pragma unroll
         for (int j = 0; j < NC / 8; ++j) {
@@ -447,20 +428,29 @@ __device__ __forceinline__ void epi_store(uint64_t (&v)[8], uint32_t base, int e
     }
 }
 template <int ACT, int RES, int F32, int NC = 16>
-__device__ __forceinline__ void epi_unit(const uint32_t (&r)[16], uint32_t bias_addr, uint32_t base, int exp, int f16, uint64_t scale2) {
+__device__ __forceinline__ void epi_unit(const uint32_t (&r)[16], uint32_t bias_addr, uint32_t base, int f16, uint64_t scale2) {
     uint64_t v[8];
     epi_bias<ACT, NC>(r, bias_addr, v, scale2);
-    if (ACT && !(exp & 8)) {
+    if (ACT) {
 #pragma unroll
         for (int i = 0; i < NC / 2; ++i) v[i] = silu2_h(v[i]);
     }
-    epi_store<RES, F32, NC>(v, base, exp, f16);
+    epi_store<RES, F32, NC>(v, base, f16);
 }
 
-// Geometry of the staging slabs, shared by the epilogue warps and the store warp.  A tile row of n_tile columns is cut
-// into chunks of 128 / 64 / 32 bytes (one tensor map per width); a tile's slab holds, chunk after chunk, all 128 rows x chunk
-// width: full 128-byte chunks first, then one 64-byte, then one 32-byte chunk (mirrors conv_tc_plan).  One TMA store (or
-// residual load) moves a whole chunk of a tile: the box of the maps is the M tile itself.
+// The epilogue chunk format: a tile row of `row_bytes` is cut into chunks of 128 / 64 / 32 bytes, one tensor map per width
+// (tmO / tmR [0], [1], [2]): full 128-byte chunks first, then at most one 64-byte and one 32-byte chunk.  The planner encodes
+// the maps and bounds the chunk count with it, the kernels lay out the staging slabs with it.
+struct EpiChunks {
+    uint32_t n128, has64, has32;
+};
+__host__ __device__ __forceinline__ EpiChunks epi_chunks(uint32_t row_bytes) {
+    return {row_bytes >> 7, (row_bytes >> 6) & 1u, (row_bytes >> 5) & 1u};
+}
+
+// Geometry of the staging slabs, shared by the epilogue warps and the store warp: a tile's slab holds, chunk after chunk
+// (epi_chunks), all 128 rows x chunk width.  One TMA store (or residual load) moves a whole chunk of a tile: the box of the
+// maps is the M tile itself.
 template <int F32>      // 0: 16-bit outputs, 1: fp32 outputs, 2: split fp16 (hi | lo) -- 4 bytes per output column like fp32
 struct EpiGeom {
     static constexpr int esize = F32 ? 4 : 2;
@@ -471,7 +461,8 @@ struct EpiGeom {
         tile_bytes = 128u * row_bytes;                                          // staging bytes of one M tile
         base = smem_u32(stg_base);                                              // slab 0
         nb = p.stg_bufs;
-        n128 = row_bytes >> 7; has64 = (row_bytes >> 6) & 1u; has32 = (row_bytes >> 5) & 1u;
+        const EpiChunks c = epi_chunks(row_bytes);
+        n128 = c.n128; has64 = c.has64; has32 = c.has32;
     }
     // TMA boxes of one tile's slab: fn(map index, byte offset in the slab, first column)
     template <typename Fn>
@@ -496,7 +487,6 @@ template <int RES, int F32>
 __device__ __forceinline__ void store_loop(const ConvTcParams& p, int total_tiles, uint64_t* sfull_bar, uint64_t* sempty_bar,
                                            uint64_t* res_bar, uint8_t* stg_base, int lane, bool pair = false) {
     if (!elect_one()) return;
-    if (B2D_EXP(p, 7)) return;                 // ablation: no slab hand-off at all
     (void)lane;
     const EpiGeom<F32> g(p, stg_base);
     const int mt = p.mt, n_tile = p.n_tile;
@@ -505,7 +495,6 @@ __device__ __forceinline__ void store_loop(const ConvTcParams& p, int total_tile
     const uint32_t rank = pair ? cluster_ctarank() : 0u;
     const int rounds = pair ? pair_rounds(p, total_tiles) : (total_tiles + mt - 1) / mt;
     const int rd0 = pair ? (int)(blockIdx.x >> 1) : (int)blockIdx.x, rd_step = pair ? (int)(gridDim.x >> 1) : (int)gridDim.x;
-    const bool no_store = B2D_EXP(p, 1) || B2D_EXP(p, 5);
     const bool perm = p.perm != 0;
     auto first_tile = [&](int rd) { return pair ? pair_tile(p, rd, (int)rank, total_tiles) : rd * mt; };
     auto valid_tiles = [&](int rd) { return pair ? 1 : min(mt, total_tiles - rd * mt); };
@@ -535,7 +524,7 @@ __device__ __forceinline__ void store_loop(const ConvTcParams& p, int total_tile
     int pend_slab = -1, pend_next = -1;                                        // slab whose stores are in flight; residual tile to load into it (or -1)
     auto release = [&](bool last) {
         if (pend_slab < 0) return;
-        if (!no_store) { if (last) tma_store_wait_read0(); else tma_store_wait_read1(); }      // the TMA unit has read the pending slab
+        if (last) tma_store_wait_read0(); else tma_store_wait_read1();      // the TMA unit has read the pending slab
         mbar_arrive_u32(sempty_u32 + (uint32_t)pend_slab * 8u);
         if (RES && pend_next >= 0) tile_io(pend_next, pend_slab, true);
         pend_slab = -1;
@@ -548,10 +537,8 @@ __device__ __forceinline__ void store_loop(const ConvTcParams& p, int total_tile
             const int c = it * mt + m, slab = c & (S - 1);
             const uint32_t use = (uint32_t)(c >> s_shift);
             mbar_wait_u32(sfull_u32 + (uint32_t)slab * 8u, use & 1u);
-            if (!no_store) {
-                tile_io(t0 + m, slab, false);
-                tma_store_commit();
-            }
+            tile_io(t0 + m, slab, false);
+            tma_store_commit();
             if (RES || S < 4) {                          // residual layers: the slab's next residual must start loading as early as possible
                 pend_slab = slab;                        // (measured: +11 us on the 96-channel residual layers when it waits a tile longer);
                 pend_next = (RES && m < nvn) ? first_tile(rdn) + m : -1;       // with fewer than four slabs a pending one starves the epilogue (+2-4 us)
@@ -609,7 +596,7 @@ __device__ __forceinline__ void epilogue_loop(const ConvTcParams& p, int total_t
     };
     const uint32_t ubytes = 16u * esize;               // bytes of one unit in a row
     int it = 0;
-    if (my_units <= 2 && !split_last && p.n_tiles_n == 1 && p.epi_path >= 1) {
+    if (my_units <= 2 && !split_last && p.n_tiles_n == 1) {
         // Narrow tiles (n_tile = 32, 48, 64, 96: the stem, the 160^2 stage, the 96-channel 3x3 layers, the head's box branch): a warp
         // owns the same one or two 16-column units of every tile, so the staging addresses and the bias pointers are loop
         // invariants and a tile is one straight-line block -- TMEM loads of the next tile in flight behind the SiLU of this
@@ -655,13 +642,13 @@ __device__ __forceinline__ void epilogue_loop(const ConvTcParams& p, int total_t
 #pragma unroll
                     for (int i = 0; i < 8; ++i) v0[i] = silu2_h(v0[i]);
                 }
-                epi_store<RES, F32, 16>(v0, ub0 + moff, 0, f16);
+                epi_store<RES, F32, 16>(v0, ub0 + moff, f16);
                 if (two) {
                     if (ACT) {
 #pragma unroll
                         for (int i = 0; i < 8; ++i) v1[i] = silu2_h(v1[i]);
                     }
-                    epi_store<RES, F32, 16>(v1, ub1 + moff, 0, f16);
+                    epi_store<RES, F32, 16>(v1, ub1 + moff, f16);
                 }
                 fence_proxy_async();                                                   // generic-proxy slab writes -> visible to the TMA store
                 __syncwarp();
@@ -678,7 +665,7 @@ __device__ __forceinline__ void epilogue_loop(const ConvTcParams& p, int total_t
         (void)rank;
         return;
     }
-    if (!split_last && p.epi_path >= 2) {
+    if (!split_last) {
         // Tile-structured path (everything except the 8 + 8 split of an odd last unit): a warp's 16-column units are the same
         // columns of every tile, a tile is one block of straight-line code per pair of units -- bias step of the pair, TMEM loads
         // of the next pair (of this tile or the next) issued behind it, SiLU + pack + staging stores -- with one slab wait in
@@ -734,13 +721,13 @@ __device__ __forceinline__ void epilogue_loop(const ConvTcParams& p, int total_t
 #pragma unroll
                         for (int i = 0; i < 8; ++i) v0[i] = silu2_h(v0[i]);
                     }
-                    epi_store<RES, F32, 16>(v0, unit_base((col0 + (uint32_t)u * ustep) * esize) + moff, 0, f16);
+                    epi_store<RES, F32, 16>(v0, unit_base((col0 + (uint32_t)u * ustep) * esize) + moff, f16);
                     if (two) {
                         if (ACT) {
 #pragma unroll
                             for (int i = 0; i < 8; ++i) v1[i] = silu2_h(v1[i]);
                         }
-                        epi_store<RES, F32, 16>(v1, unit_base((col0 + (uint32_t)(u + 1) * ustep) * esize) + moff, 0, f16);
+                        epi_store<RES, F32, 16>(v1, unit_base((col0 + (uint32_t)(u + 1) * ustep) * esize) + moff, f16);
                     }
                 }
                 fence_proxy_async();                                                   // generic-proxy slab writes -> visible to the TMA store
@@ -757,13 +744,13 @@ __device__ __forceinline__ void epilogue_loop(const ConvTcParams& p, int total_t
         }
         return;
     }
+    // Item-list path: the 8 + 8 split of an odd last unit (n_tile 16, 80, 112 ...).
     // tile walk: a CTA takes rounds blockIdx.x, + gridDim.x, ... of mt tiles; in a CTA pair (mt == 1) the pair takes two
     // consecutive tiles per round, one per CTA, and an odd last tile is computed (and stored, identically) by both
     const uint32_t rank = pair ? cluster_ctarank() : 0u;
     const int rounds = pair ? pair_rounds(p, total_tiles) : (total_tiles + mt - 1) / mt;
     const int rd0 = pair ? (int)(blockIdx.x >> 1) : (int)blockIdx.x, rd_step = pair ? (int)(gridDim.x >> 1) : (int)gridDim.x;
     const uint32_t tempty_arrive = pair ? mapa_u32(tempty_u32, 0) : tempty_u32;   // the leader's barrier gates the pair's MMAs
-    const bool ldt = !B2D_EXP(p, 4);
     const int f16 = p.f16;
     const float sc = (ACT ? 0.5f : 1.0f) * p.acc_scale;
     const uint64_t scale2 = pk2(sc, sc);
@@ -783,7 +770,6 @@ __device__ __forceinline__ void epilogue_loop(const ConvTcParams& p, int total_t
         const uint32_t tq = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(as * mt * n_tile);
         const int c_base = it * mt;
         auto item_ld = [&](int m, int u, uint32_t (&rb)[16]) {
-            if (!ldt) return;
             if (u < my_units) tmem_ld16(tq + (uint32_t)(m * n_tile + half * 16) + (uint32_t)u * ustep, rb);
             else tmem_ld8(tq + (uint32_t)(m * n_tile + split_col), rb);
         };
@@ -798,7 +784,7 @@ __device__ __forceinline__ void epilogue_loop(const ConvTcParams& p, int total_t
         auto item_do = [&](int m, int u, const uint32_t (&rb)[16]) {
             const int c = c_base + m, slab = c & (S - 1);
             const uint32_t use = (uint32_t)(c >> s_shift);
-            if (u == 0 && !B2D_EXP(p, 7)) {                                    // first item of a tile: its slab must be free (and the residual in it)
+            if (u == 0) {                                                      // first item of a tile: its slab must be free (and the residual in it)
                 B2D_TICK();
                 mbar_wait_u32(sempty_u32 + (uint32_t)slab * 8u, (use & 1u) ^ 1u);
                 if (RES) mbar_wait_u32(rbar_u32 + (uint32_t)slab * 8u, use & 1u);
@@ -806,12 +792,12 @@ __device__ __forceinline__ void epilogue_loop(const ConvTcParams& p, int total_t
             }
             const uint32_t moff = (uint32_t)slab * tile_bytes;
             B2D_TICK();
-            if (u < my_units) epi_unit<ACT, RES, F32, 16>(rb, baddr + (uint32_t)u * ustep * 4u, unit_base((uint32_t)(half + nparts * u) * ubytes) + moff, B2D_EXPW(p), f16, scale2);
-            else epi_unit<ACT, RES, F32, 8>(rb, bias_base + (uint32_t)(ch_base + split_col) * 4u, unit_base((uint32_t)split_col * esize) + moff, B2D_EXPW(p), f16, scale2);
+            if (u < my_units) epi_unit<ACT, RES, F32, 16>(rb, baddr + (uint32_t)u * ustep * 4u, unit_base((uint32_t)(half + nparts * u) * ubytes) + moff, f16, scale2);
+            else epi_unit<ACT, RES, F32, 8>(rb, bias_base + (uint32_t)(ch_base + split_col) * 4u, unit_base((uint32_t)split_col * esize) + moff, f16, scale2);
             B2D_TOCK(w_math);
-            if (u == ipt - 1 && !B2D_EXP(p, 7)) {                              // last item: hand the slab to the store warp (one arrival per warp of the quarter)
+            if (u == ipt - 1) {                                                // last item: hand the slab to the store warp (one arrival per warp of the quarter)
                 B2D_TICK();
-                if (!B2D_EXP(p, 9)) fence_proxy_async();                       // generic-proxy slab writes -> visible to the TMA store
+                fence_proxy_async();                                           // generic-proxy slab writes -> visible to the TMA store
                 __syncwarp();
                 if (lane == 0) mbar_arrive_u32(sfull_u32 + (uint32_t)slab * 8u);
                 B2D_TOCK(w_hand);
@@ -918,11 +904,6 @@ __device__ __forceinline__ uint32_t prologue(const ConvTcParams& p, const Bars& 
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
-    // Programmatic dependent launch: everything above (barrier init, TMEM allocation, constants to smem) overlapped the
-    // tail of the previous kernel in the stream; from here on its results are needed.  The next kernel may be scheduled
-    // as soon as SMs free up -- it will block at this same point until this grid has completed.
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     return *b.tmem_slot;
 }
 __device__ __forceinline__ void epilogue_exit(const ConvTcParams& p, uint32_t tmem_base, int warp) {
@@ -1044,7 +1025,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
             // without any per-MMA test, only a tap's last (possibly short, zero-padded) chunk picks its count
             int ks = 0;
             auto step = [&](auto KM) {
-                if (!B2D_EXP(p, 0)) mbar_wait_u32(full_u32 + stage * 8, phase);
+                mbar_wait_u32(full_u32 + stage * 8, phase);
                 tc_fence_after();
                 if (ks == 0) trace(p, 1, it, 2);
                 if (leader) {
@@ -1119,12 +1100,8 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_halo_kernel(const __grid_
                 for (int tap = 0; tap < 9; ++tap) {
                     mbar_wait_u32(empty_u32 + stage * 8, phase ^ 1);
                     if (elect_one()) {
-                        if (B2D_EXP(p, 2)) {
-                            mbar_arrive_u32(full_u32 + stage * 8);
-                        } else {
-                            mbar_expect_tx_u32(full_u32 + stage * 8, b_tx);
-                            tma_load_2d(&p.tmB, full_u32 + stage * 8, smem_b + (uint32_t)stage * b_bytes, tap * cin_pad + ch * 64, bn0);
-                        }
+                        mbar_expect_tx_u32(full_u32 + stage * 8, b_tx);
+                        tma_load_2d(&p.tmB, full_u32 + stage * 8, smem_b + (uint32_t)stage * b_bytes, tap * cin_pad + ch * 64, bn0);
                     }
                     if (++stage == nstages) { stage = 0; phase ^= 1; }
                 }
@@ -1150,13 +1127,9 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_halo_kernel(const __grid_
                 if (ch == 0) trace(p, 0, pit, 1);
                 if (elect_one()) {
                     const uint32_t hbar = hfull_u32 + hb * 8, dst = smem_a + (uint32_t)(hb * mt) * halo_bytes;
-                    if (B2D_EXP(p, 2)) {
-                        mbar_arrive_u32(hbar);
-                    } else {
-                        mbar_expect_tx_u32(hbar, (uint32_t)nv * p.a_tx_bytes);
-                        tma_load_4d(&p.tmA[0], hbar, dst, ch * 64, tc0.x0 - 1, perm ? tc0.n0 : tc0.y0 - 1, perm ? tc0.y0 - 1 : tc0.n0);
-                        if (nv > 1) tma_load_4d(&p.tmA[0], hbar, dst + halo_bytes, ch * 64, tc1.x0 - 1, perm ? tc1.n0 : tc1.y0 - 1, perm ? tc1.y0 - 1 : tc1.n0);
-                    }
+                    mbar_expect_tx_u32(hbar, (uint32_t)nv * p.a_tx_bytes);
+                    tma_load_4d(&p.tmA[0], hbar, dst, ch * 64, tc0.x0 - 1, perm ? tc0.n0 : tc0.y0 - 1, perm ? tc0.y0 - 1 : tc0.n0);
+                    if (nv > 1) tma_load_4d(&p.tmA[0], hbar, dst + halo_bytes, ch * 64, tc1.x0 - 1, perm ? tc1.n0 : tc1.y0 - 1, perm ? tc1.y0 - 1 : tc1.n0);
                 }
                 if (++hb == 2) { hb = 0; hphase ^= 1; }
             }
@@ -1185,7 +1158,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_halo_kernel(const __grid_
             trace(p, 1, it, 1);
             const uint32_t d_tmem = tmem_base + (uint32_t)(as * mt * n_tile);
             for (int ch = 0; ch < chunks; ++ch) {
-                if (!B2D_EXP(p, 0)) mbar_wait_u32(hfull_u32 + hb * 8, hphase);
+                mbar_wait_u32(hfull_u32 + hb * 8, hphase);
                 tc_fence_after();
                 if (ch == 0) trace(p, 1, it, 2);
                 const uint32_t a_lo_h = a_lo0 + (uint32_t)(hb * mt) * halo_units;
@@ -1197,7 +1170,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_halo_kernel(const __grid_
 #pragma unroll
                     for (int tap = 0; tap < 9; ++tap) {
                         if (b_wait) {                    // resident weights: only the first round waits for (and never releases) a stage
-                            if (!B2D_EXP(p, 0)) mbar_wait_u32(full_u32 + stage * 8, phase);
+                            mbar_wait_u32(full_u32 + stage * 8, phase);
                             tc_fence_after();
                         }
                         if (leader) {
@@ -1281,8 +1254,6 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_halo2_kernel(const __grid
     tc_fence_before();
     cluster_sync_all();                               // barriers of both CTAs initialised before anyone signals them
     tc_fence_after();
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     const uint32_t tmem_base = *b.tmem_slot;
     const uint32_t halo_bytes = p.halo_bytes;
     const uint32_t smem_a = smem_u32(smem), smem_b = smem_a + 2u * halo_bytes;
@@ -1356,7 +1327,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_halo2_kernel(const __grid
 #ifdef B2D_ENABLE_TRACE
                 w0 = clock64();
 #endif
-                if (!B2D_EXP(p, 0)) mbar_wait_u32(hfull_u32 + hb * 8, hphase);
+                mbar_wait_u32(hfull_u32 + hb * 8, hphase);
 #ifdef B2D_ENABLE_TRACE
                 wait_h += clock64() - w0;
 #endif
@@ -1371,7 +1342,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_halo2_kernel(const __grid
 #ifdef B2D_ENABLE_TRACE
                         w0 = clock64();
 #endif
-                        if (!B2D_EXP(p, 0)) mbar_wait_u32(full_u32 + stage * 8, phase);
+                        mbar_wait_u32(full_u32 + stage * 8, phase);
                         tc_fence_after();
 #ifdef B2D_ENABLE_TRACE
                         wait_b += clock64() - w0;
@@ -1470,8 +1441,6 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_pair_kernel(const __grid_
     tc_fence_before();
     cluster_sync_all();                               // barriers of both CTAs initialised before anyone signals them
     tc_fence_after();
-    asm volatile("griddepcontrol.wait;" ::: "memory");
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     const uint32_t tmem_base = *b.tmem_slot;
     const uint32_t smem_base = smem_u32(smem);
     const uint32_t full_u32 = smem_u32(b.full), empty_u32 = smem_u32(b.empty);
@@ -1704,129 +1673,6 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_dw_kernel(const __grid_co
 }
 
 // ---------------------------------------------------------------------------------------------
-// stem kernel: 3x3 (or 1x1) conv on the 4-channel network input (NHWC4 bf16, 8 bytes per pixel).
-// K = 9 taps x 4 channels = 36 is far too short for a TMA-fed pipeline, so four gather warps build
-// the im2col tiles: thread r owns row r of each of the round's mt tiles, reads its nine 8-byte input
-// pixels (zero outside the image) and writes them as one 128-byte K-major row in the SWIZZLE_128B
-// pattern (k = tap * 4 + c, zero-padded to 48).  Three K=16 MMAs per tile against the weights, which
-// stay resident in shared memory.  Bound by its output (bias + SiLU + 96 B written per pixel).
-// ---------------------------------------------------------------------------------------------
-template <int ACT, int OUT>
-__global__ void __launch_bounds__(kStemThreads, 1) conv_tc_stem_kernel(const __grid_constant__ ConvTcParams p, int nimg) {
-    extern __shared__ __align__(1024) uint8_t smem_raw[];
-    uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-    const Bars b = carve_bars(smem, p);
-    const int warp = threadIdx.x >> 5;
-    const int lane = threadIdx.x & 31;
-    const int mt = p.mt;
-    const int total_tiles = p.tiles_x * p.tiles_y * ((nimg + p.bn - 1) / p.bn);
-    const int rounds = (total_tiles + mt - 1) / mt;
-    const uint32_t stage_bytes = (uint32_t)mt * p.a_bytes;
-    uint8_t* wres = smem + (size_t)p.stages * stage_bytes;         // resident weights [n_tile][64] bf16, swizzled
-
-    {   // weights: global [n_tile][64] bf16 -> smem rows of 128 B, 16-byte piece j of row n at (j ^ (n & 7))
-        const uint4* wg = (const uint4*)p.w_raw;
-        const uint32_t wbase = smem_u32(wres);
-        for (int i = threadIdx.x; i < p.n_tile * 8; i += kStemThreads) {
-            const int n = i >> 3, j = i & 7;
-            sts128(wbase + (uint32_t)n * 128u + (uint32_t)((j ^ (n & 7)) << 4), __ldg(wg + i));
-        }
-        fence_proxy_async();
-    }
-    const uint32_t tmem_base = prologue(p, b, warp, lane, 4);        // one arrival per gather warp
-    const uint32_t smem_base = smem_u32(smem);
-    const uint32_t full_u32 = smem_u32(b.full), empty_u32 = smem_u32(b.empty);
-
-    if (warp == 1) {
-        // ===================== MMA issuer =====================
-        int stage = 0, it = 0;
-        uint32_t phase = 0;
-        const uint32_t hi = desc_hi(1024);
-        const uint32_t b_lo = desc_lo(smem_u32(wres));
-        const uint32_t idesc = p.idesc;
-        const int nstages = p.stages, n_tile = p.n_tile, kmmas = (p.taps * 4 + 15) >> 4;
-        const uint32_t tfull_u32 = smem_u32(b.tfull), tempty_u32 = smem_u32(b.tempty);
-        for (int rd = blockIdx.x; rd < rounds; rd += gridDim.x, ++it) {
-            const int as = it & 1;
-            const int nv = min(mt, total_tiles - rd * mt);
-            trace(p, 1, it, 0);
-            mbar_wait_u32(tempty_u32 + as * 8, ((it >> 1) & 1) ^ 1);
-            trace(p, 1, it, 1);
-            mbar_wait_u32(full_u32 + stage * 8, phase);
-            tc_fence_after();
-            trace(p, 1, it, 2);
-            if (elect_one()) {
-                const uint32_t d_tmem = tmem_base + (uint32_t)(as * mt * n_tile);
-                for (int m = 0; m < nv; ++m) {
-                    const uint32_t a_lo = desc_lo(smem_base + (uint32_t)stage * stage_bytes + (uint32_t)m * p.a_bytes);
-                    for (int k = 0; k < kmmas; ++k)
-                        umma_bf16(d_tmem + (uint32_t)(m * n_tile), desc64(hi, a_lo + 2 * k), desc64(hi, b_lo + 2 * k), idesc, (uint32_t)(k != 0));
-                }
-                umma_commit(empty_u32 + stage * 8);
-                umma_commit(tfull_u32 + as * 8);
-            }
-            if (++stage == nstages) { stage = 0; phase ^= 1; }
-        }
-    } else if (warp >= 12) {
-        // ===================== im2col gather (128 threads, one row of every tile of the round each) =====================
-        const int r = threadIdx.x - 384;
-        const int rx = r % p.bw, rn = (r / p.bw) % p.bn, ry = r / (p.bw * p.bn);
-        const uint32_t row = (uint32_t)r * 128u, sw = (uint32_t)(r & 7);
-        const uint2* src = (const uint2*)p.src_raw;
-        const int in_h = p.in_h, in_w = p.in_w, st = p.stride, ksz = p.ksz, pad = p.ksz >> 1;
-        const int nstages = p.stages;
-        int stage = 0, git = 0;
-        uint32_t phase = 0;
-        for (int rd = blockIdx.x; rd < rounds; rd += gridDim.x, ++git) {
-            const int t0 = rd * mt;
-            uint2 v[kMaxMt][9];
-            if (r == 0) trace(p, 0, git, 0);
-#pragma unroll
-            for (int m = 0; m < kMaxMt; ++m) {
-                if (m < mt) {
-                    const int t = t0 + m;
-                    const TileCoord tc = decode_tile(p, t < total_tiles ? t : t0);
-                    const int ox = tc.x0 + rx, oy = tc.y0 + ry, img = tc.n0 + rn;
-                    const bool valid = t < total_tiles && ox < p.W && oy < p.H && img < nimg;
-                    const uint2* ip = src + (long long)img * in_h * in_w;
-#pragma unroll
-                    for (int tap = 0; tap < 9; ++tap) {
-                        const int kh = tap / 3, kw = tap % 3;
-                        const int iy = oy * st + kh - pad, ix = ox * st + kw - pad;
-                        const bool inb = valid && kh < ksz && kw < ksz && iy >= 0 && iy < in_h && ix >= 0 && ix < in_w;
-                        v[m][tap] = inb ? __ldg(ip + (long long)iy * in_w + ix) : make_uint2(0u, 0u);
-                    }
-                }
-            }
-            if (r == 0) trace(p, 0, git, 1);
-            mbar_wait_u32(empty_u32 + stage * 8, phase ^ 1);
-            if (r == 0) trace(p, 0, git, 2);
-#pragma unroll
-            for (int m = 0; m < kMaxMt; ++m) {
-                if (m < mt) {
-                    const uint32_t a = smem_base + (uint32_t)stage * stage_bytes + (uint32_t)m * p.a_bytes + row;
-#pragma unroll
-                    for (int j = 0; j < 4; ++j)
-                        sts128(a + ((((uint32_t)j) ^ sw) << 4), make_uint4(v[m][2 * j].x, v[m][2 * j].y, v[m][2 * j + 1].x, v[m][2 * j + 1].y));
-                    sts128(a + ((4u ^ sw) << 4), make_uint4(v[m][8].x, v[m][8].y, 0u, 0u));
-                    sts128(a + ((5u ^ sw) << 4), make_uint4(0u, 0u, 0u, 0u));
-                }
-            }
-            fence_proxy_async();                                      // generic-proxy writes -> visible to the MMA's smem reads
-            __syncwarp();
-            if (lane == 0) mbar_arrive_u32(full_u32 + stage * 8);
-            if (r == 0) trace(p, 0, git, 3);
-            if (++stage == nstages) { stage = 0; phase ^= 1; }
-        }
-    } else if (warp == 3) {
-        store_loop<0, OUT>(p, total_tiles, b.sfull, b.sempty, b.res, smem + p.stg_off, lane);
-    } else if (warp >= 4) {
-        epilogue_loop<ACT, 0, OUT>(p, total_tiles, tmem_base, b.bias_s, b.tfull, b.tempty, b.sfull, b.sempty, b.res, smem + p.stg_off, warp, lane);
-    }
-    epilogue_exit(p, tmem_base, warp);
-}
-
-// ---------------------------------------------------------------------------------------------
 // stride-2 stem kernel (YOLOv8 model.0: 3x3 stride 2 on the 4-channel network input), fed by TMA.
 // Seen through a 2 x 2 space-to-depth lens the layer is a 2 x 2 stride-1 convolution over blocks of 2 x 2 input pixels
 // with 16 channels each (row phase, column phase, 4 channels): output (i, j) reads input rows 2i-1 .. 2i+1 = block row i-1
@@ -1838,9 +1684,9 @@ __global__ void __launch_bounds__(kStemThreads, 1) conv_tc_stem_kernel(const __g
 // second core matrix of a K = 16 step (row phase 1) LBO = (bw+1) * 16 bytes further, the next 8-row group (next output row)
 // SBO = 2 * LBO further.  The four taps (di, dj) are four descriptor offsets (di * SBO + dj * 16) into the one box: four
 // K = 16 MMAs per tile against resident weights whose k index is tap * 16 + row phase * 8 + column phase * 4 + channel, with
-// zeros where the 3x3 filter has no entry.  No gather warps: the 128 threads that built im2col rows from 36 scattered
-// 8-byte loads each (~5 600 cycles per four-tile round) are gone, and their warp slots go to a third epilogue warp per
-// TMEM lane quarter.  Out-of-image blocks (the zero padding) are TMA's out-of-bounds fill.
+// zeros where the 3x3 filter has no entry.  No warp builds operands, so warps 4-15 are free for the epilogue (three per
+// TMEM lane quarter when the tile width splits into thirds).  Out-of-image blocks (the zero padding) are TMA's out-of-bounds fill.  The stride-1 stem runs here in its
+// pixel-pair form (see conv_tc_plan).
 // ---------------------------------------------------------------------------------------------
 template <int ACT, int OUT>
 __global__ void __launch_bounds__(kThreads, 1) conv_tc_stem2_kernel(const __grid_constant__ ConvTcParams p, int nimg) {
@@ -2321,10 +2167,8 @@ PFN_cuTensorMapEncodeTiled_v12000 get_encode() {
     return fn;
 }
 
-int env_int(const char* name, int dflt);
-
-int encode_map(CUtensorMap* map, void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
-               const uint32_t* box, uint32_t swizzle_bytes, bool f32 = false, int promo = 3) {
+int encode_map(CUtensorMap* map, void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes, const uint32_t* box,
+               uint32_t swizzle_bytes, bool f32 = false, CUtensorMapL2promotion promo = CU_TENSOR_MAP_L2_PROMOTION_L2_256B) {
     auto enc = get_encode();
     B2D_CHECK(enc != nullptr, "cuTensorMapEncodeTiled entry point not available");
     cuuint64_t gd[5], gs[4];
@@ -2336,9 +2180,7 @@ int encode_map(CUtensorMap* map, void* base, int rank, const uint64_t* dims, con
                           : swizzle_bytes == 32  ? CU_TENSOR_MAP_SWIZZLE_32B
                                                  : CU_TENSOR_MAP_SWIZZLE_NONE;
     CUresult r = enc(map, f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, rank, base, gd, gs, bx, es, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
-                     promo == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : promo == 1 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
-                     : promo == 2 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                     promo, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     B2D_CHECK(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled failed: CUresult %d (rank %d dims %llu %llu %llu %llu box %u %u %u %u)", (int)r, rank,
               (unsigned long long)dims[0], (unsigned long long)dims[1], (unsigned long long)(rank > 2 ? dims[2] : 0),
               (unsigned long long)(rank > 3 ? dims[3] : 0), box[0], box[1], rank > 2 ? box[2] : 0, rank > 3 ? box[3] : 0);
@@ -2352,8 +2194,7 @@ int encode_act_map(CUtensorMap* map, void* base, int c, int w, int h, int n, uin
     // L2 promotion widens every request to an aligned 64/128/256-byte block.  On a dense tensor (the slice is the whole
     // pixel) that is a free prefetch of the neighbouring pixel; on a channel slice of a wider concat buffer it drags in
     // the other producers' channels -- measured 3.3x the algorithmic DRAM reads on the 48-of-192-channel slices.
-    static const int promo_slice = env_int("B2D_PROMO_SLICE", 0), promo_dense = env_int("B2D_PROMO_DENSE", 3);
-    const int promo = (uint64_t)c * (f32 ? 4u : 2u) == pix_bytes ? promo_dense : promo_slice;
+    const CUtensorMapL2promotion promo = (uint64_t)c * (f32 ? 4u : 2u) == pix_bytes ? CU_TENSOR_MAP_L2_PROMOTION_L2_256B : CU_TENSOR_MAP_L2_PROMOTION_NONE;
     if (perm) {
         uint64_t dims[4] = {(uint64_t)c, (uint64_t)w, (uint64_t)n, (uint64_t)h};
         uint64_t str[3] = {pix_bytes, img_bytes, row_bytes};
@@ -2416,9 +2257,12 @@ int conv_tc_dw_supported(int cin, int cout, int ksz, int stride, int dst_f32, in
     return cin == cout && cin % 16 == 0 && ksz == 3 && stride == 1 && !dst_f32 && !has_res;
 }
 
-// the network input: 4-channel NHWC buffer of which the first `cin` (<= 4) carry weights, 3x3 or 1x1, bf16 output
+// the network input: 4-channel NHWC buffer of which the first `cin` (<= 4) carry weights, 3x3, 16-bit output, one output-channel
+// tile (the stride-1 form computes two pixels per GEMM row: N = 2 * cout).  conv_tc_plan checks what depends on the buffers:
+// an even input size (stride 2), an even-width output buffer of its own (stride 1), a one-image 8-pixel-wide tile.
 int conv_tc_stem_supported(int src_cs, int cin, int ksz, int stride, int cout, int dst_f32, int has_res) {
-    return src_cs == 4 && cin <= 4 && (ksz == 3 || ksz == 1) && (stride == 1 || stride == 2) && cout <= 256 && !dst_f32 && !has_res;
+    return src_cs == 4 && cin <= 4 && ksz == 3 && (stride == 2 || (stride == 1 && cout % 8 == 0 && 2 * cout <= 256)) && cout <= 256 &&
+           !dst_f32 && !has_res;
 }
 
 // fused depthwise + pointwise: c a multiple of 64 (whole K chunks), one output-channel tile, 16-bit unsplit storage
@@ -2447,8 +2291,8 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
     if (!stem) {
         B2D_CHECK(conv_tc_supported(cin, ksz, stride), "conv_tc: unsupported shape cin=%d k=%d s=%d", cin, ksz, stride);
         B2D_CHECK(src_cs % 8 == 0 && src_c0 % 8 == 0, "conv_tc: source slice must be 16-byte aligned (cs=%d c0=%d)", src_cs, src_c0);
-        B2D_CHECK(stride == 1 || (src_h % 2 == 0 && src_w % 2 == 0), "conv_tc: stride-2 input must have even size");
     }
+    B2D_CHECK(stride == 1 || (src_h % 2 == 0 && src_w % 2 == 0), "conv_tc: stride-2 input must have even size");
     // Stride-1 3x3 stem (YOLOv7 model.0) through TMA: two horizontally adjacent output pixels form ONE GEMM row.  For an even x the
     // inputs of pixels x and x + 1 (input pixels x - 1 .. x + 2) lie inside the 64 contiguous, 16-byte-aligned bytes of input pixels
     // x - 2 .. x + 5 of each of the three input rows, consecutive pairs are 16 bytes apart -- the no-swizzle K-major layout again
@@ -2456,14 +2300,14 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
     // in the NHWC output.  So the layer is planned as a conv with N = 2 * cout over an image of W / 2 pair-pixels: six K = 16 MMAs
     // per tile (3 filter rows x 32 input values) against weights that hold every filter tap twice, once per pixel of the pair.
     const int cout_real = cout;
-    const bool stem1 = stem && ksz == 3 && stride == 1 && dst_c0 == 0 && dst_cs == cout && dst_w % 2 == 0 && 2 * cout <= (x2 ? 128 : 256) &&
-                       cout % 8 == 0 && env_int("B2D_STEM_S1", 1) != 0;
+    const bool stem1 = stem && stride == 1;
+    B2D_CHECK(!stem1 || (dst_c0 == 0 && dst_cs == cout && dst_w % 2 == 0 && 2 * cout <= (x2 ? 128 : 256)),
+              "conv_tc: the stride-1 stem writes an even-width buffer of its own (%d of %d channels at %d, width %d)", cout, dst_cs, dst_c0, dst_w);
     if (stem1) { cout *= 2; dst_cs *= 2; dst_w /= 2; }
     ConvTcParams& p = plan->p;
     plan->sm_count = sm_count;
     const int kmul = (x2 && !stem) ? 2 : 1;        // storage channels per real input channel
     const int kin = cin * kmul, src_cs_s = src_cs * kmul, src_c0_s = src_c0 * kmul;
-    p.in_h = src_h; p.in_w = src_w; p.src_raw = src;
     p.W = dst_w; p.H = dst_h; p.cin = kin; p.cout = cout;
     p.ksz = ksz; p.taps = ksz * ksz; p.stride = stride;
     p.act = act; p.out_f32 = dst_f32;
@@ -2479,24 +2323,18 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
     p.n_tile = cout_pad / split;
     p.n_tiles_n = split;
     if (dw) p.chunks = ceil_div(kmul * p.n_tile, 64);     // depthwise: storage chunks of one channel tile
-    // the stride-2 stem is fed by TMA through a space-to-depth view (conv_tc_stem2_kernel) when an 8-pixel-wide one-image
-    // tile fits; anything else on the 4-channel input (stride 1, 1x1, odd sizes) keeps the gather kernel
-    bool stem2 = stem1 || (stem && ksz == 3 && stride == 2 && src_h % 2 == 0 && src_w % 2 == 0 && env_int("B2D_STEM_S2D", 1) != 0);
-    pick_tile(dst_w, dst_h, max_batch, &p.bw, &p.bh, &p.bn, dw || fused);
+    // the stem (conv_tc_stem2_kernel: space-to-depth for stride 2, pixel pairs for stride 1) and the fused and depthwise
+    // kernels need 8-pixel-wide tiles, the stem one-image ones
+    pick_tile(dst_w, dst_h, max_batch, &p.bw, &p.bh, &p.bn, stem || dw || fused);
+    B2D_CHECK(!stem || p.bn == 1, "conv_tc: the stem needs a one-image tile (tile %dx%dx%d)", p.bw, p.bh, p.bn);
     // 3x3 stride-2 layers with one K chunk: the stride-2 halo kernel when an 8-pixel-wide one-image tile fits (decided below with the
     // shared-memory budget: its nine weight boxes stay resident)
-    bool s2halo = !stem && !dw && !fused && ksz == 3 && stride == 2 && kin <= 64 && cout_pad <= 256 && env_int("B2D_S2HALO", 1) != 0;
+    bool s2halo = !stem && !dw && !fused && ksz == 3 && stride == 2 && kin <= 64 && cout_pad <= 256;
     if (s2halo) {
         int w8, h8, n8;
         pick_tile(dst_w, dst_h, max_batch, &w8, &h8, &n8, true);
         if (n8 == 1) { p.bw = w8; p.bh = h8; p.bn = n8; }
         else s2halo = false;
-    }
-    if (stem2) {
-        int w8, h8, n8;
-        pick_tile(dst_w, dst_h, max_batch, &w8, &h8, &n8, true);
-        if (n8 == 1) { p.bw = w8; p.bh = h8; p.bn = n8; }
-        else { B2D_CHECK(!stem1, "conv_tc: the stride-1 stem needs a one-image tile"); stem2 = false; }
     }
     p.perm = p.bn > 1 ? 1 : 0;
     p.tiles_x = ceil_div(dst_w, p.bw);
@@ -2513,7 +2351,7 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
         p.halo_w = 2 * p.bw + 6;
         p.a_tx_bytes = (uint32_t)((p.bh + 2) * p.halo_w * 8);
         p.a_bytes = (p.a_tx_bytes + 1023u) & ~1023u;
-    } else if (stem2) {        // one tile's box: (bh + 1) block rows x 2 row phases x (bw + 1) block columns x 16 bytes
+    } else if (stem) {        // one tile's box: (bh + 1) block rows x 2 row phases x (bw + 1) block columns x 16 bytes
         p.halo_w = p.bw + 1;
         p.a_tx_bytes = (uint32_t)((p.bh + 1) * 2 * (p.bw + 1) * 16);
         p.a_bytes = (p.a_tx_bytes + 1023u) & ~1023u;
@@ -2538,27 +2376,32 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
 
     // ---- kind, tiles per round, stages, staging buffers ----
     // halo: 3x3 stride 1 on 8-pixel-wide tiles (uniform (bw+2)-row stride between 8-row groups)
-    const bool halo_ok = !stem && ksz == 3 && stride == 1 && p.bw == 8 && (dw || env_int("B2D_HALO", 1) != 0);
+    const bool halo_ok = !stem && ksz == 3 && stride == 1 && p.bw == 8;
     B2D_CHECK(!dw || halo_ok, "conv_tc: depthwise needs an 8-pixel-wide tile");
     B2D_CHECK(!fused || (p.bw == 8 && p.bh % 2 == 0 && (p.bn == 1 ? p.bh % 4 == 0 : p.bn % 2 == 0)), "conv_tc: fused depthwise + pointwise needs an 8-pixel-wide tile that splits into two even halves");
-    if (!stem2) p.halo_w = p.bw + 2;
+    if (!stem) p.halo_w = p.bw + 2;
     p.halo_kh_rows = (uint32_t)(p.bn * p.halo_w);
     const uint32_t halo_rows = (uint32_t)(p.halo_w * p.bn * (p.bh + 2));
     p.halo_bytes = (halo_rows * 128u + 1023u) & ~1023u;
-    const int mt_env = env_int("B2D_MT", 0);
+    // test hooks: B2D_MT caps the M tiles per round and lifts the balance rule, B2D_PAIR = 2 forces CTA pairs (0 forbids them),
+    // so that small batches run the variants the planner picks at large ones
+    const int mt_env = env_int("B2D_MT", 0), pair_env = env_int("B2D_PAIR", 1);
+    const bool force_pair = pair_env == 2;
     const int mt_cap = stem ? 4 : 2;
-    int best_kind = -1, best_mt = 1, best_stages = 0, best_bufs = 1, best_bres = 0;
+    bool planned = false;
+    ConvKind best_kind = CONV_GENERIC;
+    int best_mt = 1, best_stages = 0, best_bufs = 1, best_bres = 0;
     const uint32_t dw_bytes = fused ? (((uint32_t)p.chunks * (9 * 64 + 64) * 4 + 1023u) & ~1023u) : 0u;   // depthwise weights + bias in shared memory
     if (s2halo) {
         // resident weights (nine boxes), two staging buffers if they fit, the rest phase-box slots (at least the four of one tile)
         const uint32_t box = ((uint32_t)((p.bw + 1) * (p.bh + 1)) * 128u + 1023u) & ~1023u;
         const uint32_t wres = 9u * p.b_bytes;
-        int bufs = env_int("B2D_STG2", 1) != 0 ? 2 : 1;
+        int bufs = 2;
         while (bufs >= 1 && avail < wres + (uint32_t)bufs * tile_stg + slab_bars(1, bufs) + 4u * box) --bufs;
         if (bufs >= 1 && split == 1) {
             int slots = (int)((avail - wres - (uint32_t)bufs * tile_stg - slab_bars(1, bufs)) / box);
             if (slots > 8) slots = 8;
-            best_kind = 6; best_mt = 1; best_stages = slots; best_bufs = bufs; best_bres = 1;
+            planned = true; best_kind = CONV_S2HALO; best_mt = 1; best_stages = slots; best_bufs = bufs; best_bres = 1;
             p.halo_w = p.bw + 1;
             p.halo_bytes = box;
         } else {
@@ -2578,22 +2421,25 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
         int st = (int)((avail - fixed - tile_stg - slab_bars(1, 1)) / p.b_bytes);
         if (st >= p.chunks) { st = p.chunks; best_bres = 1; }
         if (st > kMaxStages) st = kMaxStages;
-        best_bufs = (avail >= fixed + 2u * tile_stg + slab_bars(1, 2) + (uint32_t)st * p.b_bytes && env_int("B2D_STG2", 1) != 0) ? 2 : 1;
-        best_kind = 5; best_mt = 1; best_stages = st;
+        best_bufs = avail >= fixed + 2u * tile_stg + slab_bars(1, 2) + (uint32_t)st * p.b_bytes ? 2 : 1;
+        planned = true; best_kind = CONV_DWPW; best_mt = 1; best_stages = st;
     }
-    for (int mt = mt_cap; mt >= 1 && best_kind < 0; mt >>= 1) {
+    // the halo kernel falls back to the generic one when its buffers do not fit
+    const ConvKind first_kind = stem ? CONV_STEM : dw ? CONV_DEPTHWISE : halo_ok ? CONV_HALO : CONV_GENERIC;
+    const int nkinds = first_kind == CONV_HALO ? 2 : 1;
+    for (int mt = mt_cap; mt >= 1 && !planned; mt >>= 1) {
         if (mt_env > 0 && mt > mt_env) continue;
         if (mt > 1 && (split > 1 || 2 * mt * p.n_tile > 512)) continue;
         if (mt > 1 && !stem && mt_env == 0 && total_tiles < 4 * mt * sm_count) continue;   // keep enough rounds per SM for balance (B2D_MT forces)
-        for (int kind = (stem ? 2 : halo_ok ? 1 : 0); kind >= (stem ? 2 : dw ? 1 : 0) && best_kind < 0; --kind) {
-            for (int bufs = 2; bufs >= 1 && best_kind < 0; --bufs) {
-                if (bufs == 2 && env_int("B2D_STG2", 1) == 0) continue;
+        for (int ki = 0; ki < nkinds && !planned; ++ki) {
+            const ConvKind kind = ki == 0 ? first_kind : CONV_GENERIC;
+            for (int bufs = 2; bufs >= 1 && !planned; --bufs) {
                 const uint32_t stg = (uint32_t)bufs * mt * tile_stg + slab_bars(mt, bufs);
                 if (stg + 4096 > avail) continue;
                 const uint32_t room = avail - stg;
                 int stages = 0, min_stages = 0;
                 bool bres = false;
-                if (kind == 0) {
+                if (kind == CONV_GENERIC) {
                     const uint32_t sb = (uint32_t)mt * p.a_bytes + p.b_bytes;
                     stages = (int)(room / sb);
                     const int ksteps = p.taps * p.chunks;
@@ -2601,15 +2447,15 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
                     // a second staging buffer is worth more than a deep ring when a round has few k-steps (memory-bound 1x1 layers)
                     min_stages = (bufs == 2 || mt > 1) ? 4 : 2;
                     if (ksteps < min_stages) min_stages = ksteps < 2 ? 2 : ksteps;
-                } else if (kind == 1) {
+                } else if (kind == CONV_HALO || kind == CONV_DEPTHWISE) {
                     const uint32_t fixed = 2u * mt * p.halo_bytes;
                     stages = room > fixed ? (int)((room - fixed) / p.b_bytes) : 0;
                     min_stages = (bufs == 2 || mt > 1) ? 4 : 3;
                     // resident weights: every (chunk, tap) weight box gets its own stage, loaded once per CTA.  The narrow 3x3
                     // layers are bound by the TMA unit's request rate and the per-round weight refetch was a third of it.
-                    bres = !dw && split == 1 && 9 * p.chunks <= kMaxStages && stages >= 9 * p.chunks && env_int("B2D_BRES", 1) != 0;
+                    bres = kind == CONV_HALO && split == 1 && 9 * p.chunks <= kMaxStages && stages >= 9 * p.chunks;
                     if (bres) stages = 9 * p.chunks;
-                } else {
+                } else {                                // CONV_STEM: resident weights
                     const uint32_t sb = (uint32_t)mt * p.a_bytes;
                     stages = room > p.b_bytes ? (int)((room - p.b_bytes) / sb) : 0;
                     if (stages > 4) stages = 4;
@@ -2617,21 +2463,21 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
                 }
                 if (stages > kMaxStages) stages = kMaxStages;
                 if (stages < min_stages) continue;
-                best_kind = kind; best_mt = mt; best_stages = stages; best_bufs = bufs; best_bres = bres ? 1 : 0;
+                planned = true; best_kind = kind; best_mt = mt; best_stages = stages; best_bufs = bufs; best_bres = bres ? 1 : 0;
             }
         }
     }
-    B2D_CHECK(best_kind >= 0, "conv_tc: no shared-memory configuration fits (n_tile %d)", p.n_tile);
-    p.kind = dw ? 3 : stem2 ? 4 : best_kind; p.mt = best_mt; p.stages = best_stages; p.stg_bufs = best_bufs; p.b_res = best_bres;
+    B2D_CHECK(planned, "conv_tc: no shared-memory configuration fits (n_tile %d)", p.n_tile);
+    p.kind = best_kind; p.mt = best_mt; p.stages = best_stages; p.stg_bufs = best_bufs; p.b_res = best_bres;
     // CTA pairs for wide halo layers: weight stages shrink to half a tile per CTA (so the ring gets deeper)
     p.pair = 0;
-    if (p.kind == 1 && split == 1 && p.n_tile >= env_int("B2D_PAIR_MIN_N", 128) && p.n_tile % 32 == 0 && (total_tiles >= 2 * sm_count || env_int("B2D_PAIR", 1) == 2) && env_int("B2D_PAIR", 1) != 0) {
+    if (p.kind == CONV_HALO && split == 1 && p.n_tile >= 128 && p.n_tile % 32 == 0 && (total_tiles >= 2 * sm_count || force_pair) && pair_env != 0) {
         p.pair = 1;
         p.mt = 1;
         p.b_res = 0;
         p.b_tx_bytes = (uint32_t)(p.n_tile / 2) * 128u;
         p.b_bytes = (p.b_tx_bytes + 1023u) & ~1023u;
-        if (avail > 2u * tile_stg + 2u * p.halo_bytes + 6u * p.b_bytes + slab_bars(1, 2) && env_int("B2D_STG2", 1) != 0) p.stg_bufs = 2;
+        if (avail > 2u * tile_stg + 2u * p.halo_bytes + 6u * p.b_bytes + slab_bars(1, 2)) p.stg_bufs = 2;
         const uint32_t room = avail - (uint32_t)p.stg_bufs * tile_stg - 2u * p.halo_bytes - slab_bars(1, p.stg_bufs);
         int st = (int)(room / p.b_bytes);
         p.stages = st > kMaxStages ? kMaxStages : st;
@@ -2643,63 +2489,55 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
     const int k_total = cin * p.taps;
     // ... and the 3x3 stride-1 layers that run here because their tiles are not 8 pixels wide (288 -> 288 at 20 x 20, two N = 144
     // tiles): 41.6 -> 35 us each with the pair's halved weight traffic (gpurun_out/r2bg), N / 2 = 72 rows per CTA.
-    const bool pair_short_k = k_total < env_int("B2D_PAIRG_MAX_K", 576) || (stride == 2 && cin <= 96) || (ksz == 3 && stride == 1 && env_int("B2D_PAIRG_3X3", 1) != 0);
-    if (p.kind == 0 && !stem && p.n_tile >= env_int("B2D_PAIRG_MIN_N", 128) && p.n_tile % 16 == 0 && p.mt == 1 &&
-        (pair_short_k || env_int("B2D_PAIR", 1) == 2) &&
-        (total_tiles >= 2 * sm_count || env_int("B2D_PAIR", 1) == 2) && env_int("B2D_PAIR", 1) != 0 && env_int("B2D_PAIRG", 1) != 0) {
+    const bool pair_short_k = k_total < 576 || (stride == 2 && cin <= 96) || (ksz == 3 && stride == 1);
+    if (p.kind == CONV_GENERIC && p.n_tile >= 128 && p.n_tile % 16 == 0 && p.mt == 1 && (pair_short_k || force_pair) &&
+        (total_tiles >= 2 * sm_count || force_pair) && pair_env != 0) {
         p.pair = 1;
         p.b_tx_bytes = (uint32_t)(p.n_tile / 2) * 128u;
         p.b_bytes = (p.b_tx_bytes + 1023u) & ~1023u;
         const uint32_t sb = p.a_bytes + p.b_bytes;
-        if (avail > 2u * tile_stg + 4u * sb + slab_bars(1, 2) && env_int("B2D_STG2", 1) != 0) p.stg_bufs = 2;
+        if (avail > 2u * tile_stg + 4u * sb + slab_bars(1, 2)) p.stg_bufs = 2;
         const uint32_t room = avail - (uint32_t)p.stg_bufs * tile_stg - slab_bars(1, p.stg_bufs);
         int st = (int)(room / sb);
         const int ksteps = p.taps * p.chunks;
         if (st > 2 * ksteps) st = 2 * ksteps;
         p.stages = st > kMaxStages ? kMaxStages : st;
     }
-    if (best_kind == 1 || best_kind == 5) p.a_tx_bytes = halo_rows * 128u;
-    if (best_kind == 6) p.a_tx_bytes = (uint32_t)((p.bw + 1) * (p.bh + 1)) * 128u;
     const uint32_t stg_bytes = (uint32_t)p.stg_bufs * p.mt * tile_stg;
-    uint32_t operand_bytes;
-    if (p.kind == 0) operand_bytes = (uint32_t)p.stages * ((uint32_t)p.mt * p.a_bytes + p.b_bytes);
-    else if (p.kind == 1 || p.kind == 3) operand_bytes = 2u * p.mt * p.halo_bytes + (uint32_t)p.stages * p.b_bytes;
-    else if (p.kind == 5) operand_bytes = 2u * p.halo_bytes + 2u * p.a_bytes + (uint32_t)p.stages * p.b_bytes + dw_bytes;
-    else if (p.kind == 6) operand_bytes = (uint32_t)p.stages * p.halo_bytes + 9u * p.b_bytes;
-    else operand_bytes = (uint32_t)p.stages * p.mt * p.a_bytes + p.b_bytes;
+    uint32_t operand_bytes = 0;
+    switch (p.kind) {
+        case CONV_GENERIC: operand_bytes = (uint32_t)p.stages * ((uint32_t)p.mt * p.a_bytes + p.b_bytes); break;
+        case CONV_HALO:
+        case CONV_DEPTHWISE:
+            p.a_tx_bytes = halo_rows * 128u;
+            operand_bytes = 2u * p.mt * p.halo_bytes + (uint32_t)p.stages * p.b_bytes;
+            break;
+        case CONV_STEM: operand_bytes = (uint32_t)p.stages * p.mt * p.a_bytes + p.b_bytes; break;
+        case CONV_DWPW:
+            p.a_tx_bytes = halo_rows * 128u;
+            operand_bytes = 2u * p.halo_bytes + 2u * p.a_bytes + (uint32_t)p.stages * p.b_bytes + dw_bytes;
+            break;
+        case CONV_S2HALO:
+            p.a_tx_bytes = (uint32_t)((p.bw + 1) * (p.bh + 1)) * 128u;
+            operand_bytes = (uint32_t)p.stages * p.halo_bytes + 9u * p.b_bytes;
+            break;
+    }
     p.stg_off = operand_bytes;                                   // 1 KiB aligned: every operand slot is a multiple of 1 KiB
     p.dw_off = operand_bytes - dw_bytes;
     p.bar_off = p.stg_off + stg_bytes;
     plan->smem_bytes = (size_t)p.bar_off + tail_fixed + slab_bars(p.mt, p.stg_bufs) + 1024 /*align slack*/;
     B2D_CHECK(plan->smem_bytes <= 227 * 1024, "conv_tc: %zu bytes of shared memory needed", plan->smem_bytes);
-    {   // epilogue chunks: a row of n_tile columns cut into 128 / 64 / 32-byte pieces
-        uint32_t done = 0, off = 0;
-        int n = 0;
-        const uint32_t spans[3] = {128, 64, 32};
-        for (int si = 0; si < 3; ++si)
-            while (row_bytes - done >= spans[si]) {
-                B2D_CHECK(n < kMaxEpiChunks, "conv_tc: n_tile %d needs too many epilogue chunks", p.n_tile);
-                p.epi[n].col0 = (uint16_t)(done / esize);
-                p.epi[n].cols = (uint16_t)(spans[si] / esize);
-                p.epi[n].span = (uint16_t)spans[si];
-                p.epi[n].map = (uint16_t)si;
-                p.epi[n].off = off;
-                off += 128u * spans[si];
-                done += spans[si];
-                ++n;
-            }
-        B2D_CHECK(done == row_bytes, "conv_tc: n_tile %d is not a multiple of 32 bytes", p.n_tile);
-        p.epi_nchunks = n;
-    }
+    // epilogue chunks (epi_chunks): at most six, which bounds fp32 tiles at 192 columns
+    const EpiChunks epi = epi_chunks(row_bytes);
+    B2D_CHECK(epi.n128 + epi.has64 + epi.has32 <= 6, "conv_tc: n_tile %d needs too many epilogue chunks", p.n_tile);
+    B2D_CHECK(row_bytes % 32 == 0, "conv_tc: n_tile %d is not a multiple of 32 bytes", p.n_tile);
     p.has_res = res ? 1 : 0;
     // Epilogue warps per TMEM lane quarter.  A warp's epilogue is a chain of dependent instructions (TMEM load -> bias FMA ->
     // MUFU.TANH -> FMA -> pack -> shared store) that issues about one instruction per six cycles; with two warps per scheduler
     // the epilogue ran at 3-4.5 outputs per clock per SM against 15 for the same code with eight warps per scheduler
     // (role traces, profiles/r2_role_traces.txt).  A third warp per quarter takes every third 16-column unit when the tile
-    // width allows an even split (48, 96, 144, 192 ...); the stem's 16 warps are taken (gather warps).
-    p.epi_parts = fused ? 1 : ((!stem || stem2) && (p.n_tile >> 4) % 3 == 0 && env_int("B2D_EPI3", 1) != 0) ? 3 : 2;   // fused: warps 8-15 compute the depthwise stage
-    p.exp = env_int("B2D_EXP", 0);
-    p.epi_path = env_int("B2D_EPI_PATH", 2);      // 0: item-list epilogue everywhere, 1: + straight-line path for one- and two-unit warps, 2: + tile-structured path for wide tiles
+    // width allows an even split (48, 96, 144, 192 ...).
+    p.epi_parts = fused ? 1 : (p.n_tile >> 4) % 3 == 0 ? 3 : 2;   // fused: warps 8-15 compute the depthwise stage
     p.trace = nullptr;
     if (getenv("B2D_TRACE")) {
         B2D_CUDA(cudaMalloc(&plan->trace_dev, sizeof(long long) * kTraceRoles * kTraceTiles * kTraceEvents));
@@ -2715,7 +2553,7 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
 
     // ---- weights: fp32 [cout][cin][k][k] -> bf16 [cout_pad][kh][kw][cin_pad] (zero padded) ----
     const int cin_pad = p.chunks * 64;
-    const size_t ktot = stem1 ? 128 : stem ? 64 : (size_t)p.taps * cin_pad;     // stem: k = tap * 4 + c, one 128-byte row per output channel
+    const size_t ktot = stem1 ? 128 : stem ? 64 : (size_t)p.taps * cin_pad;     // stem: one or two 128-byte rows per output channel
     const int dw_chunks = p.chunks * split;                       // depthwise: 64-channel chunks over all channels
     std::vector<uint16_t> wp(dw ? (size_t)dw_chunks * 9 * 16 * 64 : (size_t)cout_pad * ktot, 0);
     if (dw && x2) {
@@ -2746,12 +2584,10 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
                         const int kh = t / 3, kw = t % 3;
                         for (int half = 0; half < 2; ++half)
                             wp[(size_t)(half * cout_real + o) * ktot + (size_t)(kh * 32 + (kw + 1 + half) * 4 + c)] = v;
-                    } else if (stem2) {      // tap (kh, kw) -> block (di, dj), phase (rp, px): k = (di * 2 + dj) * 16 + rp * 8 + px * 4 + c
+                    } else if (stem) {      // tap (kh, kw) -> block (di, dj), phase (rp, px): k = (di * 2 + dj) * 16 + rp * 8 + px * 4 + c
                         const int kh = t / 3, kw = t % 3;
                         const int di = kh == 0 ? 0 : 1, rp = kh == 1 ? 0 : 1, dj = kw == 0 ? 0 : 1, px = kw == 1 ? 0 : 1;
                         wp[(size_t)o * ktot + (size_t)((di * 2 + dj) * 16 + rp * 8 + px * 4 + c)] = v;
-                    } else if (stem) {
-                        wp[(size_t)o * ktot + (size_t)t * 4 + c] = v;
                     } else if (kmul == 2) {      // the weight sits under the channel's hi and lo position
                         const size_t k = (size_t)t * cin_pad + 16 * (c / 8) + (c % 8);
                         wp[(size_t)o * ktot + k] = v;
@@ -2805,16 +2641,16 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
             if (encode_map(&p.tmB, plan->w_dev, 2, dims, str, box, 128)) return -1;
         }
         const uint64_t pix = (uint64_t)src_cs_s * 2, rowb = (uint64_t)src_w * pix, imgb = (uint64_t)src_h * rowb;
-        if (p.kind == 1 || p.kind == 3 || p.kind == 5) {
+        if (p.kind == CONV_HALO || p.kind == CONV_DEPTHWISE || p.kind == CONV_DWPW) {
             if (encode_act_map(&p.tmA[0], (void*)(src + src_c0_s), kin, src_w, src_h, max_batch, pix, rowb, imgb, 64u, (uint32_t)p.halo_w,
-                               (uint32_t)(p.bh + 2), (uint32_t)p.bn, perm, p.kind == 5 ? 0 : 128))    // fused: read by threads, plain rows
+                               (uint32_t)(p.bh + 2), (uint32_t)p.bn, perm, p.kind == CONV_DWPW ? 0 : 128))    // fused: read by threads, plain rows
                 return -1;
         } else if (stride == 1) {
             if (encode_act_map(&p.tmA[0], (void*)(src + src_c0_s), kin, src_w, src_h, max_batch, pix, rowb, imgb, 64u, (uint32_t)p.bw, (uint32_t)p.bh,
                                (uint32_t)p.bn, perm, 128))
                 return -1;
         } else {
-            const uint32_t hb = p.kind == 6 ? 1u : 0u;           // stride-2 halo kernel: one more column and row per phase box
+            const uint32_t hb = p.kind == CONV_S2HALO ? 1u : 0u;           // stride-2 halo kernel: one more column and row per phase box
             for (int py = 0; py < 2; ++py)
                 for (int px = 0; px < 2; ++px) {
                     const __nv_bfloat16* base = src + ((size_t)py * src_w + px) * src_cs_s + src_c0_s;
@@ -2829,7 +2665,7 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
         uint64_t str[3] = {(uint64_t)src_w * 8, (uint64_t)src_h * src_w * 8, (uint64_t)src_h * src_w * 8 * (uint64_t)max_batch};
         uint32_t box[4] = {(uint32_t)p.halo_w * 4u, (uint32_t)(p.bh + 2), 1u, 1u};
         if (encode_map(&p.tmA[0], (void*)src, 4, dims, str, box, 0)) return -1;
-    } else if (stem2) {        // (8-byte pixels of one input row as 16-bit elements | row phase | block row | image), un-swizzled box
+    } else if (stem) {        // (8-byte pixels of one input row as 16-bit elements | row phase | block row | image), un-swizzled box
         uint64_t dims[4] = {(uint64_t)src_w * 4, 2u, (uint64_t)src_h / 2, (uint64_t)max_batch};
         uint64_t str[3] = {(uint64_t)src_w * 8, (uint64_t)src_w * 16, (uint64_t)src_h * src_w * 8};
         uint32_t box[4] = {(uint32_t)(p.bw + 1) * 8u, 2u, (uint32_t)(p.bh + 1), 1u};
@@ -2838,8 +2674,7 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
     {   // output / residual maps: the box is one M tile, one map per chunk width
         const uint32_t sbn = (uint32_t)p.bn, sbh = (uint32_t)p.bh;
         const uint32_t spans[3] = {128, 64, 32};
-        bool used[3] = {false, false, false};
-        for (int k = 0; k < p.epi_nchunks; ++k) used[p.epi[k].map] = true;
+        const bool used[3] = {epi.n128 > 0, epi.has64 != 0, epi.has32 != 0};
         const uint64_t pix = (uint64_t)dst_cs * esize, rowb = (uint64_t)dst_w * pix, imgb = (uint64_t)dst_h * rowb;
         for (int si = 0; si < 3; ++si) {
             if (!used[si]) continue;
@@ -2860,21 +2695,20 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
 namespace {
 typedef void (*ConvKernel)(const ConvTcParams, int);
 // (kind, act, res, out) -> instantiation; out: 0 16-bit, 1 fp32 (never with a residual), 2 split fp16
-ConvKernel pick_kernel(int kind, int pair, int act, int res, int out) {
+ConvKernel pick_kernel(ConvKind kind, int pair, int act, int res, int out) {
 #define B2D_PICK(K)                                                        \
     if (out == 1) return act ? K<1, 0, 1> : K<0, 0, 1>;                    \
     if (out == 2 && res) return act ? K<1, 1, 2> : K<0, 1, 2>;             \
     if (out == 2) return act ? K<1, 0, 2> : K<0, 0, 2>;                    \
     if (res) return act ? K<1, 1, 0> : K<0, 1, 0>;                         \
     return act ? K<1, 0, 0> : K<0, 0, 0>;
-    if (kind == 2) return out == 2 ? (act ? conv_tc_stem_kernel<1, 2> : conv_tc_stem_kernel<0, 2>) : (act ? conv_tc_stem_kernel<1, 0> : conv_tc_stem_kernel<0, 0>);
-    if (kind == 6) { B2D_PICK(conv_tc_s2halo_kernel) }
-    if (kind == 5) return act ? conv_tc_dwpw_kernel<1, 0> : conv_tc_dwpw_kernel<0, 0>;
-    if (kind == 4) return out == 2 ? (act ? conv_tc_stem2_kernel<1, 2> : conv_tc_stem2_kernel<0, 2>) : (act ? conv_tc_stem2_kernel<1, 0> : conv_tc_stem2_kernel<0, 0>);
-    if (kind == 3) return out == 2 ? (act ? conv_tc_dw_kernel<1, 2> : conv_tc_dw_kernel<0, 2>) : (act ? conv_tc_dw_kernel<1, 0> : conv_tc_dw_kernel<0, 0>);
-    if (kind == 1 && pair) { B2D_PICK(conv_tc_halo2_kernel) }
-    if (kind == 0 && pair) { B2D_PICK(conv_tc_pair_kernel) }
-    if (kind == 1) { B2D_PICK(conv_tc_halo_kernel) }
+    if (kind == CONV_S2HALO) { B2D_PICK(conv_tc_s2halo_kernel) }
+    if (kind == CONV_DWPW) return act ? conv_tc_dwpw_kernel<1, 0> : conv_tc_dwpw_kernel<0, 0>;
+    if (kind == CONV_STEM) return out == 2 ? (act ? conv_tc_stem2_kernel<1, 2> : conv_tc_stem2_kernel<0, 2>) : (act ? conv_tc_stem2_kernel<1, 0> : conv_tc_stem2_kernel<0, 0>);
+    if (kind == CONV_DEPTHWISE) return out == 2 ? (act ? conv_tc_dw_kernel<1, 2> : conv_tc_dw_kernel<0, 2>) : (act ? conv_tc_dw_kernel<1, 0> : conv_tc_dw_kernel<0, 0>);
+    if (kind == CONV_HALO && pair) { B2D_PICK(conv_tc_halo2_kernel) }
+    if (kind == CONV_GENERIC && pair) { B2D_PICK(conv_tc_pair_kernel) }
+    if (kind == CONV_HALO) { B2D_PICK(conv_tc_halo_kernel) }
     B2D_PICK(conv_tc_kernel)
 #undef B2D_PICK
 }
@@ -2888,10 +2722,6 @@ int conv_tc_launch(const ConvTcPlan* plan, int n, cudaStream_t stream) {
     p.rev_last = p.rev ? tiles / p.n_tiles_n - 1 : -1;
     const int rounds = ceil_div(tiles, p.mt);
     int grid = rounds < plan->sm_count ? rounds : plan->sm_count;
-    {   // debug: B2D_GRID caps the number of CTAs (per-SM vs chip-wide bottleneck experiments)
-        static const int cap = env_int("B2D_GRID", 0);
-        if (cap > 0 && grid > cap) grid = cap;
-    }
     if (grid < 1) return 0;
     if (p.pair) {
         const int prs = ceil_div(tiles / p.n_tiles_n, 2) * p.n_tiles_n;      // rounds of a pair (see pair_rounds)
@@ -2903,24 +2733,16 @@ int conv_tc_launch(const ConvTcPlan* plan, int n, cudaStream_t stream) {
     {
         cudaLaunchConfig_t cfg{};
         cfg.gridDim = dim3((unsigned)grid);
-        cfg.blockDim = dim3(p.kind == 2 ? kStemThreads : kThreads);
+        cfg.blockDim = dim3(kThreads);
         cfg.dynamicSmemBytes = plan->smem_bytes;
         cfg.stream = stream;
-        cudaLaunchAttribute attr[2];
-        int na = 0;
-        static const int pdl = env_int("B2D_PDL", 0);   // measured neutral to slightly negative on B200 for this kernel chain
-        if (pdl) {
-            attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-            attr[na].val.programmaticStreamSerializationAllowed = 1;
-            ++na;
-        }
+        cudaLaunchAttribute attr[1];
         if (p.pair) {
-            attr[na].id = cudaLaunchAttributeClusterDimension;
-            attr[na].val.clusterDim.x = 2; attr[na].val.clusterDim.y = 1; attr[na].val.clusterDim.z = 1;
-            ++na;
+            attr[0].id = cudaLaunchAttributeClusterDimension;
+            attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
         }
         cfg.attrs = attr;
-        cfg.numAttrs = na;
+        cfg.numAttrs = p.pair ? 1 : 0;
         B2D_CUDA(cudaLaunchKernelEx(&cfg, k, p, n));
     }
     if (p.trace && getenv("B2D_TRACE_DUMP")) {
@@ -2959,8 +2781,17 @@ void conv_tc_free(ConvTcPlan* plan) {
 
 int conv_tc_describe(const ConvTcPlan* plan, char* buf, int buflen) {
     const ConvTcParams& p = plan->p;
-    static const char* kinds[9] = {"", "-halo", "-stem", "-depthwise", "-halo-pair", "-pair", "-stem-s2d", "-dw3x3+pw", "-s2halo"};
+    const char* name = "";
+    switch (p.kind) {
+        case CONV_GENERIC: name = p.pair ? "-pair" : ""; break;
+        case CONV_HALO: name = p.pair ? "-halo-pair" : "-halo"; break;
+        case CONV_DEPTHWISE: name = "-depthwise"; break;
+        case CONV_STEM: name = p.stride == 1 ? "-stem-pairs" : "-stem-s2d"; break;
+        case CONV_DWPW: name = "-dw3x3+pw"; break;
+        case CONV_S2HALO: name = "-s2halo"; break;
+    }
+    const int cin = p.x2 && p.kind != CONV_STEM ? p.cin / 2 : p.cin;     // split storage doubles K, except on the network input
     return snprintf(buf, buflen, "tcgen05%s conv k%d s%d cin %d cout %d -> %dx%d | tile %dx%dx%d x%d n_tile %d x%d stages %d%s stg %d tmem %u smem %zu",
-                    p.kind == 4 && p.stride == 1 ? "-stem-pairs" : kinds[p.pair ? (p.kind == 0 ? 5 : 4) : p.kind == 4 ? 6 : p.kind == 5 ? 7 : p.kind == 6 ? 8 : p.kind], p.ksz, p.stride, (p.x2 && p.kind != 2) ? p.cin / 2 : p.cin, p.cout, p.H, p.W, p.bw, p.bh, p.bn, p.mt, p.n_tile, p.n_tiles_n, p.stages,
+                    name, p.ksz, p.stride, cin, p.cout, p.H, p.W, p.bw, p.bh, p.bn, p.mt, p.n_tile, p.n_tiles_n, p.stages,
                     p.b_res ? " (resident)" : "", p.stg_bufs, p.tmem_cols, plan->smem_bytes);
 }

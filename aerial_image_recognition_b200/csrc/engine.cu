@@ -234,14 +234,13 @@ int launch_fwd_op(b2d_engine* e, int i, int n, cudaStream_t s) {
 // write-after-write between channel ranges of the same buffer.  Independent chains -- the six branches of the
 // detect head, head level 0 against the rest of the PAN path -- become parallel branches of the graph, so one
 // kernel's CTAs start on the SMs another kernel's tail has already left (each persistent kernel holds a whole SM, so
-// nothing else can hide the ~6 us of prologue and tail per launch).  B2D_STREAMS=1 keeps a single chain.
+// nothing else can hide the ~6 us of prologue and tail per launch).
 struct Range { int buf, c0, c1; };
 static bool overlaps(const Range& a, const Range& b) { return a.buf == b.buf && a.buf >= 0 && a.c0 < b.c1 && b.c0 < a.c1; }
 
 int capture_ops(b2d_engine* e, int n) {
     const int nops = (int)e->ops.size();
-    static const int ns_env = getenv("B2D_STREAMS") ? atoi(getenv("B2D_STREAMS")) : 3;
-    const int ns = ns_env < 1 ? 1 : (ns_env > 8 ? 8 : ns_env);
+    const int ns = 3;                                        // capture streams
     while ((int)e->side_streams.size() < ns - 1) {
         cudaStream_t s;
         B2D_CUDA(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
@@ -337,16 +336,6 @@ int b2d_create(int device, int max_batch, b2d_engine** out) {
     B2D_CHECK(prop.major == 10, "b2d_create: device %d is sm_%d%d; this library is built for sm_100a (B200) only", device, prop.major,
               prop.minor);
     DeviceGuard guard(device);
-    {   // Experiment knob: B2D_L2_FETCH = 32 / 64 / 128 sets cudaLimitMaxL2FetchGranularity (driver default 64; measured
-        // neutral for this kernel chain, profiles/r1_l2_fetch_granularity.txt), unset leaves the default.
-        const char* g = getenv("B2D_L2_FETCH");
-        const int gran = g ? atoi(g) : 0;
-        if (gran > 0) cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t)gran);
-        size_t got = 0;
-        cudaDeviceGetLimit(&got, cudaLimitMaxL2FetchGranularity);
-        if (getenv("B2D_VERBOSE")) fprintf(stderr, "b2det: L2 fetch granularity %zu bytes\n", got);
-        cudaGetLastError();
-    }
     b2d_engine* e = new b2d_engine();
     e->device = device;
     e->max_batch = max_batch;
@@ -543,16 +532,12 @@ int b2d_plan_finalize(b2d_engine* e) {
             op.h = sb.h; op.w = sb.w; op.src_cs = sb.c; op.src_c0 = d.src_c0;
             op.oh = db.h; op.ow = db.w; op.dst_cs = db.c; op.dst_c0 = d.dst_c0; op.c = d.cout; op.k = d.k; op.stride = d.stride;
         }
-        if (op.kind == OP_CONV_TC) {        // B2D_REV: 1 (default) odd ops walk backwards, 0 nobody, 2 everybody
-            static const int rev_mode = getenv("B2D_REV") ? atoi(getenv("B2D_REV")) : 1;
-            op.tc.p.rev = rev_mode == 2 ? 1 : rev_mode == 1 ? (int)(i & 1) : 0;
-        }
+        if (op.kind == OP_CONV_TC) op.tc.p.rev = (int)(i & 1);     // odd ops walk their tiles backwards (see conv_tc_launch)
     }
-    // Depthwise 3x3 followed by the 1x1 conv that is its only reader -> one kernel in forward() (B2D_FUSE_DWPW=0 keeps the pair).
+    // Depthwise 3x3 followed by the 1x1 conv that is its only reader -> one kernel in forward().
     e->fused_at.assign(e->descs.size(), -1);
     e->fused_plans.reserve(e->descs.size());
-    static const bool fuse_dwpw = getenv("B2D_FUSE_DWPW") ? atoi(getenv("B2D_FUSE_DWPW")) != 0 : true;
-    for (size_t i = 0; fuse_dwpw && i + 1 < e->descs.size(); ++i) {
+    for (size_t i = 0; i + 1 < e->descs.size(); ++i) {
         const OpDesc& d0 = e->descs[i];
         const OpDesc& d1 = e->descs[i + 1];
         if (d0.kind_req != 1 || d1.kind_req != 0 || d1.k != 1 || d1.stride != 1 || d1.res >= 0) continue;
@@ -661,7 +646,7 @@ int b2d_forward(b2d_engine* e, int n, void* stream) {
     B2D_CHECK(n > 0 && n <= e->max_batch, "forward: n=%d outside [1,%d]", n, e->max_batch);
     B2D_ENTER(e);
     cudaStream_t st = (cudaStream_t)stream;
-    static const bool use_graph = (getenv("B2D_GRAPH") ? atoi(getenv("B2D_GRAPH")) != 0 : true) && !getenv("B2D_TRACE");
+    static const bool use_graph = !getenv("B2D_TRACE");      // conv_tc_launch resets and reads back the role trace per launch
     auto it = e->fwd_graphs.find(n);
     if (use_graph && it != e->fwd_graphs.end()) {
         B2D_CUDA(cudaGraphLaunch(it->second, st));

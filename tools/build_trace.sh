@@ -1,4 +1,4 @@
-# trace/ablation build of the library (role timelines, B2D_EXP ablation bits) -> tools/ubench/build/libb2det_trace.so
+# trace build of the library (per-role timelines, B2D_TRACE / B2D_TRACE_DUMP) -> tools/ubench/build/libb2det_trace.so
 set -e
 cd "$(dirname "$0")/../aerial_image_recognition_b200/csrc"
 mkdir -p ../../tools/ubench/build/tr
