@@ -35,6 +35,12 @@
 // warp-uniformly and elect one lane around the asynchronous instructions.  Pipelines: smem ring
 // (full/empty mbarriers) TMA -> MMA; two TMEM accumulator stages (tmem_full/tmem_empty) MMA ->
 // epilogue; one or two staging slabs epilogue -> TMA store.
+//
+// CTA pairs: the generic and halo kernels have a second form (template argument PAIR = 1) for wide output tiles, in which the
+// two CTAs of a cluster compute two M tiles with one stream of cta_group::2 MMAs (M = 256) issued by the leader, each CTA
+// loading its own A and half of every weight box.  The forms share their main loops; what differs is written as
+// `if constexpr (PAIR)` or as the PAIR form of a PTX wrapper.  RoundSched is the one description of which rounds and tiles
+// a CTA computes, used by every role of every kernel.
 #include "common.cuh"
 
 #include <cudaTypedefs.h>
@@ -68,8 +74,11 @@ __device__ __forceinline__ void mbar_wait_u32(uint32_t addr, uint32_t parity) {
         "DONE:\n\t"
         "}" ::"r"(addr), "r"(parity) : "memory");
 }
+// PAIR = 1 selects the CTA-pair form of an instruction (see cluster_ctarank below): here `addr` is a shared::cluster address
+template <int PAIR = 0>
 __device__ __forceinline__ void mbar_expect_tx_u32(uint32_t addr, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(addr), "r"(bytes) : "memory");
+    if constexpr (PAIR) asm volatile("mbarrier.arrive.expect_tx.shared::cluster.b64 _, [%0], %1;" ::"r"(addr), "r"(bytes) : "memory");
+    else asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(addr), "r"(bytes) : "memory");
 }
 // one lane of a converged warp (always the same one for a full mask)
 __device__ __forceinline__ bool elect_one() {
@@ -85,17 +94,38 @@ __device__ __forceinline__ bool elect_one() {
 __device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
+// PAIR: `bar` is the leader's barrier (a shared::cluster address), the completion is signalled there
+template <int PAIR = 0>
 __device__ __forceinline__ void tma_load_4d(const CUtensorMap* map, uint32_t bar, uint32_t dst_smem, int c0, int c1, int c2, int c3) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];" ::"r"(dst_smem),
-        "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-        : "memory");
+    if constexpr (PAIR)
+        asm volatile(
+            "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];" ::"r"(dst_smem),
+            "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
+            : "memory");
+    else
+        asm volatile(
+            "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];" ::"r"(dst_smem),
+            "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
+            : "memory");
 }
+template <int PAIR = 0>
 __device__ __forceinline__ void tma_load_2d(const CUtensorMap* map, uint32_t bar, uint32_t dst_smem, int c0, int c1) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(dst_smem),
-        "l"(map), "r"(bar), "r"(c0), "r"(c1)
-        : "memory");
+    if constexpr (PAIR)
+        asm volatile(
+            "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(dst_smem),
+            "l"(map), "r"(bar), "r"(c0), "r"(c1)
+            : "memory");
+    else
+        asm volatile(
+            "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(dst_smem),
+            "l"(map), "r"(bar), "r"(c0), "r"(c1)
+            : "memory");
+}
+// 4-D activation box at channel c, pixel (x, y) of image n: the map's last two dimensions are (image, y) when `perm`
+// (tiles spanning several images, see encode_act_map)
+template <int PAIR = 0>
+__device__ __forceinline__ void tma_load_act(const CUtensorMap* map, uint32_t bar, uint32_t dst_smem, int c, int x, int y, int n, bool perm) {
+    tma_load_4d<PAIR>(map, bar, dst_smem, c, x, perm ? n : y, perm ? y : n);
 }
 __device__ __forceinline__ void tma_store_4d(const CUtensorMap* map, uint32_t src_smem, int c0, int c1, int c2, int c3) {
     asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(map), "r"(src_smem),
@@ -113,29 +143,53 @@ __device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap* map) {
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
+template <int PAIR = 0>
 __device__ __forceinline__ void tmem_alloc(uint32_t* dst_smem, uint32_t cols) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    if constexpr (PAIR) {
+        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(cols) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+    } else {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(cols) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
 }
+template <int PAIR = 0>
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
+    if constexpr (PAIR) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
+    else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
 }
+// PAIR: arrives on the barrier at this offset in both CTAs
+template <int PAIR = 0>
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
+    if constexpr (PAIR)
+        asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar), "h"((uint16_t)3) : "memory");
+    else
+        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
-// D[tmem] (+)= A[smem] * B[smem]^T, bf16 x bf16 -> fp32
+// D[tmem] (+)= A[smem] * B[smem]^T, bf16 x bf16 -> fp32 (PAIR: M = 256 over the two CTAs)
+template <int PAIR = 0>
 __device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
-        "}" ::"r"(d_tmem),
-        "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-        : "memory");
+    if constexpr (PAIR)
+        asm volatile(
+            "{\n\t"
+            ".reg .pred p;\n\t"
+            "setp.ne.b32 p, %4, 0;\n\t"
+            "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t"
+            "}" ::"r"(d_tmem),
+            "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+            : "memory");
+    else
+        asm volatile(
+            "{\n\t"
+            ".reg .pred p;\n\t"
+            "setp.ne.b32 p, %4, 0;\n\t"
+            "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
+            "}" ::"r"(d_tmem),
+            "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+            : "memory");
 }
-// ---- CTA-pair (cta_group::2) forms: one MMA spans the two SMs of a 2-CTA cluster (M = 256), each CTA holding its
-// own 128 A rows and half of the B rows; the leader (cluster rank 0) issues, barriers that gate it live in its smem.
+// ---- CTA pairs (cta_group::2): one MMA spans the two SMs of a 2-CTA cluster (M = 256), each CTA holding its own 128 A
+// rows and half of the B rows; the leader (cluster rank 0) issues, barriers that gate it live in its smem.
 __device__ __forceinline__ uint32_t cluster_ctarank() {
     uint32_t r;
     asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
@@ -152,41 +206,6 @@ __device__ __forceinline__ void cluster_sync_all() {
 }
 __device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
     asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx_cluster(uint32_t cluster_addr, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cluster.b64 _, [%0], %1;" ::"r"(cluster_addr), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void tma_load_4d_2sm(const CUtensorMap* map, uint32_t cluster_bar, uint32_t dst_smem, int c0, int c1, int c2, int c3) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];" ::"r"(dst_smem),
-        "l"(map), "r"(cluster_bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-        : "memory");
-}
-__device__ __forceinline__ void tma_load_2d_2sm(const CUtensorMap* map, uint32_t cluster_bar, uint32_t dst_smem, int c0, int c1) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(dst_smem),
-        "l"(map), "r"(cluster_bar), "r"(c0), "r"(c1)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_alloc_2sm(uint32_t* dst_smem, uint32_t cols) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_2sm(uint32_t taddr, uint32_t cols) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
-__device__ __forceinline__ void umma_commit_2sm(uint32_t bar) {     // arrives on the barrier at this offset in both CTAs
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar), "h"((uint16_t)3) : "memory");
-}
-__device__ __forceinline__ void umma_bf16_2sm(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t"
-        "}" ::"r"(d_tmem),
-        "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-        : "memory");
 }
 __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
     asm volatile(
@@ -233,6 +252,15 @@ __device__ __forceinline__ uint32_t desc_lo_ns(uint32_t saddr, uint32_t lbo_byte
 
 struct TileCoord { int nt, x0, y0, n0; };
 template <int V> struct KConst { static constexpr int value = V; };
+// fn(KConst<km>{}) for a runtime count km of K = 16 steps (1-4): the MMA issue loops keep the count a compile-time constant,
+// since a per-MMA `k < km` test costs ~13 cycles per MMA on the single issuing thread (tools/ubench/mma_issue.cu, variants 32 / 33)
+template <typename Fn>
+__device__ __forceinline__ void with_ksteps(int km, Fn&& fn) {
+    if (km == 4) fn(KConst<4>{});
+    else if (km == 3) fn(KConst<3>{});
+    else if (km == 2) fn(KConst<2>{});
+    else fn(KConst<1>{});
+}
 
 // t -> (nt, x tile, y tile, image group) without hardware division: q = umulhi(t, ceil(2^32 / d)) is exact
 // for t * d < 2^32 (tile counts are far below that); the reciprocals are computed on the host.
@@ -257,18 +285,42 @@ __device__ __forceinline__ TileCoord decode_tile(const ConvTcParams& p, int t) {
     return c;
 }
 
-// CTA pairs: round `rd` of a pair = two M tiles of one output-channel tile nt, one per CTA (rank 0 / 1); an odd last M tile
-// is computed (and stored, identically) by both.  Tile index t = m * n_tiles_n + nt as everywhere else.
-__device__ __forceinline__ int pair_rounds(const ConvTcParams& p, int total_tiles) {
-    const int nn = p.n_tiles_n, mt = total_tiles / nn;
-    return ((mt + 1) >> 1) * nn;
-}
-__device__ __forceinline__ int pair_tile(const ConvTcParams& p, int rd, int rank, int total_tiles) {
-    const int nn = p.n_tiles_n;
-    if (nn == 1) return min(2 * rd + rank, total_tiles - 1);
-    const int mp = (int)__umulhi((uint32_t)rd, p.rcp_nn), nt = rd - mp * nn;
-    return min(2 * mp + rank, total_tiles / nn - 1) * nn + nt;
-}
+// The round schedule of a CTA, shared by every role of every kernel.  A single CTA takes rounds blockIdx.x, + gridDim.x, ...;
+// round rd is the mt tiles from rd * mt on (the last round may be short).  A CTA pair (PAIR, mt == 1) takes rounds
+// blockIdx.x / 2, + gridDim.x / 2, ...; its round rd is two M tiles of one output-channel tile nt, one per CTA (rank 0 / 1),
+// and an odd last M tile is computed (and stored, identically) by both.  Tile index t = m * n_tiles_n + nt as everywhere else.
+template <int PAIR>
+struct RoundSched {
+    const ConvTcParams& p;
+    int total, mt, rounds;
+    uint32_t rank;                                   // cluster rank of this CTA (PAIR), else 0
+    __device__ __forceinline__ RoundSched(const ConvTcParams& p_, int total_tiles) : p(p_), total(total_tiles) {
+        if constexpr (PAIR) {
+            rank = cluster_ctarank();
+            mt = 1;
+            rounds = ((total / p.n_tiles_n + 1) >> 1) * p.n_tiles_n;
+        } else {
+            rank = 0;
+            mt = p.mt;
+            rounds = (total + mt - 1) / mt;
+        }
+    }
+    // this CTA's first round and the step to its next one
+    __device__ __forceinline__ int rd0() const { return PAIR ? (int)(blockIdx.x >> 1) : (int)blockIdx.x; }
+    __device__ __forceinline__ int step() const { return PAIR ? (int)(gridDim.x >> 1) : (int)gridDim.x; }
+    // the first tile of round rd (a pair: this CTA's tile)
+    __device__ __forceinline__ int tile0(int rd) const {
+        if constexpr (PAIR) {
+            const int nn = p.n_tiles_n;
+            const int mp = nn == 1 ? rd : (int)__umulhi((uint32_t)rd, p.rcp_nn), nt = rd - mp * nn;
+            return min(2 * mp + (int)rank, total / nn - 1) * nn + nt;
+        } else {
+            return rd * mt;
+        }
+    }
+    // the tiles of round rd this CTA computes
+    __device__ __forceinline__ int tiles(int rd) const { return PAIR ? 1 : min(mt, total - rd * mt); }
+};
 
 // Debug trace (build with -DB2D_ENABLE_TRACE, run with B2D_TRACE=1): CTA 0 records clock64() at role
 // events of its first kTraceTiles rounds.  Compiled out of product builds.
@@ -483,21 +535,18 @@ struct EpiGeom {
 // (Until round 2 four lanes served one TMEM lane quarter each with quarter-sized boxes: 4 x the TMA instructions, and UTMASTG
 // takes uniform registers, so the compiler serialised the four lanes in a loop around every one of them -- ncu showed the
 // warp 100 % busy with 62 % of its samples in those loops and the epilogue warps waiting for free slabs on the stem.)
-template <int RES, int F32>
+template <int RES, int F32, int PAIR = 0>
 __device__ __forceinline__ void store_loop(const ConvTcParams& p, int total_tiles, uint64_t* sfull_bar, uint64_t* sempty_bar,
-                                           uint64_t* res_bar, uint8_t* stg_base, int lane, bool pair = false) {
+                                           uint64_t* res_bar, uint8_t* stg_base, int lane) {
     if (!elect_one()) return;
     (void)lane;
     const EpiGeom<F32> g(p, stg_base);
     const int mt = p.mt, n_tile = p.n_tile;
     const int S = g.nb * mt, s_shift = 31 - __clz(S);                          // S is 1, 2, 4 or 8
     const uint32_t sfull_u32 = smem_u32(sfull_bar), sempty_u32 = smem_u32(sempty_bar), rbar_u32 = smem_u32(res_bar);
-    const uint32_t rank = pair ? cluster_ctarank() : 0u;
-    const int rounds = pair ? pair_rounds(p, total_tiles) : (total_tiles + mt - 1) / mt;
-    const int rd0 = pair ? (int)(blockIdx.x >> 1) : (int)blockIdx.x, rd_step = pair ? (int)(gridDim.x >> 1) : (int)gridDim.x;
+    const RoundSched<PAIR> rs(p, total_tiles);
+    const int rd0 = rs.rd0(), rd_step = rs.step();
     const bool perm = p.perm != 0;
-    auto first_tile = [&](int rd) { return pair ? pair_tile(p, rd, (int)rank, total_tiles) : rd * mt; };
-    auto valid_tiles = [&](int rd) { return pair ? 1 : min(mt, total_tiles - rd * mt); };
     // TMA boxes of tile t: residual loads into / stores out of slab `slab`
     auto tile_io = [&](int t, int slab, bool load) {
         const TileCoord tc = decode_tile(p, t);
@@ -515,7 +564,7 @@ __device__ __forceinline__ void store_loop(const ConvTcParams& p, int total_tile
     if (RES) {                                                                 // the first S tiles' residuals: every slab is free
         for (int c = 0; c < S; ++c) {
             const int rd = rd0 + (c / mt) * rd_step, m = c % mt;
-            if (rd < rounds && m < valid_tiles(rd)) tile_io(first_tile(rd) + m, c, true);
+            if (rd < rs.rounds && m < rs.tiles(rd)) tile_io(rs.tile0(rd) + m, c, true);
         }
     }
     // Layers without a residual keep one store group in flight: tile c's stores are issued before the lane waits for tile c - 1's
@@ -529,10 +578,10 @@ __device__ __forceinline__ void store_loop(const ConvTcParams& p, int total_tile
         if (RES && pend_next >= 0) tile_io(pend_next, pend_slab, true);
         pend_slab = -1;
     };
-    for (int rd = rd0; rd < rounds; rd += rd_step, ++it) {
-        const int t0 = first_tile(rd), nv = valid_tiles(rd);
-        const int rdn = rd + g.nb * rd_step;                                   // the round whose tile m reuses tile m's slab
-        const int nvn = rdn < rounds ? valid_tiles(rdn) : 0;
+    for (int rd = rd0; rd < rs.rounds; rd += rd_step, ++it) {
+        const int t0 = rs.tile0(rd), nv = rs.tiles(rd);
+        const int rdn = rd + g.nb * rd_step;                                  // the round whose tile m reuses tile m's slab
+        const int nvn = rdn < rs.rounds ? rs.tiles(rdn) : 0;
         for (int m = 0; m < nv; ++m) {
             const int c = it * mt + m, slab = c & (S - 1);
             const uint32_t use = (uint32_t)(c >> s_shift);
@@ -541,7 +590,7 @@ __device__ __forceinline__ void store_loop(const ConvTcParams& p, int total_tile
             tma_store_commit();
             if (RES || S < 4) {                          // residual layers: the slab's next residual must start loading as early as possible
                 pend_slab = slab;                        // (measured: +11 us on the 96-channel residual layers when it waits a tile longer);
-                pend_next = (RES && m < nvn) ? first_tile(rdn) + m : -1;       // with fewer than four slabs a pending one starves the epilogue (+2-4 us)
+                pend_next = (RES && m < nvn) ? rs.tile0(rdn) + m : -1;         // with fewer than four slabs a pending one starves the epilogue (+2-4 us)
                 release(true);
             } else {
                 release(false);
@@ -559,10 +608,10 @@ __device__ __forceinline__ void store_loop(const ConvTcParams& p, int total_tile
 // one-tile staging slabs; a slab is handed to the store warp and back through the sfull / sempty mbarriers (no named
 // barriers, no TMA instruction on this path).  A round's mt tiles are drained back to back as one flat list of work
 // items, the TMEM load of the next item always in flight behind the math of the current one.
-template <int ACT, int RES, int F32>
+template <int ACT, int RES, int F32, int PAIR = 0>
 __device__ __forceinline__ void epilogue_loop(const ConvTcParams& p, int total_tiles, uint32_t tmem_base, const float* bias_s,
                                               uint64_t* tfull_bar, uint64_t* tempty_bar, uint64_t* sfull_bar, uint64_t* sempty_bar,
-                                              uint64_t* res_bar, uint8_t* stg_base, int warp, int lane, bool pair = false) {
+                                              uint64_t* res_bar, uint8_t* stg_base, int warp, int lane) {
     const int q = warp & 3;
     const int half = (warp - 4) >> 2;                  // this warp's part of the quarter's column units: 0 .. epi_parts - 1
     const int nparts = p.epi_parts;
@@ -595,6 +644,8 @@ __device__ __forceinline__ void epilogue_loop(const ConvTcParams& p, int total_t
         return row32 + ((((rem >> 4) & 1u) ^ sw32) << 4);
     };
     const uint32_t ubytes = 16u * esize;               // bytes of one unit in a row
+    // Each path below sets up its own round schedule: kept next to the path's other loop invariants, the single-CTA
+    // instantiations compile to the same instructions as when each path spelled the schedule out.
     int it = 0;
     if (my_units <= 2 && !split_last && p.n_tiles_n == 1) {
         // Narrow tiles (n_tile = 32, 48, 64, 96: the stem, the 160^2 stage, the 96-channel 3x3 layers, the head's box branch): a warp
@@ -604,17 +655,16 @@ __device__ __forceinline__ void epilogue_loop(const ConvTcParams& p, int total_t
         const bool two = my_units == 2;
         const uint32_t ub0 = unit_base((uint32_t)half * ubytes), ub1 = two ? unit_base((uint32_t)(half + nparts) * ubytes) : ub0;
         const uint32_t baddr0 = bias_base + (uint32_t)(half * 16) * 4u, baddr1 = baddr0 + (uint32_t)nparts * 64u;
-        const uint32_t rank = pair ? cluster_ctarank() : 0u;
-        const int rounds = pair ? pair_rounds(p, total_tiles) : (total_tiles + mt - 1) / mt;
-        const int rd0 = pair ? (int)(blockIdx.x >> 1) : (int)blockIdx.x, rd_step = pair ? (int)(gridDim.x >> 1) : (int)gridDim.x;
-        const uint32_t tempty_arrive = pair ? mapa_u32(tempty_u32, 0) : tempty_u32;
+        const RoundSched<PAIR> rs(p, total_tiles);
+        const int rd0 = rs.rd0(), rd_step = rs.step();
+        const uint32_t tempty_arrive = PAIR ? mapa_u32(tempty_u32, 0) : tempty_u32;
         const int f16 = p.f16;
         const float sc = (ACT ? 0.5f : 1.0f) * p.acc_scale;
         const uint64_t scale2 = pk2(sc, sc);
         const uint32_t col0 = (uint32_t)(half * 16), col1 = col0 + (uint32_t)nparts * 16u;
-        for (int rd = rd0; rd < rounds; rd += rd_step, ++it) {
+        for (int rd = rd0; rd < rs.rounds; rd += rd_step, ++it) {
             const int as = it & 1;
-            const int nv = pair ? 1 : min(mt, total_tiles - rd * mt);
+            const int nv = rs.tiles(rd);
             if (warp == 4 && lane == 0) trace(p, 2, it, 0);
             mbar_wait_u32(tfull_u32 + as * 8, (uint32_t)((it >> 1) & 1));
             tc_fence_after();
@@ -657,12 +707,11 @@ __device__ __forceinline__ void epilogue_loop(const ConvTcParams& p, int total_t
             tc_fence_before();
             __syncwarp();
             if (lane == 0) {
-                if (pair) mbar_arrive_cluster(tempty_arrive + as * 8);
+                if constexpr (PAIR) mbar_arrive_cluster(tempty_arrive + as * 8);     // the leader's barrier gates the pair's MMAs
                 else mbar_arrive_u32(tempty_u32 + as * 8);
             }
             if (warp == 4 && lane == 0) trace(p, 2, it, 2);
         }
-        (void)rank;
         return;
     }
     if (!split_last) {
@@ -671,18 +720,16 @@ __device__ __forceinline__ void epilogue_loop(const ConvTcParams& p, int total_t
         // of the next pair (of this tile or the next) issued behind it, SiLU + pack + staging stores -- with one slab wait in
         // front and one hand-off behind.  The item-list form below spends ~180 instructions per 16 columns, most of them
         // bookkeeping, and a warp issues about one instruction per six cycles.
-        const uint32_t rank = pair ? cluster_ctarank() : 0u;
-        const int rounds = pair ? pair_rounds(p, total_tiles) : (total_tiles + mt - 1) / mt;
-        const int rd0 = pair ? (int)(blockIdx.x >> 1) : (int)blockIdx.x, rd_step = pair ? (int)(gridDim.x >> 1) : (int)gridDim.x;
-        const uint32_t tempty_arrive = pair ? mapa_u32(tempty_u32, 0) : tempty_u32;
+        const RoundSched<PAIR> rs(p, total_tiles);
+        const int rd0 = rs.rd0(), rd_step = rs.step();
+        const uint32_t tempty_arrive = PAIR ? mapa_u32(tempty_u32, 0) : tempty_u32;
         const int f16 = p.f16;
         const float sc = (ACT ? 0.5f : 1.0f) * p.acc_scale;
         const uint64_t scale2 = pk2(sc, sc);
         const uint32_t col0 = (uint32_t)(half * 16), ustep = (uint32_t)nparts * 16u;
-        for (int rd = rd0; rd < rounds; rd += rd_step, ++it) {
+        for (int rd = rd0; rd < rs.rounds; rd += rd_step, ++it) {
             const int as = it & 1;
-            const int t0 = pair ? pair_tile(p, rd, (int)rank, total_tiles) : rd * mt;
-            const int nv = pair ? 1 : min(mt, total_tiles - t0);
+            const int t0 = rs.tile0(rd), nv = rs.tiles(rd);
             if (warp == 4 && lane == 0) trace(p, 2, it, 0);
             mbar_wait_u32(tfull_u32 + as * 8, (uint32_t)((it >> 1) & 1));
             tc_fence_after();
@@ -737,7 +784,7 @@ __device__ __forceinline__ void epilogue_loop(const ConvTcParams& p, int total_t
             tc_fence_before();
             __syncwarp();
             if (lane == 0) {
-                if (pair) mbar_arrive_cluster(tempty_arrive + as * 8);
+                if constexpr (PAIR) mbar_arrive_cluster(tempty_arrive + as * 8);     // the leader's barrier gates the pair's MMAs
                 else mbar_arrive_u32(tempty_u32 + as * 8);
             }
             if (warp == 4 && lane == 0) trace(p, 2, it, 2);
@@ -745,21 +792,17 @@ __device__ __forceinline__ void epilogue_loop(const ConvTcParams& p, int total_t
         return;
     }
     // Item-list path: the 8 + 8 split of an odd last unit (n_tile 16, 80, 112 ...).
-    // tile walk: a CTA takes rounds blockIdx.x, + gridDim.x, ... of mt tiles; in a CTA pair (mt == 1) the pair takes two
-    // consecutive tiles per round, one per CTA, and an odd last tile is computed (and stored, identically) by both
-    const uint32_t rank = pair ? cluster_ctarank() : 0u;
-    const int rounds = pair ? pair_rounds(p, total_tiles) : (total_tiles + mt - 1) / mt;
-    const int rd0 = pair ? (int)(blockIdx.x >> 1) : (int)blockIdx.x, rd_step = pair ? (int)(gridDim.x >> 1) : (int)gridDim.x;
-    const uint32_t tempty_arrive = pair ? mapa_u32(tempty_u32, 0) : tempty_u32;   // the leader's barrier gates the pair's MMAs
+    const RoundSched<PAIR> rs(p, total_tiles);
+    const int rd0 = rs.rd0(), rd_step = rs.step();
+    const uint32_t tempty_arrive = PAIR ? mapa_u32(tempty_u32, 0) : tempty_u32;
     const int f16 = p.f16;
     const float sc = (ACT ? 0.5f : 1.0f) * p.acc_scale;
     const uint64_t scale2 = pk2(sc, sc);
     const int split_col = (nunits - 1) * 16 + half * 8;
-    for (int rd = rd0; rd < rounds; rd += rd_step, ++it) {
+    for (int rd = rd0; rd < rs.rounds; rd += rd_step, ++it) {
         const int as = it & 1;
         const uint32_t aphase = (it >> 1) & 1;
-        const int t0 = pair ? pair_tile(p, rd, (int)rank, total_tiles) : rd * mt;
-        const int nv = pair ? 1 : min(mt, total_tiles - t0);        // valid tiles of this round
+        const int t0 = rs.tile0(rd), nv = rs.tiles(rd);
         if (warp == 4 && lane == 0) trace(p, 2, it, 0);
         mbar_wait_u32(tfull_u32 + as * 8, aphase);
         tc_fence_after();
@@ -834,7 +877,7 @@ __device__ __forceinline__ void epilogue_loop(const ConvTcParams& p, int total_t
         tc_fence_before();
         __syncwarp();
         if (lane == 0) {
-            if (pair) mbar_arrive_cluster(tempty_arrive + as * 8);
+            if constexpr (PAIR) mbar_arrive_cluster(tempty_arrive + as * 8);     // the leader's barrier gates the pair's MMAs
             else mbar_arrive_u32(tempty_u32 + as * 8);
         }
         if (warp == 4 && lane == 0) trace(p, 2, it, 2);
@@ -874,18 +917,20 @@ __device__ __forceinline__ Bars carve_bars(uint8_t* smem, const ConvTcParams& p)
     b.bias_s = (float*)(b.tmem_slot + 4);
     return b;
 }
-// common prologue: barrier init (warp 1), TMEM allocation (warp 2), bias to smem (everyone)
-__device__ __forceinline__ uint32_t prologue(const ConvTcParams& p, const Bars& b, int warp, int lane, uint32_t full_count,
-                                             uint32_t issuers = 1, uint32_t hempty_count = 0, uint32_t afull_count = 0) {
+// common prologue: barrier init (warp 1), TMEM allocation (warp 2), bias to smem (everyone).  In a CTA pair the barriers
+// that gate the leader's MMAs (full, hfull, tempty) count the arrivals of both CTAs; the leader's copies are the ones waited on.
+template <int PAIR = 0>
+__device__ __forceinline__ uint32_t prologue(const ConvTcParams& p, const Bars& b, int warp, int lane, uint32_t issuers = 1,
+                                             uint32_t hempty_count = 0, uint32_t afull_count = 0) {
     if (warp == 1 && lane == 0) {
         for (int i = 0; i < p.stages; ++i) {
-            mbar_init(&b.full[i], full_count);
+            mbar_init(&b.full[i], PAIR ? 2 : 1);             // one arrive.expect_tx per CTA
             mbar_init(&b.empty[i], issuers);
         }
         for (int i = 0; i < 2; ++i) {
             mbar_init(&b.tfull[i], issuers);
-            mbar_init(&b.tempty[i], 4 * p.epi_parts);         // one elected lane of every active epilogue warp
-            mbar_init(&b.hfull[i], 1);
+            mbar_init(&b.tempty[i], (PAIR ? 8 : 4) * p.epi_parts);     // one elected lane of every active epilogue warp
+            mbar_init(&b.hfull[i], PAIR ? 2 : 1);
             mbar_init(&b.hempty[i], hempty_count ? hempty_count : issuers);
             if (afull_count) {
                 mbar_init(&b.afull[i], afull_count);
@@ -899,35 +944,44 @@ __device__ __forceinline__ uint32_t prologue(const ConvTcParams& p, const Bars& 
         }
         fence_barrier_init();
     }
-    if (warp == 2) tmem_alloc(b.tmem_slot, p.tmem_cols);
+    if (warp == 2) tmem_alloc<PAIR>(b.tmem_slot, p.tmem_cols);
     for (int i = threadIdx.x; i < p.n_tile * p.n_tiles_n; i += blockDim.x) b.bias_s[i] = p.act ? 0.5f * p.bias[i] : p.bias[i];   // see epi_bias
     tc_fence_before();
-    __syncthreads();
+    if constexpr (PAIR) cluster_sync_all();             // barriers of both CTAs initialised before anyone signals them
+    else __syncthreads();
     tc_fence_after();
     return *b.tmem_slot;
 }
+template <int PAIR = 0>
 __device__ __forceinline__ void epilogue_exit(const ConvTcParams& p, uint32_t tmem_base, int warp) {
     tc_fence_before();
-    __syncthreads();
+    if constexpr (PAIR) cluster_sync_all();             // the peer may still signal this CTA's barriers / read its smem until here
+    else __syncthreads();
     if (warp == 2) {
         tc_fence_after();
-        tmem_dealloc(tmem_base, p.tmem_cols);
+        tmem_dealloc<PAIR>(tmem_base, p.tmem_cols);
     }
 }
 
 // ---------------------------------------------------------------------------------------------
-// generic kernel: one A box per (tap, chunk) and tile, one B box per (tap, chunk) and round
+// generic kernel: one A box per (tap, chunk) and tile, one B box per (tap, chunk) and round.
+// PAIR (1x1 and stride-2 layers with n_tile >= 128 and a short reduction, see conv_tc_plan): the two CTAs of a cluster run ONE
+// stream of cta_group::2 MMAs (M = 256), issued by the leader.  Each CTA loads the A box of its own M tile and HALF of every
+// weight box into the same stage slot, so per SM the weight traffic from L2 and the B-operand reads are halved: these layers
+// run N = 192 tiles, where a single SM needs ~105 bytes of operands per clock to keep its tensor pipe busy and L2 delivers
+// about half of that.  Barriers: full / tempty live in the leader (both CTAs arrive), empty / tfull are signalled in both CTAs
+// by the leader's multicast commits.
 // ---------------------------------------------------------------------------------------------
-template <int ACT, int RES, int F32>
+template <int ACT, int RES, int F32, int PAIR>
 __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_constant__ ConvTcParams p, int nimg) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
     const Bars b = carve_bars(smem, p);
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
-    const int mt = p.mt;
     const int total_tiles = p.tiles_x * p.tiles_y * ((nimg + p.bn - 1) / p.bn) * p.n_tiles_n;
-    const int rounds = (total_tiles + mt - 1) / mt;
+    const RoundSched<PAIR> rs(p, total_tiles);
+    const int mt = rs.mt;
     const int ksteps = p.taps * p.chunks;
     const uint32_t stage_bytes = (uint32_t)mt * p.a_bytes + p.b_bytes;
 
@@ -940,12 +994,12 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
         }
         tma_prefetch_desc(&p.tmB);
     }
-    const uint32_t tmem_base = prologue(p, b, warp, lane, 1);
+    const uint32_t tmem_base = prologue<PAIR>(p, b, warp, lane);
     const uint32_t smem_base = smem_u32(smem);
     const uint32_t full_u32 = smem_u32(b.full), empty_u32 = smem_u32(b.empty);
 
     if (warp == 0) {
-        // ===================== TMA producer =====================
+        // ===================== TMA producer (a pair: in both CTAs) =====================
         int stage = 0;
         uint32_t phase = 0;
         const int pad = p.ksz >> 1;
@@ -953,13 +1007,14 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
         const int cin_pad = chunks * 64;
         const uint32_t a_bytes = p.a_bytes;
         const bool s2 = (p.stride == 2), perm = p.perm != 0;
+        const uint32_t full_bar = PAIR ? mapa_u32(full_u32, 0) : full_u32;     // a pair's loads complete on the leader's barrier
         int pit = 0;
-        for (int rd = blockIdx.x; rd < rounds; rd += gridDim.x, ++pit) {
-            const int t0 = rd * mt;
-            const int nv = min(mt, total_tiles - t0);
+        for (int rd = rs.rd0(); rd < rs.rounds; rd += rs.step(), ++pit) {
+            const int t0 = rs.tile0(rd);
+            const int nv = rs.tiles(rd);
             const TileCoord tc0 = decode_tile(p, t0);
             const TileCoord tc1 = decode_tile(p, nv > 1 ? t0 + 1 : t0);
-            const int bn0 = tc0.nt * n_tile;
+            const int bn0 = tc0.nt * n_tile + (PAIR ? (int)rs.rank * (n_tile >> 1) : 0);   // a pair: this CTA's half of the weight rows
             const uint32_t tx_bytes = (uint32_t)nv * p.a_tx_bytes + p.b_tx_bytes;
             int kh = 0, kw = 0;
             trace(p, 0, pit, 0);
@@ -978,17 +1033,17 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
                 for (int ch = 0; ch < chunks; ++ch) {
                     mbar_wait_u32(empty_u32 + stage * 8, phase ^ 1);
                     if (elect_one()) {
-                        const uint32_t sa = smem_base + (uint32_t)stage * stage_bytes, fb = full_u32 + stage * 8;
-                        mbar_expect_tx_u32(fb, tx_bytes);
+                        const uint32_t sa = smem_base + (uint32_t)stage * stage_bytes, fb = full_bar + stage * 8;
+                        mbar_expect_tx_u32<PAIR>(fb, tx_bytes);
                         {
                             const int cy = tc0.y0 + oy;
-                            tma_load_4d(mapA, fb, sa, ch * 64, tc0.x0 + ox, perm ? tc0.n0 : cy, perm ? cy : tc0.n0);
+                            tma_load_act<PAIR>(mapA, fb, sa, ch * 64, tc0.x0 + ox, cy, tc0.n0, perm);
                         }
                         if (nv > 1) {
                             const int cy = tc1.y0 + oy;
-                            tma_load_4d(mapA, fb, sa + a_bytes, ch * 64, tc1.x0 + ox, perm ? tc1.n0 : cy, perm ? cy : tc1.n0);
+                            tma_load_act(mapA, fb, sa + a_bytes, ch * 64, tc1.x0 + ox, cy, tc1.n0, perm);
                         }
-                        tma_load_2d(&p.tmB, fb, sa + (uint32_t)mt * a_bytes, kb + ch * 64, bn0);
+                        tma_load_2d<PAIR>(&p.tmB, fb, sa + (uint32_t)mt * a_bytes, kb + ch * 64, bn0);
                     }
                     if (++stage == nstages) { stage = 0; phase ^= 1; }
                 }
@@ -996,8 +1051,8 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
             }
             trace(p, 0, pit, 1);
         }
-    } else if (warp == 1) {
-        // ===================== MMA issuer =====================
+    } else if (warp == 1 && (!PAIR || rs.rank == 0)) {
+        // ===================== MMA issuer (a pair: the leader CTA only) =====================
         // One lane issues; it is elected once, and the loop body is kept to a handful of instructions per MMA: the issue
         // interval of a lone thread (~8 cycles per dependent instruction), not the tensor pipe, bounds narrow layers.
         int stage = 0;
@@ -1012,10 +1067,10 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
         const int last_kmmas = (p.cin - (chunks - 1) * 64 + 15) >> 4;      // K=16 MMAs that carry data in the last chunk
         const int taps = p.taps;
         const uint32_t tfull_u32 = smem_u32(b.tfull), tempty_u32 = smem_u32(b.tempty);
-        for (int rd = blockIdx.x; rd < rounds; rd += gridDim.x, ++it) {
+        for (int rd = rs.rd0(); rd < rs.rounds; rd += rs.step(), ++it) {
             const int as = it & 1;
             const uint32_t aphase = (it >> 1) & 1;
-            const bool two = min(mt, total_tiles - rd * mt) > 1;
+            const bool two = rs.tiles(rd) > 1;
             trace(p, 1, it, 0);
             mbar_wait_u32(tempty_u32 + as * 8, aphase ^ 1);
             tc_fence_after();
@@ -1034,52 +1089,55 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_kernel(const __grid_const
                     const uint32_t acc0 = (uint32_t)(ks != 0);
 #pragma unroll
                     for (int k = 0; k < decltype(KM)::value; ++k)
-                        umma_bf16(d_tmem, desc64(hi, a_lo + 2 * k), desc64(hi, b_lo + 2 * k), idesc, k == 0 ? acc0 : 1u);
+                        umma_bf16<PAIR>(d_tmem, desc64(hi, a_lo + 2 * k), desc64(hi, b_lo + 2 * k), idesc, k == 0 ? acc0 : 1u);
                     if (two) {
 #pragma unroll
                         for (int k = 0; k < decltype(KM)::value; ++k)
                             umma_bf16(d_tmem + (uint32_t)n_tile, desc64(hi, a_lo + a_units + 2 * k), desc64(hi, b_lo + 2 * k), idesc, k == 0 ? acc0 : 1u);
                     }
-                    umma_commit(empty_u32 + stage * 8);                       // frees the smem slot when these MMAs retire
-                    if (ks == ksteps - 1) umma_commit(tfull_u32 + as * 8);     // accumulators complete
+                    umma_commit<PAIR>(empty_u32 + stage * 8);                 // frees the smem slot (a pair: in both CTAs) when these MMAs retire
+                    if (ks == ksteps - 1) umma_commit<PAIR>(tfull_u32 + as * 8);     // accumulators complete
                 }
                 ++ks;
                 if (++stage == nstages) { stage = 0; phase ^= 1; }
             };
             for (int tap = 0; tap < taps; ++tap) {
                 for (int ch = 0; ch < chunks - 1; ++ch) step(KConst<4>{});
-                if (last_kmmas == 4) step(KConst<4>{});
-                else if (last_kmmas == 3) step(KConst<3>{});
-                else if (last_kmmas == 2) step(KConst<2>{});
-                else step(KConst<1>{});
+                with_ksteps(last_kmmas, step);
             }
             trace(p, 1, it, 3);
         }
     } else if (warp == 3) {
-        store_loop<RES, F32>(p, total_tiles, b.sfull, b.sempty, b.res, smem + p.stg_off, lane);
+        store_loop<RES, F32, PAIR>(p, total_tiles, b.sfull, b.sempty, b.res, smem + p.stg_off, lane);
     } else if (warp >= 4) {
-        epilogue_loop<ACT, RES, F32>(p, total_tiles, tmem_base, b.bias_s, b.tfull, b.tempty, b.sfull, b.sempty, b.res, smem + p.stg_off, warp, lane);
+        epilogue_loop<ACT, RES, F32, PAIR>(p, total_tiles, tmem_base, b.bias_s, b.tfull, b.tempty, b.sfull, b.sempty, b.res, smem + p.stg_off, warp, lane);
     }
-    epilogue_exit(p, tmem_base, warp);
+    epilogue_exit<PAIR>(p, tmem_base, warp);
 }
 
 // ---------------------------------------------------------------------------------------------
 // halo kernel: 3x3 stride-1 convs on 8-pixel-wide tiles.  Per round and chunk, one halo box per tile
 // (double buffered) and nine weight boxes through the stage ring.
+// PAIR (wide layers, n_tile >= 128): the two CTAs of a cluster work on two neighbouring M tiles with ONE stream of MMAs
+// (cta_group::2, M = 256) issued by the leader.  Each CTA loads its own halo and only half of every weight tile, so per SM the
+// weight fill and the B-operand reads are halved and each MMA instruction carries twice the work -- what keeps the tensor pipe
+// fed where a single SM's issue rate and smem bandwidth could not.  One tile per CTA and round, weights never resident.
+// Barriers: full / hfull / tempty live in the leader (both CTAs arrive), empty / hempty / tfull are signalled in both CTAs by
+// the leader's multicast commits.
 // ---------------------------------------------------------------------------------------------
-template <int ACT, int RES, int F32>
+template <int ACT, int RES, int F32, int PAIR>
 __global__ void __launch_bounds__(kThreads, 1) conv_tc_halo_kernel(const __grid_constant__ ConvTcParams p, int nimg) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
     const Bars b = carve_bars(smem, p);
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
-    const int mt = p.mt;
     const int total_tiles = p.tiles_x * p.tiles_y * ((nimg + p.bn - 1) / p.bn) * p.n_tiles_n;
-    const int rounds = (total_tiles + mt - 1) / mt;
+    const RoundSched<PAIR> rs(p, total_tiles);
+    const int mt = rs.mt;
 
     if (warp == 0 && lane == 0) { tma_prefetch_desc(&p.tmA[0]); tma_prefetch_desc(&p.tmB); }
-    const uint32_t tmem_base = prologue(p, b, warp, lane, 1);
+    const uint32_t tmem_base = prologue<PAIR>(p, b, warp, lane);
     const uint32_t halo_bytes = p.halo_bytes;
     const uint32_t smem_a = smem_u32(smem), smem_b = smem_a + 2u * (uint32_t)mt * halo_bytes;   // [2][mt] halos, then the B ring
     const uint32_t full_u32 = smem_u32(b.full), empty_u32 = smem_u32(b.empty);
@@ -1092,16 +1150,18 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_halo_kernel(const __grid_
         const int nstages = p.stages, chunks = p.chunks, n_tile = p.n_tile;
         const int cin_pad = chunks * 64;
         const uint32_t b_tx = p.b_tx_bytes, b_bytes = p.b_bytes;
+        const uint32_t full_bar = PAIR ? mapa_u32(full_u32, 0) : full_u32;     // a pair's loads complete on the leader's barrier
         int pit = 0;
-        for (int rd = blockIdx.x; rd < rounds; rd += gridDim.x, ++pit) {
-            if (p.b_res && pit > 0) break;               // resident weights: the ring holds every (chunk, tap) and is filled once
-            const int bn0 = decode_tile(p, rd * mt).nt * n_tile;
+        for (int rd = rs.rd0(); rd < rs.rounds; rd += rs.step(), ++pit) {
+            if (!PAIR && p.b_res && pit > 0) break;      // resident weights: the ring holds every (chunk, tap) and is filled once
+            // a pair (one output-channel tile): this CTA's half of the weight rows
+            const int bn0 = PAIR ? (int)rs.rank * (n_tile >> 1) : decode_tile(p, rs.tile0(rd)).nt * n_tile;
             for (int ch = 0; ch < chunks; ++ch) {
                 for (int tap = 0; tap < 9; ++tap) {
                     mbar_wait_u32(empty_u32 + stage * 8, phase ^ 1);
                     if (elect_one()) {
-                        mbar_expect_tx_u32(full_u32 + stage * 8, b_tx);
-                        tma_load_2d(&p.tmB, full_u32 + stage * 8, smem_b + (uint32_t)stage * b_bytes, tap * cin_pad + ch * 64, bn0);
+                        mbar_expect_tx_u32<PAIR>(full_bar + stage * 8, b_tx);
+                        tma_load_2d<PAIR>(&p.tmB, full_bar + stage * 8, smem_b + (uint32_t)stage * b_bytes, tap * cin_pad + ch * 64, bn0);
                     }
                     if (++stage == nstages) { stage = 0; phase ^= 1; }
                 }
@@ -1115,10 +1175,11 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_halo_kernel(const __grid_
         uint32_t hphase = 0;
         const int chunks = p.chunks;
         const bool perm = p.perm != 0;
+        const uint32_t hfull_bar = PAIR ? mapa_u32(hfull_u32, 0) : hfull_u32;
         int pit = 0;
-        for (int rd = blockIdx.x; rd < rounds; rd += gridDim.x, ++pit) {
-            const int t0 = rd * mt;
-            const int nv = min(mt, total_tiles - t0);
+        for (int rd = rs.rd0(); rd < rs.rounds; rd += rs.step(), ++pit) {
+            const int t0 = rs.tile0(rd);
+            const int nv = rs.tiles(rd);
             const TileCoord tc0 = decode_tile(p, t0);
             const TileCoord tc1 = decode_tile(p, nv > 1 ? t0 + 1 : t0);
             trace(p, 0, pit, 0);
@@ -1126,16 +1187,16 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_halo_kernel(const __grid_
                 mbar_wait_u32(hempty_u32 + hb * 8, hphase ^ 1);
                 if (ch == 0) trace(p, 0, pit, 1);
                 if (elect_one()) {
-                    const uint32_t hbar = hfull_u32 + hb * 8, dst = smem_a + (uint32_t)(hb * mt) * halo_bytes;
-                    mbar_expect_tx_u32(hbar, (uint32_t)nv * p.a_tx_bytes);
-                    tma_load_4d(&p.tmA[0], hbar, dst, ch * 64, tc0.x0 - 1, perm ? tc0.n0 : tc0.y0 - 1, perm ? tc0.y0 - 1 : tc0.n0);
-                    if (nv > 1) tma_load_4d(&p.tmA[0], hbar, dst + halo_bytes, ch * 64, tc1.x0 - 1, perm ? tc1.n0 : tc1.y0 - 1, perm ? tc1.y0 - 1 : tc1.n0);
+                    const uint32_t hbar = hfull_bar + hb * 8, dst = smem_a + (uint32_t)(hb * mt) * halo_bytes;
+                    mbar_expect_tx_u32<PAIR>(hbar, (uint32_t)nv * p.a_tx_bytes);
+                    tma_load_act<PAIR>(&p.tmA[0], hbar, dst, ch * 64, tc0.x0 - 1, tc0.y0 - 1, tc0.n0, perm);
+                    if (nv > 1) tma_load_act(&p.tmA[0], hbar, dst + halo_bytes, ch * 64, tc1.x0 - 1, tc1.y0 - 1, tc1.n0, perm);
                 }
                 if (++hb == 2) { hb = 0; hphase ^= 1; }
             }
             trace(p, 0, pit, 2);
         }
-    } else if (warp == 1) {
+    } else if (warp == 1 && (!PAIR || rs.rank == 0)) {
         int stage = 0, hb = 0, it = 0;
         uint32_t phase = 0, hphase = 0;
         const bool leader = elect_one();                 // elected once; see conv_tc_kernel for why the loop is this lean
@@ -1147,11 +1208,11 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_halo_kernel(const __grid_
         const int nstages = p.stages, n_tile = p.n_tile, chunks = p.chunks;
         const int last_kmmas = (p.cin - (chunks - 1) * 64 + 15) >> 4;
         const uint32_t tfull_u32 = smem_u32(b.tfull), tempty_u32 = smem_u32(b.tempty);
-        for (int rd = blockIdx.x; rd < rounds; rd += gridDim.x, ++it) {
+        for (int rd = rs.rd0(); rd < rs.rounds; rd += rs.step(), ++it) {
             const int as = it & 1;
             const uint32_t aphase = (it >> 1) & 1;
-            const bool two = min(mt, total_tiles - rd * mt) > 1;
-            const bool b_res = p.b_res != 0, b_wait = !b_res || it == 0;
+            const bool two = rs.tiles(rd) > 1;
+            const bool b_res = !PAIR && p.b_res != 0, b_wait = !b_res || it == 0;
             trace(p, 1, it, 0);
             mbar_wait_u32(tempty_u32 + as * 8, aphase ^ 1);
             tc_fence_after();
@@ -1164,8 +1225,6 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_halo_kernel(const __grid_
                 const uint32_t a_lo_h = a_lo0 + (uint32_t)(hb * mt) * halo_units;
                 const bool last = ch == chunks - 1;
                 const int km = last ? last_kmmas : 4;                        // skip the zero-padded tail of the last chunk
-                // the K-step count is a compile-time constant of the issue loop: a per-MMA `k < km` test costs ~13 cycles
-                // per MMA on the single issuing thread (tools/ubench/mma_issue.cu, variants 32 / 33)
                 auto taps = [&](auto KM) {
 #pragma unroll
                     for (int tap = 0; tap < 9; ++tap) {
@@ -1179,365 +1238,32 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_halo_kernel(const __grid_
                             const uint32_t acc0 = tap == 0 ? (uint32_t)(ch != 0) : 1u;
 #pragma unroll
                             for (int k = 0; k < decltype(KM)::value; ++k)
-                                umma_bf16(d_tmem, desc64(hi_a, a_lo + 2 * k), desc64(hi_b, b_lo + 2 * k), idesc, k == 0 ? acc0 : 1u);
+                                umma_bf16<PAIR>(d_tmem, desc64(hi_a, a_lo + 2 * k), desc64(hi_b, b_lo + 2 * k), idesc, k == 0 ? acc0 : 1u);
                             if (two) {
 #pragma unroll
                                 for (int k = 0; k < decltype(KM)::value; ++k)
                                     umma_bf16(d_tmem + (uint32_t)n_tile, desc64(hi_a, a_lo + halo_units + 2 * k), desc64(hi_b, b_lo + 2 * k), idesc, k == 0 ? acc0 : 1u);
                             }
-                            if (!b_res) umma_commit(empty_u32 + stage * 8);
+                            if (!b_res) umma_commit<PAIR>(empty_u32 + stage * 8);
                             if (tap == 8) {
-                                umma_commit(hempty_u32 + hb * 8);                         // halo tiles free once their MMAs retire
-                                if (last) umma_commit(tfull_u32 + as * 8);
+                                umma_commit<PAIR>(hempty_u32 + hb * 8);                   // halo tiles free once their MMAs retire
+                                if (last) umma_commit<PAIR>(tfull_u32 + as * 8);
                             }
                         }
                         if (++stage == nstages) { stage = 0; phase ^= 1; }
                     }
                 };
-                if (km == 4) taps(KConst<4>{});
-                else if (km == 3) taps(KConst<3>{});
-                else if (km == 2) taps(KConst<2>{});
-                else taps(KConst<1>{});
+                with_ksteps(km, taps);
                 if (++hb == 2) { hb = 0; hphase ^= 1; }
             }
             trace(p, 1, it, 3);
         }
     } else if (warp == 3) {
-        store_loop<RES, F32>(p, total_tiles, b.sfull, b.sempty, b.res, smem + p.stg_off, lane);
+        store_loop<RES, F32, PAIR>(p, total_tiles, b.sfull, b.sempty, b.res, smem + p.stg_off, lane);
     } else if (warp >= 4) {
-        epilogue_loop<ACT, RES, F32>(p, total_tiles, tmem_base, b.bias_s, b.tfull, b.tempty, b.sfull, b.sempty, b.res, smem + p.stg_off, warp, lane);
+        epilogue_loop<ACT, RES, F32, PAIR>(p, total_tiles, tmem_base, b.bias_s, b.tfull, b.tempty, b.sfull, b.sempty, b.res, smem + p.stg_off, warp, lane);
     }
-    epilogue_exit(p, tmem_base, warp);
-}
-
-// ---------------------------------------------------------------------------------------------
-// CTA-pair halo kernel (wide layers, n_tile >= 128): two SMs of one cluster work on two neighbouring M tiles with
-// ONE stream of MMAs (cta_group::2, M = 256) issued by the leader.  Each CTA loads its own halo and only half of
-// every weight tile, so per SM the weight fill and the B-operand reads are halved and each MMA instruction carries
-// twice the work -- what keeps the tensor pipe fed where a single SM's issue rate and smem bandwidth could not.
-// Barriers: full / hfull / tempty live in the leader (both CTAs arrive), empty / hempty / tfull are signalled in
-// both CTAs by the leader's multicast commits.
-// ---------------------------------------------------------------------------------------------
-template <int ACT, int RES, int F32>
-__global__ void __launch_bounds__(kThreads, 1) conv_tc_halo2_kernel(const __grid_constant__ ConvTcParams p, int nimg) {
-    extern __shared__ __align__(1024) uint8_t smem_raw[];
-    uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-    const Bars b = carve_bars(smem, p);
-    const int warp = threadIdx.x >> 5;
-    const int lane = threadIdx.x & 31;
-    const uint32_t rank = cluster_ctarank();
-    const int total_tiles = p.tiles_x * p.tiles_y * ((nimg + p.bn - 1) / p.bn);     // n_tiles_n == 1
-    const int rounds = (total_tiles + 1) / 2;
-    const int rd0 = (int)(blockIdx.x >> 1), rd_step = (int)(gridDim.x >> 1);
-
-    if (warp == 0 && lane == 0) { tma_prefetch_desc(&p.tmA[0]); tma_prefetch_desc(&p.tmB); }
-    if (warp == 1 && lane == 0) {
-        for (int i = 0; i < p.stages; ++i) {
-            mbar_init(&b.full[i], 2);                 // one arrive.expect_tx per CTA (leader's copy is the one waited on)
-            mbar_init(&b.empty[i], 1);
-        }
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(&b.tfull[i], 1);
-            mbar_init(&b.tempty[i], 8 * p.epi_parts);     // epilogue warps of both CTAs, one arrival each
-            mbar_init(&b.hfull[i], 2);
-            mbar_init(&b.hempty[i], 1);
-        }
-        for (int i = 0; i < p.stg_bufs * p.mt; ++i) {
-            if (p.has_res) mbar_init(&b.res[i], 1);
-            mbar_init(&b.sfull[i], 4 * p.epi_parts);
-            mbar_init(&b.sempty[i], 1);
-        }
-        fence_barrier_init();
-    }
-    if (warp == 2) tmem_alloc_2sm(b.tmem_slot, p.tmem_cols);
-    for (int i = threadIdx.x; i < p.n_tile; i += blockDim.x) b.bias_s[i] = p.act ? 0.5f * p.bias[i] : p.bias[i];
-    tc_fence_before();
-    cluster_sync_all();                               // barriers of both CTAs initialised before anyone signals them
-    tc_fence_after();
-    const uint32_t tmem_base = *b.tmem_slot;
-    const uint32_t halo_bytes = p.halo_bytes;
-    const uint32_t smem_a = smem_u32(smem), smem_b = smem_a + 2u * halo_bytes;
-    const uint32_t full_u32 = smem_u32(b.full), empty_u32 = smem_u32(b.empty);
-    const uint32_t hfull_u32 = smem_u32(b.hfull), hempty_u32 = smem_u32(b.hempty);
-
-    if (warp == 0) {
-        // ===================== weight producer (both CTAs): this CTA's half of every weight box =====================
-        int stage = 0;
-        uint32_t phase = 0;
-        const int nstages = p.stages, chunks = p.chunks;
-        const int cin_pad = chunks * 64;
-        const uint32_t b_tx = p.b_tx_bytes, b_bytes = p.b_bytes;
-        const uint32_t lead_full = mapa_u32(full_u32, 0);
-        const int b_row0 = (int)rank * (p.n_tile >> 1);                      // this CTA's half of the weight rows
-        for (int rd = rd0; rd < rounds; rd += rd_step) {
-            for (int ch = 0; ch < chunks; ++ch) {
-                for (int tap = 0; tap < 9; ++tap) {
-                    mbar_wait_u32(empty_u32 + stage * 8, phase ^ 1);
-                    if (elect_one()) {
-                        mbar_expect_tx_cluster(lead_full + stage * 8, b_tx);
-                        tma_load_2d_2sm(&p.tmB, lead_full + stage * 8, smem_b + (uint32_t)stage * b_bytes, tap * cin_pad + ch * 64, b_row0);
-                    }
-                    if (++stage == nstages) { stage = 0; phase ^= 1; }
-                }
-            }
-        }
-    } else if (warp == 2) {
-        // ===================== halo producer (both CTAs; the TMEM allocator warp, idle after the prologue) =====================
-        int hb = 0;
-        uint32_t hphase = 0;
-        const int chunks = p.chunks;
-        const bool perm = p.perm != 0;
-        const uint32_t lead_hfull = mapa_u32(hfull_u32, 0);
-        for (int rd = rd0; rd < rounds; rd += rd_step) {
-            const TileCoord tc = decode_tile(p, min(2 * rd + (int)rank, total_tiles - 1));
-            for (int ch = 0; ch < chunks; ++ch) {
-                mbar_wait_u32(hempty_u32 + hb * 8, hphase ^ 1);
-                if (elect_one()) {
-                    mbar_expect_tx_cluster(lead_hfull + hb * 8, p.a_tx_bytes);
-                    tma_load_4d_2sm(&p.tmA[0], lead_hfull + hb * 8, smem_a + (uint32_t)hb * halo_bytes, ch * 64, tc.x0 - 1, perm ? tc.n0 : tc.y0 - 1,
-                                    perm ? tc.y0 - 1 : tc.n0);
-                }
-                if (++hb == 2) { hb = 0; hphase ^= 1; }
-            }
-        }
-    } else if (warp == 1 && rank == 0) {
-        // ===================== MMA issuer (leader CTA only) =====================
-        int stage = 0, hb = 0, it = 0;
-        uint32_t phase = 0, hphase = 0;
-        const bool leader = elect_one();
-        const uint32_t hi_b = desc_hi(1024), hi_a = desc_hi((uint32_t)p.halo_w * 128u);
-        const uint32_t b_units = p.b_bytes >> 4, halo_units = halo_bytes >> 4, kh_units = (p.halo_kh_rows * 128u) >> 4;
-        const uint32_t a_lo0 = desc_lo(smem_a), b_lo0 = desc_lo(smem_b);
-        const uint32_t idesc = p.idesc;                                   // M = 256
-        const int nstages = p.stages, n_tile = p.n_tile, chunks = p.chunks;
-        const int last_kmmas = (p.cin - (chunks - 1) * 64 + 15) >> 4;
-        const uint32_t tfull_u32 = smem_u32(b.tfull), tempty_u32 = smem_u32(b.tempty);
-        for (int rd = rd0; rd < rounds; rd += rd_step, ++it) {
-            const int as = it & 1;
-            const uint32_t aphase = (it >> 1) & 1;
-            trace(p, 1, it, 0);
-            mbar_wait_u32(tempty_u32 + as * 8, aphase ^ 1);
-            tc_fence_after();
-            trace(p, 1, it, 1);
-            const uint32_t d_tmem = tmem_base + (uint32_t)(as * n_tile);
-#ifdef B2D_ENABLE_TRACE
-            long long wait_b = 0, wait_h = 0, w0;
-#endif
-            for (int ch = 0; ch < chunks; ++ch) {
-#ifdef B2D_ENABLE_TRACE
-                w0 = clock64();
-#endif
-                mbar_wait_u32(hfull_u32 + hb * 8, hphase);
-#ifdef B2D_ENABLE_TRACE
-                wait_h += clock64() - w0;
-#endif
-                tc_fence_after();
-                if (ch == 0) trace(p, 1, it, 2);
-                const uint32_t a_lo_h = a_lo0 + (uint32_t)hb * halo_units;
-                const int km = (ch == chunks - 1) ? last_kmmas : 4;
-                const bool last = ch == chunks - 1;
-                auto taps = [&](auto KM) {
-#pragma unroll
-                    for (int tap = 0; tap < 9; ++tap) {
-#ifdef B2D_ENABLE_TRACE
-                        w0 = clock64();
-#endif
-                        mbar_wait_u32(full_u32 + stage * 8, phase);
-                        tc_fence_after();
-#ifdef B2D_ENABLE_TRACE
-                        wait_b += clock64() - w0;
-#endif
-                        if (leader) {
-                            const uint32_t b_lo = b_lo0 + (uint32_t)stage * b_units;
-                            const uint32_t a_lo = a_lo_h + (uint32_t)(tap / 3) * kh_units + (uint32_t)(tap % 3) * 8u;
-                            const uint32_t acc0 = tap == 0 ? (uint32_t)(ch != 0) : 1u;
-#pragma unroll
-                            for (int k = 0; k < decltype(KM)::value; ++k)
-                                umma_bf16_2sm(d_tmem, desc64(hi_a, a_lo + 2 * k), desc64(hi_b, b_lo + 2 * k), idesc, k == 0 ? acc0 : 1u);
-                            umma_commit_2sm(empty_u32 + stage * 8);
-                            if (tap == 8) {
-                                umma_commit_2sm(hempty_u32 + hb * 8);
-                                if (last) umma_commit_2sm(tfull_u32 + as * 8);
-                            }
-                        }
-                        if (++stage == nstages) { stage = 0; phase ^= 1; }
-                    }
-                };
-                if (km == 4) taps(KConst<4>{});
-                else if (km == 3) taps(KConst<3>{});
-                else if (km == 2) taps(KConst<2>{});
-                else taps(KConst<1>{});
-                if (++hb == 2) { hb = 0; hphase ^= 1; }
-            }
-            trace(p, 1, it, 3);
-#ifdef B2D_ENABLE_TRACE
-            if (p.trace && blockIdx.x == 0 && it < kTraceTiles && lane == 0) {      // reported as offsets from the first stamp: halo / weight wait cycles
-                p.trace[(0 * kTraceTiles + it) * kTraceEvents + 2] = wait_h + p.trace[kTraceTiles * kTraceEvents];
-                p.trace[(0 * kTraceTiles + it) * kTraceEvents + 3] = wait_b + p.trace[kTraceTiles * kTraceEvents];
-            }
-#endif
-        }
-    } else if (warp == 3) {
-        store_loop<RES, F32>(p, total_tiles, b.sfull, b.sempty, b.res, smem + p.stg_off, lane, true);
-    } else if (warp >= 4) {
-        epilogue_loop<ACT, RES, F32>(p, total_tiles, tmem_base, b.bias_s, b.tfull, b.tempty, b.sfull, b.sempty, b.res, smem + p.stg_off, warp, lane, true);
-    }
-    tc_fence_before();
-    cluster_sync_all();                               // the peer may still signal this CTA's barriers / read its smem until here
-    if (warp == 2) {
-        tc_fence_after();
-        tmem_dealloc_2sm(tmem_base, p.tmem_cols);
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
-// CTA-pair generic kernel (1x1 and stride-2 layers with n_tile >= 128): the generic kernel's operand feed -- one A box per
-// (tap, chunk) -- with the pair's MMA stream.  Each CTA loads the A box of its own M tile and HALF of every weight box into
-// the same stage slot; the leader issues one cta_group::2 MMA (M = 256) per K = 16 step.  Per SM the weight traffic from L2
-// and the B-operand reads are halved: these layers run N = 192 tiles, where a single SM needs ~105 bytes of operands per
-// clock to keep its tensor pipe busy and L2 delivers about half of that.
-// Barriers as in the halo pair kernel: full / tempty live in the leader (both CTAs arrive), empty / tfull are signalled in
-// both CTAs by the leader's multicast commits.
-// ---------------------------------------------------------------------------------------------
-template <int ACT, int RES, int F32>
-__global__ void __launch_bounds__(kThreads, 1) conv_tc_pair_kernel(const __grid_constant__ ConvTcParams p, int nimg) {
-    extern __shared__ __align__(1024) uint8_t smem_raw[];
-    uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-    const Bars b = carve_bars(smem, p);
-    const int warp = threadIdx.x >> 5;
-    const int lane = threadIdx.x & 31;
-    const uint32_t rank = cluster_ctarank();
-    const int total_tiles = p.tiles_x * p.tiles_y * ((nimg + p.bn - 1) / p.bn) * p.n_tiles_n;
-    const int rounds = pair_rounds(p, total_tiles);
-    const int rd0 = (int)(blockIdx.x >> 1), rd_step = (int)(gridDim.x >> 1);
-    const int ksteps = p.taps * p.chunks;
-    const uint32_t stage_bytes = p.a_bytes + p.b_bytes;
-
-    if (warp == 0 && lane == 0) {
-        tma_prefetch_desc(&p.tmA[0]);
-        if (p.stride == 2) { tma_prefetch_desc(&p.tmA[1]); tma_prefetch_desc(&p.tmA[2]); tma_prefetch_desc(&p.tmA[3]); }
-        tma_prefetch_desc(&p.tmB);
-    }
-    if (warp == 1 && lane == 0) {
-        for (int i = 0; i < p.stages; ++i) {
-            mbar_init(&b.full[i], 2);                 // one arrive.expect_tx per CTA (the leader's copy is the one waited on)
-            mbar_init(&b.empty[i], 1);
-        }
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(&b.tfull[i], 1);
-            mbar_init(&b.tempty[i], 8 * p.epi_parts);     // epilogue warps of both CTAs, one arrival each
-            mbar_init(&b.hfull[i], 1);
-            mbar_init(&b.hempty[i], 1);
-        }
-        for (int i = 0; i < p.stg_bufs * p.mt; ++i) {
-            if (p.has_res) mbar_init(&b.res[i], 1);
-            mbar_init(&b.sfull[i], 4 * p.epi_parts);
-            mbar_init(&b.sempty[i], 1);
-        }
-        fence_barrier_init();
-    }
-    if (warp == 2) tmem_alloc_2sm(b.tmem_slot, p.tmem_cols);
-    for (int i = threadIdx.x; i < p.n_tile * p.n_tiles_n; i += blockDim.x) b.bias_s[i] = p.act ? 0.5f * p.bias[i] : p.bias[i];
-    tc_fence_before();
-    cluster_sync_all();                               // barriers of both CTAs initialised before anyone signals them
-    tc_fence_after();
-    const uint32_t tmem_base = *b.tmem_slot;
-    const uint32_t smem_base = smem_u32(smem);
-    const uint32_t full_u32 = smem_u32(b.full), empty_u32 = smem_u32(b.empty);
-
-    if (warp == 0) {
-        // ===================== TMA producer (both CTAs): own A box + this CTA's half of the weight box =====================
-        int stage = 0;
-        uint32_t phase = 0;
-        const int pad = p.ksz >> 1;
-        const int nstages = p.stages, taps = p.taps, chunks = p.chunks, ksz = p.ksz, n_tile = p.n_tile;
-        const int cin_pad = chunks * 64;
-        const bool s2 = (p.stride == 2), perm = p.perm != 0;
-        const uint32_t lead_full = mapa_u32(full_u32, 0);
-        const uint32_t tx_bytes = p.a_tx_bytes + p.b_tx_bytes;
-        for (int rd = rd0; rd < rounds; rd += rd_step) {
-            const TileCoord tc = decode_tile(p, pair_tile(p, rd, (int)rank, total_tiles));
-            const int b_row0 = tc.nt * n_tile + (int)rank * (n_tile >> 1);
-            int kh = 0, kw = 0;
-            for (int tap = 0; tap < taps; ++tap) {
-                const CUtensorMap* mapA = &p.tmA[0];
-                int ox = kw - pad, oy = kh - pad;
-                if (s2) {
-                    const int dy = kh - 1, dx = kw - 1;
-                    const int py = dy & 1, px = dx & 1;
-                    mapA = &p.tmA[py * 2 + px];
-                    ox = (dx - px) / 2;
-                    oy = (dy - py) / 2;
-                }
-                const int kb = tap * cin_pad;
-                for (int ch = 0; ch < chunks; ++ch) {
-                    mbar_wait_u32(empty_u32 + stage * 8, phase ^ 1);
-                    if (elect_one()) {
-                        const uint32_t sa = smem_base + (uint32_t)stage * stage_bytes, fb = lead_full + stage * 8;
-                        mbar_expect_tx_cluster(fb, tx_bytes);
-                        const int cy = tc.y0 + oy;
-                        tma_load_4d_2sm(mapA, fb, sa, ch * 64, tc.x0 + ox, perm ? tc.n0 : cy, perm ? cy : tc.n0);
-                        tma_load_2d_2sm(&p.tmB, fb, sa + p.a_bytes, kb + ch * 64, b_row0);
-                    }
-                    if (++stage == nstages) { stage = 0; phase ^= 1; }
-                }
-                if (++kw == ksz) { kw = 0; ++kh; }
-            }
-        }
-    } else if (warp == 1 && rank == 0) {
-        // ===================== MMA issuer (leader CTA only) =====================
-        int stage = 0, it = 0;
-        uint32_t phase = 0;
-        const bool leader = elect_one();
-        const uint32_t hi = desc_hi(1024);
-        const uint32_t lo_base = desc_lo(smem_base);
-        const uint32_t stage_units = stage_bytes >> 4, a_units = p.a_bytes >> 4;
-        const uint32_t idesc = p.idesc;                                   // M = 256
-        const int nstages = p.stages, n_tile = p.n_tile, chunks = p.chunks, taps = p.taps;
-        const int last_kmmas = (p.cin - (chunks - 1) * 64 + 15) >> 4;
-        const uint32_t tfull_u32 = smem_u32(b.tfull), tempty_u32 = smem_u32(b.tempty);
-        for (int rd = rd0; rd < rounds; rd += rd_step, ++it) {
-            const int as = it & 1;
-            const uint32_t aphase = (it >> 1) & 1;
-            mbar_wait_u32(tempty_u32 + as * 8, aphase ^ 1);
-            tc_fence_after();
-            const uint32_t d_tmem = tmem_base + (uint32_t)(as * n_tile);
-            int ks = 0;
-            auto step = [&](auto KM) {
-                mbar_wait_u32(full_u32 + stage * 8, phase);
-                tc_fence_after();
-                if (leader) {
-                    const uint32_t a_lo = lo_base + (uint32_t)stage * stage_units;
-                    const uint32_t b_lo = a_lo + a_units;
-                    const uint32_t acc0 = (uint32_t)(ks != 0);
-#pragma unroll
-                    for (int k = 0; k < decltype(KM)::value; ++k)
-                        umma_bf16_2sm(d_tmem, desc64(hi, a_lo + 2 * k), desc64(hi, b_lo + 2 * k), idesc, k == 0 ? acc0 : 1u);
-                    umma_commit_2sm(empty_u32 + stage * 8);                       // frees the slot in both CTAs
-                    if (ks == ksteps - 1) umma_commit_2sm(tfull_u32 + as * 8);
-                }
-                ++ks;
-                if (++stage == nstages) { stage = 0; phase ^= 1; }
-            };
-            for (int tap = 0; tap < taps; ++tap) {
-                for (int ch = 0; ch < chunks - 1; ++ch) step(KConst<4>{});
-                if (last_kmmas == 4) step(KConst<4>{});
-                else if (last_kmmas == 3) step(KConst<3>{});
-                else if (last_kmmas == 2) step(KConst<2>{});
-                else step(KConst<1>{});
-            }
-        }
-    } else if (warp == 3) {
-        store_loop<RES, F32>(p, total_tiles, b.sfull, b.sempty, b.res, smem + p.stg_off, lane, true);
-    } else if (warp >= 4) {
-        epilogue_loop<ACT, RES, F32>(p, total_tiles, tmem_base, b.bias_s, b.tfull, b.tempty, b.sfull, b.sempty, b.res, smem + p.stg_off, warp, lane, true);
-    }
-    tc_fence_before();
-    cluster_sync_all();                               // the peer may still signal this CTA's barriers / read its smem until here
-    if (warp == 2) {
-        tc_fence_after();
-        tmem_dealloc_2sm(tmem_base, p.tmem_cols);
-    }
+    epilogue_exit<PAIR>(p, tmem_base, warp);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1562,12 +1288,12 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_dw_kernel(const __grid_co
     const Bars b = carve_bars(smem, p);
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
-    const int mt = p.mt;
     const int total_tiles = p.tiles_x * p.tiles_y * ((nimg + p.bn - 1) / p.bn) * p.n_tiles_n;
-    const int rounds = (total_tiles + mt - 1) / mt;
+    const RoundSched<0> rs(p, total_tiles);
+    const int mt = rs.mt;
 
     if (warp == 0 && lane == 0) { tma_prefetch_desc(&p.tmA[0]); tma_prefetch_desc(&p.tmB); }
-    const uint32_t tmem_base = prologue(p, b, warp, lane, 1, 2);
+    const uint32_t tmem_base = prologue(p, b, warp, lane, 2);
     const uint32_t halo_bytes = p.halo_bytes;
     const uint32_t smem_a = smem_u32(smem), smem_b = smem_a + 2u * (uint32_t)mt * halo_bytes;
     const uint32_t full_u32 = smem_u32(b.full), empty_u32 = smem_u32(b.empty);
@@ -1581,9 +1307,9 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_dw_kernel(const __grid_co
         const uint32_t b_tx = p.b_tx_bytes, b_bytes = p.b_bytes;
         const bool perm = p.perm != 0;
         int pit = 0;
-        for (int rd = blockIdx.x; rd < rounds; rd += gridDim.x, ++pit) {
-            const int t0 = rd * mt;
-            const int nv = min(mt, total_tiles - t0);
+        for (int rd = rs.rd0(); rd < rs.rounds; rd += rs.step(), ++pit) {
+            const int t0 = rs.tile0(rd);
+            const int nv = rs.tiles(rd);
             const TileCoord tc0 = decode_tile(p, t0);
             const TileCoord tc1 = decode_tile(p, nv > 1 ? t0 + 1 : t0);
             trace(p, 0, pit, 0);
@@ -1599,8 +1325,8 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_dw_kernel(const __grid_co
                 if (elect_one()) {
                     const uint32_t hbar = hfull_u32 + hb * 8, dst = smem_a + (uint32_t)(hb * mt) * halo_bytes;
                     mbar_expect_tx_u32(hbar, (uint32_t)nv * p.a_tx_bytes);
-                    tma_load_4d(&p.tmA[0], hbar, dst, gch * 64, tc0.x0 - 1, perm ? tc0.n0 : tc0.y0 - 1, perm ? tc0.y0 - 1 : tc0.n0);
-                    if (nv > 1) tma_load_4d(&p.tmA[0], hbar, dst + halo_bytes, gch * 64, tc1.x0 - 1, perm ? tc1.n0 : tc1.y0 - 1, perm ? tc1.y0 - 1 : tc1.n0);
+                    tma_load_act(&p.tmA[0], hbar, dst, gch * 64, tc0.x0 - 1, tc0.y0 - 1, tc0.n0, perm);
+                    if (nv > 1) tma_load_act(&p.tmA[0], hbar, dst + halo_bytes, gch * 64, tc1.x0 - 1, tc1.y0 - 1, tc1.n0, perm);
                 }
                 if (++hb == 2) { hb = 0; hphase ^= 1; }
             }
@@ -1620,10 +1346,10 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_dw_kernel(const __grid_co
         const int nstages = p.stages, n_tile = p.n_tile;
         const uint32_t kh_bytes = p.halo_kh_rows * 128u;
         const uint32_t tfull_u32 = smem_u32(b.tfull), tempty_u32 = smem_u32(b.tempty);
-        for (int rd = blockIdx.x; rd < rounds; rd += gridDim.x, ++it) {
+        for (int rd = rs.rd0(); rd < rs.rounds; rd += rs.step(), ++it) {
             const int as = it & 1;
             const uint32_t aphase = (it >> 1) & 1;
-            const int nv = min(mt, total_tiles - rd * mt);
+            const int nv = rs.tiles(rd);
             if (isu == 0) trace(p, 1, it, 0);
             mbar_wait_u32(tempty_u32 + as * 8, aphase ^ 1);
             tc_fence_after();
@@ -1695,9 +1421,9 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_stem2_kernel(const __grid
     const Bars b = carve_bars(smem, p);
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
-    const int mt = p.mt;
     const int total_tiles = p.tiles_x * p.tiles_y * nimg;                // bn == 1
-    const int rounds = (total_tiles + mt - 1) / mt;
+    const RoundSched<0> rs(p, total_tiles);
+    const int mt = rs.mt;
     const uint32_t tile_bytes = p.a_bytes, stage_bytes = (uint32_t)mt * tile_bytes;
     uint8_t* wres = smem + (size_t)p.stages * stage_bytes;               // resident weights [n_tile][64] 16-bit, SWIZZLE_128B
 
@@ -1715,7 +1441,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_stem2_kernel(const __grid
         }
         fence_proxy_async();
     }
-    const uint32_t tmem_base = prologue(p, b, warp, lane, 1);
+    const uint32_t tmem_base = prologue(p, b, warp, lane);
     const uint32_t smem_base = smem_u32(smem);
     const uint32_t full_u32 = smem_u32(b.full), empty_u32 = smem_u32(b.empty);
 
@@ -1724,8 +1450,8 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_stem2_kernel(const __grid
         int stage = 0, pit = 0;
         uint32_t phase = 0;
         const int nstages = p.stages;
-        for (int rd = blockIdx.x; rd < rounds; rd += gridDim.x, ++pit) {
-            const int t0 = rd * mt, nv = min(mt, total_tiles - t0);
+        for (int rd = rs.rd0(); rd < rs.rounds; rd += rs.step(), ++pit) {
+            const int t0 = rs.tile0(rd), nv = rs.tiles(rd);
             trace(p, 0, pit, 0);
             mbar_wait_u32(empty_u32 + stage * 8, phase ^ 1);
             if (elect_one()) {
@@ -1752,9 +1478,9 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_stem2_kernel(const __grid
         const uint32_t idesc = p.idesc;
         const int nstages = p.stages, n_tile = p.n_tile;
         const uint32_t tfull_u32 = smem_u32(b.tfull), tempty_u32 = smem_u32(b.tempty);
-        for (int rd = blockIdx.x; rd < rounds; rd += gridDim.x, ++it) {
+        for (int rd = rs.rd0(); rd < rs.rounds; rd += rs.step(), ++it) {
             const int as = it & 1;
-            const int nv = min(mt, total_tiles - rd * mt);
+            const int nv = rs.tiles(rd);
             trace(p, 1, it, 0);
             mbar_wait_u32(tempty_u32 + as * 8, ((it >> 1) & 1) ^ 1);
             trace(p, 1, it, 1);
@@ -1935,7 +1661,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_dwpw_kernel(const __grid_
             asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(smem_dw + (uint32_t)i * 16u), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
         }
     }
-    const uint32_t tmem_base = prologue(p, b, warp, lane, 1, 1, 8, 8);    // hempty / afull: one arrival per depthwise warp
+    const uint32_t tmem_base = prologue(p, b, warp, lane, 1, 8, 8);    // hempty / afull: one arrival per depthwise warp
     const uint32_t full_u32 = smem_u32(b.full), empty_u32 = smem_u32(b.empty);
     const uint32_t hfull_u32 = smem_u32(b.hfull), hempty_u32 = smem_u32(b.hempty);
     const uint32_t afull_u32 = smem_u32(b.afull), aempty_u32 = smem_u32(b.aempty);
@@ -1952,7 +1678,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_dwpw_kernel(const __grid_
                 if (elect_one()) {
                     const uint32_t hbar = hfull_u32 + hb * 8;
                     mbar_expect_tx_u32(hbar, p.a_tx_bytes);
-                    tma_load_4d(&p.tmA[0], hbar, smem_h + (uint32_t)hb * halo_bytes, ch * 64, tc.x0 - 1, perm ? tc.n0 : tc.y0 - 1, perm ? tc.y0 - 1 : tc.n0);
+                    tma_load_act(&p.tmA[0], hbar, smem_h + (uint32_t)hb * halo_bytes, ch * 64, tc.x0 - 1, tc.y0 - 1, tc.n0, perm);
                 }
                 if (++hb == 2) { hb = 0; hphase ^= 1; }
             }
@@ -2065,7 +1791,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_s2halo_kernel(const __gri
         for (int i = 0; i < 4; ++i) tma_prefetch_desc(&p.tmA[i]);
         tma_prefetch_desc(&p.tmB);
     }
-    const uint32_t tmem_base = prologue(p, b, warp, lane, 1);
+    const uint32_t tmem_base = prologue(p, b, warp, lane);
     const uint32_t full_u32 = smem_u32(b.full), empty_u32 = smem_u32(b.empty);
     const uint32_t wbar = smem_u32(b.hfull);                          // "weights have landed"
 
@@ -2141,10 +1867,7 @@ __global__ void __launch_bounds__(kThreads, 1) conv_tc_s2halo_kernel(const __gri
                     if (++slot == nslots) { slot = 0; phase ^= 1; }
                 }
             };
-            if (kmmas == 4) tile(KConst<4>{});
-            else if (kmmas == 3) tile(KConst<3>{});
-            else if (kmmas == 2) tile(KConst<2>{});
-            else tile(KConst<1>{});
+            with_ksteps(kmmas, tile);
         }
     } else if (warp == 3) {
         store_loop<RES, F32>(p, total_tiles, b.sfull, b.sempty, b.res, smem + p.stg_off, lane);
@@ -2469,38 +2192,33 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
     }
     B2D_CHECK(planned, "conv_tc: no shared-memory configuration fits (n_tile %d)", p.n_tile);
     p.kind = best_kind; p.mt = best_mt; p.stages = best_stages; p.stg_bufs = best_bufs; p.b_res = best_bres;
-    // CTA pairs for wide halo layers: weight stages shrink to half a tile per CTA (so the ring gets deeper)
-    p.pair = 0;
-    if (p.kind == CONV_HALO && split == 1 && p.n_tile >= 128 && p.n_tile % 32 == 0 && (total_tiles >= 2 * sm_count || force_pair) && pair_env != 0) {
-        p.pair = 1;
+    // CTA pairs (the PAIR forms of the halo and generic kernels) for layers with wide output tiles and enough tiles for 2 x 148
+    // SMs: a stage holds half a weight tile per CTA, so the ring gets deeper.
+    //   halo: 192-channel 3x3 layers and wider, n_tile a multiple of 32.
+    //   generic (1x1, stride 2), one tile per round and a SHORT reduction.  Measured per op at batch 64
+    //   (profiles/r2_pair_generic_per_op.txt): K = cin * taps < 576 gains 5-18 % (the weight tile is a large share of a short
+    //   round's operand traffic), K >= 576 loses 1-6 % (the leader's barrier round trip through the cluster per K step is no
+    //   longer hidden), so the planner pairs only the short ones ... and the 3x3 stride-1 layers that run here because their
+    //   tiles are not 8 pixels wide (288 -> 288 at 20 x 20, two N = 144 tiles): 41.6 -> 35 us each with the pair's halved weight
+    //   traffic, N / 2 = 72 rows per CTA.
+    const bool pair_short_k = cin * p.taps < 576 || (stride == 2 && cin <= 96) || (ksz == 3 && stride == 1);
+    const bool pair_kind = p.kind == CONV_HALO ? split == 1 && p.n_tile % 32 == 0
+                         : p.kind == CONV_GENERIC && p.n_tile % 16 == 0 && p.mt == 1 && (pair_short_k || force_pair);
+    p.pair = pair_kind && p.n_tile >= 128 && (total_tiles >= 2 * sm_count || force_pair) && pair_env != 0 ? 1 : 0;
+    if (p.pair) {
+        // what differs between the kinds: the halo kernel keeps its two halo buffers outside the ring, whose stages hold weights
+        // only, and keeps six of them before it takes a second staging buffer; the generic ring holds A + B and needs four
+        // stages, at most two rounds' worth
+        const bool halo = p.kind == CONV_HALO;
         p.mt = 1;
         p.b_res = 0;
         p.b_tx_bytes = (uint32_t)(p.n_tile / 2) * 128u;
         p.b_bytes = (p.b_tx_bytes + 1023u) & ~1023u;
-        if (avail > 2u * tile_stg + 2u * p.halo_bytes + 6u * p.b_bytes + slab_bars(1, 2)) p.stg_bufs = 2;
-        const uint32_t room = avail - (uint32_t)p.stg_bufs * tile_stg - 2u * p.halo_bytes - slab_bars(1, p.stg_bufs);
-        int st = (int)(room / p.b_bytes);
-        p.stages = st > kMaxStages ? kMaxStages : st;
-    }
-    // CTA pairs for generic layers (1x1, stride 2) with wide output tiles and a SHORT reduction: half a weight tile per CTA per
-    // stage.  Measured per op at batch 64 (profiles/r2_pair_generic_per_op.txt): K = cin * taps < 576 gains 5-18 % (the weight
-    // tile is a large share of a short round's operand traffic), K >= 576 loses 1-6 % (the leader's barrier round trip through
-    // the cluster per K step is no longer hidden), so the planner pairs only the short ones.
-    const int k_total = cin * p.taps;
-    // ... and the 3x3 stride-1 layers that run here because their tiles are not 8 pixels wide (288 -> 288 at 20 x 20, two N = 144
-    // tiles): 41.6 -> 35 us each with the pair's halved weight traffic (gpurun_out/r2bg), N / 2 = 72 rows per CTA.
-    const bool pair_short_k = k_total < 576 || (stride == 2 && cin <= 96) || (ksz == 3 && stride == 1);
-    if (p.kind == CONV_GENERIC && p.n_tile >= 128 && p.n_tile % 16 == 0 && p.mt == 1 && (pair_short_k || force_pair) &&
-        (total_tiles >= 2 * sm_count || force_pair) && pair_env != 0) {
-        p.pair = 1;
-        p.b_tx_bytes = (uint32_t)(p.n_tile / 2) * 128u;
-        p.b_bytes = (p.b_tx_bytes + 1023u) & ~1023u;
-        const uint32_t sb = p.a_bytes + p.b_bytes;
-        if (avail > 2u * tile_stg + 4u * sb + slab_bars(1, 2)) p.stg_bufs = 2;
-        const uint32_t room = avail - (uint32_t)p.stg_bufs * tile_stg - slab_bars(1, p.stg_bufs);
+        const uint32_t fixed = halo ? 2u * p.halo_bytes : 0u, sb = halo ? p.b_bytes : p.a_bytes + p.b_bytes, min_st = halo ? 6u : 4u;
+        if (avail > 2u * tile_stg + fixed + min_st * sb + slab_bars(1, 2)) p.stg_bufs = 2;
+        const uint32_t room = avail - (uint32_t)p.stg_bufs * tile_stg - fixed - slab_bars(1, p.stg_bufs);
         int st = (int)(room / sb);
-        const int ksteps = p.taps * p.chunks;
-        if (st > 2 * ksteps) st = 2 * ksteps;
+        if (!halo && st > 2 * p.taps * p.chunks) st = 2 * p.taps * p.chunks;
         p.stages = st > kMaxStages ? kMaxStages : st;
     }
     const uint32_t stg_bytes = (uint32_t)p.stg_bufs * p.mt * tile_stg;
@@ -2696,20 +2414,23 @@ namespace {
 typedef void (*ConvKernel)(const ConvTcParams, int);
 // (kind, act, res, out) -> instantiation; out: 0 16-bit, 1 fp32 (never with a residual), 2 split fp16
 ConvKernel pick_kernel(ConvKind kind, int pair, int act, int res, int out) {
-#define B2D_PICK(K)                                                        \
-    if (out == 1) return act ? K<1, 0, 1> : K<0, 0, 1>;                    \
-    if (out == 2 && res) return act ? K<1, 1, 2> : K<0, 1, 2>;             \
-    if (out == 2) return act ? K<1, 0, 2> : K<0, 0, 2>;                    \
-    if (res) return act ? K<1, 1, 0> : K<0, 1, 0>;                         \
-    return act ? K<1, 0, 0> : K<0, 0, 0>;
-    if (kind == CONV_S2HALO) { B2D_PICK(conv_tc_s2halo_kernel) }
+    // K<act, res, out ...>, the trailing arguments (`, pair`) for the kernels with a CTA-pair form
+#define B2D_PICK(K, ...)                                                                        \
+    if (out == 1) return act ? K<1, 0, 1 __VA_ARGS__> : K<0, 0, 1 __VA_ARGS__>;                 \
+    if (out == 2 && res) return act ? K<1, 1, 2 __VA_ARGS__> : K<0, 1, 2 __VA_ARGS__>;          \
+    if (out == 2) return act ? K<1, 0, 2 __VA_ARGS__> : K<0, 0, 2 __VA_ARGS__>;                 \
+    if (res) return act ? K<1, 1, 0 __VA_ARGS__> : K<0, 1, 0 __VA_ARGS__>;                      \
+    return act ? K<1, 0, 0 __VA_ARGS__> : K<0, 0, 0 __VA_ARGS__>;
+    if (kind == CONV_S2HALO) { B2D_PICK(conv_tc_s2halo_kernel, ) }
     if (kind == CONV_DWPW) return act ? conv_tc_dwpw_kernel<1, 0> : conv_tc_dwpw_kernel<0, 0>;
     if (kind == CONV_STEM) return out == 2 ? (act ? conv_tc_stem2_kernel<1, 2> : conv_tc_stem2_kernel<0, 2>) : (act ? conv_tc_stem2_kernel<1, 0> : conv_tc_stem2_kernel<0, 0>);
     if (kind == CONV_DEPTHWISE) return out == 2 ? (act ? conv_tc_dw_kernel<1, 2> : conv_tc_dw_kernel<0, 2>) : (act ? conv_tc_dw_kernel<1, 0> : conv_tc_dw_kernel<0, 0>);
-    if (kind == CONV_HALO && pair) { B2D_PICK(conv_tc_halo2_kernel) }
-    if (kind == CONV_GENERIC && pair) { B2D_PICK(conv_tc_pair_kernel) }
-    if (kind == CONV_HALO) { B2D_PICK(conv_tc_halo_kernel) }
-    B2D_PICK(conv_tc_kernel)
+    if (kind == CONV_HALO) {
+        if (pair) { B2D_PICK(conv_tc_halo_kernel, , 1) }
+        B2D_PICK(conv_tc_halo_kernel, , 0)
+    }
+    if (pair) { B2D_PICK(conv_tc_kernel, , 1) }
+    B2D_PICK(conv_tc_kernel, , 0)
 #undef B2D_PICK
 }
 }  // namespace
@@ -2724,7 +2445,7 @@ int conv_tc_launch(const ConvTcPlan* plan, int n, cudaStream_t stream) {
     int grid = rounds < plan->sm_count ? rounds : plan->sm_count;
     if (grid < 1) return 0;
     if (p.pair) {
-        const int prs = ceil_div(tiles / p.n_tiles_n, 2) * p.n_tiles_n;      // rounds of a pair (see pair_rounds)
+        const int prs = ceil_div(tiles / p.n_tiles_n, 2) * p.n_tiles_n;      // rounds of a pair (see RoundSched)
         grid = 2 * (prs < plan->sm_count / 2 ? prs : plan->sm_count / 2);
     }
     ConvKernel k = pick_kernel(p.kind, p.pair, p.act, p.has_res, p.out_f32 ? 1 : p.x2 ? 2 : 0);

@@ -108,11 +108,13 @@ def test_every_planned_op_matches_torch(arch, imgsz, n):
 def test_every_planned_op_large_batch_kernel_variants(arch, imgsz, n, monkeypatch):
     """The planner only picks multi-tile rounds (mt = 2 / 4) and CTA pairs when a layer has enough tiles to
     balance 148 SMs, i.e. at bench batch sizes.  Force them (B2D_MT, B2D_PAIR=2 are read at plan time) so the
-    kernels the benchmark runs -- halo-pair, two-tile halo/generic rounds, four-tile stem -- are the ones checked."""
+    kernels the benchmark runs -- the CTA-pair forms of the halo and generic kernels, two-tile halo/generic rounds, four-tile
+    stem -- are the ones checked."""
     monkeypatch.setenv("B2D_MT", "4")
     monkeypatch.setenv("B2D_PAIR", "2")
     seen = _check_every_op(arch, imgsz, n)
-    assert any("halo-pair" in d for d in seen) and any(" x2 " in d for d in seen) and any(" x4 " in d for d in seen), seen[:8]
+    assert any("halo-pair" in d for d in seen) and any("tcgen05-pair conv" in d for d in seen), seen[:8]
+    assert any(" x2 " in d for d in seen) and any(" x4 " in d for d in seen), seen[:8]
 
 
 def test_every_planned_op_matches_torch_split_fp16():
