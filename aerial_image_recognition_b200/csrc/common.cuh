@@ -157,6 +157,13 @@ int candidates_from_rows_launch(const float* rows, int n, int num_rows, int ncol
                                 b2d_det* cand, int* cand_count, int cand_cap, cudaStream_t stream);
 int select_launch(const b2d_det* cand, const int* cand_count, int cand_cap, int n, unsigned long long* keys_scratch,
                   float iou_thr, int top_k, int max_det, b2d_det* out, int* out_count, int cap, cudaStream_t stream);
+// oriented boxes (yolov8m-obb): candidates are b2d_det records plus cand_angle[slot]; prm = 2 float4 per sorted candidate
+int obb_decode_rows_launch(const HeadDesc* h, int n, float* rows, cudaStream_t stream);
+int obb_postprocess_launch(const HeadDesc* h, int n, float thr, int inclusive, float scale, b2d_det* cand, float* cand_angle,
+                           int* cand_count, int cand_cap, unsigned long long* keys_scratch, float4* prm, float iou_thr, int top_k,
+                           int max_det, b2d_obb* out, int* out_count, int cap, cudaStream_t stream);
+int obb_georef_launch(const b2d_obb* dets, const int* counts, int n, int cap, int mode, const double* params, b2d_geoobb* out,
+                      cudaStream_t stream);
 int segment_launch(const float* logits, long long npix, int c, int nc, uint8_t* labels, float* conf, cudaStream_t stream);
 int georef_launch(const b2d_det* dets, const int* counts, int n, int cap, int mode, const double* params,
                   b2d_geodet* out, cudaStream_t stream);

@@ -16,6 +16,9 @@
 #include <utility>
 #include <vector>
 
+static_assert(sizeof(b2d_det) == 32 && sizeof(b2d_geodet) == 40, "record sizes are part of the ABI");
+static_assert(sizeof(b2d_obb) == 36 && sizeof(b2d_geoobb) == 104, "record sizes are part of the ABI");
+
 static thread_local std::string g_last_error;
 
 void b2d_set_error(const char* fmt, ...) {
@@ -108,6 +111,8 @@ struct b2d_engine {
     unsigned long long* keys = nullptr;
     int cand_cap = 0;
     int cand_tiles = 0;
+    float* cand_angle = nullptr;            // oriented-box engines: the angle of each candidate slot, beside `cand`
+    float4* obb_prm = nullptr;              // ... and the rotated NMS's per-candidate Gaussians (2 float4 per key slot)
     void* dedup_scratch = nullptr;
     size_t dedup_scratch_bytes = 0;
     float conf_scale = 1.0f;                // b2d_set_conf_scale: the TTA confidence adjustment (gpu_handler.py:236)
@@ -134,16 +139,23 @@ struct b2d_engine {
 
 namespace {
 
+bool is_obb(const b2d_engine* e) { return e->head_levels > 0 && e->head.kind == B2D_HEAD_V8_OBB; }
+
 int ensure_cand(b2d_engine* e, int n, int rows) {
     int cap = rows < 32768 ? rows : 32768;
     if (e->cand && e->cand_cap >= cap && e->cand_tiles >= n) return 0;
     if (e->cand) { cudaFree(e->cand); cudaFree(e->cand_count); cudaFree(e->keys); }
+    if (e->cand_angle) { cudaFree(e->cand_angle); cudaFree(e->obb_prm); e->cand_angle = nullptr; e->obb_prm = nullptr; }
     int tiles = n > e->max_batch ? n : e->max_batch;
     int stride = 1;
     while (stride < cap) stride <<= 1;
     B2D_CUDA(cudaMalloc(&e->cand, (size_t)tiles * cap * sizeof(b2d_det)));
     B2D_CUDA(cudaMalloc(&e->cand_count, (size_t)tiles * sizeof(int)));
     B2D_CUDA(cudaMalloc(&e->keys, (size_t)tiles * stride * sizeof(unsigned long long)));
+    if (is_obb(e)) {
+        B2D_CUDA(cudaMalloc(&e->cand_angle, (size_t)tiles * cap * sizeof(float)));
+        B2D_CUDA(cudaMalloc(&e->obb_prm, (size_t)tiles * stride * 2 * sizeof(float4)));
+    }
     e->cand_cap = cap;
     e->cand_tiles = tiles;
     return 0;
@@ -361,6 +373,7 @@ void b2d_destroy(b2d_engine* e) {
         if (te.t.tmp) cudaFree(te.t.tmp);
     }
     if (e->cand) { cudaFree(e->cand); cudaFree(e->cand_count); cudaFree(e->keys); }
+    if (e->cand_angle) { cudaFree(e->cand_angle); cudaFree(e->obb_prm); }
     if (e->dedup_scratch) cudaFree(e->dedup_scratch);
     if (e->tta_luts) cudaFree(e->tta_luts);
     if (e->tta_sums) cudaFree(e->tta_sums);
@@ -484,9 +497,11 @@ int b2d_plan_head_level(b2d_engine* e, int kind, int buf, int stride, int nc, co
     HeadLevel& L = e->head.lv[e->head_levels];
     L.buf = (const float*)b.ptr; L.hw = b.h; L.c = b.c; L.stride = stride; L.nc = nc; L.kind = kind;
     for (int i = 0; i < 6; ++i) L.anchors[i] = anchors_px ? anchors_px[i] : 0.f;
+    B2D_CHECK(kind == B2D_HEAD_V8_DFL || kind == B2D_HEAD_V7_ANCHOR || kind == B2D_HEAD_V8_OBB, "plan_head_level: unknown head kind %d", kind);
     const int per = (kind == B2D_HEAD_V7_ANCHOR) ? 3 : 1;
     L.row0 = e->head.rows_total;
-    B2D_CHECK(b.c >= (kind == B2D_HEAD_V7_ANCHOR ? 3 * (nc + 5) : 64 + nc), "plan_head_level: head buffer too narrow");
+    const int need = kind == B2D_HEAD_V7_ANCHOR ? 3 * (nc + 5) : kind == B2D_HEAD_V8_OBB ? (64 + nc + 3) / 4 * 4 + 1 : 64 + nc;
+    B2D_CHECK(b.c >= need, "plan_head_level: head buffer too narrow (%d channels, the head needs %d)", b.c, need);
     e->head.rows_total += per * b.h * b.w;
     e->head.kind = kind; e->head.nc = nc;
     e->head_levels += 1;
@@ -715,6 +730,7 @@ int b2d_set_input_f32(b2d_engine* e, const float* src_dev, int n, void* stream) 
 
 int b2d_decode_rows(b2d_engine* e, int n, float* rows_dev, void* stream) {
     B2D_CHECK(e && e->finalized && e->head_levels > 0, "decode_rows: no head planned");
+    B2D_CHECK(!is_obb(e), "decode_rows: the engine has an oriented-box head; use b2d_decode_rows_obb");
     B2D_ENTER(e);
     B2D_CHECK(n > 0 && n <= e->max_batch && rows_dev, "decode_rows: bad arguments");
     return decode_rows_launch(&e->head, n, rows_dev, (cudaStream_t)stream);
@@ -723,6 +739,7 @@ int b2d_decode_rows(b2d_engine* e, int n, float* rows_dev, void* stream) {
 int b2d_postprocess(b2d_engine* e, int n, float conf_thr, int inclusive, float iou_thr, int top_k, int max_det, b2d_det* dets_dev,
                     int32_t* counts_dev, int cap, void* stream) {
     B2D_CHECK(e && e->finalized && e->head_levels > 0, "postprocess: no head planned");
+    B2D_CHECK(!is_obb(e), "postprocess: the engine has an oriented-box head; use b2d_postprocess_obb");
     B2D_ENTER(e);
     B2D_CHECK(n > 0 && n <= e->max_batch && dets_dev && counts_dev && cap > 0, "postprocess: bad arguments");
     if (ensure_cand(e, n, e->head.rows_total)) return -2;
@@ -734,6 +751,7 @@ int b2d_postprocess(b2d_engine* e, int n, float conf_thr, int inclusive, float i
 int b2d_postprocess_rows(b2d_engine* e, const float* rows_dev, int n, int num_rows, int ncol, float conf_thr, int inclusive,
                          float iou_thr, int top_k, int max_det, b2d_det* dets_dev, int32_t* counts_dev, int cap, void* stream) {
     B2D_CHECK(e && rows_dev && n > 0 && num_rows > 0 && ncol >= 5 && dets_dev && counts_dev && cap > 0, "postprocess_rows: bad arguments");
+    B2D_CHECK(!is_obb(e), "postprocess_rows: the engine has an oriented-box head; axis-aligned rows are not its output");
     B2D_ENTER(e);
     if (ensure_cand(e, n, num_rows)) return -2;
     cudaStream_t s = (cudaStream_t)stream;
@@ -755,7 +773,36 @@ int b2d_georef(b2d_engine* e, const b2d_det* dets_dev, const int32_t* counts_dev
     B2D_CHECK(e && dets_dev && counts_dev && params_dev && out_dev, "georef: bad arguments");
     B2D_ENTER(e);
     B2D_CHECK(mode >= 0 && mode <= 3, "georef: unknown mode %d", mode);
+    B2D_CHECK(!is_obb(e), "georef: the engine has an oriented-box head; use b2d_georef_obb");
     return georef_launch(dets_dev, counts_dev, n, cap, mode, params_dev, out_dev, (cudaStream_t)stream);
+}
+
+int b2d_decode_rows_obb(b2d_engine* e, int n, float* rows_dev, void* stream) {
+    B2D_CHECK(e && e->finalized && e->head_levels > 0, "decode_rows_obb: no head planned");
+    B2D_CHECK(is_obb(e), "decode_rows_obb: the engine has no oriented-box head; use b2d_decode_rows");
+    B2D_ENTER(e);
+    B2D_CHECK(n > 0 && n <= e->max_batch && rows_dev, "decode_rows_obb: bad arguments");
+    return obb_decode_rows_launch(&e->head, n, rows_dev, (cudaStream_t)stream);
+}
+
+int b2d_postprocess_obb(b2d_engine* e, int n, float conf_thr, int inclusive, float iou_thr, int top_k, int max_det, b2d_obb* dets_dev,
+                        int32_t* counts_dev, int cap, void* stream) {
+    B2D_CHECK(e && e->finalized && e->head_levels > 0, "postprocess_obb: no head planned");
+    B2D_CHECK(is_obb(e), "postprocess_obb: the engine has no oriented-box head; use b2d_postprocess");
+    B2D_ENTER(e);
+    B2D_CHECK(n > 0 && n <= e->max_batch && dets_dev && counts_dev && cap > 0, "postprocess_obb: bad arguments");
+    if (ensure_cand(e, n, e->head.rows_total)) return -2;
+    return obb_postprocess_launch(&e->head, n, conf_thr, inclusive, e->conf_scale, e->cand, e->cand_angle, e->cand_count, e->cand_cap, e->keys,
+                                  e->obb_prm, iou_thr, top_k, max_det, dets_dev, counts_dev, cap, (cudaStream_t)stream);
+}
+
+int b2d_georef_obb(b2d_engine* e, const b2d_obb* dets_dev, const int32_t* counts_dev, int n, int cap, int mode, const double* params_dev,
+                   b2d_geoobb* out_dev, void* stream) {
+    B2D_CHECK(e && dets_dev && counts_dev && params_dev && out_dev, "georef_obb: bad arguments");
+    B2D_CHECK(is_obb(e), "georef_obb: the engine has no oriented-box head; use b2d_georef");
+    B2D_CHECK(mode == B2D_GEO_BOUNDS || mode == B2D_GEO_AFFINE, "georef_obb: form %d has no oriented-box variant (bounds and affine do)", mode);
+    B2D_ENTER(e);
+    return obb_georef_launch(dets_dev, counts_dev, n, cap, mode, params_dev, out_dev, (cudaStream_t)stream);
 }
 
 static int ensure_dedup_scratch(b2d_engine* e, int count) {
@@ -861,6 +908,7 @@ int b2d_infer_tiles(b2d_engine* e, const uint8_t* src_dev, int n, int h, int w, 
                     float conf_thr, int inclusive, float iou_thr, int top_k, int max_det, b2d_det* dets_dev, int32_t* counts_dev, int cap,
                     void* stream) {
     B2D_CHECK(e != nullptr, "infer_tiles: null engine");
+    B2D_CHECK(!is_obb(e), "infer_tiles: the engine has an oriented-box head; run b2d_preprocess, b2d_forward, b2d_postprocess_obb");
     B2D_ENTER(e);
     int rc = b2d_preprocess(e, src_dev, n, h, w, pitch, img_stride, mode, bgr, B2D_OUT_BF16_NHWC4, nullptr, stream);
     if (rc) return rc;
@@ -904,6 +952,7 @@ int b2d_detect_host(b2d_engine* e, const uint8_t* tiles_host, int n, int h, int 
                     int32_t* counts_host, int cap, void* stream) {
     B2D_CHECK(e && e->finalized && tiles_host && params_host && out_host && counts_host && n > 0 && h > 0 && w > 0 && cap > 0,
               "detect_host: bad arguments");
+    B2D_CHECK(!is_obb(e), "detect_host: the engine has an oriented-box head; the host path returns axis-aligned records only");
     B2D_ENTER(e);
     cudaStream_t s = (cudaStream_t)stream;
     if (!e->copy_stream) B2D_CUDA(cudaStreamCreateWithFlags(&e->copy_stream, cudaStreamNonBlocking));

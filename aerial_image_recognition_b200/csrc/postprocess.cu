@@ -535,7 +535,322 @@ __global__ void __launch_bounds__(256) georef_kernel(const b2d_det* __restrict__
     out[(size_t)tile * cap + i] = g;
 }
 
+// ---- oriented boxes (yolov8m-obb): Ultralytics >= 8.1 OBB head, rotated NMS, corner georeferencing [EXT] ----------------
+// Decode = OBB.forward + dist2rbox: theta = (sigmoid(z) - 0.25) pi, the DFL half-differences rotated by theta around the anchor.
+// Every step is the restated fp32 arithmetic, one rounding per torch op (__f*_rn: no contraction), precise expf / sincosf.
+constexpr float kPiF = 3.14159265358979f;           // float(math.pi), the scalar of the torch expressions
+constexpr float kHalfPiF = 1.57079632679490f;       // float(math.pi / 2)
+constexpr float kProbEps = 1e-7f;
+
+__device__ __forceinline__ int obb_angle_channel(int nc) { return (64 + nc + 3) / 4 * 4; }   // graph.obb_angle_channel
+
+// MODE 0 = dense rows [n][A][7] (cx, cy, w, h, conf, cls, theta); MODE 1 = thresholded candidates + their angles
+template <int MODE>
+__global__ void __launch_bounds__(256) obb_head_kernel(HeadDesc h, float thr, int inclusive, float scale, float* rows, b2d_det* cand,
+                                                       float* cand_angle, int* cand_count, int cand_cap) {
+    const int tile = blockIdx.y;
+    const int lane = threadIdx.x & 31;
+    const int a = (blockIdx.x * blockDim.x + threadIdx.x) >> 2;        // 4 lanes per anchor, one per box side
+    const int side = threadIdx.x & 3;
+    const bool in_range = a < h.rows_total;
+    int lvl = 0;
+    if (in_range) { while (lvl + 1 < h.nlevels && a >= h.lv[lvl + 1].row0) ++lvl; }
+    const HeadLevel& L = h.lv[lvl];
+    const int cell = in_range ? a - L.row0 : 0;
+    const int gy = cell / L.hw, gx = cell - gy * L.hw;
+    const float* pix = L.buf + ((size_t)tile * L.hw * L.hw + cell) * L.c;
+    float conf = 0.f; int cls = 0;
+    bool want = in_range;
+    if (in_range) {
+        v8_scores(pix, h.nc, &conf, &cls);
+        if (MODE == 1) { conf = __fmul_rn(conf, scale); want = passes(conf, thr, inclusive); }
+    }
+    const unsigned any = __ballot_sync(0xffffffffu, want);
+    if (any == 0) return;
+    float sidev = 0.f;
+    if (want) sidev = dfl_side(pix + side * 16);
+    const unsigned m = 0xffffffffu;
+    const int bl = lane & ~3;
+    const float l = __shfl_sync(m, sidev, bl), t = __shfl_sync(m, sidev, bl + 1), r = __shfl_sync(m, sidev, bl + 2), b = __shfl_sync(m, sidev, bl + 3);
+    if (!want || side != 0) {
+        if (MODE == 0) return;
+    }
+    float cx = 0.f, cy = 0.f, w = 0.f, hh = 0.f, th = 0.f;
+    if (want && side == 0) {
+        th = __fmul_rn(__fsub_rn(sigmoid_f(__ldg(pix + obb_angle_channel(h.nc))), 0.25f), kPiF);
+        float sn, cs;
+        sincosf(th, &sn, &cs);
+        const float xf = __fdiv_rn(__fsub_rn(r, l), 2.0f), yf = __fdiv_rn(__fsub_rn(b, t), 2.0f);
+        const float x = __fsub_rn(__fmul_rn(xf, cs), __fmul_rn(yf, sn));
+        const float y = __fadd_rn(__fmul_rn(xf, sn), __fmul_rn(yf, cs));
+        const float s = (float)L.stride;
+        cx = __fmul_rn(__fadd_rn(x, (float)gx + 0.5f), s);
+        cy = __fmul_rn(__fadd_rn(y, (float)gy + 0.5f), s);
+        w = __fmul_rn(__fadd_rn(l, r), s);
+        hh = __fmul_rn(__fadd_rn(t, b), s);
+    }
+    if (MODE == 0) {
+        float* o = rows + ((size_t)tile * h.rows_total + a) * 7;
+        o[0] = cx; o[1] = cy; o[2] = w; o[3] = hh; o[4] = conf; o[5] = (float)cls; o[6] = th;
+        return;
+    }
+    const bool emit = want && side == 0;
+    const unsigned em = __ballot_sync(0xffffffffu, emit);
+    if (!em) return;
+    int base = 0;
+    const int leader = __ffs(em) - 1;
+    if (lane == leader) base = atomicAdd(&cand_count[tile], __popc(em));
+    base = __shfl_sync(0xffffffffu, base, leader);
+    if (emit) {
+        const int slot = base + __popc(em & ((1u << lane) - 1));
+        if (slot < cand_cap) {
+            b2d_det d;
+            d.cx = cx; d.cy = cy; d.w = w; d.h = hh; d.conf = conf; d.cls = cls; d.tile = tile; d.anchor = a;
+            cand[(size_t)tile * cand_cap + slot] = d;
+            cand_angle[(size_t)tile * cand_cap + slot] = th;
+        }
+    }
+}
+
+// regularize_rboxes: w >= h, theta in [0, pi) -- torch's `%` on floats is fmod with the sign of the divisor
+__device__ __forceinline__ b2d_obb obb_record(const b2d_det& d, float th) {
+    b2d_obb o;
+    o.cx = d.cx; o.cy = d.cy;
+    const bool keep = d.w > d.h;
+    o.w = keep ? d.w : d.h;
+    o.h = keep ? d.h : d.w;
+    const float t = keep ? th : __fadd_rn(th, kHalfPiF);
+    float md = fmodf(t, kPiF);
+    if (md != 0.f && md < 0.f) md = __fadd_rn(md, kPiF);
+    o.theta = md;
+    o.conf = d.conf; o.cls = d.cls; o.tile = d.tile; o.anchor = d.anchor;
+    return o;
+}
+
+// ProbIoU fast NMS, one CTA per tile.  Phase 1 turns every sorted candidate (at most kMaxNms, Ultralytics' max_nms) into its
+// Gaussian once -- class-offset centre, covariance (A, B, C) and P = max(A B - C^2, 0) of the log term -- in global scratch.
+// Phase 2 walks the candidates in blocks of 1024: thread j tests the earlier candidates i < j, staged chunk by chunk through
+// shared memory, and leaves at its first suppressor (fast NMS: a suppressed box still suppresses, so the tests are independent and
+// there is no serial keep scan).  Survivors are compacted in order; the walk stops when max_det are kept.  No pair is skipped.
+constexpr int kObbThreads = 1024;
+constexpr int kMaxNms = 30000;
+
+__device__ __forceinline__ bool probiou_suppresses(const float4 pi, const float2 qi, const float4 pj, const float2 qj, float thr) {
+    // batch_probiou(obb1 = box i, obb2 = box j); p = (x, y, A, B), q = (C, P)
+    const float a12 = __fadd_rn(pi.z, pj.z), b12 = __fadd_rn(pi.w, pj.w), c12 = __fadd_rn(qi.x, qj.x);
+    const float dy = __fsub_rn(pi.y, pj.y), dx = __fsub_rn(pi.x, pj.x);
+    const float den = __fsub_rn(__fmul_rn(a12, b12), __fmul_rn(c12, c12));
+    const float dene = __fadd_rn(den, kProbEps);
+    const float t1 = __fmul_rn(__fdiv_rn(__fadd_rn(__fmul_rn(a12, __fmul_rn(dy, dy)), __fmul_rn(b12, __fmul_rn(dx, dx))), dene), 0.25f);
+    const float t2 = __fmul_rn(__fdiv_rn(__fmul_rn(__fmul_rn(c12, __fsub_rn(pj.x, pi.x)), dy), dene), 0.5f);
+    const float t3 = __fmul_rn(logf(__fadd_rn(__fdiv_rn(den, __fadd_rn(__fmul_rn(4.0f, __fsqrt_rn(__fmul_rn(qi.y, qj.y))), kProbEps)), kProbEps)), 0.5f);
+    const float bd = fminf(fmaxf(__fadd_rn(__fadd_rn(t1, t2), t3), kProbEps), 100.0f);
+    const float hd = __fsqrt_rn(__fadd_rn(__fsub_rn(1.0f, expf(-bd)), kProbEps));
+    const float iou = __fsub_rn(1.0f, hd);
+    return !(iou < thr);            // kept iff every earlier ProbIoU < thr (a NaN suppresses, as torch's max propagates it)
+}
+
+__global__ void __launch_bounds__(kObbThreads) obb_select_kernel(const b2d_det* __restrict__ cand, const float* __restrict__ cand_angle,
+                                                                  const int* __restrict__ cand_count, int cand_cap,
+                                                                  const unsigned long long* __restrict__ keys_scratch, int keys_stride,
+                                                                  float4* __restrict__ prm, float iou_thr, int top_k, int max_det,
+                                                                  b2d_obb* __restrict__ out, int* __restrict__ out_count, int cap) {
+    __shared__ float4 sp[kObbThreads];
+    __shared__ float2 sq[kObbThreads];
+    __shared__ int warp_n[kObbThreads / 32];
+    __shared__ int s_nk;
+    const int tile = blockIdx.x;
+    const int tid = threadIdx.x;
+    int cnt = cand_count[tile];
+    if (cnt > cand_cap) cnt = cand_cap;
+    const b2d_det* tc = cand + (size_t)tile * cand_cap;
+    const float* ta = cand_angle + (size_t)tile * cand_cap;
+    b2d_obb* to = out + (size_t)tile * cap;
+    const unsigned long long* keys = keys_scratch + (size_t)tile * keys_stride;
+    if (!(iou_thr > 0.f)) {
+        int m = cnt;
+        if (top_k > 0 && m > top_k) m = top_k;
+        if (m > cap) m = cap;
+        for (int i = tid; i < m; i += blockDim.x) {
+            const int s = (int)(keys[i] & 0x7FFF);
+            to[i] = obb_record(tc[s], ta[s]);
+        }
+        if (tid == 0) out_count[tile] = m;
+        return;
+    }
+    if (max_det > cap) max_det = cap;
+    const int m = cnt < kMaxNms ? cnt : kMaxNms;
+    float4* tp = prm + (size_t)tile * keys_stride * 2;
+    for (int i = tid; i < m; i += blockDim.x) {
+        const int s = (int)(keys[i] & 0x7FFF);
+        const b2d_det d = tc[s];
+        const float off = __fmul_rn((float)d.cls, 7680.0f);
+        const float a = __fdiv_rn(__fmul_rn(d.w, d.w), 12.0f), b = __fdiv_rn(__fmul_rn(d.h, d.h), 12.0f);
+        float sn, cs;
+        sincosf(ta[s], &sn, &cs);
+        const float c2 = __fmul_rn(cs, cs), s2 = __fmul_rn(sn, sn);
+        const float A = __fadd_rn(__fmul_rn(a, c2), __fmul_rn(b, s2));
+        const float B = __fadd_rn(__fmul_rn(a, s2), __fmul_rn(b, c2));
+        const float Cc = __fmul_rn(__fmul_rn(__fsub_rn(a, b), cs), sn);
+        const float P = fmaxf(__fsub_rn(__fmul_rn(A, B), __fmul_rn(Cc, Cc)), 0.f);
+        tp[2 * i] = make_float4(__fadd_rn(d.cx, off), __fadd_rn(d.cy, off), A, B);
+        tp[2 * i + 1] = make_float4(Cc, P, 0.f, 0.f);
+    }
+    if (tid == 0) s_nk = 0;
+    __syncthreads();
+    for (int jb = 0; jb < m; jb += kObbThreads) {
+        const int j = jb + tid;
+        bool alive = j < m;
+        float4 pj = make_float4(0.f, 0.f, 0.f, 0.f);
+        float2 qj = make_float2(0.f, 0.f);
+        if (alive) {
+            pj = tp[2 * j];
+            const float4 q = tp[2 * j + 1];
+            qj = make_float2(q.x, q.y);
+        }
+        for (int ib = 0; ib <= jb; ib += kObbThreads) {
+            if (!__syncthreads_or(alive)) break;            // every box of the block already suppressed
+            const int i = ib + tid;
+            if (i < m) {
+                sp[tid] = tp[2 * i];
+                const float4 q = tp[2 * i + 1];
+                sq[tid] = make_float2(q.x, q.y);
+            }
+            __syncthreads();
+            if (alive) {
+                const int end = min(kObbThreads, j - ib);   // i < j
+                for (int k = 0; k < end; ++k)
+                    if (probiou_suppresses(sp[k], sq[k], pj, qj, iou_thr)) { alive = false; break; }
+            }
+        }
+        // compact the survivors of this block in order
+        const unsigned bal = __ballot_sync(0xffffffffu, alive);
+        if ((tid & 31) == 0) warp_n[tid >> 5] = __popc(bal);
+        __syncthreads();
+        const int nk = s_nk;
+        int before = 0, total = 0;
+        for (int w = 0; w < kObbThreads / 32; ++w) {
+            const int c = warp_n[w];
+            before += (w < (tid >> 5)) ? c : 0;
+            total += c;
+        }
+        if (alive) {
+            const int slot = nk + before + __popc(bal & ((1u << (tid & 31)) - 1));
+            if (slot < max_det) {
+                const int s = (int)(keys[j] & 0x7FFF);
+                to[slot] = obb_record(tc[s], ta[s]);
+            }
+        }
+        __syncthreads();
+        if (tid == 0) s_nk = min(nk + total, max_det);
+        __syncthreads();
+        if (s_nk >= max_det) break;
+    }
+    if (tid == 0) out_count[tile] = s_nk;
+}
+
+// xywhr2xyxyxyxy in fp32: v1 = (w/2 cos, w/2 sin), v2 = (-h/2 sin, h/2 cos); corners c+v1+v2, c+v1-v2, c-v1-v2, c-v1+v2
+__device__ __forceinline__ void obb_corners(float cx, float cy, float w, float h, float th, float* px, float* py) {
+    const float sn = sinf(th), cs = cosf(th);
+    const float w2 = __fdiv_rn(w, 2.0f), h2 = __fdiv_rn(-h, 2.0f), h2p = __fdiv_rn(h, 2.0f);
+    const float v1x = __fmul_rn(w2, cs), v1y = __fmul_rn(w2, sn);
+    const float v2x = __fmul_rn(h2, sn), v2y = __fmul_rn(h2p, cs);
+    px[0] = __fadd_rn(__fadd_rn(cx, v1x), v2x); py[0] = __fadd_rn(__fadd_rn(cy, v1y), v2y);
+    px[1] = __fsub_rn(__fadd_rn(cx, v1x), v2x); py[1] = __fsub_rn(__fadd_rn(cy, v1y), v2y);
+    px[2] = __fsub_rn(__fsub_rn(cx, v1x), v2x); py[2] = __fsub_rn(__fsub_rn(cy, v1y), v2y);
+    px[3] = __fadd_rn(__fsub_rn(cx, v1x), v2x); py[3] = __fadd_rn(__fsub_rn(cy, v1y), v2y);
+}
+
+__global__ void __launch_bounds__(256) obb_georef_kernel(const b2d_obb* __restrict__ dets, const int* __restrict__ counts, int cap, int mode,
+                                                          const double* __restrict__ params, b2d_geoobb* __restrict__ out) {
+    const int tile = blockIdx.y;
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= counts[tile] || i >= cap) return;
+    const b2d_obb d = dets[(size_t)tile * cap + i];
+    const double* P = params + (size_t)tile * B2D_GEO_PARAMS;
+    b2d_geoobb g;
+    g.conf = d.conf; g.theta = d.theta; g.cls = d.cls; g.tile = tile;
+    float px[5], py[5];
+    if (mode == B2D_GEO_BOUNDS) {
+        // simple_detector.py:487-494 applied to the centre and to each corner; w, h scaled like x_img (model -> crop pixels)
+        obb_corners(d.cx, d.cy, d.w, d.h, d.theta, px, py);
+        px[4] = d.cx; py[4] = d.cy;
+        const double ms = P[5] > 0.0 ? P[5] : 640.0;
+        g.w = (float)__dmul_rn(__ddiv_rn((double)d.w, ms), P[4]);
+        g.h = (float)__dmul_rn(__ddiv_rn((double)d.h, ms), P[4]);
+        double gx[5], gy[5];
+#pragma unroll
+        for (int k = 0; k < 5; ++k) {
+            const double xf = __ddiv_rn((double)px[k], ms), yf = __ddiv_rn((double)py[k], ms);
+            gx[k] = __dadd_rn(P[0], __dmul_rn(xf, __dsub_rn(P[1], P[0])));
+            gy[k] = __dsub_rn(P[3], __dmul_rn(yf, __dsub_rn(P[3], P[2])));
+        }
+        g.x = gx[4]; g.y = gy[4];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) { g.corners[2 * k] = gx[k]; g.corners[2 * k + 1] = gy[k]; }
+    } else {
+        // affine: undo the letterbox in fp32 (centre - pad, / gain; w, h / gain; no clipping), corners in fp32, then the window
+        // offset and the 6-term geotransform in fp64.  P = gt[0..5], win_x, win_y, pad_x, pad_y, gain
+        const float padx = (float)P[8], pady = (float)P[9], gain = (float)P[10];
+        const float cx = __fdiv_rn(__fsub_rn(d.cx, padx), gain), cy = __fdiv_rn(__fsub_rn(d.cy, pady), gain);
+        g.w = __fdiv_rn(d.w, gain);
+        g.h = __fdiv_rn(d.h, gain);
+        obb_corners(cx, cy, g.w, g.h, d.theta, px, py);
+        px[4] = cx; py[4] = cy;
+        double gx[5], gy[5];
+#pragma unroll
+        for (int k = 0; k < 5; ++k) {
+            const double X = __dadd_rn((double)px[k], P[6]), Y = __dadd_rn((double)py[k], P[7]);
+            gx[k] = __dadd_rn(__dadd_rn(P[0], __dmul_rn(X, P[1])), __dmul_rn(Y, P[2]));
+            gy[k] = __dadd_rn(__dadd_rn(P[3], __dmul_rn(X, P[4])), __dmul_rn(Y, P[5]));
+        }
+        g.x = gx[4]; g.y = gy[4];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) { g.corners[2 * k] = gx[k]; g.corners[2 * k + 1] = gy[k]; }
+    }
+    out[(size_t)tile * cap + i] = g;
+}
+
 }  // namespace
+
+int obb_decode_rows_launch(const HeadDesc* h, int n, float* rows, cudaStream_t stream) {
+    if (n <= 0) return 0;
+    dim3 grid(ceil_div(h->rows_total * 4, 256), n);
+    obb_head_kernel<0><<<grid, 256, 0, stream>>>(*h, 0.f, 1, 1.f, rows, nullptr, nullptr, nullptr, 0);
+    B2D_LAUNCH_CHECK();
+    return 0;
+}
+
+int obb_postprocess_launch(const HeadDesc* h, int n, float thr, int inclusive, float scale, b2d_det* cand, float* cand_angle,
+                           int* cand_count, int cand_cap, unsigned long long* keys_scratch, float4* prm, float iou_thr, int top_k,
+                           int max_det, b2d_obb* out, int* out_count, int cap, cudaStream_t stream) {
+    if (n <= 0) return 0;
+    B2D_CHECK(cand_cap <= 32768, "postprocess_obb: candidate capacity %d exceeds the 15-bit slot field", cand_cap);
+    B2D_CUDA(cudaMemsetAsync(cand_count, 0, sizeof(int) * n, stream));
+    dim3 grid(ceil_div(h->rows_total * 4, 256), n);
+    obb_head_kernel<1><<<grid, 256, 0, stream>>>(*h, thr, inclusive, scale, nullptr, cand, cand_angle, cand_count, cand_cap);
+    B2D_LAUNCH_CHECK();
+    int stride = 1;
+    while (stride < cand_cap) stride <<= 1;
+    if (b2d_func_smem_optin((const void*)sort_keys_kernel, kSortSmemKeys * 8)) return -2;
+    int need = 1;
+    while (need < cand_cap && need < kSortSmemKeys) need <<= 1;
+    sort_keys_kernel<<<n, kSortThreads, (size_t)need * 8, stream>>>(cand, cand_count, cand_cap, keys_scratch, stride, (iou_thr > 0.f) || (top_k > 0));
+    B2D_LAUNCH_CHECK();
+    obb_select_kernel<<<n, kObbThreads, 0, stream>>>(cand, cand_angle, cand_count, cand_cap, keys_scratch, stride, prm, iou_thr, top_k, max_det,
+                                                     out, out_count, cap);
+    B2D_LAUNCH_CHECK();
+    return 0;
+}
+
+int obb_georef_launch(const b2d_obb* dets, const int* counts, int n, int cap, int mode, const double* params, b2d_geoobb* out,
+                      cudaStream_t stream) {
+    if (n <= 0 || cap <= 0) return 0;
+    dim3 grid(ceil_div(cap, 256), n);
+    obb_georef_kernel<<<grid, 256, 0, stream>>>(dets, counts, cap, mode, params, out);
+    B2D_LAUNCH_CHECK();
+    return 0;
+}
 
 int decode_rows_launch(const HeadDesc* h, int n, float* rows, cudaStream_t stream) {
     if (n <= 0) return 0;

@@ -32,6 +32,15 @@ GEODET_DTYPE = np.dtype([("x", "<f8"), ("y", "<f8"), ("conf", "<f4"), ("x_img", 
 DET_DTYPE = np.dtype([("cx", "<f4"), ("cy", "<f4"), ("w", "<f4"), ("h", "<f4"), ("conf", "<f4"),
                       ("cls", "<i4"), ("tile", "<i4"), ("anchor", "<i4")])
 assert GEODET_DTYPE.itemsize == GEODET_BYTES and DET_DTYPE.itemsize == 4 * DET_WORDS
+# oriented boxes (arch "yolov8m-obb"): b2d_obb / b2d_geoobb
+OBB_WORDS = 9
+GEOOBB_BYTES = 104
+OBB_DTYPE = np.dtype([("cx", "<f4"), ("cy", "<f4"), ("w", "<f4"), ("h", "<f4"), ("theta", "<f4"), ("conf", "<f4"),
+                      ("cls", "<i4"), ("tile", "<i4"), ("anchor", "<i4")])
+GEOOBB_DTYPE = np.dtype([("x", "<f8"), ("y", "<f8"), ("corners", "<f8", (4, 2)), ("conf", "<f4"), ("w", "<f4"), ("h", "<f4"),
+                         ("theta", "<f4"), ("cls", "<i4"), ("tile", "<i4")])
+assert OBB_DTYPE.itemsize == 4 * OBB_WORDS and GEOOBB_DTYPE.itemsize == GEOOBB_BYTES
+HEAD_KIND = {"v8_dfl": 0, "v7_anchor": 1, "v8_obb": 2}
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -53,6 +62,7 @@ class Engine:
         torch.cuda.set_device(self.device)
         self.graph = graph if graph is not None else build(arch, nc, imgsz)
         self.arch = self.graph.arch
+        self.is_obb = self.graph.head.get("kind") == "v8_obb"     # oriented boxes: the *_obb entry points, OBB_DTYPE records
         self.imgsz = self.graph.imgsz
         self.max_batch = int(max_batch)
         self.weights_seed = seed if weights is None else None
@@ -101,7 +111,7 @@ class Engine:
             else:
                 raise ValueError(op.kind)
             self.op_names.append(op.tag or op.weight)
-        kind = 0 if g.head["kind"] == "v8_dfl" else 1            # "seg" (config C5) has no detection levels: see segment()
+        kind = HEAD_KIND.get(g.head["kind"], -1)                 # "seg" (config C5) has no detection levels: see segment()
         for lv in g.head["levels"]:
             anc = None
             if "anchors" in lv:
@@ -201,6 +211,12 @@ class Engine:
         return (labels, conf) if with_conf else labels
 
     def decode_rows(self, n: int) -> torch.Tensor:
+        """Dense rows [n, A, 6] (cx, cy, w, h, conf, cls); on an oriented-box engine [n, A, 7] with theta (radians, not
+        regularized) as the last column."""
+        if self.is_obb:
+            rows = torch.empty((n, self.num_rows, 7), dtype=torch.float32, device=self.device)
+            _lib.check(self.lib.b2d_decode_rows_obb(self.h, n, _ptr(rows), self.stream), "decode_rows_obb")
+            return rows
         rows = torch.empty((n, self.num_rows, 6), dtype=torch.float32, device=self.device)
         _lib.check(self.lib.b2d_decode_rows(self.h, n, _ptr(rows), self.stream), "decode_rows")
         return rows
@@ -208,9 +224,18 @@ class Engine:
     def postprocess(self, n: int, conf_thr: float = 0.3, inclusive: bool = True, iou_thr: float = 0.0, top_k: int = 0,
                     max_det: int = 300, cap: Optional[int] = None, rows: Optional[torch.Tensor] = None
                     ) -> Tuple[torch.Tensor, torch.Tensor]:
-        """Returns (dets float32 [n, cap, 8] -- view ints with .view(torch.int32) --, counts int32 [n])."""
+        """Returns (dets float32 [n, cap, 8] -- view ints with .view(torch.int32) --, counts int32 [n]).  On an oriented-box engine
+        dets is [n, cap, 9] ``OBB_DTYPE`` records (regularized boxes after Ultralytics' rotated NMS when iou_thr > 0)."""
         if cap is None:
             cap = max_det if iou_thr > 0 else (top_k if top_k > 0 else min(self.num_rows if rows is None else rows.shape[1], 32768))
+        if self.is_obb:
+            if rows is not None:
+                raise ValueError("postprocess(rows=...) takes axis-aligned rows; an oriented-box engine post-processes its own head maps")
+            dets = torch.empty((n, cap, OBB_WORDS), dtype=torch.float32, device=self.device)
+            counts = torch.empty((n,), dtype=torch.int32, device=self.device)
+            _lib.check(self.lib.b2d_postprocess_obb(self.h, n, conf_thr, int(inclusive), iou_thr, top_k, max_det, _ptr(dets),
+                                                    _ptr(counts), cap, self.stream), "postprocess_obb")
+            return dets, counts
         dets = torch.empty((n, cap, DET_WORDS), dtype=torch.float32, device=self.device)
         counts = torch.empty((n,), dtype=torch.int32, device=self.device)
         if rows is None:
@@ -225,9 +250,15 @@ class Engine:
         return dets, counts
 
     def georef(self, dets: torch.Tensor, counts: torch.Tensor, params: torch.Tensor, mode: str = "bounds") -> torch.Tensor:
-        """params: float64 CUDA [n, 16].  Returns uint8 [n, cap, 40] (``GEODET_DTYPE`` records)."""
+        """params: float64 CUDA [n, 16].  Returns uint8 [n, cap, 40] (``GEODET_DTYPE`` records); on an oriented-box engine uint8
+        [n, cap, 104] (``GEOOBB_DTYPE``: centre and four corners), forms "bounds" and "affine" only."""
         n, cap = dets.shape[0], dets.shape[1]
         assert params.dtype == torch.float64 and tuple(params.shape) == (n, GEO_PARAMS) and params.is_cuda
+        if self.is_obb:
+            out = torch.zeros((n, cap, GEOOBB_BYTES), dtype=torch.uint8, device=self.device)
+            _lib.check(self.lib.b2d_georef_obb(self.h, _ptr(dets), _ptr(counts), n, cap, GEO[mode], _ptr(params.contiguous()), _ptr(out),
+                                               self.stream), "georef_obb")
+            return out
         out = torch.zeros((n, cap, GEODET_BYTES), dtype=torch.uint8, device=self.device)
         _lib.check(self.lib.b2d_georef(self.h, _ptr(dets), _ptr(counts), n, cap, GEO[mode], _ptr(params.contiguous()), _ptr(out),
                                        self.stream), "georef")
@@ -347,6 +378,8 @@ class Engine:
                     iou_thr: float = 0.0, top_k: int = 0, max_det: int = 300, cap: Optional[int] = None, geo: str = "bounds"):
         """Host tiles in, host records out, in ONE C call (``b2d_detect_host``): ``tiles`` uint8 [n,h,w,3] (NumPy array or CPU
         tensor; any n, pinned memory overlaps the copies), ``params`` float64 [n,16].  Returns one ``GEODET_DTYPE`` array per tile."""
+        if self.is_obb:
+            raise _lib.B2DError("detect_host returns axis-aligned records; on an oriented-box engine use infer() + georef()")
         t = _host_array(tiles, np.uint8)
         p = _host_array(params, np.float64)
         n, h, w, _ = t.shape
@@ -378,6 +411,14 @@ class Engine:
             self.set_conf_scale(1.0)
 
 
+def require_axis_aligned(engine, who: str) -> None:
+    """The front-ends that mirror the reference (GPUHandler and its test-time augmentation, SimpleDetector, InferenceSession,
+    MosaicDetector) return axis-aligned records; built on an oriented-box engine they stop here instead of misreading its output."""
+    if getattr(engine, "is_obb", False):
+        raise ValueError(f"{who} handles axis-aligned detections only; {engine.arch!r} is an oriented-box model: "
+                         "use Engine.infer / Engine.postprocess and Engine.georef, which return OBB_DTYPE / GEOOBB_DTYPE records")
+
+
 def _host_array(x, dtype) -> np.ndarray:
     a = x.numpy() if isinstance(x, torch.Tensor) else np.asarray(x)
     assert a.dtype == dtype
@@ -393,5 +434,18 @@ def dets_to_numpy(dets: torch.Tensor, counts: torch.Tensor):
 
 def geodets_to_numpy(geo: torch.Tensor, counts: torch.Tensor):
     g = geo.cpu().numpy().view(GEODET_DTYPE)[..., 0]
+    c = counts.cpu().numpy()
+    return [g[i, :c[i]].copy() for i in range(len(c))]
+
+
+def obbs_to_numpy(dets: torch.Tensor, counts: torch.Tensor):
+    """Device (dets, counts) of an oriented-box engine -> list of structured arrays (``OBB_DTYPE``), one per tile."""
+    d = dets.cpu().numpy().view(np.uint8).reshape(dets.shape[0], dets.shape[1], 4 * OBB_WORDS).view(OBB_DTYPE)[..., 0]
+    c = counts.cpu().numpy()
+    return [d[i, :c[i]].copy() for i in range(len(c))]
+
+
+def geoobbs_to_numpy(geo: torch.Tensor, counts: torch.Tensor):
+    g = geo.cpu().numpy().view(GEOOBB_DTYPE)[..., 0]
     c = counts.cpu().numpy()
     return [g[i, :c[i]].copy() for i in range(len(c))]

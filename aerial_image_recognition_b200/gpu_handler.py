@@ -23,7 +23,7 @@ import numpy as np
 import torch
 
 from . import tta as _tta
-from .engine import GEO_PARAMS, GEODET_BYTES, GEODET_DTYPE, Engine, geodets_to_numpy
+from .engine import GEO_PARAMS, GEODET_BYTES, GEODET_DTYPE, Engine, geodets_to_numpy, require_axis_aligned
 from .session import InferenceSession, arch_from_model_path, resolve_weights
 
 
@@ -70,6 +70,7 @@ class TileStager:
     the event of the copy that last read it, so the host fills batch i+1 while batch i is in flight."""
 
     def __init__(self, engine):
+        require_axis_aligned(engine, "TileStager")
         self.engine = engine
         self._stage = {}            # (h, w, channels) -> two pinned uint8 [max_batch, h, w, channels] buffers
         self._free = {}             # same key -> the events after which they may be overwritten

@@ -7,11 +7,13 @@ The reference never builds a graph itself: it hands an ``.onnx`` file to
 to be stated somewhere; this module states it as data that the C-ABI plan
 builder (``engine.py`` -> ``b2d_plan_*``) consumes one op at a time.
 
-Three architectures are described:
+Four architectures are described:
 
 * ``yolov8m`` with ``nc=2`` and the Ultralytics 8.3.x depthwise cls branch -- the
   "tokyo" checkpoint, recovered from the training log in
   ``x_arch/01_train_tokyo.ipynb:1 (cell 15 output)`` (SURVEY.md Appendix A.1).
+* ``yolov8m-obb`` -- the same backbone and neck with Ultralytics' oriented-box head (``build_yolov8m_obb``), the family of
+  the published overhead-imagery (DOTAv1) checkpoints.
 * ``yolov7`` canonical deploy graph -- the stand-in for the missing ITCVD
   model named at ``_script/config.py:25`` (SURVEY.md Appendix A.4).
 
@@ -127,7 +129,7 @@ class Graph:
         n = 0
         for cout, cing, k, g in self.wshapes.values():
             n += cout * cing * k * k + cout
-        return n + (16 if self.arch == "yolov8m" else 0)  # + the DFL arange conv
+        return n + (16 if self.arch in ("yolov8m", "yolov8m-obb") else 0)  # + the DFL arange conv
 
 
 def op_weights(op: Op, w) -> Tuple:
@@ -173,8 +175,82 @@ def _c2f(g: Graph, name, src: Ref, dst: Ref, n, shortcut, hw, order=None):
 
 def build_yolov8m(nc: int = 2, imgsz: int = 640) -> Graph:
     """YOLOv8m, Ultralytics 8.3.4 head (SURVEY.md Appendix A.1)."""
+    g, feats = _yolov8m_body("yolov8m", nc, imgsz)
+    # Detect head (8.3.x: box branch dense, cls branch depthwise-separable)
+    levels = []
+    c2, c3 = 64, 192
+    for i, (feat, ch, hw, stride) in enumerate(feats):
+        # box 64 | cls nc | padding up to a multiple of 32 fp32 channels: a pixel is then a whole number of 128-byte lines and the box
+        # branch's 256-byte rows start on a line (with 68 channels = 272 bytes every store straddled three lines: cv2.0.2 50 -> 35 us)
+        hc = ((64 + nc + 31) // 32) * 32
+        out = g.buf(f"head{i}", hw, hw, hc, f32=True)
+        _v8_box_branch(g, i, feat, ch, hw, out)
+        d0 = g.buf(f"h{i}.d0", hw, hw, ch)
+        e0 = g.buf(f"h{i}.e0", hw, hw, c3)
+        d1 = g.buf(f"h{i}.d1", hw, hw, c3)
+        e1 = g.buf(f"h{i}.e1", hw, hw, c3)
+        g.conv(f"model.22.cv3.{i}.0.0", Ref(feat, 0, ch), Ref(d0, 0, ch), 3, 1, groups=ch)
+        g.conv(f"model.22.cv3.{i}.0.1", Ref(d0, 0, ch), Ref(e0, 0, c3), 1, 1)
+        g.conv(f"model.22.cv3.{i}.1.0", Ref(e0, 0, c3), Ref(d1, 0, c3), 3, 1, groups=c3)
+        g.conv(f"model.22.cv3.{i}.1.1", Ref(d1, 0, c3), Ref(e1, 0, c3), 1, 1)
+        g.conv(f"model.22.cv3.{i}.2", Ref(e1, 0, c3), Ref(out, 64, nc), 1, 1, act=ACT_NONE)
+        levels.append({"buf": out, "hw": hw, "stride": stride, "c": hc})
+    g.head = {"kind": "v8_dfl", "levels": levels, "reg_max": 16, "nc": nc,
+              "anchors_total": sum(l["hw"] ** 2 for l in levels)}
+    return g
+
+
+def obb_angle_channel(nc: int) -> int:
+    """Channel of the angle logit in a ``yolov8m-obb`` head map: the first 16-byte-aligned fp32 channel after box 64 | cls nc
+    (a conv writes its output slice through a tensor map whose base must be 16-byte aligned).  The C library places it the same way."""
+    return (64 + nc + 3) // 4 * 4
+
+
+def build_yolov8m_obb(nc: int = 15, imgsz: int = 640) -> Graph:
+    """YOLOv8m-OBB, the oriented-box head of Ultralytics >= 8.1 [EXT] on the YOLOv8m backbone and neck (identical to
+    ``build_yolov8m`` up to model.21).  Per level: the box branch cv2 as in v8, a dense cls branch cv3 (Conv 3x3, Conv 3x3,
+    Conv2d 1x1 with c3 = max(192, min(nc, 100)) channels, as in the published v8 OBB checkpoints) and an angle branch cv4 (Conv 3x3,
+    Conv 3x3, Conv2d 1x1 -> 1 with 48 = max(192 // 4, 1) channels).  The head map of a level is fp32 [box 64 | cls nc | pad | angle | pad]
+    (angle at ``obb_angle_channel(nc)``, width a multiple of 32 channels).  Ultralytics' ``OBB.forward`` runs cv4 over all three
+    levels before ``Detect.forward`` runs cv2 / cv3, and the ops are listed in that order (the ONNX reader maps by order)."""
+    g, feats = _yolov8m_body("yolov8m-obb", nc, imgsz)
+    c3, c4 = max(192, min(nc, 100)), 48
+    ac = obb_angle_channel(nc)
+    hc = ((ac + 1 + 31) // 32) * 32
+    outs = [g.buf(f"head{i}", hw, hw, hc, f32=True) for i, (_, _, hw, _) in enumerate(feats)]
+    for i, (feat, ch, hw, _) in enumerate(feats):
+        a = g.buf(f"h{i}.a0", hw, hw, c4)
+        b = g.buf(f"h{i}.a1", hw, hw, c4)
+        g.conv(f"model.22.cv4.{i}.0", Ref(feat, 0, ch), Ref(a, 0, c4), 3, 1)
+        g.conv(f"model.22.cv4.{i}.1", Ref(a, 0, c4), Ref(b, 0, c4), 3, 1)
+        g.conv(f"model.22.cv4.{i}.2", Ref(b, 0, c4), Ref(outs[i], ac, 1), 1, 1, act=ACT_NONE)
+    levels = []
+    for i, (feat, ch, hw, stride) in enumerate(feats):
+        _v8_box_branch(g, i, feat, ch, hw, outs[i])
+        a = g.buf(f"h{i}.c0", hw, hw, c3)
+        b = g.buf(f"h{i}.c1", hw, hw, c3)
+        g.conv(f"model.22.cv3.{i}.0", Ref(feat, 0, ch), Ref(a, 0, c3), 3, 1)
+        g.conv(f"model.22.cv3.{i}.1", Ref(a, 0, c3), Ref(b, 0, c3), 3, 1)
+        g.conv(f"model.22.cv3.{i}.2", Ref(b, 0, c3), Ref(outs[i], 64, nc), 1, 1, act=ACT_NONE)
+        levels.append({"buf": outs[i], "hw": hw, "stride": stride, "c": hc})
+    g.head = {"kind": "v8_obb", "levels": levels, "reg_max": 16, "nc": nc, "angle_c": ac,
+              "anchors_total": sum(l["hw"] ** 2 for l in levels)}
+    return g
+
+
+def _v8_box_branch(g: Graph, i: int, feat: str, ch: int, hw: int, out: str) -> None:
+    c2 = 64
+    a = g.buf(f"h{i}.b0", hw, hw, c2)
+    b = g.buf(f"h{i}.b1", hw, hw, c2)
+    g.conv(f"model.22.cv2.{i}.0", Ref(feat, 0, ch), Ref(a, 0, c2), 3, 1)
+    g.conv(f"model.22.cv2.{i}.1", Ref(a, 0, c2), Ref(b, 0, c2), 3, 1)
+    g.conv(f"model.22.cv2.{i}.2", Ref(b, 0, c2), Ref(out, 0, 64), 1, 1, act=ACT_NONE)
+
+
+def _yolov8m_body(arch: str, nc: int, imgsz: int):
+    """YOLOv8m backbone and neck (model.0 - model.21); returns the graph and (buffer, channels, size, stride) of P3, P4, P5."""
     assert imgsz % 32 == 0
-    g = Graph("yolov8m", nc, imgsz)
+    g = Graph(arch, nc, imgsz)
     s1, s2, s3, s4, s5 = (imgsz // 2, imgsz // 4, imgsz // 8, imgsz // 16, imgsz // 32)
     g.buf("input", imgsz, imgsz, 4)
     # concat buffers of the FPN/PAN, allocated up front so producers can target them
@@ -221,33 +297,7 @@ def build_yolov8m(nc: int = 2, imgsz: int = 640) -> Graph:
     g.conv("model.19", Ref(x18, 0, 384), Ref(cat20, 0, 384), 3, 2)
     x21 = g.buf("x21", s5, s5, 576)                         # P5 out
     _c2f(g, "model.21", Ref(cat20, 0, 960), Ref(x21, 0, 576), 2, False, s5)
-
-    # Detect head (8.3.x: box branch dense, cls branch depthwise-separable)
-    levels = []
-    c2, c3 = 64, 192
-    for i, (feat, ch, hw, stride) in enumerate(((x15, 192, s3, 8), (x18, 384, s4, 16), (x21, 576, s5, 32))):
-        # box 64 | cls nc | padding up to a multiple of 32 fp32 channels: a pixel is then a whole number of 128-byte lines and the box
-        # branch's 256-byte rows start on a line (with 68 channels = 272 bytes every store straddled three lines: cv2.0.2 50 -> 35 us)
-        hc = ((64 + nc + 31) // 32) * 32
-        out = g.buf(f"head{i}", hw, hw, hc, f32=True)
-        a = g.buf(f"h{i}.b0", hw, hw, c2)
-        b = g.buf(f"h{i}.b1", hw, hw, c2)
-        g.conv(f"model.22.cv2.{i}.0", Ref(feat, 0, ch), Ref(a, 0, c2), 3, 1)
-        g.conv(f"model.22.cv2.{i}.1", Ref(a, 0, c2), Ref(b, 0, c2), 3, 1)
-        g.conv(f"model.22.cv2.{i}.2", Ref(b, 0, c2), Ref(out, 0, 64), 1, 1, act=ACT_NONE)
-        d0 = g.buf(f"h{i}.d0", hw, hw, ch)
-        e0 = g.buf(f"h{i}.e0", hw, hw, c3)
-        d1 = g.buf(f"h{i}.d1", hw, hw, c3)
-        e1 = g.buf(f"h{i}.e1", hw, hw, c3)
-        g.conv(f"model.22.cv3.{i}.0.0", Ref(feat, 0, ch), Ref(d0, 0, ch), 3, 1, groups=ch)
-        g.conv(f"model.22.cv3.{i}.0.1", Ref(d0, 0, ch), Ref(e0, 0, c3), 1, 1)
-        g.conv(f"model.22.cv3.{i}.1.0", Ref(e0, 0, c3), Ref(d1, 0, c3), 3, 1, groups=c3)
-        g.conv(f"model.22.cv3.{i}.1.1", Ref(d1, 0, c3), Ref(e1, 0, c3), 1, 1)
-        g.conv(f"model.22.cv3.{i}.2", Ref(e1, 0, c3), Ref(out, 64, nc), 1, 1, act=ACT_NONE)
-        levels.append({"buf": out, "hw": hw, "stride": stride, "c": hc})
-    g.head = {"kind": "v8_dfl", "levels": levels, "reg_max": 16, "nc": nc,
-              "anchors_total": sum(l["hw"] ** 2 for l in levels)}
-    return g
+    return g, ((x15, 192, s3, 8), (x18, 384, s4, 16), (x21, 576, s5, 32))
 
 
 # ---------------------------------------------------------------------------------
@@ -475,6 +525,8 @@ def build_xunet(nc: int = 4, imgsz: int = 256) -> Graph:
 def build(arch: str, nc: Optional[int] = None, imgsz: int = 640) -> Graph:
     if arch in ("yolov8m", "v8", "yolov8m_tokyo"):
         return build_yolov8m(2 if nc is None else nc, imgsz)
+    if arch in ("yolov8m-obb", "yolov8m_obb"):
+        return build_yolov8m_obb(15 if nc is None else nc, imgsz)
     if arch in ("yolov7", "v7", "yolov7_itcvd"):
         return build_yolov7(1 if nc is None else nc, imgsz)
     if arch in ("xunet", "ramp_xunet"):

@@ -152,6 +152,8 @@ class MosaicDetector:
 
     def __init__(self, engine, geotransform: Sequence[float], win: int = 640, stride: int = 512, conf: float = 0.4,
                  nms_conf: float = 0.25, iou: float = 0.7, max_det: int = 300, dedup_thr: float = 1.0, fill: int = 114):
+        from .engine import require_axis_aligned
+        require_axis_aligned(engine, "MosaicDetector")
         self.eng = engine
         self.gt = tuple(float(v) for v in geotransform)
         self.win, self.stride = win, stride

@@ -242,7 +242,12 @@ def load_onnx_weights(path: str, g: Graph, by_name: bool = True) -> Dict[str, np
             continue
         convs.append((nd, wt, inits.get(nd.inputs[2]) if len(nd.inputs) > 2 else None))
     if len(convs) != len(names):
-        raise ValueError(f"{path}: {len(convs)} Conv nodes with weights in the file, the {g.arch} graph has {len(names)} convolutions")
+        # name the first layer where the file and the graph part ways (e.g. a depthwise cls branch, or no OBB angle branch cv4)
+        k = next((i for i, (name, (_nd, wt, _bs)) in enumerate(zip(names, convs)) if tuple(wt.shape) != _expected_shape(g, name)),
+                 min(len(names), len(convs)))
+        where = (f"; the first that differs is Conv node {convs[k][0].name or convs[k][0].outputs[0]!r} with shape {tuple(convs[k][1].shape)} "
+                 f"where the graph runs {names[k]} {_expected_shape(g, names[k])}") if k < min(len(names), len(convs)) else ""
+        raise ValueError(f"{path}: {len(convs)} Conv nodes with weights in the file, the {g.arch} graph has {len(names)} convolutions{where}")
     for name, (nd, wt, bs) in zip(names, convs):
         put(name, wt, bs, f"Conv node {nd.name or nd.outputs[0]!r}")
         _check_conv_node(path, g, name, nd)
@@ -308,7 +313,7 @@ def write_conv_onnx(path: str, g: Graph, w: Dict[str, np.ndarray], named: bool =
         parts.append(_enc_field(5, _enc_tensor(bn, w[name + ".bias"].astype(dt))))
         prev = outn
         k += 1
-    if g.arch == "yolov8m":
+    if g.arch in ("yolov8m", "yolov8m-obb"):
         node = _enc_field(1, prev.encode()) + _enc_field(1, b"model.22.dfl.conv.weight") + _enc_field(2, b"/model.22/dfl/conv/Conv_output_0")
         node += _enc_field(3, b"/model.22/dfl/conv/Conv") + _enc_field(4, b"Conv")
         parts.append(_enc_field(1, node))

@@ -17,7 +17,7 @@ from typing import Dict, List, Optional, Union
 import numpy as np
 import torch
 
-from .engine import Engine
+from .engine import Engine, require_axis_aligned
 
 
 class _Input:
@@ -87,6 +87,7 @@ class InferenceSession:
             arch = arch or arch_from_model_path(model_path)
             weights = resolve_weights(model_path, arch, weights)
             engine = Engine(arch, weights=weights, max_batch=max_batch, device=device, seed=seed, precision=precision)
+        require_axis_aligned(engine, "InferenceSession")
         self.engine = engine
         self._inputs = [_Input("images", [None, 3, engine.imgsz, engine.imgsz])]
 

@@ -20,7 +20,9 @@ architecture.  The generator is deterministic in ``(arch, nc, seed)``.
   i.e. a discrete Gaussian around ``d`` with std 0.7, plus a small random part --
   and the last cls / objectness bias is placed so that about 6 % of the v8
   anchors (~500 of 8400 per tile) clear conf 0.25 (2 % of the 25200 v7 rows
-  clear the reference's 0.3, ``simple_detector.py:30``).
+  clear the reference's 0.3, ``simple_detector.py:30``);
+* the oriented-box head's angle logits (``yolov8m-obb``, cv4) get mean 0 and std ``ANGLE_STD`` = 1.5, so that the decoded
+  angle (sigmoid(z) - 0.25) * pi covers most of (-pi/4, 3pi/4) and the rotated NMS sees truly rotated boxes.
 """
 from __future__ import annotations
 
@@ -36,6 +38,7 @@ PREACT_STD = 4.0          # LSUV target of every SiLU conv (see the module docst
 CAL_SIZE, CAL_TILES = 640, 2
 DFL_SIGMA_D, DFL_D0, DFL_NOISE = 1.0, 1.5, 0.25
 CLS_STD, V8_PASS_FRACTION, V7_PASS_FRACTION = 2.0, 0.06, 0.02
+ANGLE_STD = 1.5                # OBB angle logits (yolov8m-obb)
 GENERATOR_VERSION = 2          # part of the seed: bump when the recipe changes
 
 _CACHE: Dict[Tuple, Dict[str, np.ndarray]] = {}
@@ -72,9 +75,13 @@ def _snap(v, bits: int = 12):
 def _final_layers(graph: Graph):
     if graph.head["kind"] == "seg":        # segmentation stand-in: the logits layer is scaled like every other conv
         return set(), set()
-    if graph.head["kind"] == "v8_dfl":
+    if graph.head["kind"] in ("v8_dfl", "v8_obb"):
         return {f"model.22.cv2.{i}.2" for i in range(3)}, {f"model.22.cv3.{i}.2" for i in range(3)}
     return set(), {f"model.105.m.{i}" for i in range(3)}
+
+
+def _angle_layers(graph: Graph):
+    return {f"model.22.cv4.{i}.2" for i in range(3)} if graph.head["kind"] == "v8_obb" else set()
 
 
 def make_synthetic_weights(graph: Graph, seed: int = 0, calibrate: bool = True) -> Dict[str, np.ndarray]:
@@ -167,7 +174,8 @@ def _calibrate_single_thread(graph: Graph, w: Dict[str, np.ndarray], seed: int) 
     g = build(graph.arch, graph.nc, 256 if graph.arch == "xunet" else CAL_SIZE)
     cal_size = g.imgsz
     box_final, cls_final = _final_layers(g)
-    v8 = g.head["kind"] == "v8_dfl"
+    v8 = g.head["kind"] in ("v8_dfl", "v8_obb")
+    angle_final = _angle_layers(g)
     x = torch.from_numpy(make_tiles(CAL_TILES, cal_size, seed=seed + 7919).astype(np.float32) / 255.0).permute(0, 3, 1, 2)
     bufs = {n: torch.zeros(CAL_TILES, b.c, b.h, b.w) for n, b in g.bufs.items()}
     bufs["input"][:, :3] = x
@@ -211,6 +219,11 @@ def _calibrate_single_thread(graph: Graph, w: Dict[str, np.ndarray], seed: int) 
                         bb = b.reshape(3, no)
                         bb[:, 4] = _snap(bb[:, 4] + shift)
                         b = bb.reshape(-1)
+                elif name in angle_final:
+                    # theta = (sigmoid(z) - 0.25) pi: logits of std ANGLE_STD around 0 spread theta over most of (-pi/4, 3pi/4)
+                    s1 = _quantised_scale(ANGLE_STD / float(y.std()))
+                    sc[:] = s1
+                    b[:] = _snap(-float(y.numpy().astype(np.float64).mean()) * s1)
                 else:
                     sc[:] = _quantised_scale(PREACT_STD / float(y.std()))
                 w[name + ".weight"] = round_to_bf16(w[name + ".weight"] * inv(op, sc)[:, None, None, None])   # model order

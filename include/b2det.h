@@ -50,6 +50,27 @@ typedef struct b2d_geodet {
     int32_t tile;
 } b2d_geodet;
 
+/* One oriented detection of a yolov8m-obb engine in model-input pixel space (36 bytes): Ultralytics' regularized
+ * rotated box (w >= h, theta in [0, pi), radians, the rotation of the w side from +x towards +y).                       */
+typedef struct b2d_obb {
+    float cx, cy, w, h, theta;
+    float conf;           /* best class score                                              */
+    int32_t cls;
+    int32_t tile;
+    int32_t anchor;       /* anchor index inside the tile (stable tie-break key)          */
+} b2d_obb;
+
+/* One georeferenced oriented detection (104 bytes): centre and the four corners (Ultralytics xywhr2xyxyxyxy order:
+ * c+v1+v2, c+v1-v2, c-v1-v2, c-v1+v2 with v1 along w, v2 along h) in lon/lat or CRS units, box size in the
+ * georeferenced form's pixels (bounds: crop pixels; affine: source-window pixels).                                     */
+typedef struct b2d_geoobb {
+    double x, y;
+    double corners[8];    /* x0, y0, x1, y1, x2, y2, x3, y3                                */
+    float conf, w, h, theta;
+    int32_t cls;
+    int32_t tile;
+} b2d_geoobb;
+
 /* ---- enums ----------------------------------------------------------------------------- */
 enum { B2D_ACT_NONE = 0, B2D_ACT_SILU = 1 };
 enum { B2D_CONV_AUTO = 0, B2D_CONV_TCGEN05 = 1 };   /* one backend: a shape the tensor-core kernels cannot run fails b2d_plan_finalize */
@@ -61,7 +82,10 @@ enum {
     B2D_RESIZE_LETTERBOX = 3     /* Ultralytics LetterBox, pad 114 -- x_arch/02_analyze_images:1 (cell 6) */
 };
 enum { B2D_OUT_BF16_NHWC4 = 0, B2D_OUT_F32_NCHW = 1, B2D_OUT_U8_NHWC = 2, B2D_OUT_F16_NHWC4 = 3 };
-enum { B2D_HEAD_V8_DFL = 0, B2D_HEAD_V7_ANCHOR = 1 };
+/* head kinds: v8 DFL boxes, v7 anchor boxes, v8 oriented boxes (DFL distances + one angle logit per anchor, Ultralytics >= 8.1
+ * OBB head; the angle logit is the fp32 channel (64 + nc + 3) / 4 * 4 of the head map, the first 16-byte-aligned one after the
+ * 64 DFL logits and the nc class logits)                                                                                   */
+enum { B2D_HEAD_V8_DFL = 0, B2D_HEAD_V7_ANCHOR = 1, B2D_HEAD_V8_OBB = 2 };
 /* georeferencing forms */
 enum {
     B2D_GEO_BOUNDS = 0,      /* simple_detector.py:487-494 : params = west,east,south,north,crop_size   */
@@ -106,7 +130,9 @@ int b2d_plan_dwconv(b2d_engine* e, int src, int src_c0, int dst, int dst_c0, int
                     const float* weight_host, const float* bias_host);
 int b2d_plan_maxpool(b2d_engine* e, int src, int src_c0, int dst, int dst_c0, int c, int k, int stride);
 int b2d_plan_upsample2x(b2d_engine* e, int src, int src_c0, int dst, int dst_c0, int c);
-/* head level: fp32 buffer `buf` [.,hw,hw,c]; anchors_px: 6 floats (v7) or NULL (v8).     */
+/* head level: fp32 buffer `buf` [.,hw,hw,c]; anchors_px: 6 floats (v7) or NULL (v8, v8 OBB).
+ * An engine planned with B2D_HEAD_V8_OBB levels answers only the *_obb stage entry points below, any other engine only
+ * the axis-aligned ones; a call of the other family fails with a message.                   */
 int b2d_plan_head_level(b2d_engine* e, int kind, int buf, int stride, int nc, const float* anchors_px);
 int b2d_plan_finalize(b2d_engine* e);
 void* b2d_buffer_ptr(b2d_engine* e, int buf);
@@ -173,6 +199,22 @@ int b2d_detect_host(b2d_engine* e, const uint8_t* tiles_host, int n, int h, int 
  * Replaces simple_detector.py:484-502, gpu_handler.py:178-190, pixel_to_geo.                 */
 int b2d_georef(b2d_engine* e, const b2d_det* dets_dev, const int32_t* counts_dev, int n, int cap,
                int mode, const double* params_dev, b2d_geodet* out_dev, void* stream);
+
+/* ---- oriented boxes (engines planned with B2D_HEAD_V8_OBB) --------------------------------
+ * Ultralytics >= 8.1 OBB semantics [EXT]: decode theta = (sigmoid(z) - 0.25) pi and dist2rbox; rotated NMS =
+ * non_max_suppression(rotated=True): class-offset boxes (+7680 cls), descending confidence, keep j iff
+ * ProbIoU(i, j) < iou_thr for EVERY earlier i ("fast NMS": a suppressed box still suppresses), at most max_det
+ * (<= 30000 candidates enter); results regularized (regularize_rboxes).                                        */
+/* Dense decode: rows_dev fp32 [n][A][7] = cx, cy, w, h, conf (max class), cls, theta (not regularized).            */
+int b2d_decode_rows_obb(b2d_engine* e, int n, float* rows_dev, void* stream);
+/* Decode + filter + (iou_thr > 0) rotated NMS, arguments as b2d_postprocess; dets_dev: b2d_obb [n][cap].          */
+int b2d_postprocess_obb(b2d_engine* e, int n, float conf_thr, int inclusive, float iou_thr, int top_k,
+                        int max_det, b2d_obb* dets_dev, int32_t* counts_dev, int cap, void* stream);
+/* Georeference centre and corners, arguments as b2d_georef; modes B2D_GEO_BOUNDS (per-point interpolation) and
+ * B2D_GEO_AFFINE (letterbox undone on centre and size, no clipping; fp32 corners; window offset + geotransform
+ * in fp64).  The other two forms are refused.                                                                   */
+int b2d_georef_obb(b2d_engine* e, const b2d_obb* dets_dev, const int32_t* counts_dev, int n, int cap,
+                   int mode, const double* params_dev, b2d_geoobb* out_dev, void* stream);
 
 /* Greedy centre-distance dedup in a metric CRS.  Replaces SimpleDetector._remove_duplicates
  * (simple_detector.py:558-596, inclusive=1) and ResultsManager.remove_duplicates
