@@ -147,8 +147,21 @@ int preprocess_launch(const ResizeTables* t, const uint8_t* src, int n, int pitc
 
 int input_from_f32_launch(const float* src, int n, int h, int w, void* dst, cudaStream_t stream, int f16 = 0);
 
-struct HeadLevel { const float* buf; int hw, c, stride, nc, kind; float anchors[6]; int row0; };
+struct HeadLevel { const float* buf; int hw, c, stride; float anchors[6]; int row0; };
 struct HeadDesc { HeadLevel lv[3]; int nlevels; int kind; int nc; int rows_total; };
+
+// OBB head: the angle logit sits at the first 16-byte-aligned fp32 channel after the 64 DFL and nc class channels
+// (graph.obb_angle_channel)
+__host__ __device__ inline int obb_angle_channel(int nc) { return (64 + nc + 3) / 4 * 4; }
+
+// Candidates per tile: sort keys carry the candidate slot in a 15-bit field
+constexpr int kMaxCand = 32768;
+// Sort keys per tile: the candidate capacity rounded up to a power of two
+static inline int keys_stride(int cand_cap) {
+    int s = 1;
+    while (s < cand_cap) s <<= 1;
+    return s;
+}
 
 int decode_rows_launch(const HeadDesc* h, int n, float* rows, cudaStream_t stream);
 int candidates_from_head_launch(const HeadDesc* h, int n, float thr, int inclusive, float scale, b2d_det* cand, int* cand_count,

@@ -142,13 +142,12 @@ namespace {
 bool is_obb(const b2d_engine* e) { return e->head_levels > 0 && e->head.kind == B2D_HEAD_V8_OBB; }
 
 int ensure_cand(b2d_engine* e, int n, int rows) {
-    int cap = rows < 32768 ? rows : 32768;
+    int cap = rows < kMaxCand ? rows : kMaxCand;
     if (e->cand && e->cand_cap >= cap && e->cand_tiles >= n) return 0;
     if (e->cand) { cudaFree(e->cand); cudaFree(e->cand_count); cudaFree(e->keys); }
     if (e->cand_angle) { cudaFree(e->cand_angle); cudaFree(e->obb_prm); e->cand_angle = nullptr; e->obb_prm = nullptr; }
     int tiles = n > e->max_batch ? n : e->max_batch;
-    int stride = 1;
-    while (stride < cap) stride <<= 1;
+    const int stride = keys_stride(cap);
     B2D_CUDA(cudaMalloc(&e->cand, (size_t)tiles * cap * sizeof(b2d_det)));
     B2D_CUDA(cudaMalloc(&e->cand_count, (size_t)tiles * sizeof(int)));
     B2D_CUDA(cudaMalloc(&e->keys, (size_t)tiles * stride * sizeof(unsigned long long)));
@@ -495,12 +494,12 @@ int b2d_plan_head_level(b2d_engine* e, int kind, int buf, int stride, int nc, co
     B2D_CHECK(e->head_levels == 0 || (e->head.kind == kind && e->head.nc == nc), "plan_head_level: inconsistent head");
     const Buffer& b = e->bufs[buf];
     HeadLevel& L = e->head.lv[e->head_levels];
-    L.buf = (const float*)b.ptr; L.hw = b.h; L.c = b.c; L.stride = stride; L.nc = nc; L.kind = kind;
+    L.buf = (const float*)b.ptr; L.hw = b.h; L.c = b.c; L.stride = stride;
     for (int i = 0; i < 6; ++i) L.anchors[i] = anchors_px ? anchors_px[i] : 0.f;
     B2D_CHECK(kind == B2D_HEAD_V8_DFL || kind == B2D_HEAD_V7_ANCHOR || kind == B2D_HEAD_V8_OBB, "plan_head_level: unknown head kind %d", kind);
     const int per = (kind == B2D_HEAD_V7_ANCHOR) ? 3 : 1;
     L.row0 = e->head.rows_total;
-    const int need = kind == B2D_HEAD_V7_ANCHOR ? 3 * (nc + 5) : kind == B2D_HEAD_V8_OBB ? (64 + nc + 3) / 4 * 4 + 1 : 64 + nc;
+    const int need = kind == B2D_HEAD_V7_ANCHOR ? 3 * (nc + 5) : kind == B2D_HEAD_V8_OBB ? obb_angle_channel(nc) + 1 : 64 + nc;
     B2D_CHECK(b.c >= need, "plan_head_level: head buffer too narrow (%d channels, the head needs %d)", b.c, need);
     e->head.rows_total += per * b.h * b.w;
     e->head.kind = kind; e->head.nc = nc;

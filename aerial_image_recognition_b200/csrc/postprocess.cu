@@ -45,25 +45,58 @@ __device__ __forceinline__ float dfl_side(const float* p) {
     return e / s;
 }
 
-__device__ __forceinline__ void v8_scores(const float* pix, int nc, float* conf, int* cls) {
-    float best = -1.f;
-    int bi = 0;
-    for (int k = 0; k < nc; ++k) {
-        const float s = sigmoid_f(__ldg(pix + 64 + k));
-        if (s > best) { best = s; bi = k; }
-    }
-    *conf = best; *cls = bi;
+__device__ __forceinline__ bool passes(float conf, float thr, int inclusive) { return inclusive ? (conf >= thr) : (conf > thr); }
+
+// The pyramid level of head row `a`: rows are numbered level by level
+__device__ __forceinline__ const HeadLevel& head_level(const HeadDesc& h, int a, bool in_range) {
+    int lvl = 0;
+    if (in_range) { while (lvl + 1 < h.nlevels && a >= h.lv[lvl + 1].row0) ++lvl; }
+    return h.lv[lvl];
 }
 
-__device__ __forceinline__ Row v8_box(float side, int lane_side, int gx, int gy, float stride, unsigned mask, int base_lane) {
-    // gather l,t,r,b from the 4 lanes of this anchor
-    const float l = __shfl_sync(mask, side, base_lane + 0);
-    const float t = __shfl_sync(mask, side, base_lane + 1);
-    const float r = __shfl_sync(mask, side, base_lane + 2);
-    const float b = __shfl_sync(mask, side, base_lane + 3);
-    (void)lane_side;
+// v8 anchor `a` (DFL and OBB heads): its grid cell and its logits in the NHWC map of its level
+struct V8Anchor { const float* pix; int gx, gy; float stride; };
+
+__device__ __forceinline__ V8Anchor v8_anchor(const HeadDesc& h, int tile, int a, bool in_range) {
+    const HeadLevel& L = head_level(h, a, in_range);
+    const int cell = in_range ? a - L.row0 : 0;
+    V8Anchor v;
+    v.gy = cell / L.hw; v.gx = cell - v.gy * L.hw;
+    v.pix = L.buf + ((size_t)tile * L.hw * L.hw + cell) * L.c;
+    v.stride = (float)L.stride;
+    return v;
+}
+
+// Best class, the threshold (MODE 1) and the DFL distances l, t, r, b of a v8 anchor, whose 4 lanes decode one side each and
+// then gather all four.  Returns false, on every lane, when no anchor of the warp is wanted: the caller leaves.
+template <int MODE>
+__device__ __forceinline__ bool v8_sides(const float* pix, int nc, bool in_range, float thr, int inclusive, float scale, float* conf,
+                                         int* cls, bool* want, float* ltrb) {
+    float best = 0.f;
+    int bi = 0;
+    *want = in_range;
+    if (in_range) {
+        best = -1.f;
+        for (int k = 0; k < nc; ++k) {
+            const float s = sigmoid_f(__ldg(pix + 64 + k));
+            if (s > best) { best = s; bi = k; }
+        }
+        if (MODE == 1) { best = __fmul_rn(best, scale); *want = passes(best, thr, inclusive); }   // scale: gpu_handler.py:236-238
+    }
+    *conf = best; *cls = bi;
+    // the 4 lanes of an anchor agree on `want`; decode only where some anchor of the warp needs it
+    if (__ballot_sync(0xffffffffu, *want) == 0) return false;
+    const int side = threadIdx.x & 3, base_lane = (threadIdx.x & 31) & ~3;
+    const float d = *want ? dfl_side(pix + side * 16) : 0.f;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) ltrb[k] = __shfl_sync(0xffffffffu, d, base_lane + k);
+    return true;
+}
+
+// dist2bbox: the anchor point minus (l, t) and plus (r, b), as centre and size in pixels
+__device__ __forceinline__ Row v8_box(const float* ltrb, int gx, int gy, float stride) {
     const float ax = (float)gx + 0.5f, ay = (float)gy + 0.5f;
-    const float x1 = __fsub_rn(ax, l), y1 = __fsub_rn(ay, t), x2 = __fadd_rn(ax, r), y2 = __fadd_rn(ay, b);
+    const float x1 = __fsub_rn(ax, ltrb[0]), y1 = __fsub_rn(ay, ltrb[1]), x2 = __fadd_rn(ax, ltrb[2]), y2 = __fadd_rn(ay, ltrb[3]);
     Row o;
     o.cx = __fmul_rn(__fmul_rn(__fadd_rn(x1, x2), 0.5f), stride);
     o.cy = __fmul_rn(__fmul_rn(__fadd_rn(y1, y2), 0.5f), stride);
@@ -93,100 +126,65 @@ __device__ __forceinline__ Row v7_row(const float* cell, int nc, int gx, int gy,
     return o;
 }
 
-__device__ __forceinline__ bool passes(float conf, float thr, int inclusive) { return inclusive ? (conf >= thr) : (conf > thr); }
+// Warp-aggregated append to a tile's candidate list: one atomicAdd per warp, slots in lane order.  Every lane of the warp must
+// call it, converged (full-mask ballot and shuffle).  Returns the lane's slot, or -1 when it does not emit or the list is full.
+__device__ __forceinline__ int append_candidate(bool emit, int& cand_count, int cand_cap) {
+    const unsigned em = __ballot_sync(0xffffffffu, emit);
+    if (!em) return -1;
+    const int lane = threadIdx.x & 31;
+    const int leader = __ffs(em) - 1;
+    int base = 0;
+    if (lane == leader) base = atomicAdd(&cand_count, __popc(em));
+    base = __shfl_sync(0xffffffffu, base, leader);
+    const int slot = base + __popc(em & ((1u << lane) - 1));
+    return emit && slot < cand_cap ? slot : -1;
+}
 
 // Shared body: MODE 0 = dense rows, MODE 1 = thresholded candidates.
 template <int MODE>
-__global__ void __launch_bounds__(256) head_kernel(HeadDesc h, int n, float thr, int inclusive, float scale, float* rows, b2d_det* cand,
+__global__ void __launch_bounds__(256) head_kernel(HeadDesc h, float thr, int inclusive, float scale, float* rows, b2d_det* cand,
                                                    int* cand_count, int cand_cap) {
     const int tile = blockIdx.y;
-    const int lane = threadIdx.x & 31;
+    int a;
+    bool out;       // this lane stores anchor a's row (MODE 0) or emits it as a candidate (MODE 1)
+    Row r;
     if (h.kind == B2D_HEAD_V8_DFL) {
-        // 4 lanes per anchor
-        const int a = (blockIdx.x * blockDim.x + threadIdx.x) >> 2;    // anchor index inside the tile
-        const int side = threadIdx.x & 3;
+        a = (blockIdx.x * blockDim.x + threadIdx.x) >> 2;    // 4 lanes per anchor, one per box side
         const bool in_range = a < h.rows_total;
-        int lvl = 0;
-        if (in_range) { while (lvl + 1 < h.nlevels && a >= h.lv[lvl + 1].row0) ++lvl; }
-        const HeadLevel& L = h.lv[lvl];
-        const int cell = in_range ? a - L.row0 : 0;
-        const int gy = cell / L.hw, gx = cell - gy * L.hw;
-        const float* pix = L.buf + ((size_t)tile * L.hw * L.hw + cell) * L.c;
-        float conf = 0.f; int cls = 0;
-        bool want = in_range;
-        if (in_range) {
-            v8_scores(pix, h.nc, &conf, &cls);
-            if (MODE == 1) { conf = __fmul_rn(conf, scale); want = passes(conf, thr, inclusive); }   // scale: gpu_handler.py:236-238
-        }
-        // the 4 lanes of an anchor agree on `want`; decode only where some anchor of the warp needs it
-        const unsigned any = __ballot_sync(0xffffffffu, want);
-        if (any == 0) return;
-        float sidev = 0.f;
-        if (want) sidev = dfl_side(pix + side * 16);
-        Row r = v8_box(sidev, side, gx, gy, (float)L.stride, 0xffffffffu, lane & ~3);
+        const V8Anchor v = v8_anchor(h, tile, a, in_range);
+        float conf, ltrb[4]; int cls; bool want;
+        if (!v8_sides<MODE>(v.pix, h.nc, in_range, thr, inclusive, scale, &conf, &cls, &want, ltrb)) return;
+        r = v8_box(ltrb, v.gx, v.gy, v.stride);
         r.conf = conf; r.cls = cls;
-        if (MODE == 0) {
-            if (in_range && side == 0) {
-                float* o = rows + ((size_t)tile * h.rows_total + a) * 6;
-                o[0] = r.cx; o[1] = r.cy; o[2] = r.w; o[3] = r.h; o[4] = r.conf; o[5] = (float)r.cls;
-            }
-        } else {
-            const bool emit = want && side == 0;
-            const unsigned em = __ballot_sync(0xffffffffu, emit);
-            if (em) {
-                int base = 0;
-                const int leader = __ffs(em) - 1;
-                if (lane == leader) base = atomicAdd(&cand_count[tile], __popc(em));
-                base = __shfl_sync(0xffffffffu, base, leader);
-                if (emit) {
-                    const int slot = base + __popc(em & ((1u << lane) - 1));
-                    if (slot < cand_cap) {
-                        b2d_det d;
-                        d.cx = r.cx; d.cy = r.cy; d.w = r.w; d.h = r.h; d.conf = r.conf; d.cls = r.cls; d.tile = tile; d.anchor = a;
-                        cand[(size_t)tile * cand_cap + slot] = d;
-                    }
-                }
-            }
-        }
+        out = want && (threadIdx.x & 3) == 0;
     } else {
-        const int a = blockIdx.x * blockDim.x + threadIdx.x;   // row index inside the tile
+        a = blockIdx.x * blockDim.x + threadIdx.x;   // row index inside the tile
         const bool in_range = a < h.rows_total;
-        int lvl = 0;
-        if (in_range) { while (lvl + 1 < h.nlevels && a >= h.lv[lvl + 1].row0) ++lvl; }
-        const HeadLevel& L = h.lv[lvl];
+        const HeadLevel& L = head_level(h, a, in_range);
         const int no = h.nc + 5;
         const int rel = in_range ? a - L.row0 : 0;
         const int cells = L.hw * L.hw;
         const int ai = rel / cells, cell = rel - ai * cells;     // rows ordered anchor, y, x inside a level
         const int gy = cell / L.hw, gx = cell - gy * L.hw;
-        Row r; r.conf = -1.f;
+        r.conf = -1.f;
         if (in_range) {
             const float* p = L.buf + ((size_t)tile * cells + cell) * L.c + ai * no;
             r = v7_row(p, h.nc, gx, gy, (float)L.stride, L.anchors[2 * ai], L.anchors[2 * ai + 1]);
             if (MODE == 1) r.conf = __fmul_rn(r.conf, scale);
         }
-        if (MODE == 0) {
-            if (in_range) {
-                float* o = rows + ((size_t)tile * h.rows_total + a) * 6;
-                o[0] = r.cx; o[1] = r.cy; o[2] = r.w; o[3] = r.h; o[4] = r.conf; o[5] = (float)r.cls;
-            }
-        } else {
-            const bool emit = in_range && passes(r.conf, thr, inclusive);
-            const unsigned em = __ballot_sync(0xffffffffu, emit);
-            if (em) {
-                int base = 0;
-                const int leader = __ffs(em) - 1;
-                if (lane == leader) base = atomicAdd(&cand_count[tile], __popc(em));
-                base = __shfl_sync(0xffffffffu, base, leader);
-                if (emit) {
-                    const int slot = base + __popc(em & ((1u << lane) - 1));
-                    if (slot < cand_cap) {
-                        b2d_det d;
-                        d.cx = r.cx; d.cy = r.cy; d.w = r.w; d.h = r.h; d.conf = r.conf; d.cls = r.cls; d.tile = tile; d.anchor = a;
-                        cand[(size_t)tile * cand_cap + slot] = d;
-                    }
-                }
-            }
+        out = in_range && (MODE == 0 || passes(r.conf, thr, inclusive));
+    }
+    if (MODE == 0) {
+        if (out) {
+            float* o = rows + ((size_t)tile * h.rows_total + a) * 6;
+            o[0] = r.cx; o[1] = r.cy; o[2] = r.w; o[3] = r.h; o[4] = r.conf; o[5] = (float)r.cls;
+        }
+    } else {
+        const int slot = append_candidate(out, cand_count[tile], cand_cap);
+        if (slot >= 0) {
+            b2d_det d;
+            d.cx = r.cx; d.cy = r.cy; d.w = r.w; d.h = r.h; d.conf = r.conf; d.cls = r.cls; d.tile = tile; d.anchor = a;
+            cand[(size_t)tile * cand_cap + slot] = d;
         }
     }
 }
@@ -196,26 +194,16 @@ __global__ void __launch_bounds__(256) rows_filter_kernel(const float* __restric
                                                            int inclusive, float scale, b2d_det* cand, int* cand_count, int cand_cap) {
     const int tile = blockIdx.y;
     const int a = blockIdx.x * blockDim.x + threadIdx.x;
-    const int lane = threadIdx.x & 31;
     const bool in_range = a < num_rows;
     const float* p = rows + ((size_t)tile * num_rows + (in_range ? a : 0)) * ncol;
     const float conf = in_range ? __fmul_rn(__ldg(p + 4), scale) : -1.f;
-    const bool emit = in_range && passes(conf, thr, inclusive);
-    const unsigned em = __ballot_sync(0xffffffffu, emit);
-    if (!em) return;
-    int base = 0;
-    const int leader = __ffs(em) - 1;
-    if (lane == leader) base = atomicAdd(&cand_count[tile], __popc(em));
-    base = __shfl_sync(0xffffffffu, base, leader);
-    if (emit) {
-        const int slot = base + __popc(em & ((1u << lane) - 1));
-        if (slot < cand_cap) {
-            b2d_det d;
-            d.cx = __ldg(p); d.cy = __ldg(p + 1); d.w = __ldg(p + 2); d.h = __ldg(p + 3); d.conf = conf;
-            d.cls = (ncol > 5) ? (int)__ldg(p + 5) : 0;
-            d.tile = tile; d.anchor = a;
-            cand[(size_t)tile * cand_cap + slot] = d;
-        }
+    const int slot = append_candidate(in_range && passes(conf, thr, inclusive), cand_count[tile], cand_cap);
+    if (slot >= 0) {
+        b2d_det d;
+        d.cx = __ldg(p); d.cy = __ldg(p + 1); d.w = __ldg(p + 2); d.h = __ldg(p + 3); d.conf = conf;
+        d.cls = (ncol > 5) ? (int)__ldg(p + 5) : 0;
+        d.tile = tile; d.anchor = a;
+        cand[(size_t)tile * cand_cap + slot] = d;
     }
 }
 
@@ -224,7 +212,6 @@ constexpr int kSelCand = 256;                     // candidates per NMS chunk
 constexpr int kSelParts = 4;                      // thread groups sharing a chunk's work (= 64-bit words of a suppression mask)
 constexpr int kSelThreads = kSelCand * kSelParts;
 static_assert(kSelParts == kSelCand / 64, "one part per mask word");
-constexpr int kSmemKeys = 2048;
 constexpr int kMaxDet = 512;
 
 __device__ void bitonic_sort(unsigned long long* keys, int n2) {
@@ -351,6 +338,16 @@ __global__ void __launch_bounds__(kSortThreads) sort_keys_kernel(const b2d_det* 
         for (int i = threadIdx.x; i < cnt; i += blockDim.x) out[i] = keys[i];
 }
 
+// No NMS: the first min(cnt, top_k, cap) candidates in key order, each slot s converted by rec(s)
+template <class Out, class Rec>
+__device__ __forceinline__ void copy_top_k(const unsigned long long* keys, int cnt, int top_k, int cap, Out* to, int* out_count, Rec rec) {
+    int m = cnt;
+    if (top_k > 0 && m > top_k) m = top_k;
+    if (m > cap) m = cap;
+    for (int i = threadIdx.x; i < m; i += blockDim.x) to[i] = rec((int)(keys[i] & 0x7FFF));
+    if (threadIdx.x == 0) *out_count = m;
+}
+
 __global__ void __launch_bounds__(kSelThreads) select_kernel(const b2d_det* __restrict__ cand, const int* __restrict__ cand_count,
                                                               int cand_cap, const unsigned long long* __restrict__ keys_scratch, int keys_stride,
                                                               float iou_thr, int top_k, int max_det, b2d_det* out, int* out_count,
@@ -378,11 +375,7 @@ __global__ void __launch_bounds__(kSelThreads) select_kernel(const b2d_det* __re
     const unsigned long long* keys = keys_scratch + (size_t)tile * keys_stride;     // sorted by sort_keys_kernel
 
     if (!(iou_thr > 0.f)) {
-        int m = cnt;
-        if (top_k > 0 && m > top_k) m = top_k;
-        if (m > cap) m = cap;
-        for (int i = tid; i < m; i += blockDim.x) to[i] = tc[(int)(keys[i] & 0x7FFF)];
-        if (tid == 0) out_count[tile] = m;
+        copy_top_k(keys, cnt, top_k, cap, to, &out_count[tile], [&](int s) { return tc[s]; });
         return;
     }
 
@@ -482,6 +475,22 @@ __global__ void __launch_bounds__(kSelThreads) select_kernel(const b2d_det* __re
 }
 
 // ---- georef -------------------------------------------------------------------------------------
+// Bounds form, simple_detector.py:487-494 -- P = west, east, south, north, crop_size, model_size: model pixel (x, y) -> lon / lat
+__device__ __forceinline__ double geo_model_size(const double* P) { return P[5] > 0.0 ? P[5] : 640.0; }
+
+__device__ __forceinline__ void geo_bounds(const double* P, double x, double y, double* gx, double* gy) {
+    const double ms = geo_model_size(P);
+    const double xf = __ddiv_rn(x, ms), yf = __ddiv_rn(y, ms);
+    *gx = __dadd_rn(P[0], __dmul_rn(xf, __dsub_rn(P[1], P[0])));
+    *gy = __dsub_rn(P[3], __dmul_rn(yf, __dsub_rn(P[3], P[2])));
+}
+
+// 6-term geotransform P[0..5] of the window-relative pixel (X, Y)
+__device__ __forceinline__ void geo_affine(const double* P, double X, double Y, double* gx, double* gy) {
+    *gx = __dadd_rn(__dadd_rn(P[0], __dmul_rn(X, P[1])), __dmul_rn(Y, P[2]));
+    *gy = __dadd_rn(__dadd_rn(P[3], __dmul_rn(X, P[4])), __dmul_rn(Y, P[5]));
+}
+
 __global__ void __launch_bounds__(256) georef_kernel(const b2d_det* __restrict__ dets, const int* __restrict__ counts, int cap, int mode,
                                                       const double* __restrict__ params, b2d_geodet* __restrict__ out) {
     const int tile = blockIdx.y;
@@ -493,13 +502,10 @@ __global__ void __launch_bounds__(256) georef_kernel(const b2d_det* __restrict__
     g.conf = d.conf; g.tile = tile; g.x_yolo = d.cx; g.y_yolo = d.cy; g.x_img = 0.f; g.y_img = 0.f;
     const double x = (double)d.cx, y = (double)d.cy;
     if (mode == B2D_GEO_BOUNDS) {
-        // simple_detector.py:487-494 -- P = west, east, south, north, crop_size, model_size
-        const double ms = P[5] > 0.0 ? P[5] : 640.0;
-        const double xf = __ddiv_rn(x, ms), yf = __ddiv_rn(y, ms);
-        g.x_img = (float)__dmul_rn(xf, P[4]);
-        g.y_img = (float)__dmul_rn(yf, P[4]);
-        g.x = __dadd_rn(P[0], __dmul_rn(xf, __dsub_rn(P[1], P[0])));
-        g.y = __dsub_rn(P[3], __dmul_rn(yf, __dsub_rn(P[3], P[2])));
+        const double ms = geo_model_size(P);
+        g.x_img = (float)__dmul_rn(__ddiv_rn(x, ms), P[4]);
+        g.y_img = (float)__dmul_rn(__ddiv_rn(y, ms), P[4]);
+        geo_bounds(P, x, y, &g.x, &g.y);
     } else if (mode == B2D_GEO_GPUHANDLER) {
         // gpu_handler.py:182-190 -- P = lon_min, lat_min, lon_max, lat_max; keeps the *864/864 round trip
         const double x864 = __dmul_rn(__ddiv_rn(x, 640.0), 864.0), y864 = __dmul_rn(__ddiv_rn(y, 640.0), 864.0);
@@ -529,8 +535,7 @@ __global__ void __launch_bounds__(256) georef_kernel(const b2d_det* __restrict__
         const double cxp = __dadd_rn(__ddiv_rn((double)__fadd_rn(x1, x2), 2.0), P[6]);
         const double cyp = __dadd_rn(__ddiv_rn((double)__fadd_rn(y1, y2), 2.0), P[7]);
         g.x_img = (float)cxp; g.y_img = (float)cyp;
-        g.x = __dadd_rn(__dadd_rn(P[0], __dmul_rn(cxp, P[1])), __dmul_rn(cyp, P[2]));
-        g.y = __dadd_rn(__dadd_rn(P[3], __dmul_rn(cxp, P[4])), __dmul_rn(cyp, P[5]));
+        geo_affine(P, cxp, cyp, &g.x, &g.y);
     }
     out[(size_t)tile * cap + i] = g;
 }
@@ -542,50 +547,32 @@ constexpr float kPiF = 3.14159265358979f;           // float(math.pi), the scala
 constexpr float kHalfPiF = 1.57079632679490f;       // float(math.pi / 2)
 constexpr float kProbEps = 1e-7f;
 
-__device__ __forceinline__ int obb_angle_channel(int nc) { return (64 + nc + 3) / 4 * 4; }   // graph.obb_angle_channel
-
 // MODE 0 = dense rows [n][A][7] (cx, cy, w, h, conf, cls, theta); MODE 1 = thresholded candidates + their angles
 template <int MODE>
 __global__ void __launch_bounds__(256) obb_head_kernel(HeadDesc h, float thr, int inclusive, float scale, float* rows, b2d_det* cand,
                                                        float* cand_angle, int* cand_count, int cand_cap) {
     const int tile = blockIdx.y;
-    const int lane = threadIdx.x & 31;
     const int a = (blockIdx.x * blockDim.x + threadIdx.x) >> 2;        // 4 lanes per anchor, one per box side
     const int side = threadIdx.x & 3;
     const bool in_range = a < h.rows_total;
-    int lvl = 0;
-    if (in_range) { while (lvl + 1 < h.nlevels && a >= h.lv[lvl + 1].row0) ++lvl; }
-    const HeadLevel& L = h.lv[lvl];
-    const int cell = in_range ? a - L.row0 : 0;
-    const int gy = cell / L.hw, gx = cell - gy * L.hw;
-    const float* pix = L.buf + ((size_t)tile * L.hw * L.hw + cell) * L.c;
-    float conf = 0.f; int cls = 0;
-    bool want = in_range;
-    if (in_range) {
-        v8_scores(pix, h.nc, &conf, &cls);
-        if (MODE == 1) { conf = __fmul_rn(conf, scale); want = passes(conf, thr, inclusive); }
-    }
-    const unsigned any = __ballot_sync(0xffffffffu, want);
-    if (any == 0) return;
-    float sidev = 0.f;
-    if (want) sidev = dfl_side(pix + side * 16);
-    const unsigned m = 0xffffffffu;
-    const int bl = lane & ~3;
-    const float l = __shfl_sync(m, sidev, bl), t = __shfl_sync(m, sidev, bl + 1), r = __shfl_sync(m, sidev, bl + 2), b = __shfl_sync(m, sidev, bl + 3);
+    const V8Anchor v = v8_anchor(h, tile, a, in_range);
+    float conf, ltrb[4]; int cls; bool want;
+    if (!v8_sides<MODE>(v.pix, h.nc, in_range, thr, inclusive, scale, &conf, &cls, &want, ltrb)) return;
+    const float l = ltrb[0], t = ltrb[1], r = ltrb[2], b = ltrb[3];
     if (!want || side != 0) {
         if (MODE == 0) return;
     }
     float cx = 0.f, cy = 0.f, w = 0.f, hh = 0.f, th = 0.f;
     if (want && side == 0) {
-        th = __fmul_rn(__fsub_rn(sigmoid_f(__ldg(pix + obb_angle_channel(h.nc))), 0.25f), kPiF);
+        th = __fmul_rn(__fsub_rn(sigmoid_f(__ldg(v.pix + obb_angle_channel(h.nc))), 0.25f), kPiF);
         float sn, cs;
         sincosf(th, &sn, &cs);
         const float xf = __fdiv_rn(__fsub_rn(r, l), 2.0f), yf = __fdiv_rn(__fsub_rn(b, t), 2.0f);
         const float x = __fsub_rn(__fmul_rn(xf, cs), __fmul_rn(yf, sn));
         const float y = __fadd_rn(__fmul_rn(xf, sn), __fmul_rn(yf, cs));
-        const float s = (float)L.stride;
-        cx = __fmul_rn(__fadd_rn(x, (float)gx + 0.5f), s);
-        cy = __fmul_rn(__fadd_rn(y, (float)gy + 0.5f), s);
+        const float s = v.stride;
+        cx = __fmul_rn(__fadd_rn(x, (float)v.gx + 0.5f), s);
+        cy = __fmul_rn(__fadd_rn(y, (float)v.gy + 0.5f), s);
         w = __fmul_rn(__fadd_rn(l, r), s);
         hh = __fmul_rn(__fadd_rn(t, b), s);
     }
@@ -594,21 +581,12 @@ __global__ void __launch_bounds__(256) obb_head_kernel(HeadDesc h, float thr, in
         o[0] = cx; o[1] = cy; o[2] = w; o[3] = hh; o[4] = conf; o[5] = (float)cls; o[6] = th;
         return;
     }
-    const bool emit = want && side == 0;
-    const unsigned em = __ballot_sync(0xffffffffu, emit);
-    if (!em) return;
-    int base = 0;
-    const int leader = __ffs(em) - 1;
-    if (lane == leader) base = atomicAdd(&cand_count[tile], __popc(em));
-    base = __shfl_sync(0xffffffffu, base, leader);
-    if (emit) {
-        const int slot = base + __popc(em & ((1u << lane) - 1));
-        if (slot < cand_cap) {
-            b2d_det d;
-            d.cx = cx; d.cy = cy; d.w = w; d.h = hh; d.conf = conf; d.cls = cls; d.tile = tile; d.anchor = a;
-            cand[(size_t)tile * cand_cap + slot] = d;
-            cand_angle[(size_t)tile * cand_cap + slot] = th;
-        }
+    const int slot = append_candidate(want && side == 0, cand_count[tile], cand_cap);
+    if (slot >= 0) {
+        b2d_det d;
+        d.cx = cx; d.cy = cy; d.w = w; d.h = hh; d.conf = conf; d.cls = cls; d.tile = tile; d.anchor = a;
+        cand[(size_t)tile * cand_cap + slot] = d;
+        cand_angle[(size_t)tile * cand_cap + slot] = th;
     }
 }
 
@@ -668,14 +646,7 @@ __global__ void __launch_bounds__(kObbThreads) obb_select_kernel(const b2d_det* 
     b2d_obb* to = out + (size_t)tile * cap;
     const unsigned long long* keys = keys_scratch + (size_t)tile * keys_stride;
     if (!(iou_thr > 0.f)) {
-        int m = cnt;
-        if (top_k > 0 && m > top_k) m = top_k;
-        if (m > cap) m = cap;
-        for (int i = tid; i < m; i += blockDim.x) {
-            const int s = (int)(keys[i] & 0x7FFF);
-            to[i] = obb_record(tc[s], ta[s]);
-        }
-        if (tid == 0) out_count[tile] = m;
+        copy_top_k(keys, cnt, top_k, cap, to, &out_count[tile], [&](int s) { return obb_record(tc[s], ta[s]); });
         return;
     }
     if (max_det > cap) max_det = cap;
@@ -771,23 +742,16 @@ __global__ void __launch_bounds__(256) obb_georef_kernel(const b2d_obb* __restri
     b2d_geoobb g;
     g.conf = d.conf; g.theta = d.theta; g.cls = d.cls; g.tile = tile;
     float px[5], py[5];
+    double gx[5], gy[5];
     if (mode == B2D_GEO_BOUNDS) {
-        // simple_detector.py:487-494 applied to the centre and to each corner; w, h scaled like x_img (model -> crop pixels)
+        // the bounds form applied to the centre and to each corner; w, h scaled like x_img (model -> crop pixels)
         obb_corners(d.cx, d.cy, d.w, d.h, d.theta, px, py);
         px[4] = d.cx; py[4] = d.cy;
-        const double ms = P[5] > 0.0 ? P[5] : 640.0;
+        const double ms = geo_model_size(P);
         g.w = (float)__dmul_rn(__ddiv_rn((double)d.w, ms), P[4]);
         g.h = (float)__dmul_rn(__ddiv_rn((double)d.h, ms), P[4]);
-        double gx[5], gy[5];
 #pragma unroll
-        for (int k = 0; k < 5; ++k) {
-            const double xf = __ddiv_rn((double)px[k], ms), yf = __ddiv_rn((double)py[k], ms);
-            gx[k] = __dadd_rn(P[0], __dmul_rn(xf, __dsub_rn(P[1], P[0])));
-            gy[k] = __dsub_rn(P[3], __dmul_rn(yf, __dsub_rn(P[3], P[2])));
-        }
-        g.x = gx[4]; g.y = gy[4];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) { g.corners[2 * k] = gx[k]; g.corners[2 * k + 1] = gy[k]; }
+        for (int k = 0; k < 5; ++k) geo_bounds(P, (double)px[k], (double)py[k], &gx[k], &gy[k]);
     } else {
         // affine: undo the letterbox in fp32 (centre - pad, / gain; w, h / gain; no clipping), corners in fp32, then the window
         // offset and the 6-term geotransform in fp64.  P = gt[0..5], win_x, win_y, pad_x, pad_y, gain
@@ -797,18 +761,25 @@ __global__ void __launch_bounds__(256) obb_georef_kernel(const b2d_obb* __restri
         g.h = __fdiv_rn(d.h, gain);
         obb_corners(cx, cy, g.w, g.h, d.theta, px, py);
         px[4] = cx; py[4] = cy;
-        double gx[5], gy[5];
 #pragma unroll
-        for (int k = 0; k < 5; ++k) {
-            const double X = __dadd_rn((double)px[k], P[6]), Y = __dadd_rn((double)py[k], P[7]);
-            gx[k] = __dadd_rn(__dadd_rn(P[0], __dmul_rn(X, P[1])), __dmul_rn(Y, P[2]));
-            gy[k] = __dadd_rn(__dadd_rn(P[3], __dmul_rn(X, P[4])), __dmul_rn(Y, P[5]));
-        }
-        g.x = gx[4]; g.y = gy[4];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) { g.corners[2 * k] = gx[k]; g.corners[2 * k + 1] = gy[k]; }
+        for (int k = 0; k < 5; ++k) geo_affine(P, __dadd_rn((double)px[k], P[6]), __dadd_rn((double)py[k], P[7]), &gx[k], &gy[k]);
     }
+    g.x = gx[4]; g.y = gy[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) { g.corners[2 * k] = gx[k]; g.corners[2 * k + 1] = gy[k]; }
     out[(size_t)tile * cap + i] = g;
+}
+
+// Sorts each tile's candidates into keys (tile stride keys_stride(cand_cap)): by confidence, else in slot order
+int sort_keys_launch(const b2d_det* cand, const int* cand_count, int cand_cap, int n, unsigned long long* keys, int by_conf,
+                     cudaStream_t stream) {
+    B2D_CHECK(cand_cap <= kMaxCand, "postprocess: candidate capacity %d exceeds the 15-bit slot field", cand_cap);
+    if (b2d_func_smem_optin((const void*)sort_keys_kernel, kSortSmemKeys * 8)) return -2;
+    int need = 1;
+    while (need < cand_cap && need < kSortSmemKeys) need <<= 1;       // keys that can occur, capped by the smem variant
+    sort_keys_kernel<<<n, kSortThreads, (size_t)need * 8, stream>>>(cand, cand_count, cand_cap, keys, keys_stride(cand_cap), by_conf);
+    B2D_LAUNCH_CHECK();
+    return 0;
 }
 
 }  // namespace
@@ -825,20 +796,13 @@ int obb_postprocess_launch(const HeadDesc* h, int n, float thr, int inclusive, f
                            int* cand_count, int cand_cap, unsigned long long* keys_scratch, float4* prm, float iou_thr, int top_k,
                            int max_det, b2d_obb* out, int* out_count, int cap, cudaStream_t stream) {
     if (n <= 0) return 0;
-    B2D_CHECK(cand_cap <= 32768, "postprocess_obb: candidate capacity %d exceeds the 15-bit slot field", cand_cap);
     B2D_CUDA(cudaMemsetAsync(cand_count, 0, sizeof(int) * n, stream));
     dim3 grid(ceil_div(h->rows_total * 4, 256), n);
     obb_head_kernel<1><<<grid, 256, 0, stream>>>(*h, thr, inclusive, scale, nullptr, cand, cand_angle, cand_count, cand_cap);
     B2D_LAUNCH_CHECK();
-    int stride = 1;
-    while (stride < cand_cap) stride <<= 1;
-    if (b2d_func_smem_optin((const void*)sort_keys_kernel, kSortSmemKeys * 8)) return -2;
-    int need = 1;
-    while (need < cand_cap && need < kSortSmemKeys) need <<= 1;
-    sort_keys_kernel<<<n, kSortThreads, (size_t)need * 8, stream>>>(cand, cand_count, cand_cap, keys_scratch, stride, (iou_thr > 0.f) || (top_k > 0));
-    B2D_LAUNCH_CHECK();
-    obb_select_kernel<<<n, kObbThreads, 0, stream>>>(cand, cand_angle, cand_count, cand_cap, keys_scratch, stride, prm, iou_thr, top_k, max_det,
-                                                     out, out_count, cap);
+    if (int rc = sort_keys_launch(cand, cand_count, cand_cap, n, keys_scratch, (iou_thr > 0.f) || (top_k > 0), stream)) return rc;
+    obb_select_kernel<<<n, kObbThreads, 0, stream>>>(cand, cand_angle, cand_count, cand_cap, keys_scratch, keys_stride(cand_cap), prm,
+                                                     iou_thr, top_k, max_det, out, out_count, cap);
     B2D_LAUNCH_CHECK();
     return 0;
 }
@@ -856,7 +820,7 @@ int decode_rows_launch(const HeadDesc* h, int n, float* rows, cudaStream_t strea
     if (n <= 0) return 0;
     const int per = (h->kind == B2D_HEAD_V8_DFL) ? 4 : 1;
     dim3 grid(ceil_div(h->rows_total * per, 256), n);
-    head_kernel<0><<<grid, 256, 0, stream>>>(*h, n, 0.f, 1, 1.f, rows, nullptr, nullptr, 0);
+    head_kernel<0><<<grid, 256, 0, stream>>>(*h, 0.f, 1, 1.f, rows, nullptr, nullptr, 0);
     B2D_LAUNCH_CHECK();
     return 0;
 }
@@ -867,7 +831,7 @@ int candidates_from_head_launch(const HeadDesc* h, int n, float thr, int inclusi
     B2D_CUDA(cudaMemsetAsync(cand_count, 0, sizeof(int) * n, stream));
     const int per = (h->kind == B2D_HEAD_V8_DFL) ? 4 : 1;
     dim3 grid(ceil_div(h->rows_total * per, 256), n);
-    head_kernel<1><<<grid, 256, 0, stream>>>(*h, n, thr, inclusive, scale, nullptr, cand, cand_count, cand_cap);
+    head_kernel<1><<<grid, 256, 0, stream>>>(*h, thr, inclusive, scale, nullptr, cand, cand_count, cand_cap);
     B2D_LAUNCH_CHECK();
     return 0;
 }
@@ -885,19 +849,10 @@ int candidates_from_rows_launch(const float* rows, int n, int num_rows, int ncol
 int select_launch(const b2d_det* cand, const int* cand_count, int cand_cap, int n, unsigned long long* keys_scratch, float iou_thr,
                   int top_k, int max_det, b2d_det* out, int* out_count, int cap, cudaStream_t stream) {
     if (n <= 0) return 0;
-    B2D_CHECK(cand_cap <= 32768, "select: candidate capacity %d exceeds the 15-bit slot field", cand_cap);
     B2D_CHECK(!(iou_thr > 0.f) || max_det <= kMaxDet, "select: max_det %d exceeds the NMS kernel's %d kept boxes per tile", max_det, kMaxDet);
-    int stride = 1;
-    while (stride < cand_cap) stride <<= 1;
-    {
-        if (b2d_func_smem_optin((const void*)sort_keys_kernel, kSortSmemKeys * 8)) return -2;
-        int need = 1;
-        while (need < cand_cap && need < kSortSmemKeys) need <<= 1;       // keys that can occur, capped by the smem variant
-        sort_keys_kernel<<<n, kSortThreads, (size_t)need * 8, stream>>>(cand, cand_count, cand_cap, keys_scratch, stride, (iou_thr > 0.f) || (top_k > 0));
-        B2D_LAUNCH_CHECK();
-    }
-    select_kernel<<<n, kSelThreads, 0, stream>>>(cand, cand_count, cand_cap, keys_scratch, stride, iou_thr, top_k, max_det, out,
-                                                 out_count, cap);
+    if (int rc = sort_keys_launch(cand, cand_count, cand_cap, n, keys_scratch, (iou_thr > 0.f) || (top_k > 0), stream)) return rc;
+    select_kernel<<<n, kSelThreads, 0, stream>>>(cand, cand_count, cand_cap, keys_scratch, keys_stride(cand_cap), iou_thr, top_k, max_det,
+                                                 out, out_count, cap);
     B2D_LAUNCH_CHECK();
     return 0;
 }

@@ -47,6 +47,12 @@ def _ptr(t: Optional[torch.Tensor]):
     return C.c_void_p(0 if t is None else t.data_ptr())
 
 
+def _default_cap(iou_thr: float, top_k: int, max_det: int, rows: int) -> int:
+    """Output records per tile when the caller gives no cap: max_det with NMS, else top_k, else every candidate the engine keeps
+    (one per row, at most 32768: the slot field of the sort keys)."""
+    return max_det if iou_thr > 0 else (top_k if top_k > 0 else min(rows, 32768))
+
+
 class Engine:
     def __init__(self, arch: str = "yolov8m", weights: Optional[Dict[str, np.ndarray]] = None, max_batch: int = 64,
                  device: int = 0, seed: int = 0, conv_impl: str = "auto", imgsz: int = 640, nc: Optional[int] = None,
@@ -227,7 +233,7 @@ class Engine:
         """Returns (dets float32 [n, cap, 8] -- view ints with .view(torch.int32) --, counts int32 [n]).  On an oriented-box engine
         dets is [n, cap, 9] ``OBB_DTYPE`` records (regularized boxes after Ultralytics' rotated NMS when iou_thr > 0)."""
         if cap is None:
-            cap = max_det if iou_thr > 0 else (top_k if top_k > 0 else min(self.num_rows if rows is None else rows.shape[1], 32768))
+            cap = _default_cap(iou_thr, top_k, max_det, self.num_rows if rows is None else rows.shape[1])
         if self.is_obb:
             if rows is not None:
                 raise ValueError("postprocess(rows=...) takes axis-aligned rows; an oriented-box engine post-processes its own head maps")
@@ -385,7 +391,7 @@ class Engine:
         n, h, w, _ = t.shape
         assert p.shape == (n, GEO_PARAMS)
         if cap is None:
-            cap = max_det if iou_thr > 0 else (top_k if top_k > 0 else min(self.num_rows, 32768))
+            cap = _default_cap(iou_thr, top_k, max_det, self.num_rows)
         out = np.zeros((n, cap), dtype=GEODET_DTYPE)
         counts = np.zeros((n,), dtype=np.int32)
         _lib.check(self.lib.b2d_detect_host(self.h, C.c_void_p(t.ctypes.data), n, h, w, RESIZE[resize], int(bgr), conf_thr,
