@@ -154,8 +154,11 @@ struct HeadDesc { HeadLevel lv[3]; int nlevels; int kind; int nc; int rows_total
 // (graph.obb_angle_channel)
 __host__ __device__ inline int obb_angle_channel(int nc) { return (64 + nc + 3) / 4 * 4; }
 
-// Candidates per tile: sort keys carry the candidate slot in a 15-bit field
-constexpr int kMaxCand = 32768;
+// Candidates per tile: one per row, and the sort keys carry the anchor and the candidate slot in 16-bit fields
+// (postprocess.cu, sort_key), so a tile may have at most this many rows
+constexpr int kMaxCand = 65536;
+// Ultralytics' max_nms: NMS looks at the best this many candidates of a tile only (both NMS kernels)
+constexpr int kMaxNms = 30000;
 // Sort keys per tile: the candidate capacity rounded up to a power of two
 static inline int keys_stride(int cand_cap) {
     int s = 1;

@@ -141,8 +141,11 @@ namespace {
 
 bool is_obb(const b2d_engine* e) { return e->head_levels > 0 && e->head.kind == B2D_HEAD_V8_OBB; }
 
+// Room for every row of a tile to be a candidate: a tile's candidates are never truncated, larger tiles are refused
 int ensure_cand(b2d_engine* e, int n, int rows) {
-    int cap = rows < kMaxCand ? rows : kMaxCand;
+    B2D_CHECK(rows <= kMaxCand, "postprocess: %d rows per tile exceed the limit of %d (the sort key's 16-bit anchor and slot fields)",
+              rows, kMaxCand);
+    const int cap = rows;
     if (e->cand && e->cand_cap >= cap && e->cand_tiles >= n) return 0;
     if (e->cand) { cudaFree(e->cand); cudaFree(e->cand_count); cudaFree(e->keys); }
     if (e->cand_angle) { cudaFree(e->cand_angle); cudaFree(e->obb_prm); e->cand_angle = nullptr; e->obb_prm = nullptr; }
@@ -741,7 +744,7 @@ int b2d_postprocess(b2d_engine* e, int n, float conf_thr, int inclusive, float i
     B2D_CHECK(!is_obb(e), "postprocess: the engine has an oriented-box head; use b2d_postprocess_obb");
     B2D_ENTER(e);
     B2D_CHECK(n > 0 && n <= e->max_batch && dets_dev && counts_dev && cap > 0, "postprocess: bad arguments");
-    if (ensure_cand(e, n, e->head.rows_total)) return -2;
+    if (int rc = ensure_cand(e, n, e->head.rows_total)) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     if (candidates_from_head_launch(&e->head, n, conf_thr, inclusive, e->conf_scale, e->cand, e->cand_count, e->cand_cap, s)) return -2;
     return select_launch(e->cand, e->cand_count, e->cand_cap, n, e->keys, iou_thr, top_k, max_det, dets_dev, counts_dev, cap, s);
@@ -752,7 +755,7 @@ int b2d_postprocess_rows(b2d_engine* e, const float* rows_dev, int n, int num_ro
     B2D_CHECK(e && rows_dev && n > 0 && num_rows > 0 && ncol >= 5 && dets_dev && counts_dev && cap > 0, "postprocess_rows: bad arguments");
     B2D_CHECK(!is_obb(e), "postprocess_rows: the engine has an oriented-box head; axis-aligned rows are not its output");
     B2D_ENTER(e);
-    if (ensure_cand(e, n, num_rows)) return -2;
+    if (int rc = ensure_cand(e, n, num_rows)) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     if (candidates_from_rows_launch(rows_dev, n, num_rows, ncol, conf_thr, inclusive, e->conf_scale, e->cand, e->cand_count, e->cand_cap, s)) return -2;
     return select_launch(e->cand, e->cand_count, e->cand_cap, n, e->keys, iou_thr, top_k, max_det, dets_dev, counts_dev, cap, s);
@@ -790,7 +793,7 @@ int b2d_postprocess_obb(b2d_engine* e, int n, float conf_thr, int inclusive, flo
     B2D_CHECK(is_obb(e), "postprocess_obb: the engine has no oriented-box head; use b2d_postprocess");
     B2D_ENTER(e);
     B2D_CHECK(n > 0 && n <= e->max_batch && dets_dev && counts_dev && cap > 0, "postprocess_obb: bad arguments");
-    if (ensure_cand(e, n, e->head.rows_total)) return -2;
+    if (int rc = ensure_cand(e, n, e->head.rows_total)) return rc;
     return obb_postprocess_launch(&e->head, n, conf_thr, inclusive, e->conf_scale, e->cand, e->cand_angle, e->cand_count, e->cand_cap, e->keys,
                                   e->obb_prm, iou_thr, top_k, max_det, dets_dev, counts_dev, cap, (cudaStream_t)stream);
 }

@@ -250,13 +250,21 @@ __device__ __forceinline__ bool iou_gt(const float4& a, float aa, const float4& 
 constexpr int kSortThreads = 1024;
 constexpr int kSortSmemKeys = 16384;
 
+// Key of candidate slot i: high word = confidence, descending; low word = anchor (16 bits) | slot (16 bits).  The confidence is
+// mapped to an unsigned that orders like the float (negatives: all bits flipped; the rest: sign bit set), after -0.0 became +0.0
+// so the two zeros tie, and complemented so that the ascending sort gives descending confidence.  Anchors are unique in a tile,
+// so equal confidences keep anchor order.  Needs anchors and slots < kMaxCand (ensure_cand refuses larger tiles).
 __device__ __forceinline__ unsigned long long sort_key(const b2d_det* tc, int i, int cnt, int by_conf) {
     if (i >= cnt) return ~0ull;
-    const unsigned a = (unsigned)tc[i].anchor & 0x1FFFFu;
-    const unsigned long long lo = ((unsigned long long)a << 15) | (unsigned long long)(i & 0x7FFF);
-    return by_conf ? (((unsigned long long)(~__float_as_uint(tc[i].conf)) << 32) | lo)     // conf desc, anchor asc
-                   : lo;                                                                    // row order
+    const unsigned long long lo = ((unsigned long long)((unsigned)tc[i].anchor & 0xFFFFu) << 16) | (unsigned)(i & 0xFFFF);
+    if (!by_conf) return lo;                                                                // row order
+    const unsigned u = __float_as_uint(__fadd_rn(tc[i].conf, 0.0f));
+    const unsigned ordered = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+    return ((unsigned long long)(~ordered) << 32) | lo;                                    // conf desc, anchor asc
 }
+
+// The candidate slot a sorted key refers to
+__device__ __forceinline__ int key_slot(unsigned long long key) { return (int)(key & 0xFFFFu); }
 
 template <int KPT>
 __device__ void bitonic_sort_regs(const b2d_det* tc, int cnt, int by_conf, unsigned long long* smem, unsigned long long* out) {
@@ -344,7 +352,7 @@ __device__ __forceinline__ void copy_top_k(const unsigned long long* keys, int c
     int m = cnt;
     if (top_k > 0 && m > top_k) m = top_k;
     if (m > cap) m = cap;
-    for (int i = threadIdx.x; i < m; i += blockDim.x) to[i] = rec((int)(keys[i] & 0x7FFF));
+    for (int i = threadIdx.x; i < m; i += blockDim.x) to[i] = rec(key_slot(keys[i]));
     if (threadIdx.x == 0) *out_count = m;
 }
 
@@ -383,6 +391,7 @@ __global__ void __launch_bounds__(kSelThreads) select_kernel(const b2d_det* __re
     // One tile has one CTA, so the work of a chunk is spread over four thread groups ("parts") of 256: part p tests candidate c
     // against the kept boxes k = p, p + 4, ... and builds word p of c's suppression mask.
     if (max_det > cap) max_det = cap;                       // max_det <= kMaxDet is checked by select_launch
+    if (cnt > kMaxNms) cnt = kMaxNms;                       // Ultralytics' max_nms cut of the sorted list
     const int c = tid & (kSelCand - 1), part = tid / kSelCand;
     if (tid == 0) s_nk = 0;
     __syncthreads();
@@ -395,7 +404,7 @@ __global__ void __launch_bounds__(kSelThreads) select_kernel(const b2d_det* __re
         float4 bx = make_float4(0.f, 0.f, 0.f, 0.f);
         float ar = 0.f;
         if (valid) {
-            d = tc[(int)(keys[i] & 0x7FFF)];
+            d = tc[key_slot(keys[i])];
             // xywh2xyxy then + cls * max_wh, as Ultralytics
             const float hw = __fmul_rn(d.w, 0.5f), hh = __fmul_rn(d.h, 0.5f);
             const float off = __fmul_rn((float)d.cls, 7680.0f);
@@ -611,7 +620,6 @@ __device__ __forceinline__ b2d_obb obb_record(const b2d_det& d, float th) {
 // shared memory, and leaves at its first suppressor (fast NMS: a suppressed box still suppresses, so the tests are independent and
 // there is no serial keep scan).  Survivors are compacted in order; the walk stops when max_det are kept.  No pair is skipped.
 constexpr int kObbThreads = 1024;
-constexpr int kMaxNms = 30000;
 
 __device__ __forceinline__ bool probiou_suppresses(const float4 pi, const float2 qi, const float4 pj, const float2 qj, float thr) {
     // batch_probiou(obb1 = box i, obb2 = box j); p = (x, y, A, B), q = (C, P)
@@ -653,7 +661,7 @@ __global__ void __launch_bounds__(kObbThreads) obb_select_kernel(const b2d_det* 
     const int m = cnt < kMaxNms ? cnt : kMaxNms;
     float4* tp = prm + (size_t)tile * keys_stride * 2;
     for (int i = tid; i < m; i += blockDim.x) {
-        const int s = (int)(keys[i] & 0x7FFF);
+        const int s = key_slot(keys[i]);
         const b2d_det d = tc[s];
         const float off = __fmul_rn((float)d.cls, 7680.0f);
         const float a = __fdiv_rn(__fmul_rn(d.w, d.w), 12.0f), b = __fdiv_rn(__fmul_rn(d.h, d.h), 12.0f);
@@ -708,7 +716,7 @@ __global__ void __launch_bounds__(kObbThreads) obb_select_kernel(const b2d_det* 
         if (alive) {
             const int slot = nk + before + __popc(bal & ((1u << (tid & 31)) - 1));
             if (slot < max_det) {
-                const int s = (int)(keys[j] & 0x7FFF);
+                const int s = key_slot(keys[j]);
                 to[slot] = obb_record(tc[s], ta[s]);
             }
         }
@@ -773,7 +781,7 @@ __global__ void __launch_bounds__(256) obb_georef_kernel(const b2d_obb* __restri
 // Sorts each tile's candidates into keys (tile stride keys_stride(cand_cap)): by confidence, else in slot order
 int sort_keys_launch(const b2d_det* cand, const int* cand_count, int cand_cap, int n, unsigned long long* keys, int by_conf,
                      cudaStream_t stream) {
-    B2D_CHECK(cand_cap <= kMaxCand, "postprocess: candidate capacity %d exceeds the 15-bit slot field", cand_cap);
+    B2D_CHECK(cand_cap <= kMaxCand, "postprocess: candidate capacity %d exceeds the sort key's 16-bit slot field", cand_cap);
     if (b2d_func_smem_optin((const void*)sort_keys_kernel, kSortSmemKeys * 8)) return -2;
     int need = 1;
     while (need < cand_cap && need < kSortSmemKeys) need <<= 1;       // keys that can occur, capped by the smem variant

@@ -48,9 +48,9 @@ def _ptr(t: Optional[torch.Tensor]):
 
 
 def _default_cap(iou_thr: float, top_k: int, max_det: int, rows: int) -> int:
-    """Output records per tile when the caller gives no cap: max_det with NMS, else top_k, else every candidate the engine keeps
-    (one per row, at most 32768: the slot field of the sort keys)."""
-    return max_det if iou_thr > 0 else (top_k if top_k > 0 else min(rows, 32768))
+    """Output records per tile when the caller gives no cap: max_det with NMS, else top_k, else one per row (every row may pass;
+    post-processing refuses tiles of more than 65536 rows)."""
+    return max_det if iou_thr > 0 else (top_k if top_k > 0 else rows)
 
 
 class Engine:

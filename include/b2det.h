@@ -168,7 +168,11 @@ int b2d_decode_rows(b2d_engine* e, int n, float* rows_dev, void* stream);
  *  - reference filter: `rows[:,4] >= thr` (inclusive=1), simple_detector.py:480, output in
  *    row order; top_k > 0 keeps the k best per tile (gpu_handler.py:173);
  *  - iou_thr > 0: Ultralytics NMS [EXT] (class-offset boxes, suppress iff IoU > thr, at most
- *    max_det per tile, output in descending confidence).
+ *    max_det per tile, output in descending confidence); like Ultralytics' max_nms, only the
+ *    30000 best candidates of a tile enter the NMS.
+ * Order: descending confidence as floats compare (+0.0 and -0.0 equal), equal confidences in
+ * ascending anchor (row) order.  Every passing row is a candidate: a tile of more than 65536
+ * rows is refused, never truncated.
  * dets_dev: [n][cap]; counts_dev: int32 [n] (number written per tile, <= cap).               */
 int b2d_postprocess(b2d_engine* e, int n, float conf_thr, int inclusive, float iou_thr, int top_k,
                     int max_det, b2d_det* dets_dev, int32_t* counts_dev, int cap, void* stream);
