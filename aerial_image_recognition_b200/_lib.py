@@ -58,6 +58,8 @@ SIGNATURES = {
     "b2d_seam_closure": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_double, c_int, c_void_p, c_void_p]),
     "b2d_utm_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "b2d_cut_windows": (c_int, [c_void_p, c_void_p, c_int, c_int, c_ll, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "b2d_resize_windows": (c_int, [c_void_p, c_void_p, c_int, c_int, c_ll, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p,
+                                   c_void_p]),
     "b2d_resize_table": (c_int, [c_int, c_int, c_int, c_void_p, c_void_p, P(c_int)]),
     "b2d_tta_clahe": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_double, c_int, c_int, c_void_p, c_void_p]),
     "b2d_tta_lut": (c_int, [c_void_p, c_void_p, c_int, c_ll, c_void_p, c_int, c_void_p, c_void_p]),

@@ -135,6 +135,32 @@ int upsample2x_launch(const __nv_bfloat16* src, int h, int w, int src_cs, int sr
 // ---------------------------------------------------------------------------------------
 // pre / post processing
 // ---------------------------------------------------------------------------------------
+// OpenCV INTER_LINEAR (cv::resize, 8-bit): source taps (i0, i1) and 11-bit coefficients (a0, a1) of output index d, where
+// scale = in_size / out_size.  Horizontal taps outside the image zero the fraction (fx = 0, sx clamped); the vertical pass
+// keeps the fraction and clamps the two row indices separately.  The two rules give the same bytes on every down-scale
+// and differ in the edge rows of an up-scale.  One IEEE rounding per operation on host and device (no contraction), so
+// the host tables and the device-computed coefficients are the same numbers.
+__host__ __device__ inline void cv2_linear_coef(int d, double scale, int in_size, int vertical, int* i0, int* i1, int* a0, int* a1) {
+#ifdef __CUDA_ARCH__
+    float f = (float)__dadd_rn(__dmul_rn(__dadd_rn((double)d, 0.5), scale), -0.5);
+#else
+    float f = (float)(((double)d + 0.5) * scale - 0.5);     // x86-64 host code has no FMA to contract into
+#endif
+    int s = (int)floorf(f);
+    f -= (float)s;
+    if (vertical) {
+        *i0 = s < 0 ? 0 : (s > in_size - 1 ? in_size - 1 : s);
+        *i1 = s + 1 < 0 ? 0 : (s + 1 > in_size - 1 ? in_size - 1 : s + 1);
+    } else {
+        if (s < 0) { f = 0.f; s = 0; }
+        if (s >= in_size - 1) { f = 0.f; s = in_size - 1; }
+        *i0 = s;
+        *i1 = s + 1 < in_size ? s + 1 : in_size - 1;
+    }
+    *a0 = (int)lrintf((1.f - f) * 2048.f);
+    *a1 = (int)lrintf(f * 2048.f);
+}
+
 struct ResizeTables {     // device tables for one (mode, in_h, in_w, out)
     int mode, in_h, in_w, out_h, out_w, left, top;   // left/top: letterbox placement
     int ksize_x, ksize_y;
@@ -144,6 +170,11 @@ struct ResizeTables {     // device tables for one (mode, in_h, in_w, out)
 };
 int preprocess_launch(const ResizeTables* t, const uint8_t* src, int n, int pitch, long long img_stride,
                       int bgr, int out_kind, void* dst, int out_size, cudaStream_t stream);
+// host: the cv2 INTER_LINEAR table of one axis (cv2_linear_coef for every output index), ofs / coef [out_size][2]
+void cv2_linear_axis_table(int in_size, int out_size, int vertical, int32_t* ofs, int32_t* coef);
+// mosaic windows (x0, y0, w0, h0) -> cv2 INTER_LINEAR by imgsz / win, centred on an imgsz x imgsz canvas of `fill`
+int resize_windows_launch(const uint8_t* mosaic, int mh, int mw, long long pitch, const int32_t* origins, int n, int win, int imgsz,
+                          int fill, int bgr, int out_kind, void* dst, cudaStream_t stream);
 
 int input_from_f32_launch(const float* src, int n, int h, int w, void* dst, cudaStream_t stream, int f16 = 0);
 

@@ -207,7 +207,10 @@ int get_tables(b2d_engine* e, int mode, int h, int w, int out, int n, const Resi
         t.ksize_x = kx; t.ksize_y = ky;
         std::vector<int32_t> xb(2 * (size_t)t.out_w), xk((size_t)kx * t.out_w), yb(2 * (size_t)t.out_h), yk((size_t)ky * t.out_h);
         B2D_CHECK(b2d_resize_table(tmode, w, t.out_w, xb.data(), xk.data(), &kx) == 0, "resize table failed");
-        B2D_CHECK(b2d_resize_table(tmode, h, t.out_h, yb.data(), yk.data(), &ky) == 0, "resize table failed");
+        if (tmode == B2D_RESIZE_CV2_LINEAR)       // the row taps follow OpenCV's vertical rule (cv2_linear_coef)
+            cv2_linear_axis_table(h, t.out_h, 1, yb.data(), yk.data());
+        else
+            B2D_CHECK(b2d_resize_table(tmode, h, t.out_h, yb.data(), yk.data(), &ky) == 0, "resize table failed");
         if (upload_i32(&t.xb, xb) || upload_i32(&t.xk, xk) || upload_i32(&t.yb, yb) || upload_i32(&t.yk, yk)) return -2;
         if (mode == B2D_RESIZE_PIL_BICUBIC && t.in_w != t.out_w) {
             t.tmp_bytes = (size_t)n * t.in_h * t.out_w * 3;
@@ -849,6 +852,27 @@ int b2d_cut_windows(b2d_engine* e, const uint8_t* mosaic_dev, int mh, int mw, lo
     B2D_CHECK(e && mosaic_dev && origins_dev && dst_dev && n > 0, "cut_windows: bad arguments");
     B2D_ENTER(e);
     return cut_windows_launch(mosaic_dev, mh, mw, pitch, origins_dev, n, win, fill, dst_dev, (cudaStream_t)stream);
+}
+
+int b2d_resize_windows(b2d_engine* e, const uint8_t* mosaic_dev, int mh, int mw, long long pitch, const int32_t* origins_dev, int n,
+                       int win, int fill, int bgr, int out_kind, void* dst_dev, void* stream) {
+    B2D_CHECK(e && mosaic_dev && origins_dev && n > 0, "resize_windows: bad arguments");
+    B2D_CHECK(win > 0, "resize_windows: window size %d must be positive", win);
+    B2D_CHECK(mh > 0 && mw > 0 && pitch >= 3LL * mw, "resize_windows: mosaic %dx%d with pitch %lld", mh, mw, pitch);
+    B2D_CHECK(fill >= 0 && fill <= 255, "resize_windows: fill %d outside 0..255", fill);
+    B2D_ENTER(e);
+    const int imgsz = e->bufs.empty() ? 640 : e->bufs[0].h;
+    if (dst_dev == nullptr) {
+        if (out_kind == B2D_OUT_BF16_NHWC4 && e->f16) out_kind = B2D_OUT_F16_NHWC4;   // the engine's own input format
+        B2D_CHECK((out_kind == B2D_OUT_BF16_NHWC4 || out_kind == B2D_OUT_F16_NHWC4) && !e->bufs.empty() && e->bufs[0].c == 4 && !e->bufs[0].f32,
+                  "resize_windows: dst NULL needs the planned 16-bit NHWC4 input buffer");
+        B2D_CHECK(n <= e->max_batch, "resize_windows: n=%d exceeds max_batch %d", n, e->max_batch);
+        dst_dev = e->bufs[0].ptr;
+    }
+    B2D_CHECK(out_kind == B2D_OUT_U8_NHWC || out_kind == B2D_OUT_BF16_NHWC4 || out_kind == B2D_OUT_F16_NHWC4,
+              "resize_windows: out_kind %d is neither uint8 NHWC nor a 16-bit NHWC4 network input", out_kind);
+    return resize_windows_launch(mosaic_dev, mh, mw, pitch, origins_dev, n, win, imgsz, fill, bgr, out_kind, dst_dev,
+                                 (cudaStream_t)stream);
 }
 
 int b2d_set_conf_scale(b2d_engine* e, float scale) {

@@ -18,6 +18,7 @@
 // L1/L2-resident rows.
 #include "common.cuh"
 
+#include <limits.h>
 #include <math.h>
 #include <string.h>
 #include <vector>
@@ -239,6 +240,127 @@ __global__ void __launch_bounds__(256) cut_windows_kernel(const uint8_t* __restr
     o[0] = r; o[1] = g; o[2] = b;
 }
 
+// ---- windows of any size: cut + cv2 INTER_LINEAR + centred letterbox, one launch per batch ----------------------
+// A CTA owns one window and walks bands of kBandRows canvas rows.  Per band, warp 0 computes each row's vertical taps
+// and maps the distinct source rows they touch to slots; those rows are copied into shared memory with 16-byte loads,
+// kStageRows at a time, and resampled horizontally into int16 rows (the `s >> 4` of the vertical sum); then every
+// thread writes canvas pixels from two slot rows.  Each source row a band needs is read once per band (a row shared
+// by two bands is read twice); the horizontal taps are computed once per CTA.  All coefficients come from
+// cv2_linear_coef, so nothing is uploaded per window size.
+constexpr int kBandRows = 4;
+constexpr int kBandSlots = 2 * kBandRows;   // distinct source rows a band can touch
+constexpr int kStageRows = 4;
+
+struct WindowGeom { int nw, nh, left, top; };
+
+// The geometry of mosaic.window_geometry: one gain g = imgsz / win, Python round() = rint()
+__device__ __forceinline__ WindowGeom window_geom(int w0, int h0, int win, int imgsz) {
+    const double g = __ddiv_rn((double)imgsz, (double)win);
+    WindowGeom r;
+    r.nw = max(1, (int)rint(__dmul_rn((double)w0, g)));
+    r.nh = max(1, (int)rint(__dmul_rn((double)h0, g)));
+    r.left = (int)rint(__dadd_rn((double)(imgsz - r.nw) * 0.5, -0.1));
+    r.top = (int)rint(__dadd_rn((double)(imgsz - r.nh) * 0.5, -0.1));
+    return r;
+}
+
+__host__ __device__ inline int raw_pitch(int win) { return (win * 3 + 15 + 15) / 16 * 16; }   // one source row + its 16-byte misalignment
+
+static inline size_t resize_windows_smem(int win, int imgsz) {
+    return (size_t)imgsz * sizeof(int4) + (size_t)kBandSlots * imgsz * sizeof(uint2) + (size_t)kStageRows * raw_pitch(win);
+}
+
+__global__ void __launch_bounds__(256) resize_windows_kernel(const uint8_t* __restrict__ mosaic, int mh, int mw, long long pitch,
+                                                             const int32_t* __restrict__ origins, int win, int imgsz, int groups,
+                                                             int fill, int bgr, int out_kind, void* dst) {
+    extern __shared__ __align__(16) uint8_t smem[];
+    int4* xtab = reinterpret_cast<int4*>(smem);                                    // [imgsz] byte offsets of the two taps, a0, a1
+    uint2* hrow = reinterpret_cast<uint2*>(smem + (size_t)imgsz * sizeof(int4));   // [kBandSlots][imgsz] three int16 per pixel
+    uint8_t* raw = smem + (size_t)imgsz * (sizeof(int4) + kBandSlots * sizeof(uint2));   // [kStageRows][rp] source bytes
+    __shared__ int4 vtab[kBandRows];            // slot of each tap, b0, b1
+    __shared__ int slot_row[kBandSlots];
+    __shared__ int nslots;
+    const int rp = raw_pitch(win);
+    const int i = blockIdx.x / groups, grp = blockIdx.x % groups;
+    const int x0 = origins[4 * i], y0 = origins[4 * i + 1], w0 = origins[4 * i + 2], h0 = origins[4 * i + 3];
+    const bool ok = w0 >= 1 && w0 <= win && h0 >= 1 && h0 <= win && x0 >= 0 && y0 >= 0 && x0 <= mw - w0 && y0 <= mh - h0;
+    WindowGeom gm = window_geom(ok ? w0 : win, ok ? h0 : win, win, imgsz);
+    if (!ok) gm.nw = gm.nh = 0;             // a window the caller should have refused: all fill, nothing read
+    const double sx = __ddiv_rn((double)w0, (double)gm.nw), sy = __ddiv_rn((double)h0, (double)gm.nh);
+    for (int rx = threadIdx.x; rx < gm.nw; rx += blockDim.x) {
+        int i0, i1, a0, a1;
+        cv2_linear_coef(rx, sx, w0, 0, &i0, &i1, &a0, &a1);
+        xtab[rx] = make_int4(3 * i0, 3 * i1, a0, a1);
+    }
+    const int nbands = (imgsz + kBandRows - 1) / kBandRows;
+    const uint8_t fb = (uint8_t)fill;
+    for (int band = grp; band < nbands; band += groups) {
+        const int yb = band * kBandRows;
+        if (threadIdx.x < 32) {
+            // lane t < 2 kBandRows holds tap (t & 1) of band row t >> 1; inactive taps (pad rows) hold INT_MAX
+            const int lane = threadIdx.x, ry = yb + (lane >> 1) - gm.top;
+            int r0 = INT_MAX, r1 = INT_MAX, b0 = 0, b1 = 0;
+            if (lane < kBandSlots && yb + (lane >> 1) < imgsz && ry >= 0 && ry < gm.nh) cv2_linear_coef(ry, sy, h0, 1, &r0, &r1, &b0, &b1);
+            const int v = (lane & 1) ? r1 : r0;
+            int first = v != INT_MAX, rank = 0;
+            for (int k = 0; k < kBandSlots; ++k) {
+                const int u = __shfl_sync(0xffffffffu, v, k);
+                int ufirst = u != INT_MAX;
+                for (int j = 0; j < k; ++j) ufirst &= __shfl_sync(0xffffffffu, v, j) != u;
+                if (k < lane && u == v) first = 0;
+                if (ufirst && u < v) ++rank;
+            }
+            if (lane < kBandSlots && first) slot_row[rank] = v;
+            const int slot_other = __shfl_xor_sync(0xffffffffu, rank, 1);
+            const unsigned firsts = __ballot_sync(0xffffffffu, lane < kBandSlots && first);
+            if (lane < kBandSlots && !(lane & 1)) vtab[lane >> 1] = make_int4(rank, slot_other, b0, b1);
+            if (lane == 0) nslots = __popc(firsts);
+        }
+        __syncthreads();
+        const int ns = nslots;
+        for (int s0 = 0; s0 < ns; s0 += kStageRows) {
+            const int cnt = min(kStageRows, ns - s0);
+            // 16-byte loads of the aligned run that holds bytes [x0 * 3, (x0 + w0) * 3) of each staged row.  The bytes read
+            // before and after the row share a 16-byte block with bytes of the row, so they lie inside the mosaic's allocation.
+            const int nch_max = (w0 * 3 + 30) >> 4;
+            for (int p = threadIdx.x; p < cnt * nch_max; p += blockDim.x) {
+                const int q = p / nch_max, c = p - q * nch_max;
+                const uintptr_t a = (uintptr_t)(mosaic + (long long)(y0 + slot_row[s0 + q]) * pitch + (long long)x0 * 3);
+                if (c < (int)(((a & 15) + w0 * 3 + 15) >> 4))
+                    reinterpret_cast<uint4*>(raw + q * rp)[c] = __ldg(reinterpret_cast<const uint4*>(a & ~(uintptr_t)15) + c);
+            }
+            __syncthreads();
+            for (int p = threadIdx.x; p < cnt * gm.nw; p += blockDim.x) {
+                const int q = p / gm.nw, rx = p - q * gm.nw;
+                const uint8_t* a = mosaic + (long long)(y0 + slot_row[s0 + q]) * pitch + (long long)x0 * 3;
+                const uint8_t* r = raw + q * rp + ((uintptr_t)a & 15);
+                const int4 t = xtab[rx];
+                const int c0 = (r[t.x] * t.z + r[t.y] * t.w) >> 4;
+                const int c1 = (r[t.x + 1] * t.z + r[t.y + 1] * t.w) >> 4;
+                const int c2 = (r[t.x + 2] * t.z + r[t.y + 2] * t.w) >> 4;
+                hrow[(size_t)(s0 + q) * imgsz + rx] = make_uint2((uint32_t)c0 | ((uint32_t)c1 << 16), (uint32_t)c2);
+            }
+            __syncthreads();
+        }
+        for (int p = threadIdx.x; p < kBandRows * imgsz; p += blockDim.x) {
+            const int t = p / imgsz, x = p - t * imgsz, y = yb + t;
+            if (y >= imgsz) break;
+            const int rx = x - gm.left, ry = y - gm.top;
+            uint8_t o[3] = {fb, fb, fb};
+            if (rx >= 0 && rx < gm.nw && ry >= 0 && ry < gm.nh) {
+                const int4 v = vtab[t];
+                const uint2 h0v = hrow[(size_t)v.x * imgsz + rx], h1v = hrow[(size_t)v.y * imgsz + rx];
+                const int s0[3] = {(int)(h0v.x & 0xffffu), (int)(h0v.x >> 16), (int)h0v.y};
+                const int s1[3] = {(int)(h1v.x & 0xffffu), (int)(h1v.x >> 16), (int)h1v.y};
+#pragma unroll
+                for (int c = 0; c < 3; ++c) o[c] = clip8((((v.z * s0[c]) >> 16) + ((v.w * s1[c]) >> 16) + 2) >> 2);
+            }
+            emit_pixel(out_kind, dst, i, y, x, imgsz, imgsz, o[0], o[1], o[2], bgr);
+        }
+        __syncthreads();
+    }
+}
+
 
 // ---- f32 NCHW in [0,1] (the tensor the reference hands to session.run) -> 16-bit NHWC4 network input ---------
 __global__ void __launch_bounds__(256) input_from_f32_kernel(const float* __restrict__ src, int n, int h, int w, uint2* __restrict__ dst,
@@ -330,6 +452,30 @@ int cut_windows_launch(const uint8_t* mosaic, int mh, int mw, long long pitch, c
     return 0;
 }
 
+int resize_windows_launch(const uint8_t* mosaic, int mh, int mw, long long pitch, const int32_t* origins, int n, int win, int imgsz,
+                          int fill, int bgr, int out_kind, void* dst, cudaStream_t stream) {
+    if (n <= 0) return 0;
+    const size_t smem = resize_windows_smem(win, imgsz);
+    int dev = 0, optin = 0;
+    cudaFuncAttributes fa;
+    B2D_CUDA(cudaGetDevice(&dev));
+    B2D_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    B2D_CUDA(cudaFuncGetAttributes(&fa, (const void*)resize_windows_kernel));
+    const int dyn_max = optin - (int)fa.sharedSizeBytes;
+    B2D_CHECK(smem <= (size_t)dyn_max, "resize_windows: window %d on a %d canvas needs %zu bytes of shared memory, the device allows %d",
+              win, imgsz, smem, dyn_max);
+    // opted in once per device at the largest size, so a later call with a larger window needs no second opt-in
+    if (smem > 48 * 1024 && b2d_func_smem_optin((const void*)resize_windows_kernel, dyn_max)) return -2;
+    // a CTA walks every groups-th band of one window: the horizontal taps are computed once per CTA, and a batch of
+    // 64 windows is 1024 CTAs
+    const int nbands = (imgsz + kBandRows - 1) / kBandRows;
+    const int groups = nbands < 16 ? nbands : 16;
+    B2D_CHECK((long long)n * groups < (1LL << 31), "resize_windows: %d windows", n);
+    resize_windows_kernel<<<n * groups, 256, smem, stream>>>(mosaic, mh, mw, pitch, origins, win, imgsz, groups, fill, bgr, out_kind, dst);
+    B2D_LAUNCH_CHECK();
+    return 0;
+}
+
 // ---------------------------------------------------------------------------------------------
 // host-side coefficient tables (same arithmetic as Pillow's precompute_coeffs / normalize_coeffs_8bpc
 // and OpenCV's resize() table set-up; mirrored in aerial_image_recognition_b200/resample.py)
@@ -381,20 +527,18 @@ extern "C" int b2d_resize_table(int mode, int in_size, int out_size, int32_t* bo
     if (mode == B2D_RESIZE_CV2_LINEAR) {
         if (ksize_out) *ksize_out = 2;
         if (!bounds_out || !coef_out) return 0;
-        const double scale = (double)in_size / (double)out_size;
-        for (int d = 0; d < out_size; ++d) {
-            float f = (float)((d + 0.5) * scale - 0.5);
-            int s = (int)floorf(f);
-            f -= (float)s;
-            if (s < 0) { f = 0.f; s = 0; }
-            if (s >= in_size - 1) { f = 0.f; s = in_size - 1; }
-            const float c0 = 1.f - f;
-            bounds_out[2 * d] = s;
-            bounds_out[2 * d + 1] = s + 1 < in_size ? s + 1 : in_size - 1;
-            coef_out[2 * d] = (int32_t)lrintf(c0 * 2048.f);
-            coef_out[2 * d + 1] = (int32_t)lrintf(f * 2048.f);
-        }
+        cv2_linear_axis_table(in_size, out_size, 0, bounds_out, coef_out);
         return 0;
     }
     return -1;
+}
+
+void cv2_linear_axis_table(int in_size, int out_size, int vertical, int32_t* ofs, int32_t* coef) {
+    const double scale = (double)in_size / (double)out_size;
+    for (int d = 0; d < out_size; ++d) {
+        int i0, i1, a0, a1;
+        cv2_linear_coef(d, scale, in_size, vertical, &i0, &i1, &a0, &a1);
+        ofs[2 * d] = i0; ofs[2 * d + 1] = i1;
+        coef[2 * d] = a0; coef[2 * d + 1] = a1;
+    }
 }

@@ -308,6 +308,38 @@ class Engine:
                                             _ptr(origins.contiguous()), n, win, fill, _ptr(out), self.stream), "cut_windows")
         return out
 
+    def resize_windows(self, mosaic: torch.Tensor, origins, win: int, fill: int = 114, bgr: bool = False, out: str = "engine", *,
+                       checked: bool = False) -> Optional[torch.Tensor]:
+        """Windows of any size ``win`` resampled from the mosaic into ``imgsz`` x ``imgsz`` canvases in one launch
+        (``mosaic.window_geometry``: one gain ``imgsz / win``, cv2 INTER_LINEAR, centred on ``fill``).  mosaic uint8 CUDA
+        [H, W, 3] (row pitch may exceed 3 W); origins int32 [n, 4] = (x0, y0, w0, h0), NumPy or CUDA.  out='engine' fills the
+        network input (n <= max_batch) and returns None; 'u8' returns uint8 [n, imgsz, imgsz, 3].  The windows are checked
+        against ``win`` and the mosaic first (which reads CUDA origins back to the host); ``checked=True`` skips that for
+        origins the caller has already checked with ``mosaic.check_windows``."""
+        from .mosaic import check_windows
+        assert mosaic.dtype == torch.uint8 and mosaic.is_cuda and mosaic.dim() == 3 and mosaic.shape[2] == 3
+        assert mosaic.stride(2) == 1 and mosaic.stride(1) == 3
+        if win <= 0:
+            raise ValueError(f"resize_windows: window size {win} must be positive")
+        if not checked:
+            check_windows(origins.cpu().numpy() if isinstance(origins, torch.Tensor) else np.asarray(origins), win,
+                          mosaic.shape[0], mosaic.shape[1])
+        if not isinstance(origins, torch.Tensor):
+            origins = torch.from_numpy(np.ascontiguousarray(origins, dtype=np.int32)).to(self.device)
+        assert origins.dtype == torch.int32 and origins.is_cuda and origins.dim() == 2 and origins.shape[1] == 4
+        origins = origins.contiguous()
+        n = origins.shape[0]
+        S = self.imgsz
+        if out == "u8":
+            dst, kind = torch.empty((n, S, S, 3), dtype=torch.uint8, device=self.device), 2
+        elif out == "engine":
+            dst, kind = None, 0
+        else:
+            raise ValueError(f"resize_windows: out must be 'engine' or 'u8', not {out!r}")
+        _lib.check(self.lib.b2d_resize_windows(self.h, _ptr(mosaic), mosaic.shape[0], mosaic.shape[1], mosaic.stride(0), _ptr(origins),
+                                               n, win, fill, int(bgr), kind, _ptr(dst), self.stream), "resize_windows")
+        return dst
+
     # ---- test-time-augmentation views (gpu_handler.py:94-140, gpu_handler_archive.py:67-122) ---------
     def _u8(self, images: torch.Tensor) -> torch.Tensor:
         assert images.dtype == torch.uint8 and images.is_cuda and images.dim() == 4 and images.shape[3] == 3

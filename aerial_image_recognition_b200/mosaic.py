@@ -8,8 +8,10 @@ Ancestor in the reference: the notebook loop at ``x_arch/02_analyze_images:1 (ce
 (``simple_detector.py:540-596``).  BASELINE config C4: 40k x 40k, window 640, stride 512.
 
 Decisions where the reference leaves a choice (stated in DESIGN.md):
-* windows are model-sized (640) so no resampling happens; edge windows are clipped like the
-  notebook's ``min()`` and centred on a 114 canvas (Ultralytics LetterBox without up-scaling);
+* windows are model-sized (640) by default, so no resampling happens; edge windows are clipped like the
+  notebook's ``min()`` and centred on a 114 canvas (Ultralytics LetterBox without up-scaling).  Any other
+  window size is resampled by one gain ``imgsz / win`` for every window (``window_geometry``), so an object
+  has the same size in the network input wherever it lies in the mosaic;
 * the window grid is y-outer / x-inner, and that order is the global tie-break of the dedup;
 * shards are contiguous bands of window rows (fewest seams).  Each window belongs to exactly one
   rank, so the only cross-rank interaction is the dedup of detections that sit in the overlap
@@ -82,17 +84,53 @@ def seam_flags_device(py, rank: int, covers: Sequence[Tuple[int, int]], margin_p
     return flag.to(torch.uint8)
 
 
-def affine_params(windows: np.ndarray, geotransform: Sequence[float], win: int = 640) -> np.ndarray:
+def window_geometry(windows: np.ndarray, win: int, imgsz: int):
+    """Letterbox geometry of every window at one gain ``g = imgsz / win``: (new_w, new_h, left, top) int64 [n] each, and g.
+
+    Ultralytics LetterBox (center=True) with ``r = g``: ``new = max(1, round(w0 * g))``, ``left = round((imgsz - new_w) / 2 - 0.1)``
+    (Python ``round`` = ``rint``).  This is Ultralytics' own ``r = min(imgsz / h0, imgsz / w0)`` on every window clipped on at
+    most one axis; a corner window clipped on both keeps the gain of its neighbours, so objects keep one scale across the
+    mosaic.  ``max(1, ...)`` keeps the one-pixel slivers of a grid with ``W % stride == 1``.  ``b2d_resize_windows`` restates it."""
+    w = np.asarray(windows)
+    g = imgsz / win
+    new_w = np.maximum(1, np.rint(w[:, 2].astype(np.float64) * g)).astype(np.int64)
+    new_h = np.maximum(1, np.rint(w[:, 3].astype(np.float64) * g)).astype(np.int64)
+    left = np.rint((imgsz - new_w) / 2 - 0.1).astype(np.int64)
+    top = np.rint((imgsz - new_h) / 2 - 0.1).astype(np.int64)
+    return new_w, new_h, left, top, g
+
+
+def check_windows(windows: np.ndarray, win: int, height: int, width: int) -> None:
+    """Raise ValueError unless every window has 1 <= w0, h0 <= win and lies inside a height x width mosaic."""
+    if win <= 0:
+        raise ValueError(f"window size {win} must be positive")
+    w = np.asarray(windows, dtype=np.int64).reshape(-1, 4)
+    x0, y0, w0, h0 = w.T
+    bad = (w0 < 1) | (w0 > win) | (h0 < 1) | (h0 > win) | (x0 < 0) | (y0 < 0) | (x0 + w0 > width) | (y0 + h0 > height)
+    if bad.any():
+        k = int(np.flatnonzero(bad)[0])
+        raise ValueError(f"window {k} (x0, y0, w0, h0) = {tuple(int(v) for v in w[k])} needs 1 <= w0, h0 <= {win} and to lie "
+                         f"inside the {height} x {width} mosaic")
+
+
+def affine_params(windows: np.ndarray, geotransform: Sequence[float], win: int = 640, imgsz: Optional[int] = None) -> np.ndarray:
     """float64 [n,16] georef parameters for B2D_GEO_AFFINE: gt[6], win_x, win_y, pad_x, pad_y, gain,
-    w0, h0 (the letterbox undo of Ultralytics ``scale_boxes``; gain is 1 for model-sized windows)."""
+    w0, h0 (the letterbox undo of Ultralytics ``scale_boxes``).  ``imgsz=None`` means model-sized windows: gain 1 and the
+    centring pad.  With ``imgsz`` the pad and gain are ``window_geometry``'s."""
     n = len(windows)
     p = np.zeros((n, 16), dtype=np.float64)
     p[:, 0:6] = np.asarray(geotransform, dtype=np.float64)
     p[:, 6] = windows[:, 0]
     p[:, 7] = windows[:, 1]
-    p[:, 8] = (win - windows[:, 2]) // 2
-    p[:, 9] = (win - windows[:, 3]) // 2
-    p[:, 10] = 1.0
+    if imgsz is None:
+        p[:, 8] = (win - windows[:, 2]) // 2
+        p[:, 9] = (win - windows[:, 3]) // 2
+        p[:, 10] = 1.0
+    else:
+        _, _, left, top, g = window_geometry(windows, win, imgsz)
+        p[:, 8] = left
+        p[:, 9] = top
+        p[:, 10] = g
     p[:, 11] = windows[:, 2]
     p[:, 12] = windows[:, 3]
     return p
@@ -180,14 +218,24 @@ class MosaicDetector:
         local[:, 1] -= y_offset
         # every per-window table goes to the device once; the batch loop below queues kernels only (no host
         # synchronisation: a boolean-mask gather per batch would stall the launch queue ~100 times per mosaic)
-        params_all = torch.from_numpy(affine_params(windows, self.gt, self.win)).to(dev)
+        resample = self.win != eng.imgsz
+        if resample:
+            # windows of another size are resampled from the mosaic straight into the network input: checked once here,
+            # since the per-batch launches below leave the origins on the device
+            check_windows(local, self.win, mosaic.shape[0], mosaic.shape[1])
+        params_all = torch.from_numpy(affine_params(windows, self.gt, self.win, eng.imgsz if resample else None)).to(dev)
         org_all = torch.from_numpy(local).to(dev)
         ids_all = torch.from_numpy(ids).to(dev)
         for s in range(0, len(windows), B):
             e = min(s + B, len(windows))
             n = e - s
-            tiles = eng.cut_windows(mosaic, org_all[s:e], self.win, self.fill)
-            dets, counts = eng.infer(tiles, "identity", False, self.nms_conf, False, self.iou, 0, self.max_det)
+            if resample:
+                eng.resize_windows(mosaic, org_all[s:e], self.win, self.fill, checked=True)
+                eng.forward(n)
+                dets, counts = eng.postprocess(n, self.nms_conf, False, self.iou, 0, self.max_det)
+            else:
+                tiles = eng.cut_windows(mosaic, org_all[s:e], self.win, self.fill)
+                dets, counts = eng.infer(tiles, "identity", False, self.nms_conf, False, self.iou, 0, self.max_det)
             geo = eng.georef(dets, counts, params_all[s:e], "affine")
             outs.append((geo, dets, counts, ids_all[s:e]))
         if not outs:

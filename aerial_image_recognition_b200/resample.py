@@ -72,13 +72,15 @@ def pil_bicubic_table(in_size: int, out_size: int) -> Tuple[np.ndarray, np.ndarr
 
 
 @lru_cache(maxsize=64)
-def cv2_linear_table(in_size: int, out_size: int) -> Tuple[np.ndarray, np.ndarray]:
-    """(ofs int32 [out,2] = (i0, i1), coef int16 [out,2]) for one axis.
+def cv2_linear_table(in_size: int, out_size: int, vertical: bool = False) -> Tuple[np.ndarray, np.ndarray]:
+    """(ofs int32 [out,2] = (i0, i1), coef int16 [out,2]) for one axis (``cv2_linear_coef`` in ``csrc/common.cuh``).
 
-    The same table serves the horizontal and the vertical pass: OpenCV clamps the
-    horizontal taps by zeroing the fraction and the vertical taps by clipping the
-    row index, which coincide for every size where ``fx`` stays inside the image
-    (all down-scales); the index clamp below reproduces both.
+    OpenCV clamps the two passes differently.  Horizontally, a tap outside the
+    image zeroes the fraction and clamps the index.  Vertically
+    (``vertical=True``), the fraction is kept and the two row indices are
+    clamped separately.  The tables agree on every down-scale and differ in the
+    edge rows of an up-scale, where the vertical sum's two ``>> 16`` truncations
+    round differently.
     """
     scale = np.float64(in_size) / np.float64(out_size)
     ofs = np.zeros((out_size, 2), dtype=np.int32)
@@ -87,14 +89,17 @@ def cv2_linear_table(in_size: int, out_size: int) -> Tuple[np.ndarray, np.ndarra
         f = np.float32((d + 0.5) * scale - 0.5)
         s = int(math.floor(float(f)))
         f = np.float32(f - np.float32(s))
-        if s < 0:
-            f, s = np.float32(0.0), 0
-        if s >= in_size - 1:
-            f, s = np.float32(0.0), in_size - 1
+        if vertical:
+            ofs[d] = (min(max(s, 0), in_size - 1), min(max(s + 1, 0), in_size - 1))
+        else:
+            if s < 0:
+                f, s = np.float32(0.0), 0
+            if s >= in_size - 1:
+                f, s = np.float32(0.0), in_size - 1
+            ofs[d] = (s, min(s + 1, in_size - 1))
         c0 = np.float32(1.0) - f
         a0 = int(np.rint(np.float32(c0 * np.float32(2048.0))))
         a1 = int(np.rint(np.float32(f * np.float32(2048.0))))
-        ofs[d] = (s, min(s + 1, in_size - 1))
         coef[d] = (a0, a1)
     return ofs, coef
 
@@ -136,7 +141,7 @@ def emulate_pil_bicubic(img: np.ndarray, out_h: int, out_w: int) -> np.ndarray:
 def emulate_cv2_linear(img: np.ndarray, out_h: int, out_w: int) -> np.ndarray:
     h, w, c = img.shape
     xo, xa = cv2_linear_table(w, out_w)
-    yo, yb = cv2_linear_table(h, out_h)
+    yo, yb = cv2_linear_table(h, out_h, vertical=True)
     s = img.astype(np.int32)
     rows = s[:, xo[:, 0], :] * xa[:, 0].astype(np.int32)[None, :, None] + s[:, xo[:, 1], :] * xa[:, 1].astype(np.int32)[None, :, None]
     r0 = rows[yo[:, 0]] >> 4

@@ -246,6 +246,18 @@ int b2d_utm_forward(b2d_engine* e, const double* lon_dev, const double* lat_dev,
 int b2d_cut_windows(b2d_engine* e, const uint8_t* mosaic_dev, int mh, int mw, long long pitch,
                     const int32_t* origins_dev, int n, int win, int fill, uint8_t* dst_dev, void* stream);
 
+/* Windows of any size `win`, resampled from the mosaic straight into an imgsz x imgsz canvas (imgsz = the
+ * engine's input side) in one launch: Ultralytics LetterBox with one gain g = imgsz / win for every window,
+ * new_w = max(1, rint(w0 g)), left = rint((imgsz - new_w) / 2 - 0.1) (same for h / top), cv2 INTER_LINEAR from
+ * w0 x h0 to new_w x new_h, the rest `fill`.  At g = 1 the bytes equal b2d_cut_windows'.  origins_dev as there;
+ * `bgr` swaps R and B.  out_kind B2D_OUT_U8_NHWC: dst uint8 [n][imgsz][imgsz][3].  B2D_OUT_BF16_NHWC4 (or
+ * B2D_OUT_F16_NHWC4) with dst_dev == NULL writes the engine's own input buffer (raw pixel values, n <= max_batch).
+ * The origins stay on the device, so they are not checked here: a window with w0 or h0 outside 1..win, or one
+ * reaching outside the mosaic, comes out as a canvas of `fill` (Engine.resize_windows refuses them).            */
+int b2d_resize_windows(b2d_engine* e, const uint8_t* mosaic_dev, int mh, int mw, long long pitch,
+                       const int32_t* origins_dev, int n, int win, int fill, int bgr, int out_kind, void* dst_dev,
+                       void* stream);
+
 /* Host-only: the integer coefficient table one axis of b2d_preprocess uses (mode PIL_BICUBIC or
  * CV2_LINEAR).  bounds_out int32 [out][2], coef_out int32 [out][ksize]; pass NULLs to query ksize. */
 int b2d_resize_table(int mode, int in_size, int out_size, int32_t* bounds_out, int32_t* coef_out, int* ksize_out);

@@ -2,7 +2,7 @@
 window 640, stride 512 = 20 % overlap -> 79 x 79 = 6241 windows), window rows sharded across the
 ranks, cross-shard seam dedup through the NCCL all-gather of mosaic.MosaicDetector.
 
-    python tools/mosaic_bench.py [--size 40000] [--repeat 2]
+    python tools/mosaic_bench.py [--size 40000] [--repeat 2] [--win 640 --stride 512]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P tools/mosaic_bench.py
 
 Every rank materialises only its own band of the mosaic, on the device, from a small pool of
@@ -11,7 +11,9 @@ not depend on the sharding); no host traffic on the data path.  Timing: CUDA eve
 run (cut windows -> preprocess -> network -> NMS -> georef -> local dedup -> seam exchange -> merge),
 max over ranks.  Rank 0 prints one JSON line with windows/s, the number of detections before and after
 dedup, the seam records exchanged and an order-independent checksum of the result, which must be
-identical for every world size.
+identical for every world size.  ``--win`` / ``--stride`` run another window grid: windows other than
+the model input are resampled from the mosaic into the network input (``b2d_resize_windows``), e.g. the reference
+notebook's 1200 / 600.
 """
 from __future__ import annotations
 
@@ -33,6 +35,8 @@ def main():
     ap.add_argument("--size", type=int, default=40000)
     ap.add_argument("--repeat", type=int, default=2)
     ap.add_argument("--batch", type=int, default=64)
+    ap.add_argument("--win", type=int, default=640)
+    ap.add_argument("--stride", type=int, default=512)
     ap.add_argument("--dump", default="")
     ap.add_argument("--dump-raw", default="", help="debug: save every rank's raw (pre-dedup) detections to <prefix>.rank<r>.npz")
     args = ap.parse_args()
@@ -49,9 +53,9 @@ def main():
     H = W = args.size
     eng = Engine("yolov8m", max_batch=args.batch, device=local, seed=0)
     pool = torch.from_numpy(synth.mosaic_block_pool(77)).to(eng.device)
-    windows, ids, cover = M.shard_windows(H, W, rank, world)
+    windows, ids, cover = M.shard_windows(H, W, rank, world, args.win, args.stride)
     band = synth.mosaic_band_device(pool, H, W, cover[0], cover[1], 5)
-    det = M.MosaicDetector(eng, GT, conf=0.4, dedup_thr=1.0)
+    det = M.MosaicDetector(eng, GT, win=args.win, stride=args.stride, conf=0.4, dedup_thr=1.0)
     det.profile = bool(os.environ.get("B2D_MOSAIC_PROFILE"))
 
     def barrier():
@@ -86,8 +90,8 @@ def main():
     if args.dump:
         np.save(f"{args.dump}.rank{rank}.npy", out)
     if rank == 0:
-        nwin = len(M.window_grid(H, W))
-        print(json.dumps({"workload": f"C4: synthetic {H}x{W} mosaic, window 640 stride 512, {nwin} windows, YOLOv8m (seeded synthetic weights), "
+        nwin = len(M.window_grid(H, W, args.win, args.stride))
+        print(json.dumps({"workload": f"C4: synthetic {H}x{W} mosaic, window {args.win} stride {args.stride}, {nwin} windows, YOLOv8m (seeded synthetic weights), "
                                       f"conf>0.4, 1 m dedup, row bands over {world} rank(s)",
                           "n_gpus": world, "windows": nwin, "ms_per_mosaic": float(mx[0]), "windows_per_s": nwin / (float(mx[0]) * 1e-3),
                           "detections_raw": int(stats[2]), "detections_after_dedup": int(stats[1]), "seam_records_exchanged": int(stats[3]),
