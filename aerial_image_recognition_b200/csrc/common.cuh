@@ -7,6 +7,8 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include <memory>
+
 #include "../../include/b2det.h"
 
 void b2d_set_error(const char* fmt, ...);
@@ -31,6 +33,42 @@ void b2d_set_error(const char* fmt, ...);
 #define B2D_LAUNCH_CHECK() B2D_CUDA(cudaGetLastError())
 
 static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
+
+// The one owner of a cudaMalloc (Pinned = false) or cudaMallocHost (Pinned = true) block: freed by its destructor, moved,
+// never copied.  bytes() is always the size of the block it holds, 0 when it holds none.
+template <class T, bool Pinned>
+class CudaBlock {
+  public:
+    T* get() const { return ptr_.get(); }
+    size_t bytes() const { return bytes_; }
+    void reset() { ptr_.reset(); bytes_ = 0; }
+    // Grow-only: keeps the block when it holds `bytes`, else frees it and allocates `bytes`.  A refused allocation leaves
+    // the owner empty and returns -2 with the error set, like B2D_CUDA.
+    int reserve(size_t bytes) {
+        if (bytes <= bytes_) return 0;
+        reset();
+        void* p = nullptr;
+        const cudaError_t err = Pinned ? cudaMallocHost(&p, bytes) : cudaMalloc(&p, bytes);
+        if (err != cudaSuccess) {
+            cudaGetLastError();      // the refusal is reported here; the next launch check must not report it again
+            b2d_set_error("%s:%d %s(%zu bytes) -> %s", __FILE__, __LINE__, Pinned ? "cudaMallocHost" : "cudaMalloc", bytes,
+                          cudaGetErrorString(err));
+            return -2;
+        }
+        ptr_.reset(static_cast<T*>(p));
+        bytes_ = bytes;
+        return 0;
+    }
+
+  private:
+    struct Free {
+        void operator()(T* p) const { Pinned ? cudaFreeHost(p) : cudaFree(p); }
+    };
+    std::unique_ptr<T, Free> ptr_;
+    size_t bytes_ = 0;
+};
+template <class T> using DeviceBlock = CudaBlock<T, false>;
+template <class T> using PinnedBlock = CudaBlock<T, true>;
 
 // Opt a kernel in to more than 48 KB of dynamic shared memory on the CURRENT device, once per (device, kernel): the
 // attribute is per device, so a process-global "done" flag would leave the second GPU of a process without it
@@ -98,10 +136,10 @@ struct ConvTcPlan {
     ConvTcParams p;
     size_t smem_bytes;
     int sm_count;
-    __nv_bfloat16* w_dev;   // packed weights (owned)
-    float* bias_dev;        // owned
-    float* dw_dev;          // owned (fused depthwise + pointwise plans)
-    long long* trace_dev;   // owned, debug only
+    DeviceBlock<__nv_bfloat16> w_dev;   // packed weights
+    DeviceBlock<float> bias_dev;
+    DeviceBlock<float> dw_dev;          // fused depthwise + pointwise plans
+    DeviceBlock<long long> trace_dev;   // debug only
 };
 
 // fused depthwise 3x3 (c channels, source slice) + pointwise 1x1 (c -> cout, destination slice), both with bias and optional SiLU
@@ -117,7 +155,6 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch,
 int conv_tc_dw_supported(int cin, int cout, int ksz, int stride, int dst_f32, int has_res);
 int conv_tc_dwpw_supported(int c, int cout, int dst_f32, int x2);
 int conv_tc_launch(const ConvTcPlan* plan, int n, cudaStream_t stream);
-void conv_tc_free(ConvTcPlan* plan);
 int conv_tc_describe(const ConvTcPlan* plan, char* buf, int buflen);
 
 // ---------------------------------------------------------------------------------------

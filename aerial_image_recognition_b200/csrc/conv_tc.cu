@@ -2000,7 +2000,7 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
     // Channel arguments are REAL channel counts.  In split-fp16 storage (x2) a 16-bit buffer keeps 2 x 16 bits per channel
     // ([hi x 8 | lo x 8] groups, see split2): the A operand then has K = 2 * cin storage channels against weights packed twice,
     // and 16-bit outputs / residuals are 4 bytes per channel like fp32 ones.  The network input (stem) is never split.
-    memset(plan, 0, sizeof(*plan));
+    *plan = ConvTcPlan{};
     const bool dw = depthwise != 0;
     const bool fused = fuse != nullptr;       // this 1x1 conv reads the depthwise 3x3 of fuse->src computed in the same kernel (src is unused)
     B2D_CHECK(!x2 || f16, "conv_tc: split storage is fp16");
@@ -2258,8 +2258,8 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
     p.epi_parts = fused ? 1 : (p.n_tile >> 4) % 3 == 0 ? 3 : 2;   // fused: warps 8-15 compute the depthwise stage
     p.trace = nullptr;
     if (getenv("B2D_TRACE")) {
-        B2D_CUDA(cudaMalloc(&plan->trace_dev, sizeof(long long) * kTraceRoles * kTraceTiles * kTraceEvents));
-        p.trace = plan->trace_dev;
+        if (plan->trace_dev.reserve(sizeof(long long) * kTraceRoles * kTraceTiles * kTraceEvents)) return -2;
+        p.trace = plan->trace_dev.get();
     }
     uint32_t cols = 32;
     while (cols < (uint32_t)(2 * p.mt * p.n_tile)) cols *= 2;
@@ -2317,12 +2317,12 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
     }
     std::vector<float> bp(cout_pad, 0.f);
     for (int o = 0; o < cout; ++o) bp[o] = b_host ? b_host[o % cout_real] : 0.f;      // stride-1 stem: both pixels of a pair
-    B2D_CUDA(cudaMalloc(&plan->w_dev, wp.size() * 2));
-    B2D_CUDA(cudaMemcpy(plan->w_dev, wp.data(), wp.size() * 2, cudaMemcpyHostToDevice));
-    B2D_CUDA(cudaMalloc(&plan->bias_dev, bp.size() * 4));
-    B2D_CUDA(cudaMemcpy(plan->bias_dev, bp.data(), bp.size() * 4, cudaMemcpyHostToDevice));
-    p.bias = plan->bias_dev;
-    p.w_raw = plan->w_dev;
+    if (plan->w_dev.reserve(wp.size() * 2)) return -2;
+    B2D_CUDA(cudaMemcpy(plan->w_dev.get(), wp.data(), wp.size() * 2, cudaMemcpyHostToDevice));
+    if (plan->bias_dev.reserve(bp.size() * 4)) return -2;
+    B2D_CUDA(cudaMemcpy(plan->bias_dev.get(), bp.data(), bp.size() * 4, cudaMemcpyHostToDevice));
+    p.bias = plan->bias_dev.get();
+    p.w_raw = plan->w_dev.get();
     if (fused) {
         // [chunk][tap][64] fp32 then [chunks * 64] bias; values rounded to the 16-bit weight format like every packed weight, and
         // halved for SiLU layers (silu2_h takes v / 2; the scaling is exact)
@@ -2338,9 +2338,9 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
             }
             dwc[(size_t)p.chunks * 9 * 64 + c] = hs * (fuse->b ? fuse->b[c] : 0.f);
         }
-        B2D_CUDA(cudaMalloc(&plan->dw_dev, dwc.size() * 4));
-        B2D_CUDA(cudaMemcpy(plan->dw_dev, dwc.data(), dwc.size() * 4, cudaMemcpyHostToDevice));
-        p.dw_w = plan->dw_dev;
+        if (plan->dw_dev.reserve(dwc.size() * 4)) return -2;
+        B2D_CUDA(cudaMemcpy(plan->dw_dev.get(), dwc.data(), dwc.size() * 4, cudaMemcpyHostToDevice));
+        p.dw_w = plan->dw_dev.get();
         p.dw_act = fuse->act;
     }
 
@@ -2351,12 +2351,12 @@ int conv_tc_plan(ConvTcPlan* plan, int sm_count, int max_batch, const __nv_bfloa
             uint64_t dims[2] = {64u, (uint64_t)dw_chunks * 9 * 16};
             uint64_t str[1] = {128u};
             uint32_t box[2] = {64u, 144u};
-            if (encode_map(&p.tmB, plan->w_dev, 2, dims, str, box, 128)) return -1;
+            if (encode_map(&p.tmB, plan->w_dev.get(), 2, dims, str, box, 128)) return -1;
         } else {
             uint64_t dims[2] = {(uint64_t)ktot, (uint64_t)cout_pad};
             uint64_t str[1] = {(uint64_t)ktot * 2};
             uint32_t box[2] = {64u, (uint32_t)(p.pair ? p.n_tile / 2 : p.n_tile)};
-            if (encode_map(&p.tmB, plan->w_dev, 2, dims, str, box, 128)) return -1;
+            if (encode_map(&p.tmB, plan->w_dev.get(), 2, dims, str, box, 128)) return -1;
         }
         const uint64_t pix = (uint64_t)src_cs_s * 2, rowb = (uint64_t)src_w * pix, imgb = (uint64_t)src_h * rowb;
         if (p.kind == CONV_HALO || p.kind == CONV_DEPTHWISE || p.kind == CONV_DWPW) {
@@ -2487,17 +2487,6 @@ int conv_tc_launch(const ConvTcPlan* plan, int n, cudaStream_t stream) {
     }
     B2D_LAUNCH_CHECK();
     return 0;
-}
-
-void conv_tc_free(ConvTcPlan* plan) {
-    if (plan->w_dev) cudaFree(plan->w_dev);
-    if (plan->bias_dev) cudaFree(plan->bias_dev);
-    if (plan->trace_dev) cudaFree(plan->trace_dev);
-    if (plan->dw_dev) cudaFree(plan->dw_dev);
-    plan->dw_dev = nullptr;
-    plan->trace_dev = nullptr;
-    plan->w_dev = nullptr;
-    plan->bias_dev = nullptr;
 }
 
 int conv_tc_describe(const ConvTcPlan* plan, char* buf, int buflen) {

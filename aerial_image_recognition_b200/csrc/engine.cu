@@ -13,6 +13,7 @@
 #include <mutex>
 #include <set>
 #include <string>
+#include <type_traits>
 #include <utility>
 #include <vector>
 
@@ -62,9 +63,32 @@ struct DeviceGuard {
 
 struct Buffer {
     int h, w, c, f32;
-    void* ptr;
-    size_t bytes;
+    DeviceBlock<void> ptr;
 };
+
+// Owners of the engine's streams, events and graph executables
+struct CudaDestroy {
+    void operator()(cudaStream_t s) const { cudaStreamDestroy(s); }
+    void operator()(cudaEvent_t ev) const { cudaEventDestroy(ev); }
+    void operator()(cudaGraphExec_t g) const { cudaGraphExecDestroy(g); }
+};
+using Stream = std::unique_ptr<std::remove_pointer_t<cudaStream_t>, CudaDestroy>;
+using Event = std::unique_ptr<std::remove_pointer_t<cudaEvent_t>, CudaDestroy>;
+using GraphExec = std::unique_ptr<std::remove_pointer_t<cudaGraphExec_t>, CudaDestroy>;
+
+// every stream the engine creates is non-blocking, every event has timing disabled
+int create(Stream& s) {
+    cudaStream_t raw;
+    B2D_CUDA(cudaStreamCreateWithFlags(&raw, cudaStreamNonBlocking));
+    s.reset(raw);
+    return 0;
+}
+int create(Event& ev) {
+    cudaEvent_t raw;
+    B2D_CUDA(cudaEventCreateWithFlags(&raw, cudaEventDisableTiming));
+    ev.reset(raw);
+    return 0;
+}
 
 enum OpKind { OP_CONV_TC, OP_MAXPOOL, OP_UPSAMPLE, OP_POOLCHAIN, OP_NOP };
 
@@ -84,7 +108,12 @@ struct Op {
     __nv_bfloat16* chain_dst[3]; int chain_c0[3]; int chain_stages; int fused_into;
 };
 
-struct TableEntry { ResizeTables t; int canvas; };
+struct TableEntry {     // t is what the kernels take; its pointers are views of the blocks beside it
+    ResizeTables t;
+    int canvas;
+    DeviceBlock<int32_t> xb, xk, yb, yk;
+    DeviceBlock<uint8_t> tmp;
+};
 
 }  // namespace
 
@@ -105,36 +134,34 @@ struct b2d_engine {
     HeadDesc head{};
     int head_levels = 0;
     std::vector<TableEntry> tables;
-    // post-processing scratch
-    b2d_det* cand = nullptr;
-    int* cand_count = nullptr;
-    unsigned long long* keys = nullptr;
+    // post-processing scratch; cand_cap and cand_tiles are 0 until every block below is held at their size
+    DeviceBlock<b2d_det> cand;
+    DeviceBlock<int> cand_count;
+    DeviceBlock<unsigned long long> keys;
     int cand_cap = 0;
     int cand_tiles = 0;
-    float* cand_angle = nullptr;            // oriented-box engines: the angle of each candidate slot, beside `cand`
-    float4* obb_prm = nullptr;              // ... and the rotated NMS's per-candidate Gaussians (2 float4 per key slot)
-    void* dedup_scratch = nullptr;
-    size_t dedup_scratch_bytes = 0;
+    DeviceBlock<float> cand_angle;          // oriented-box engines: the angle of each candidate slot, beside `cand`
+    DeviceBlock<float4> obb_prm;            // ... and the rotated NMS's per-candidate Gaussians (2 float4 per key slot)
+    DeviceBlock<void> dedup_scratch;
     float conf_scale = 1.0f;                // b2d_set_conf_scale: the TTA confidence adjustment (gpu_handler.py:236)
     // test-time-augmentation scratch: CLAHE tile tables / per-image byte tables, per-image grey sums
-    uint8_t* tta_luts = nullptr;
-    size_t tta_luts_bytes = 0;
-    unsigned long long* tta_sums = nullptr;
-    int tta_sums_n = 0;
+    DeviceBlock<uint8_t> tta_luts;
+    DeviceBlock<unsigned long long> tta_sums;
     // b2d_detect_host: two staging slots (tiles, params, records, counts), a copy stream and the events that order them
     struct HostSlot {
-        uint8_t* tiles = nullptr; size_t tiles_bytes = 0;
-        double* params = nullptr; b2d_det* dets = nullptr; b2d_geodet* geo = nullptr; int32_t* counts = nullptr; int cap = 0;
-        double* params_pin = nullptr; b2d_geodet* geo_pin = nullptr; int32_t* counts_pin = nullptr;   // pinned host staging
-        cudaEvent_t loaded = nullptr, drained = nullptr;
+        DeviceBlock<uint8_t> tiles;
+        // cap is 0 until every record block is held at its size
+        DeviceBlock<double> params; DeviceBlock<b2d_det> dets; DeviceBlock<b2d_geodet> geo; DeviceBlock<int32_t> counts; int cap = 0;
+        PinnedBlock<double> params_pin; PinnedBlock<b2d_geodet> geo_pin; PinnedBlock<int32_t> counts_pin;   // pinned host staging
+        Event loaded, drained;
     } host_slot[2];
-    cudaStream_t copy_stream = nullptr;
+    Stream copy_stream;
     // forward() as a CUDA graph per batch size: the ~94 launches of a step replay without per-launch driver work
-    std::map<int, cudaGraphExec_t> fwd_graphs;
+    std::map<int, GraphExec> fwd_graphs;
     std::map<int, int> fwd_calls;
-    cudaStream_t cap_stream = nullptr;      // capture happens here (the caller's stream may be the legacy default stream)
-    std::vector<cudaStream_t> side_streams; // further capture streams: independent ops become parallel graph branches
-    std::vector<cudaEvent_t> cap_events;    // one per op + fork / join events (capture only)
+    Stream cap_stream;                      // capture happens here (the caller's stream may be the legacy default stream)
+    std::vector<Stream> side_streams;       // further capture streams: independent ops become parallel graph branches
+    std::vector<Event> cap_events;          // one per op + fork / join events (capture only)
 };
 
 namespace {
@@ -146,79 +173,75 @@ int ensure_cand(b2d_engine* e, int n, int rows) {
     B2D_CHECK(rows <= kMaxCand, "postprocess: %d rows per tile exceed the limit of %d (the sort key's 16-bit anchor and slot fields)",
               rows, kMaxCand);
     const int cap = rows;
-    if (e->cand && e->cand_cap >= cap && e->cand_tiles >= n) return 0;
-    if (e->cand) { cudaFree(e->cand); cudaFree(e->cand_count); cudaFree(e->keys); }
-    if (e->cand_angle) { cudaFree(e->cand_angle); cudaFree(e->obb_prm); e->cand_angle = nullptr; e->obb_prm = nullptr; }
-    int tiles = n > e->max_batch ? n : e->max_batch;
+    if (e->cand_cap >= cap && e->cand_tiles >= n) return 0;
+    e->cand_cap = e->cand_tiles = 0;          // every old block goes before any new one is allocated
+    e->cand.reset(); e->cand_count.reset(); e->keys.reset(); e->cand_angle.reset(); e->obb_prm.reset();
+    const int tiles = n > e->max_batch ? n : e->max_batch;
     const int stride = keys_stride(cap);
-    B2D_CUDA(cudaMalloc(&e->cand, (size_t)tiles * cap * sizeof(b2d_det)));
-    B2D_CUDA(cudaMalloc(&e->cand_count, (size_t)tiles * sizeof(int)));
-    B2D_CUDA(cudaMalloc(&e->keys, (size_t)tiles * stride * sizeof(unsigned long long)));
-    if (is_obb(e)) {
-        B2D_CUDA(cudaMalloc(&e->cand_angle, (size_t)tiles * cap * sizeof(float)));
-        B2D_CUDA(cudaMalloc(&e->obb_prm, (size_t)tiles * stride * 2 * sizeof(float4)));
-    }
+    if (e->cand.reserve((size_t)tiles * cap * sizeof(b2d_det)) || e->cand_count.reserve((size_t)tiles * sizeof(int)) ||
+        e->keys.reserve((size_t)tiles * stride * sizeof(unsigned long long)))
+        return -2;
+    if (is_obb(e) && (e->cand_angle.reserve((size_t)tiles * cap * sizeof(float)) ||
+                      e->obb_prm.reserve((size_t)tiles * stride * 2 * sizeof(float4))))
+        return -2;
     e->cand_cap = cap;
     e->cand_tiles = tiles;
     return 0;
 }
 
-int upload_i32(int32_t** dst, const std::vector<int32_t>& v) {
-    B2D_CUDA(cudaMalloc(dst, v.size() * sizeof(int32_t)));
-    B2D_CUDA(cudaMemcpy(*dst, v.data(), v.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+int upload_i32(DeviceBlock<int32_t>& dst, const std::vector<int32_t>& v) {
+    if (dst.reserve(v.size() * sizeof(int32_t))) return -2;
+    B2D_CUDA(cudaMemcpy(dst.get(), v.data(), v.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
     return 0;
 }
 
 int get_tables(b2d_engine* e, int mode, int h, int w, int out, int n, const ResizeTables** result) {
-    for (auto& te : e->tables)
-        if (te.t.mode == mode && te.t.in_h == h && te.t.in_w == w && te.canvas == out) {
-            ResizeTables& t = te.t;
-            if (mode == B2D_RESIZE_PIL_BICUBIC && t.in_w != t.out_w) {
-                const size_t need = (size_t)n * t.in_h * t.out_w * 3;
-                if (need > t.tmp_bytes) {
-                    if (t.tmp) cudaFree(t.tmp);
-                    B2D_CUDA(cudaMalloc(&t.tmp, need));
-                    t.tmp_bytes = need;
-                }
+    TableEntry* te = nullptr;
+    for (auto& x : e->tables)
+        if (x.t.mode == mode && x.t.in_h == h && x.t.in_w == w && x.canvas == out) { te = &x; break; }
+    if (!te) {
+        TableEntry ne{};
+        ResizeTables& t = ne.t;
+        t.mode = mode; t.in_h = h; t.in_w = w; t.out_h = out; t.out_w = out;
+        if (mode == B2D_RESIZE_IDENTITY) {
+            B2D_CHECK(h == out && w == out, "preprocess: identity mode needs %dx%d input, got %dx%d", out, out, h, w);
+        } else {
+            int tmode = mode;
+            if (mode == B2D_RESIZE_LETTERBOX) {
+                // Ultralytics LetterBox(auto=False, scaleup=True, center=True); Python round() = rint()
+                const double r = fmin((double)out / h, (double)out / w);
+                t.out_w = (int)rint(w * r);
+                t.out_h = (int)rint(h * r);
+                const double dw = (out - t.out_w) / 2.0, dh = (out - t.out_h) / 2.0;
+                t.left = (int)rint(dw - 0.1);
+                t.top = (int)rint(dh - 0.1);
+                tmode = B2D_RESIZE_CV2_LINEAR;
             }
-            *result = &t;
-            return 0;
+            int kx = 0, ky = 0;
+            b2d_resize_table(tmode, w, t.out_w, nullptr, nullptr, &kx);
+            b2d_resize_table(tmode, h, t.out_h, nullptr, nullptr, &ky);
+            t.ksize_x = kx; t.ksize_y = ky;
+            std::vector<int32_t> xb(2 * (size_t)t.out_w), xk((size_t)kx * t.out_w), yb(2 * (size_t)t.out_h), yk((size_t)ky * t.out_h);
+            B2D_CHECK(b2d_resize_table(tmode, w, t.out_w, xb.data(), xk.data(), &kx) == 0, "resize table failed");
+            if (tmode == B2D_RESIZE_CV2_LINEAR)       // the row taps follow OpenCV's vertical rule (cv2_linear_coef)
+                cv2_linear_axis_table(h, t.out_h, 1, yb.data(), yk.data());
+            else
+                B2D_CHECK(b2d_resize_table(tmode, h, t.out_h, yb.data(), yk.data(), &ky) == 0, "resize table failed");
+            if (upload_i32(ne.xb, xb) || upload_i32(ne.xk, xk) || upload_i32(ne.yb, yb) || upload_i32(ne.yk, yk)) return -2;
+            t.xb = ne.xb.get(); t.xk = ne.xk.get(); t.yb = ne.yb.get(); t.yk = ne.yk.get();
         }
-    ResizeTables t;
-    memset(&t, 0, sizeof(t));
-    t.mode = mode; t.in_h = h; t.in_w = w; t.out_h = out; t.out_w = out;
-    if (mode == B2D_RESIZE_IDENTITY) {
-        B2D_CHECK(h == out && w == out, "preprocess: identity mode needs %dx%d input, got %dx%d", out, out, h, w);
-    } else {
-        int tmode = mode;
-        if (mode == B2D_RESIZE_LETTERBOX) {
-            // Ultralytics LetterBox(auto=False, scaleup=True, center=True); Python round() = rint()
-            const double r = fmin((double)out / h, (double)out / w);
-            t.out_w = (int)rint(w * r);
-            t.out_h = (int)rint(h * r);
-            const double dw = (out - t.out_w) / 2.0, dh = (out - t.out_h) / 2.0;
-            t.left = (int)rint(dw - 0.1);
-            t.top = (int)rint(dh - 0.1);
-            tmode = B2D_RESIZE_CV2_LINEAR;
-        }
-        int kx = 0, ky = 0;
-        b2d_resize_table(tmode, w, t.out_w, nullptr, nullptr, &kx);
-        b2d_resize_table(tmode, h, t.out_h, nullptr, nullptr, &ky);
-        t.ksize_x = kx; t.ksize_y = ky;
-        std::vector<int32_t> xb(2 * (size_t)t.out_w), xk((size_t)kx * t.out_w), yb(2 * (size_t)t.out_h), yk((size_t)ky * t.out_h);
-        B2D_CHECK(b2d_resize_table(tmode, w, t.out_w, xb.data(), xk.data(), &kx) == 0, "resize table failed");
-        if (tmode == B2D_RESIZE_CV2_LINEAR)       // the row taps follow OpenCV's vertical rule (cv2_linear_coef)
-            cv2_linear_axis_table(h, t.out_h, 1, yb.data(), yk.data());
-        else
-            B2D_CHECK(b2d_resize_table(tmode, h, t.out_h, yb.data(), yk.data(), &ky) == 0, "resize table failed");
-        if (upload_i32(&t.xb, xb) || upload_i32(&t.xk, xk) || upload_i32(&t.yb, yb) || upload_i32(&t.yk, yk)) return -2;
-        if (mode == B2D_RESIZE_PIL_BICUBIC && t.in_w != t.out_w) {
-            t.tmp_bytes = (size_t)n * t.in_h * t.out_w * 3;
-            B2D_CUDA(cudaMalloc(&t.tmp, t.tmp_bytes));
-        }
+        ne.canvas = out;
+        e->tables.push_back(std::move(ne));
+        te = &e->tables.back();
     }
-    e->tables.push_back({t, out});
-    *result = &e->tables.back().t;
+    ResizeTables& t = te->t;
+    if (mode == B2D_RESIZE_PIL_BICUBIC && t.in_w != t.out_w) {
+        const int rc = te->tmp.reserve((size_t)n * t.in_h * t.out_w * 3);
+        t.tmp = te->tmp.get();
+        t.tmp_bytes = te->tmp.bytes();
+        if (rc) return rc;
+    }
+    *result = &t;
     return 0;
 }
 
@@ -258,17 +281,13 @@ static bool overlaps(const Range& a, const Range& b) { return a.buf == b.buf && 
 int capture_ops(b2d_engine* e, int n) {
     const int nops = (int)e->ops.size();
     const int ns = 3;                                        // capture streams
-    while ((int)e->side_streams.size() < ns - 1) {
-        cudaStream_t s;
-        B2D_CUDA(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
-        e->side_streams.push_back(s);
-    }
-    while ((int)e->cap_events.size() < nops + 2 * ns) {
-        cudaEvent_t ev;
-        B2D_CUDA(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-        e->cap_events.push_back(ev);
-    }
-    auto stream_of = [&](int k) { return k == 0 ? e->cap_stream : e->side_streams[k - 1]; };
+    e->side_streams.resize(ns - 1);
+    for (auto& s : e->side_streams)
+        if (!s && create(s)) return -2;
+    e->cap_events.resize(nops + 2 * ns);
+    for (auto& ev : e->cap_events)
+        if (!ev && create(ev)) return -2;
+    auto stream_of = [&](int k) { return k == 0 ? e->cap_stream.get() : e->side_streams[k - 1].get(); };
     // reads / writes of every launched op (a fused pool chain writes its followers' outputs too)
     std::vector<std::vector<Range>> rd(nops), wr(nops);
     for (int i = 0; i < nops; ++i) {
@@ -290,8 +309,8 @@ int capture_ops(b2d_engine* e, int n) {
     std::vector<int> where(nops, -1), last_on(ns, -1);
     std::vector<bool> joined(ns, false);
     joined[0] = true;
-    cudaEvent_t fork_ev = e->cap_events[nops];
-    B2D_CUDA(cudaEventRecord(fork_ev, e->cap_stream));
+    cudaEvent_t fork_ev = e->cap_events[nops].get();
+    B2D_CUDA(cudaEventRecord(fork_ev, e->cap_stream.get()));
     for (int i = 0; i < nops; ++i) {
         if (e->ops[i].kind == OP_NOP || (i > 0 && e->fused_at[i - 1] >= 0)) continue;
         std::vector<int> deps;
@@ -320,16 +339,16 @@ int capture_ops(b2d_engine* e, int n) {
             joined[k] = true;
         }
         for (int j : deps)
-            if (where[j] != k) B2D_CUDA(cudaStreamWaitEvent(s, e->cap_events[j], 0));
+            if (where[j] != k) B2D_CUDA(cudaStreamWaitEvent(s, e->cap_events[j].get(), 0));
         if (int r = launch_fwd_op(e, i, n, s)) return r;
-        B2D_CUDA(cudaEventRecord(e->cap_events[i], s));
+        B2D_CUDA(cudaEventRecord(e->cap_events[i].get(), s));
         where[i] = k;
         last_on[k] = i;
     }
     for (int t = 1; t < ns; ++t)
         if (joined[t]) {
-            B2D_CUDA(cudaEventRecord(e->cap_events[nops + 1 + t], stream_of(t)));
-            B2D_CUDA(cudaStreamWaitEvent(e->cap_stream, e->cap_events[nops + 1 + t], 0));
+            B2D_CUDA(cudaEventRecord(e->cap_events[nops + 1 + t].get(), stream_of(t)));
+            B2D_CUDA(cudaStreamWaitEvent(e->cap_stream.get(), e->cap_events[nops + 1 + t].get(), 0));
         }
     return 0;
 }
@@ -363,38 +382,7 @@ int b2d_create(int device, int max_batch, b2d_engine** out) {
 
 void b2d_destroy(b2d_engine* e) {
     if (!e) return;
-    B2D_ENTER(e);
-    for (auto& op : e->ops) {
-        if (op.kind == OP_CONV_TC) conv_tc_free(&op.tc);
-    }
-    for (auto& fp : e->fused_plans) conv_tc_free(&fp);
-    for (auto& b : e->bufs)
-        if (b.ptr) cudaFree(b.ptr);
-    for (auto& te : e->tables) {
-        if (te.t.xb) cudaFree(te.t.xb);
-        if (te.t.xk) cudaFree(te.t.xk);
-        if (te.t.yb) cudaFree(te.t.yb);
-        if (te.t.yk) cudaFree(te.t.yk);
-        if (te.t.tmp) cudaFree(te.t.tmp);
-    }
-    if (e->cand) { cudaFree(e->cand); cudaFree(e->cand_count); cudaFree(e->keys); }
-    if (e->cand_angle) { cudaFree(e->cand_angle); cudaFree(e->obb_prm); }
-    if (e->dedup_scratch) cudaFree(e->dedup_scratch);
-    if (e->tta_luts) cudaFree(e->tta_luts);
-    if (e->tta_sums) cudaFree(e->tta_sums);
-    for (auto& hs : e->host_slot) {
-        if (hs.tiles) cudaFree(hs.tiles);
-        if (hs.params) {
-            cudaFree(hs.params); cudaFree(hs.dets); cudaFree(hs.geo); cudaFree(hs.counts);
-            cudaFreeHost(hs.params_pin); cudaFreeHost(hs.geo_pin); cudaFreeHost(hs.counts_pin);
-        }
-        if (hs.loaded) { cudaEventDestroy(hs.loaded); cudaEventDestroy(hs.drained); }
-    }
-    if (e->copy_stream) cudaStreamDestroy(e->copy_stream);
-    for (auto& kv : e->fwd_graphs) cudaGraphExecDestroy(kv.second);
-    if (e->cap_stream) cudaStreamDestroy(e->cap_stream);
-    for (auto st : e->side_streams) cudaStreamDestroy(st);
-    for (auto ev : e->cap_events) cudaEventDestroy(ev);
+    B2D_ENTER(e);      // declared before the delete, so every member is released with the engine's device current
     delete e;
 }
 
@@ -414,14 +402,13 @@ int b2d_plan_buffer(b2d_engine* e, int h, int w, int c, int is_f32) {
     B2D_CHECK(e && !e->finalized, "plan_buffer: engine finalized or null");
     B2D_CHECK(h > 0 && w > 0 && c > 0, "plan_buffer: bad shape");
     B2D_ENTER(e);
-    Buffer b{h, w, c, is_f32, nullptr, 0};
+    Buffer b{h, w, c, is_f32};
     // bytes per channel: 4 (fp32 head maps), 2 (bf16 / fp16), or 2 + 2 in split storage -- except buffer 0, the network
     // input, which holds raw pixel values (exact in 16 bits) in every mode
     const bool split = e->x2 && !is_f32 && !e->bufs.empty();
-    b.bytes = (size_t)e->max_batch * h * w * c * ((is_f32 || split) ? 4 : 2);
-    B2D_CUDA(cudaMalloc(&b.ptr, b.bytes));
-    B2D_CUDA(cudaMemset(b.ptr, 0, b.bytes));
-    e->bufs.push_back(b);
+    if (b.ptr.reserve((size_t)e->max_batch * h * w * c * ((is_f32 || split) ? 4 : 2))) return -2;
+    B2D_CUDA(cudaMemset(b.ptr.get(), 0, b.ptr.bytes()));
+    e->bufs.push_back(std::move(b));
     return (int)e->bufs.size() - 1;
 }
 
@@ -500,7 +487,7 @@ int b2d_plan_head_level(b2d_engine* e, int kind, int buf, int stride, int nc, co
     B2D_CHECK(e->head_levels == 0 || (e->head.kind == kind && e->head.nc == nc), "plan_head_level: inconsistent head");
     const Buffer& b = e->bufs[buf];
     HeadLevel& L = e->head.lv[e->head_levels];
-    L.buf = (const float*)b.ptr; L.hw = b.h; L.c = b.c; L.stride = stride;
+    L.buf = (const float*)b.ptr.get(); L.hw = b.h; L.c = b.c; L.stride = stride;
     for (int i = 0; i < 6; ++i) L.anchors[i] = anchors_px ? anchors_px[i] : 0.f;
     B2D_CHECK(kind == B2D_HEAD_V8_DFL || kind == B2D_HEAD_V7_ANCHOR || kind == B2D_HEAD_V8_OBB, "plan_head_level: unknown head kind %d", kind);
     const int per = (kind == B2D_HEAD_V7_ANCHOR) ? 3 : 1;
@@ -524,7 +511,7 @@ int b2d_plan_finalize(b2d_engine* e) {
         const Buffer& sb = e->bufs[d.src];
         const Buffer& db = e->bufs[d.dst];
         if (d.kind_req == 0) {
-            const __nv_bfloat16* res = d.res >= 0 ? (const __nv_bfloat16*)e->bufs[d.res].ptr : nullptr;
+            const __nv_bfloat16* res = d.res >= 0 ? (const __nv_bfloat16*)e->bufs[d.res].ptr.get() : nullptr;
             const int res_cs = d.res >= 0 ? e->bufs[d.res].c : 0;
             const bool tc = (conv_tc_supported(d.cin, d.k, d.stride) && sb.c % 8 == 0 && d.src_c0 % 8 == 0) ||
                             (conv_tc_stem_supported(sb.c, d.cin, d.k, d.stride, d.cout, db.f32, d.res >= 0) && d.src_c0 == 0);
@@ -535,20 +522,20 @@ int b2d_plan_finalize(b2d_engine* e) {
             op.kind = OP_CONV_TC;
             // the network input holds raw 0..255 pixel values: the reference's `/ 255.0` is the stem's accumulator scale
             const float acc_scale = d.src == 0 ? 1.0f / 255.0f : 1.0f;
-            if (conv_tc_plan(&op.tc, e->sm_count, e->max_batch, (const __nv_bfloat16*)sb.ptr, sb.h, sb.w, sb.c, d.src_c0, d.cin,
-                             db.ptr, db.h, db.w, db.c, d.dst_c0, d.cout, db.f32, d.k, d.stride, d.act, d.w.data(), d.b.data(), res,
+            if (conv_tc_plan(&op.tc, e->sm_count, e->max_batch, (const __nv_bfloat16*)sb.ptr.get(), sb.h, sb.w, sb.c, d.src_c0, d.cin,
+                             db.ptr.get(), db.h, db.w, db.c, d.dst_c0, d.cout, db.f32, d.k, d.stride, d.act, d.w.data(), d.b.data(), res,
                              res_cs, d.res_c0, 0, e->f16, e->x2, acc_scale))
                 return -1;
         } else if (d.kind_req == 1) {
             B2D_CHECK(conv_tc_dw_supported(d.cin, d.cout, 3, 1, db.f32, 0) && sb.c % 8 == 0 && d.src_c0 % 8 == 0,
                       "plan_finalize: op %zu (depthwise, %d channels) has no tcgen05 kernel", i, d.cin);
             op.kind = OP_CONV_TC;
-            if (conv_tc_plan(&op.tc, e->sm_count, e->max_batch, (const __nv_bfloat16*)sb.ptr, sb.h, sb.w, sb.c, d.src_c0, d.cin, db.ptr, db.h,
+            if (conv_tc_plan(&op.tc, e->sm_count, e->max_batch, (const __nv_bfloat16*)sb.ptr.get(), sb.h, sb.w, sb.c, d.src_c0, d.cin, db.ptr.get(), db.h,
                              db.w, db.c, d.dst_c0, d.cout, 0, 3, 1, d.act, d.w.data(), d.b.data(), nullptr, 0, 0, 1, e->f16, e->x2))
                 return -1;
         } else {
             op.kind = d.kind_req == 2 ? OP_MAXPOOL : OP_UPSAMPLE;
-            op.src = (const __nv_bfloat16*)sb.ptr; op.dst = (__nv_bfloat16*)db.ptr;
+            op.src = (const __nv_bfloat16*)sb.ptr.get(); op.dst = (__nv_bfloat16*)db.ptr.get();
             op.h = sb.h; op.w = sb.w; op.src_cs = sb.c; op.src_c0 = d.src_c0;
             op.oh = db.h; op.ow = db.w; op.dst_cs = db.c; op.dst_c0 = d.dst_c0; op.c = d.cout; op.k = d.k; op.stride = d.stride;
         }
@@ -576,14 +563,14 @@ int b2d_plan_finalize(b2d_engine* e) {
             if (j != i && dj.dst == d0.dst && dj.dst_c0 < d0.dst_c0 + d0.cout && d0.dst_c0 < dj.dst_c0 + dj.cout) other_reader = true;   // or another writer
         }
         if (other_reader) continue;
-        DwFuse fz{(const __nv_bfloat16*)sb.ptr, sb.c, d0.src_c0, d0.w.data(), d0.b.data(), d0.act};
+        DwFuse fz{(const __nv_bfloat16*)sb.ptr.get(), sb.c, d0.src_c0, d0.w.data(), d0.b.data(), d0.act};
         ConvTcPlan fp;
-        if (conv_tc_plan(&fp, e->sm_count, e->max_batch, nullptr, sb.h, sb.w, 0, 0, d1.cin, db.ptr, db.h, db.w, db.c, d1.dst_c0, d1.cout, 0, 1, 1,
+        if (conv_tc_plan(&fp, e->sm_count, e->max_batch, nullptr, sb.h, sb.w, 0, 0, d1.cin, db.ptr.get(), db.h, db.w, db.c, d1.dst_c0, d1.cout, 0, 1, 1,
                          d1.act, d1.w.data(), d1.b.data(), nullptr, 0, 0, 0, e->f16, 0, 1.0f, &fz))
             return -1;
         fp.p.rev = e->ops[i].tc.p.rev;
         e->fused_at[i] = (int)e->fused_plans.size();
-        e->fused_plans.push_back(fp);
+        e->fused_plans.push_back(std::move(fp));
         ++i;
     }
     for (auto& d : e->descs) { d.w.clear(); d.w.shrink_to_fit(); }
@@ -616,8 +603,8 @@ int b2d_plan_finalize(b2d_engine* e) {
     return 0;
 }
 
-void* b2d_buffer_ptr(b2d_engine* e, int buf) { return (e && buf >= 0 && buf < (int)e->bufs.size()) ? e->bufs[buf].ptr : nullptr; }
-size_t b2d_buffer_bytes(b2d_engine* e, int buf) { return (e && buf >= 0 && buf < (int)e->bufs.size()) ? e->bufs[buf].bytes : 0; }
+void* b2d_buffer_ptr(b2d_engine* e, int buf) { return (e && buf >= 0 && buf < (int)e->bufs.size()) ? e->bufs[buf].ptr.get() : nullptr; }
+size_t b2d_buffer_bytes(b2d_engine* e, int buf) { return (e && buf >= 0 && buf < (int)e->bufs.size()) ? e->bufs[buf].ptr.bytes() : 0; }
 int b2d_num_anchors(b2d_engine* e) { return e ? e->head.rows_total : -1; }
 int b2d_num_ops(b2d_engine* e) { return e ? (int)e->ops.size() : -1; }
 int b2d_num_kernels_per_forward(b2d_engine* e) {
@@ -669,14 +656,14 @@ int b2d_forward(b2d_engine* e, int n, void* stream) {
     static const bool use_graph = !getenv("B2D_TRACE");      // conv_tc_launch resets and reads back the role trace per launch
     auto it = e->fwd_graphs.find(n);
     if (use_graph && it != e->fwd_graphs.end()) {
-        B2D_CUDA(cudaGraphLaunch(it->second, st));
+        B2D_CUDA(cudaGraphLaunch(it->second.get(), st));
         return 0;
     }
     // the first call of a batch size runs eagerly (function attributes, lazy module loading); the second is captured
     const bool capture = use_graph && e->fwd_calls[n]++ >= 1;
     if (capture) {
-        if (!e->cap_stream) B2D_CUDA(cudaStreamCreateWithFlags(&e->cap_stream, cudaStreamNonBlocking));
-        B2D_CUDA(cudaStreamBeginCapture(e->cap_stream, cudaStreamCaptureModeThreadLocal));
+        if (!e->cap_stream && create(e->cap_stream)) return -2;
+        B2D_CUDA(cudaStreamBeginCapture(e->cap_stream.get(), cudaStreamCaptureModeThreadLocal));
     }
     int rc = 0;
     if (!capture) {
@@ -687,11 +674,11 @@ int b2d_forward(b2d_engine* e, int n, void* stream) {
     }
     if (capture) {
         cudaGraph_t g = nullptr;
-        cudaError_t err = cudaStreamEndCapture(e->cap_stream, &g);
+        cudaError_t err = cudaStreamEndCapture(e->cap_stream.get(), &g);
         if (rc == 0 && err == cudaSuccess && g) {
             cudaGraphExec_t ex = nullptr;
             if (cudaGraphInstantiate(&ex, g, 0) == cudaSuccess) {
-                e->fwd_graphs[n] = ex;
+                e->fwd_graphs[n].reset(ex);
                 cudaGraphDestroy(g);
                 B2D_CUDA(cudaGraphLaunch(ex, st));
                 return 0;
@@ -719,7 +706,7 @@ int b2d_preprocess(b2d_engine* e, const uint8_t* src_dev, int n, int h, int w, i
         B2D_CHECK((out_kind == B2D_OUT_BF16_NHWC4 || out_kind == B2D_OUT_F16_NHWC4) && !e->bufs.empty() && e->bufs[0].c == 4 && !e->bufs[0].f32,
                   "preprocess: dst NULL needs the planned 16-bit NHWC4 input buffer");
         B2D_CHECK(n <= e->max_batch, "preprocess: n=%d exceeds max_batch %d", n, e->max_batch);
-        dst_dev = e->bufs[0].ptr;
+        dst_dev = e->bufs[0].ptr.get();
     }
     const ResizeTables* t = nullptr;
     if (get_tables(e, mode, h, w, out, n, &t)) return -1;
@@ -730,7 +717,7 @@ int b2d_set_input_f32(b2d_engine* e, const float* src_dev, int n, void* stream) 
     B2D_CHECK(e && src_dev && n > 0 && n <= e->max_batch, "set_input_f32: bad arguments");
     B2D_ENTER(e);
     B2D_CHECK(!e->bufs.empty() && e->bufs[0].c == 4 && !e->bufs[0].f32, "set_input_f32: no planned bf16 NHWC4 input buffer");
-    return input_from_f32_launch(src_dev, n, e->bufs[0].h, e->bufs[0].w, e->bufs[0].ptr, (cudaStream_t)stream, e->f16);
+    return input_from_f32_launch(src_dev, n, e->bufs[0].h, e->bufs[0].w, e->bufs[0].ptr.get(), (cudaStream_t)stream, e->f16);
 }
 
 int b2d_decode_rows(b2d_engine* e, int n, float* rows_dev, void* stream) {
@@ -749,8 +736,8 @@ int b2d_postprocess(b2d_engine* e, int n, float conf_thr, int inclusive, float i
     B2D_CHECK(n > 0 && n <= e->max_batch && dets_dev && counts_dev && cap > 0, "postprocess: bad arguments");
     if (int rc = ensure_cand(e, n, e->head.rows_total)) return rc;
     cudaStream_t s = (cudaStream_t)stream;
-    if (candidates_from_head_launch(&e->head, n, conf_thr, inclusive, e->conf_scale, e->cand, e->cand_count, e->cand_cap, s)) return -2;
-    return select_launch(e->cand, e->cand_count, e->cand_cap, n, e->keys, iou_thr, top_k, max_det, dets_dev, counts_dev, cap, s);
+    if (candidates_from_head_launch(&e->head, n, conf_thr, inclusive, e->conf_scale, e->cand.get(), e->cand_count.get(), e->cand_cap, s)) return -2;
+    return select_launch(e->cand.get(), e->cand_count.get(), e->cand_cap, n, e->keys.get(), iou_thr, top_k, max_det, dets_dev, counts_dev, cap, s);
 }
 
 int b2d_postprocess_rows(b2d_engine* e, const float* rows_dev, int n, int num_rows, int ncol, float conf_thr, int inclusive,
@@ -760,8 +747,8 @@ int b2d_postprocess_rows(b2d_engine* e, const float* rows_dev, int n, int num_ro
     B2D_ENTER(e);
     if (int rc = ensure_cand(e, n, num_rows)) return rc;
     cudaStream_t s = (cudaStream_t)stream;
-    if (candidates_from_rows_launch(rows_dev, n, num_rows, ncol, conf_thr, inclusive, e->conf_scale, e->cand, e->cand_count, e->cand_cap, s)) return -2;
-    return select_launch(e->cand, e->cand_count, e->cand_cap, n, e->keys, iou_thr, top_k, max_det, dets_dev, counts_dev, cap, s);
+    if (candidates_from_rows_launch(rows_dev, n, num_rows, ncol, conf_thr, inclusive, e->conf_scale, e->cand.get(), e->cand_count.get(), e->cand_cap, s)) return -2;
+    return select_launch(e->cand.get(), e->cand_count.get(), e->cand_cap, n, e->keys.get(), iou_thr, top_k, max_det, dets_dev, counts_dev, cap, s);
 }
 
 int b2d_segment(b2d_engine* e, int buf, int n, int nc, uint8_t* labels_dev, float* conf_dev, void* stream) {
@@ -770,7 +757,7 @@ int b2d_segment(b2d_engine* e, int buf, int n, int nc, uint8_t* labels_dev, floa
     const Buffer& b = e->bufs[buf];
     B2D_CHECK(b.f32, "segment: buffer %d is not an fp32 logits buffer", buf);
     B2D_ENTER(e);
-    return segment_launch((const float*)b.ptr, (long long)n * b.h * b.w, b.c, nc, labels_dev, conf_dev, (cudaStream_t)stream);
+    return segment_launch((const float*)b.ptr.get(), (long long)n * b.h * b.w, b.c, nc, labels_dev, conf_dev, (cudaStream_t)stream);
 }
 
 int b2d_georef(b2d_engine* e, const b2d_det* dets_dev, const int32_t* counts_dev, int n, int cap, int mode, const double* params_dev,
@@ -797,8 +784,8 @@ int b2d_postprocess_obb(b2d_engine* e, int n, float conf_thr, int inclusive, flo
     B2D_ENTER(e);
     B2D_CHECK(n > 0 && n <= e->max_batch && dets_dev && counts_dev && cap > 0, "postprocess_obb: bad arguments");
     if (int rc = ensure_cand(e, n, e->head.rows_total)) return rc;
-    return obb_postprocess_launch(&e->head, n, conf_thr, inclusive, e->conf_scale, e->cand, e->cand_angle, e->cand_count, e->cand_cap, e->keys,
-                                  e->obb_prm, iou_thr, top_k, max_det, dets_dev, counts_dev, cap, (cudaStream_t)stream);
+    return obb_postprocess_launch(&e->head, n, conf_thr, inclusive, e->conf_scale, e->cand.get(), e->cand_angle.get(), e->cand_count.get(), e->cand_cap,
+                                  e->keys.get(), e->obb_prm.get(), iou_thr, top_k, max_det, dets_dev, counts_dev, cap, (cudaStream_t)stream);
 }
 
 int b2d_georef_obb(b2d_engine* e, const b2d_obb* dets_dev, const int32_t* counts_dev, int n, int cap, int mode, const double* params_dev,
@@ -810,23 +797,13 @@ int b2d_georef_obb(b2d_engine* e, const b2d_obb* dets_dev, const int32_t* counts
     return obb_georef_launch(dets_dev, counts_dev, n, cap, mode, params_dev, out_dev, (cudaStream_t)stream);
 }
 
-static int ensure_dedup_scratch(b2d_engine* e, int count) {
-    const size_t need = dedup_scratch_bytes(count);
-    if (need > e->dedup_scratch_bytes) {
-        if (e->dedup_scratch) cudaFree(e->dedup_scratch);
-        B2D_CUDA(cudaMalloc(&e->dedup_scratch, need));
-        e->dedup_scratch_bytes = need;
-    }
-    return 0;
-}
-
 int b2d_dedup(b2d_engine* e, const double* x_dev, const double* y_dev, const float* conf_dev, const long long* tiebreak_dev, int count,
               double thr, int inclusive, uint8_t* keep_dev, void* stream) {
     B2D_CHECK(e && (count == 0 || (x_dev && y_dev && conf_dev && keep_dev)), "dedup: bad arguments");
     B2D_ENTER(e);
     if (count == 0) return 0;
-    if (ensure_dedup_scratch(e, count)) return -2;
-    return dedup_launch(x_dev, y_dev, conf_dev, tiebreak_dev, count, thr, inclusive, keep_dev, e->dedup_scratch, e->dedup_scratch_bytes,
+    if (e->dedup_scratch.reserve(dedup_scratch_bytes(count))) return -2;
+    return dedup_launch(x_dev, y_dev, conf_dev, tiebreak_dev, count, thr, inclusive, keep_dev, e->dedup_scratch.get(), e->dedup_scratch.bytes(),
                         (cudaStream_t)stream);
 }
 
@@ -835,8 +812,8 @@ int b2d_seam_closure(b2d_engine* e, const double* x_dev, const double* y_dev, in
     B2D_CHECK(e && (count == 0 || (x_dev && y_dev && flag_dev)), "seam_closure: bad arguments");
     B2D_ENTER(e);
     if (count == 0) return 0;
-    if (ensure_dedup_scratch(e, count)) return -2;
-    return closure_launch(x_dev, y_dev, count, thr, inclusive, flag_dev, e->dedup_scratch, e->dedup_scratch_bytes, (cudaStream_t)stream);
+    if (e->dedup_scratch.reserve(dedup_scratch_bytes(count))) return -2;
+    return closure_launch(x_dev, y_dev, count, thr, inclusive, flag_dev, e->dedup_scratch.get(), e->dedup_scratch.bytes(), (cudaStream_t)stream);
 }
 
 int b2d_utm_forward(b2d_engine* e, const double* lon_dev, const double* lat_dev, int count, int zone, int north, double* x_dev,
@@ -867,7 +844,7 @@ int b2d_resize_windows(b2d_engine* e, const uint8_t* mosaic_dev, int mh, int mw,
         B2D_CHECK((out_kind == B2D_OUT_BF16_NHWC4 || out_kind == B2D_OUT_F16_NHWC4) && !e->bufs.empty() && e->bufs[0].c == 4 && !e->bufs[0].f32,
                   "resize_windows: dst NULL needs the planned 16-bit NHWC4 input buffer");
         B2D_CHECK(n <= e->max_batch, "resize_windows: n=%d exceeds max_batch %d", n, e->max_batch);
-        dst_dev = e->bufs[0].ptr;
+        dst_dev = e->bufs[0].ptr.get();
     }
     B2D_CHECK(out_kind == B2D_OUT_U8_NHWC || out_kind == B2D_OUT_BF16_NHWC4 || out_kind == B2D_OUT_F16_NHWC4,
               "resize_windows: out_kind %d is neither uint8 NHWC nor a 16-bit NHWC4 network input", out_kind);
@@ -878,22 +855,6 @@ int b2d_resize_windows(b2d_engine* e, const uint8_t* mosaic_dev, int mh, int mw,
 int b2d_set_conf_scale(b2d_engine* e, float scale) {
     B2D_CHECK(e && scale > 0.f, "set_conf_scale: bad arguments");
     e->conf_scale = scale;
-    return 0;
-}
-
-static int ensure_tta(b2d_engine* e, size_t lut_bytes, int n) {
-    if (lut_bytes > e->tta_luts_bytes) {
-        if (e->tta_luts) cudaFree(e->tta_luts);
-        e->tta_luts = nullptr; e->tta_luts_bytes = 0;
-        B2D_CUDA(cudaMalloc(&e->tta_luts, lut_bytes));
-        e->tta_luts_bytes = lut_bytes;
-    }
-    if (n > e->tta_sums_n) {
-        if (e->tta_sums) cudaFree(e->tta_sums);
-        e->tta_sums = nullptr; e->tta_sums_n = 0;
-        B2D_CUDA(cudaMalloc(&e->tta_sums, (size_t)n * sizeof(unsigned long long)));
-        e->tta_sums_n = n;
-    }
     return 0;
 }
 
@@ -911,8 +872,8 @@ int b2d_tta_clahe(b2d_engine* e, const uint8_t* src_dev, int n, int h, int w, do
     B2D_CHECK(e && src_dev && dst_dev && n > 0 && h > 0 && w > 0 && tiles_x > 0 && tiles_y > 0, "tta_clahe: bad arguments");
     B2D_ENTER(e);
     B2D_CHECK(aligned4(src_dev, dst_dev), "tta_clahe: pointers must be 4-byte aligned");
-    if (ensure_tta(e, (size_t)n * tiles_x * tiles_y * 256, 0)) return -2;
-    return tta_clahe_launch(src_dev, n, h, w, clip_limit, tiles_x, tiles_y, e->tta_luts, dst_dev, (cudaStream_t)stream);
+    if (e->tta_luts.reserve((size_t)n * tiles_x * tiles_y * 256)) return -2;
+    return tta_clahe_launch(src_dev, n, h, w, clip_limit, tiles_x, tiles_y, e->tta_luts.get(), dst_dev, (cudaStream_t)stream);
 }
 
 int b2d_tta_lut(b2d_engine* e, const uint8_t* src_dev, int n, long long img_bytes, const uint8_t* lut_dev, int per_image,
@@ -926,8 +887,8 @@ int b2d_tta_contrast(b2d_engine* e, const uint8_t* src_dev, int n, int h, int w,
     B2D_CHECK(e && src_dev && dst_dev && n > 0 && h > 0 && w > 0, "tta_contrast: bad arguments");
     B2D_ENTER(e);
     B2D_CHECK(aligned4(src_dev, dst_dev), "tta_contrast: pointers must be 4-byte aligned");
-    if (ensure_tta(e, (size_t)n * 256, n)) return -2;
-    return tta_contrast_launch(src_dev, n, h, w, factor, e->tta_sums, e->tta_luts, dst_dev, (cudaStream_t)stream);
+    if (e->tta_luts.reserve((size_t)n * 256) || e->tta_sums.reserve((size_t)n * sizeof(unsigned long long))) return -2;
+    return tta_contrast_launch(src_dev, n, h, w, factor, e->tta_sums.get(), e->tta_luts.get(), dst_dev, (cudaStream_t)stream);
 }
 
 int b2d_infer_tiles(b2d_engine* e, const uint8_t* src_dev, int n, int h, int w, int pitch, long long img_stride, int mode, int bgr,
@@ -944,30 +905,17 @@ int b2d_infer_tiles(b2d_engine* e, const uint8_t* src_dev, int n, int h, int w, 
 
 static int ensure_host_slot(b2d_engine* e, int slot, size_t tiles_bytes, int cap) {
     auto& hs = e->host_slot[slot];
-    if (!hs.loaded) {
-        B2D_CUDA(cudaEventCreateWithFlags(&hs.loaded, cudaEventDisableTiming));
-        B2D_CUDA(cudaEventCreateWithFlags(&hs.drained, cudaEventDisableTiming));
-    }
-    if (tiles_bytes > hs.tiles_bytes) {
-        if (hs.tiles) cudaFree(hs.tiles);
-        hs.tiles = nullptr; hs.tiles_bytes = 0;
-        B2D_CUDA(cudaMalloc(&hs.tiles, tiles_bytes));
-        hs.tiles_bytes = tiles_bytes;
-    }
+    if ((!hs.loaded && create(hs.loaded)) || (!hs.drained && create(hs.drained)) || hs.tiles.reserve(tiles_bytes)) return -2;
     if (cap > hs.cap) {
-        if (hs.params) {
-            cudaFree(hs.params); cudaFree(hs.dets); cudaFree(hs.geo); cudaFree(hs.counts);
-            cudaFreeHost(hs.params_pin); cudaFreeHost(hs.geo_pin); cudaFreeHost(hs.counts_pin);
-        }
-        hs.params = nullptr; hs.cap = 0;
+        hs.cap = 0;             // every old record block goes before any new one is allocated; the device ones come first
+        hs.params.reset(); hs.dets.reset(); hs.geo.reset(); hs.counts.reset();
+        hs.params_pin.reset(); hs.geo_pin.reset(); hs.counts_pin.reset();
         const size_t nb = (size_t)e->max_batch;
-        B2D_CUDA(cudaMalloc(&hs.params, nb * B2D_GEO_PARAMS * sizeof(double)));
-        B2D_CUDA(cudaMalloc(&hs.dets, nb * cap * sizeof(b2d_det)));
-        B2D_CUDA(cudaMalloc(&hs.geo, nb * cap * sizeof(b2d_geodet)));
-        B2D_CUDA(cudaMalloc(&hs.counts, nb * sizeof(int32_t)));
-        B2D_CUDA(cudaMallocHost(&hs.params_pin, nb * B2D_GEO_PARAMS * sizeof(double)));
-        B2D_CUDA(cudaMallocHost(&hs.geo_pin, nb * cap * sizeof(b2d_geodet)));
-        B2D_CUDA(cudaMallocHost(&hs.counts_pin, nb * sizeof(int32_t)));
+        if (hs.params.reserve(nb * B2D_GEO_PARAMS * sizeof(double)) || hs.dets.reserve(nb * cap * sizeof(b2d_det)) ||
+            hs.geo.reserve(nb * cap * sizeof(b2d_geodet)) || hs.counts.reserve(nb * sizeof(int32_t)) ||
+            hs.params_pin.reserve(nb * B2D_GEO_PARAMS * sizeof(double)) || hs.geo_pin.reserve(nb * cap * sizeof(b2d_geodet)) ||
+            hs.counts_pin.reserve(nb * sizeof(int32_t)))
+            return -2;
         hs.cap = cap;
     }
     return 0;
@@ -981,7 +929,8 @@ int b2d_detect_host(b2d_engine* e, const uint8_t* tiles_host, int n, int h, int 
     B2D_CHECK(!is_obb(e), "detect_host: the engine has an oriented-box head; the host path returns axis-aligned records only");
     B2D_ENTER(e);
     cudaStream_t s = (cudaStream_t)stream;
-    if (!e->copy_stream) B2D_CUDA(cudaStreamCreateWithFlags(&e->copy_stream, cudaStreamNonBlocking));
+    if (!e->copy_stream && create(e->copy_stream)) return -2;
+    cudaStream_t cs = e->copy_stream.get();
     const size_t img_bytes = (size_t)h * w * 3;
     const int mb = e->max_batch;
     for (int slot = 0; slot < 2; ++slot)
@@ -992,35 +941,34 @@ int b2d_detect_host(b2d_engine* e, const uint8_t* tiles_host, int n, int h, int 
     int rc = 0, k = 0, prev_i0 = -1, prev_nb = 0;
     auto flush = [&](int slot, int i0, int nb) -> int {
         auto& hs = e->host_slot[slot];
-        B2D_CUDA(cudaEventSynchronize(hs.drained));
-        memcpy(out_host + (size_t)i0 * cap, hs.geo_pin, (size_t)nb * cap * sizeof(b2d_geodet));
-        memcpy(counts_host + i0, hs.counts_pin, (size_t)nb * sizeof(int32_t));
+        B2D_CUDA(cudaEventSynchronize(hs.drained.get()));
+        memcpy(out_host + (size_t)i0 * cap, hs.geo_pin.get(), (size_t)nb * cap * sizeof(b2d_geodet));
+        memcpy(counts_host + i0, hs.counts_pin.get(), (size_t)nb * sizeof(int32_t));
         return 0;
     };
     for (int i0 = 0; i0 < n && rc == 0; i0 += mb, ++k) {
         const int nb = n - i0 < mb ? n - i0 : mb;
         auto& hs = e->host_slot[k & 1];
         // copy stream: wait until the chunk that used this slot two iterations ago has been consumed, then load
-        if (k >= 2) B2D_CUDA(cudaStreamWaitEvent(e->copy_stream, hs.drained, 0));
-        memcpy(hs.params_pin, params_host + (size_t)i0 * B2D_GEO_PARAMS, (size_t)nb * B2D_GEO_PARAMS * sizeof(double));
-        B2D_CUDA(cudaMemcpyAsync(hs.tiles, tiles_host + (size_t)i0 * img_bytes, (size_t)nb * img_bytes, cudaMemcpyHostToDevice, e->copy_stream));
-        B2D_CUDA(cudaMemcpyAsync(hs.params, hs.params_pin, (size_t)nb * B2D_GEO_PARAMS * sizeof(double), cudaMemcpyHostToDevice,
-                                 e->copy_stream));
-        B2D_CUDA(cudaEventRecord(hs.loaded, e->copy_stream));
-        B2D_CUDA(cudaStreamWaitEvent(s, hs.loaded, 0));
-        rc = b2d_infer_tiles(e, hs.tiles, nb, h, w, w * 3, (long long)img_bytes, mode, bgr, conf_thr, inclusive, iou_thr, top_k, max_det,
-                             hs.dets, hs.counts, cap, s);
-        if (rc == 0) rc = b2d_georef(e, hs.dets, hs.counts, nb, cap, geo_mode, hs.params, hs.geo, s);
+        if (k >= 2) B2D_CUDA(cudaStreamWaitEvent(cs, hs.drained.get(), 0));
+        memcpy(hs.params_pin.get(), params_host + (size_t)i0 * B2D_GEO_PARAMS, (size_t)nb * B2D_GEO_PARAMS * sizeof(double));
+        B2D_CUDA(cudaMemcpyAsync(hs.tiles.get(), tiles_host + (size_t)i0 * img_bytes, (size_t)nb * img_bytes, cudaMemcpyHostToDevice, cs));
+        B2D_CUDA(cudaMemcpyAsync(hs.params.get(), hs.params_pin.get(), (size_t)nb * B2D_GEO_PARAMS * sizeof(double), cudaMemcpyHostToDevice, cs));
+        B2D_CUDA(cudaEventRecord(hs.loaded.get(), cs));
+        B2D_CUDA(cudaStreamWaitEvent(s, hs.loaded.get(), 0));
+        rc = b2d_infer_tiles(e, hs.tiles.get(), nb, h, w, w * 3, (long long)img_bytes, mode, bgr, conf_thr, inclusive, iou_thr, top_k, max_det,
+                             hs.dets.get(), hs.counts.get(), cap, s);
+        if (rc == 0) rc = b2d_georef(e, hs.dets.get(), hs.counts.get(), nb, cap, geo_mode, hs.params.get(), hs.geo.get(), s);
         if (rc) break;
-        B2D_CUDA(cudaMemcpyAsync(hs.geo_pin, hs.geo, (size_t)nb * cap * sizeof(b2d_geodet), cudaMemcpyDeviceToHost, s));
-        B2D_CUDA(cudaMemcpyAsync(hs.counts_pin, hs.counts, (size_t)nb * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-        B2D_CUDA(cudaEventRecord(hs.drained, s));
+        B2D_CUDA(cudaMemcpyAsync(hs.geo_pin.get(), hs.geo.get(), (size_t)nb * cap * sizeof(b2d_geodet), cudaMemcpyDeviceToHost, s));
+        B2D_CUDA(cudaMemcpyAsync(hs.counts_pin.get(), hs.counts.get(), (size_t)nb * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+        B2D_CUDA(cudaEventRecord(hs.drained.get(), s));
         if (prev_i0 >= 0 && flush((k & 1) ^ 1, prev_i0, prev_nb)) return -2;
         prev_i0 = i0; prev_nb = nb;
     }
     if (rc == 0 && prev_i0 >= 0 && flush((k - 1) & 1, prev_i0, prev_nb)) return -2;
     cudaError_t err = cudaStreamSynchronize(s);
-    cudaStreamSynchronize(e->copy_stream);
+    cudaStreamSynchronize(cs);
     if (rc) return rc;
     B2D_CUDA(err);
     return 0;
