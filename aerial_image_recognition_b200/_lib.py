@@ -54,6 +54,7 @@ SIGNATURES = {
     "b2d_decode_rows_obb": (c_int, [c_void_p, c_int, c_void_p, c_void_p]),
     "b2d_postprocess_obb": (c_int, [c_void_p, c_int, c_float, c_int, c_float, c_int, c_int, c_void_p, c_void_p, c_int, c_void_p]),
     "b2d_georef_obb": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    "b2d_mosaic_nms_obb": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_float, c_float, c_void_p, c_void_p]),
     "b2d_dedup": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_double, c_int, c_void_p, c_void_p]),
     "b2d_seam_closure": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_double, c_int, c_void_p, c_void_p]),
     "b2d_utm_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),

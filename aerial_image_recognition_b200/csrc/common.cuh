@@ -70,6 +70,38 @@ class CudaBlock {
 template <class T> using DeviceBlock = CudaBlock<T, false>;
 template <class T> using PinnedBlock = CudaBlock<T, true>;
 
+// Hashed uniform grid (dedup.cu; the mosaic-wide oriented-box merge in postprocess.cu): an open-addressing table of
+// 2^k cell keys (linear probing), each slot the head of a linked list of points, built with one atomicExch per point.
+// Cell indices are biased by 2^31 so that no in-range cell packs to the empty-slot sentinel 0xFFFF...F (cell (-1, -1) did
+// with plain two's-complement packing: points there were inserted but never found, so their duplicates survived).
+constexpr long long kCellBias = 1ll << 31, kCellMax = (1ll << 31) - 2;
+__device__ __forceinline__ unsigned long long pack_cell(long long cx, long long cy) {
+    return ((unsigned long long)(cx + kCellBias) << 32) | (unsigned long long)(cy + kCellBias);
+}
+__device__ __forceinline__ unsigned hash_cell(unsigned long long k) {
+    k ^= k >> 33; k *= 0xff51afd7ed558ccdULL; k ^= k >> 33; k *= 0xc4ceb9fe1a85ec53ULL; k ^= k >> 33;
+    return (unsigned)k;
+}
+// The slot holding cell `key`, claimed if the cell has none yet (the table must have an empty slot)
+__device__ __forceinline__ unsigned cell_claim(long long* cell_key, unsigned cap_mask, unsigned long long key) {
+    unsigned slot = hash_cell(key) & cap_mask;
+    while (true) {
+        const long long prev = atomicCAS((unsigned long long*)&cell_key[slot], (unsigned long long)-1LL, key);
+        if (prev == -1LL || (unsigned long long)prev == key) return slot;
+        slot = (slot + 1) & cap_mask;
+    }
+}
+// The first point of cell `key`'s list, -1 for a cell without points
+__device__ __forceinline__ int cell_first(const long long* cell_key, const int* cell_head, unsigned cap_mask, unsigned long long key) {
+    unsigned slot = hash_cell(key) & cap_mask;
+    while (true) {
+        const long long k = cell_key[slot];
+        if (k == -1LL) return -1;
+        if ((unsigned long long)k == key) return cell_head[slot];
+        slot = (slot + 1) & cap_mask;
+    }
+}
+
 // Opt a kernel in to more than 48 KB of dynamic shared memory on the CURRENT device, once per (device, kernel): the
 // attribute is per device, so a process-global "done" flag would leave the second GPU of a process without it
 // (engine.cu; thread-safe).
@@ -248,6 +280,10 @@ int obb_postprocess_launch(const HeadDesc* h, int n, float thr, int inclusive, f
                            int max_det, b2d_obb* out, int* out_count, int cap, cudaStream_t stream);
 int obb_georef_launch(const b2d_obb* dets, const int* counts, int n, int cap, int mode, const double* params, b2d_geoobb* out,
                       cudaStream_t stream);
+// mosaic-wide ProbIoU fast NMS over n windows' records [n][cap] (n * cap fits an int), keep [n][cap]
+size_t mosaic_nms_obb_scratch_bytes(int total);
+int mosaic_nms_obb_launch(const b2d_obb* dets, const int* counts, const double* params, int n, int cap, float conf_thr, float iou_thr,
+                          uint8_t* keep, void* scratch, size_t scratch_bytes, cudaStream_t stream);
 int segment_launch(const float* logits, long long npix, int c, int nc, uint8_t* labels, float* conf, cudaStream_t stream);
 int georef_launch(const b2d_det* dets, const int* counts, int n, int cap, int mode, const double* params,
                   b2d_geodet* out, cudaStream_t stream);

@@ -27,18 +27,9 @@ struct DedupTable {
     unsigned cap_mask;
 };
 
-// Cell indices are biased by 2^31 so that no in-range cell packs to the empty-slot sentinel 0xFFFF...F (cell (-1, -1) did
-// with plain two's-complement packing: points there were inserted but never found, so their duplicates survived).
-constexpr long long kCellBias = 1ll << 31, kCellMax = (1ll << 31) - 2;
-__device__ __forceinline__ unsigned long long pack_cell(long long cx, long long cy) {
-    return ((unsigned long long)(cx + kCellBias) << 32) | (unsigned long long)(cy + kCellBias);
-}
+// The cell packing, hash and table probes are common.cuh's (pack_cell, cell_claim, cell_first).
 __device__ __forceinline__ bool cell_in_range(long long cx, long long cy) {
     return cx > -kCellMax && cx < kCellMax && cy > -kCellMax && cy < kCellMax;
-}
-__device__ __forceinline__ unsigned hash_cell(unsigned long long k) {
-    k ^= k >> 33; k *= 0xff51afd7ed558ccdULL; k ^= k >> 33; k *= 0xc4ceb9fe1a85ec53ULL; k ^= k >> 33;
-    return (unsigned)k;
 }
 
 __global__ void dedup_init_kernel(DedupTable t, int n, unsigned cap) {
@@ -56,13 +47,7 @@ __global__ void dedup_build_kernel(DedupTable t, const double* __restrict__ x, c
         t.flag[1] = 1;
         return;                                                               // the host reports the error; the point stays unlinked
     }
-    const unsigned long long key = pack_cell((long long)fx, (long long)fy);
-    unsigned slot = hash_cell(key) & t.cap_mask;
-    while (true) {
-        const long long prev = atomicCAS((unsigned long long*)&t.cell_key[slot], (unsigned long long)-1LL, key);
-        if (prev == -1LL || (unsigned long long)prev == key) break;
-        slot = (slot + 1) & t.cap_mask;
-    }
+    const unsigned slot = cell_claim(t.cell_key, t.cap_mask, pack_cell((long long)fx, (long long)fy));
     t.next[i] = atomicExch(&t.cell_head[slot], i);
 }
 
@@ -79,15 +64,7 @@ __global__ void dedup_round_kernel(DedupTable t, const double* __restrict__ x, c
     bool removed = false, wait = false;
     for (int dx = -1; dx <= 1 && !removed; ++dx)
         for (int dy = -1; dy <= 1 && !removed; ++dy) {
-            const unsigned long long key = pack_cell(cx + dx, cy + dy);
-            unsigned slot = hash_cell(key) & t.cap_mask;
-            int head = -1;
-            while (true) {
-                const long long k = t.cell_key[slot];
-                if (k == -1LL) break;
-                if ((unsigned long long)k == key) { head = t.cell_head[slot]; break; }
-                slot = (slot + 1) & t.cap_mask;
-            }
+            const int head = cell_first(t.cell_key, t.cell_head, t.cap_mask, pack_cell(cx + dx, cy + dy));
             for (int j = head; j >= 0; j = t.next[j]) {
                 if (j == i) continue;
                 const float cj = conf[j];
@@ -176,15 +153,7 @@ __global__ void closure_hook_kernel(DedupTable t, const double* __restrict__ x, 
     int m = li;
     for (int dx = -1; dx <= 1; ++dx)
         for (int dy = -1; dy <= 1; ++dy) {
-            const unsigned long long key = pack_cell(cx + dx, cy + dy);
-            unsigned slot = hash_cell(key) & t.cap_mask;
-            int head = -1;
-            while (true) {
-                const long long k = t.cell_key[slot];
-                if (k == -1LL) break;
-                if ((unsigned long long)k == key) { head = t.cell_head[slot]; break; }
-                slot = (slot + 1) & t.cap_mask;
-            }
+            const int head = cell_first(t.cell_key, t.cell_head, t.cap_mask, pack_cell(cx + dx, cy + dy));
             for (int j = head; j >= 0; j = t.next[j]) {
                 if (j == i) continue;
                 const double ddx = __dsub_rn(xi, x[j]), ddy = __dsub_rn(yi, y[j]);

@@ -5,6 +5,7 @@
 // is built op by op through b2d_plan_* and executed by b2d_forward as a fixed launch sequence.
 #include "common.cuh"
 
+#include <limits.h>
 #include <math.h>
 #include <stdarg.h>
 #include <string.h>
@@ -143,6 +144,7 @@ struct b2d_engine {
     DeviceBlock<float> cand_angle;          // oriented-box engines: the angle of each candidate slot, beside `cand`
     DeviceBlock<float4> obb_prm;            // ... and the rotated NMS's per-candidate Gaussians (2 float4 per key slot)
     DeviceBlock<void> dedup_scratch;
+    DeviceBlock<void> mosaic_nms_scratch;   // b2d_mosaic_nms_obb: per-record frame, Gaussian and grid links, the cell table
     float conf_scale = 1.0f;                // b2d_set_conf_scale: the TTA confidence adjustment (gpu_handler.py:236)
     // test-time-augmentation scratch: CLAHE tile tables / per-image byte tables, per-image grey sums
     DeviceBlock<uint8_t> tta_luts;
@@ -795,6 +797,21 @@ int b2d_georef_obb(b2d_engine* e, const b2d_obb* dets_dev, const int32_t* counts
     B2D_CHECK(mode == B2D_GEO_BOUNDS || mode == B2D_GEO_AFFINE, "georef_obb: form %d has no oriented-box variant (bounds and affine do)", mode);
     B2D_ENTER(e);
     return obb_georef_launch(dets_dev, counts_dev, n, cap, mode, params_dev, out_dev, (cudaStream_t)stream);
+}
+
+int b2d_mosaic_nms_obb(b2d_engine* e, const b2d_obb* dets_dev, const int32_t* counts_dev, const double* params_dev, int n, int cap,
+                       float conf_thr, float iou_thr, uint8_t* keep_dev, void* stream) {
+    B2D_CHECK(e, "mosaic_nms_obb: bad arguments");
+    B2D_CHECK(is_obb(e), "mosaic_nms_obb: the engine has no oriented-box head; the merge takes b2d_obb records");
+    B2D_CHECK(iou_thr > 0.f && iou_thr < 1.f, "mosaic_nms_obb: iou_thr %g is outside (0, 1)", (double)iou_thr);
+    B2D_CHECK(n >= 0 && cap > 0, "mosaic_nms_obb: bad arguments (n %d, cap %d)", n, cap);
+    B2D_CHECK((long long)n * cap <= INT_MAX, "mosaic_nms_obb: %d windows x %d records exceed the %d records of one call", n, cap, INT_MAX);
+    B2D_ENTER(e);
+    if (n == 0) return 0;
+    B2D_CHECK(dets_dev && counts_dev && params_dev && keep_dev, "mosaic_nms_obb: bad arguments");
+    if (e->mosaic_nms_scratch.reserve(mosaic_nms_obb_scratch_bytes(n * cap))) return -2;
+    return mosaic_nms_obb_launch(dets_dev, counts_dev, params_dev, n, cap, conf_thr, iou_thr, keep_dev, e->mosaic_nms_scratch.get(),
+                                 e->mosaic_nms_scratch.bytes(), (cudaStream_t)stream);
 }
 
 int b2d_dedup(b2d_engine* e, const double* x_dev, const double* y_dev, const float* conf_dev, const long long* tiebreak_dev, int count,

@@ -621,15 +621,32 @@ __device__ __forceinline__ b2d_obb obb_record(const b2d_det& d, float th) {
 // there is no serial keep scan).  Survivors are compacted in order; the walk stops when max_det are kept.  No pair is skipped.
 constexpr int kObbThreads = 1024;
 
-__device__ __forceinline__ bool probiou_suppresses(const float4 pi, const float2 qi, const float4 pj, const float2 qj, float thr) {
-    // batch_probiou(obb1 = box i, obb2 = box j); p = (x, y, A, B), q = (C, P)
-    const float a12 = __fadd_rn(pi.z, pj.z), b12 = __fadd_rn(pi.w, pj.w), c12 = __fadd_rn(qi.x, qj.x);
-    const float dy = __fsub_rn(pi.y, pj.y), dx = __fsub_rn(pi.x, pj.x);
+// batch_probiou's Gaussian of a box (_get_covariance_matrix): a = w^2 / 12, b = h^2 / 12, A = a cos^2 + b sin^2,
+// B = a sin^2 + b cos^2, C = (a - b) cos sin, and P = max(A B - C^2, 0) of the log term
+struct ObbGauss { float A, B, C, P; };
+__device__ __forceinline__ ObbGauss obb_gaussian(float w, float h, float th) {
+    const float a = __fdiv_rn(__fmul_rn(w, w), 12.0f), b = __fdiv_rn(__fmul_rn(h, h), 12.0f);
+    float sn, cs;
+    sincosf(th, &sn, &cs);
+    const float c2 = __fmul_rn(cs, cs), s2 = __fmul_rn(sn, sn);
+    ObbGauss g;
+    g.A = __fadd_rn(__fmul_rn(a, c2), __fmul_rn(b, s2));
+    g.B = __fadd_rn(__fmul_rn(a, s2), __fmul_rn(b, c2));
+    g.C = __fmul_rn(__fmul_rn(__fsub_rn(a, b), cs), sn);
+    g.P = fmaxf(__fsub_rn(__fmul_rn(g.A, g.B), __fmul_rn(g.C, g.C)), 0.f);
+    return g;
+}
+
+// batch_probiou(obb1 = box i, obb2 = box j) >= thr, from the centre difference (dx, dy) = (x_i - x_j, y_i - y_j) and the two
+// Gaussians (A, B, C, P).  batch_probiou's x2 - x1 is -dx, exactly (round-to-nearest is symmetric).
+__device__ __forceinline__ bool probiou_suppresses(float dx, float dy, float Ai, float Bi, float Ci, float Pi, float Aj, float Bj,
+                                                   float Cj, float Pj, float thr) {
+    const float a12 = __fadd_rn(Ai, Aj), b12 = __fadd_rn(Bi, Bj), c12 = __fadd_rn(Ci, Cj);
     const float den = __fsub_rn(__fmul_rn(a12, b12), __fmul_rn(c12, c12));
     const float dene = __fadd_rn(den, kProbEps);
     const float t1 = __fmul_rn(__fdiv_rn(__fadd_rn(__fmul_rn(a12, __fmul_rn(dy, dy)), __fmul_rn(b12, __fmul_rn(dx, dx))), dene), 0.25f);
-    const float t2 = __fmul_rn(__fdiv_rn(__fmul_rn(__fmul_rn(c12, __fsub_rn(pj.x, pi.x)), dy), dene), 0.5f);
-    const float t3 = __fmul_rn(logf(__fadd_rn(__fdiv_rn(den, __fadd_rn(__fmul_rn(4.0f, __fsqrt_rn(__fmul_rn(qi.y, qj.y))), kProbEps)), kProbEps)), 0.5f);
+    const float t2 = __fmul_rn(__fdiv_rn(__fmul_rn(__fmul_rn(c12, -dx), dy), dene), 0.5f);
+    const float t3 = __fmul_rn(logf(__fadd_rn(__fdiv_rn(den, __fadd_rn(__fmul_rn(4.0f, __fsqrt_rn(__fmul_rn(Pi, Pj))), kProbEps)), kProbEps)), 0.5f);
     const float bd = fminf(fmaxf(__fadd_rn(__fadd_rn(t1, t2), t3), kProbEps), 100.0f);
     const float hd = __fsqrt_rn(__fadd_rn(__fsub_rn(1.0f, expf(-bd)), kProbEps));
     const float iou = __fsub_rn(1.0f, hd);
@@ -664,16 +681,9 @@ __global__ void __launch_bounds__(kObbThreads) obb_select_kernel(const b2d_det* 
         const int s = key_slot(keys[i]);
         const b2d_det d = tc[s];
         const float off = __fmul_rn((float)d.cls, 7680.0f);
-        const float a = __fdiv_rn(__fmul_rn(d.w, d.w), 12.0f), b = __fdiv_rn(__fmul_rn(d.h, d.h), 12.0f);
-        float sn, cs;
-        sincosf(ta[s], &sn, &cs);
-        const float c2 = __fmul_rn(cs, cs), s2 = __fmul_rn(sn, sn);
-        const float A = __fadd_rn(__fmul_rn(a, c2), __fmul_rn(b, s2));
-        const float B = __fadd_rn(__fmul_rn(a, s2), __fmul_rn(b, c2));
-        const float Cc = __fmul_rn(__fmul_rn(__fsub_rn(a, b), cs), sn);
-        const float P = fmaxf(__fsub_rn(__fmul_rn(A, B), __fmul_rn(Cc, Cc)), 0.f);
-        tp[2 * i] = make_float4(__fadd_rn(d.cx, off), __fadd_rn(d.cy, off), A, B);
-        tp[2 * i + 1] = make_float4(Cc, P, 0.f, 0.f);
+        const ObbGauss g = obb_gaussian(d.w, d.h, ta[s]);
+        tp[2 * i] = make_float4(__fadd_rn(d.cx, off), __fadd_rn(d.cy, off), g.A, g.B);
+        tp[2 * i + 1] = make_float4(g.C, g.P, 0.f, 0.f);
     }
     if (tid == 0) s_nk = 0;
     __syncthreads();
@@ -698,8 +708,12 @@ __global__ void __launch_bounds__(kObbThreads) obb_select_kernel(const b2d_det* 
             __syncthreads();
             if (alive) {
                 const int end = min(kObbThreads, j - ib);   // i < j
-                for (int k = 0; k < end; ++k)
-                    if (probiou_suppresses(sp[k], sq[k], pj, qj, iou_thr)) { alive = false; break; }
+                for (int k = 0; k < end; ++k) {
+                    const float4 pi = sp[k];
+                    const float2 qi = sq[k];
+                    if (probiou_suppresses(__fsub_rn(pi.x, pj.x), __fsub_rn(pi.y, pj.y), pi.z, pi.w, qi.x, qi.y, pj.z, pj.w, qj.x, qj.y,
+                                           iou_thr)) { alive = false; break; }
+                }
             }
         }
         // compact the survivors of this block in order
@@ -740,6 +754,25 @@ __device__ __forceinline__ void obb_corners(float cx, float cy, float w, float h
     px[3] = __fadd_rn(__fsub_rn(cx, v1x), v2x); py[3] = __fadd_rn(__fsub_rn(cy, v1y), v2y);
 }
 
+// B2D_GEO_AFFINE's letterbox undo of an oriented box (Ultralytics scale_boxes without clipping): centre (x - pad) / gain and
+// size / gain in fp32, theta unchanged; P = gt[0..5], win_x, win_y, pad_x, pad_y, gain.  The window offset is added in fp64
+// by source_px.  obb_georef_kernel and the mosaic merge (mosaic_nms_prep_kernel) both map boxes with these two, so the merged
+// boxes and the georeferenced footprints are in one frame.
+struct ObbUndo { float cx, cy, w, h; };
+__device__ __forceinline__ ObbUndo obb_affine_undo(const b2d_obb& d, const double* P) {
+    const float padx = (float)P[8], pady = (float)P[9], gain = (float)P[10];
+    ObbUndo u;
+    u.cx = __fdiv_rn(__fsub_rn(d.cx, padx), gain);
+    u.cy = __fdiv_rn(__fsub_rn(d.cy, pady), gain);
+    u.w = __fdiv_rn(d.w, gain);
+    u.h = __fdiv_rn(d.h, gain);
+    return u;
+}
+// a window pixel (fp32) in the mosaic's pixel frame: + (win_x, win_y) in fp64
+__device__ __forceinline__ double2 source_px(float px, float py, const double* P) {
+    return make_double2(__dadd_rn((double)px, P[6]), __dadd_rn((double)py, P[7]));
+}
+
 __global__ void __launch_bounds__(256) obb_georef_kernel(const b2d_obb* __restrict__ dets, const int* __restrict__ counts, int cap, int mode,
                                                           const double* __restrict__ params, b2d_geoobb* __restrict__ out) {
     const int tile = blockIdx.y;
@@ -761,21 +794,174 @@ __global__ void __launch_bounds__(256) obb_georef_kernel(const b2d_obb* __restri
 #pragma unroll
         for (int k = 0; k < 5; ++k) geo_bounds(P, (double)px[k], (double)py[k], &gx[k], &gy[k]);
     } else {
-        // affine: undo the letterbox in fp32 (centre - pad, / gain; w, h / gain; no clipping), corners in fp32, then the window
-        // offset and the 6-term geotransform in fp64.  P = gt[0..5], win_x, win_y, pad_x, pad_y, gain
-        const float padx = (float)P[8], pady = (float)P[9], gain = (float)P[10];
-        const float cx = __fdiv_rn(__fsub_rn(d.cx, padx), gain), cy = __fdiv_rn(__fsub_rn(d.cy, pady), gain);
-        g.w = __fdiv_rn(d.w, gain);
-        g.h = __fdiv_rn(d.h, gain);
-        obb_corners(cx, cy, g.w, g.h, d.theta, px, py);
-        px[4] = cx; py[4] = cy;
+        // affine: undo the letterbox in fp32, corners in fp32, then the window offset and the 6-term geotransform in fp64
+        const ObbUndo u = obb_affine_undo(d, P);
+        g.w = u.w;
+        g.h = u.h;
+        obb_corners(u.cx, u.cy, u.w, u.h, d.theta, px, py);
+        px[4] = u.cx; py[4] = u.cy;
 #pragma unroll
-        for (int k = 0; k < 5; ++k) geo_affine(P, __dadd_rn((double)px[k], P[6]), __dadd_rn((double)py[k], P[7]), &gx[k], &gy[k]);
+        for (int k = 0; k < 5; ++k) {
+            const double2 m = source_px(px[k], py[k], P);
+            geo_affine(P, m.x, m.y, &gx[k], &gy[k]);
+        }
     }
     g.x = gx[4]; g.y = gy[4];
 #pragma unroll
     for (int k = 0; k < 4; ++k) { g.corners[2 * k] = gx[k]; g.corners[2 * k + 1] = gy[k]; }
     out[(size_t)tile * cap + i] = g;
+}
+
+// ---- mosaic-wide oriented-box merge (b2d_mosaic_nms_obb) -------------------------------------------------------------
+// Ultralytics' DOTA slice merge, fast NMS over every window's records in the mosaic's pixel frame: record j is suppressed iff
+// an eligible record i of the same class and higher priority (confidence descending, then lower index k = row * cap + slot)
+// has ProbIoU(i, j) >= thr.  The fate of j depends on its higher-priority neighbours only, not on theirs, so there is no sort
+// and no rounds: keep starts as "eligible", and every examined pair that suppresses stores 0 into the keep byte of its
+// lower-priority member.  The store is idempotent and the set of pairs examined does not depend on scheduling, so the result
+// is deterministic.  Which pairs must be examined:
+//
+// A record is REGULAR when X, Y, w', h', theta are finite, |X|, |Y| < 2^31, its short side s = min(w', h') >= 1 px, its
+// long side L <= kMnmsAspect s and L <= the grid's reach (below).  For two regular boxes (exact arithmetic first), with
+// S = Sigma_i + Sigma_j and d = the centre difference:
+//   t1 + t2 = 1/4 d^T S^-1 d * det S / (det S + eps)  >=  |d|^2 / (4 lmax(S)) * (1 - eps / det S),
+//   lmax(S) <= lmax(Sigma_i) + lmax(Sigma_j) = (L_i^2 + L_j^2) / 12,
+//   det S >= (sqrt det Sigma_i + sqrt det Sigma_j)^2 >= 4 sqrt(P_i P_j)   (Minkowski), so t3 >= 1/2 ln(1 / (1 + eps / (4 sqrt(P_i P_j)))),
+// and s >= 1 gives P >= 1/144, det S >= 1/36: eps / det S <= 3.6e-6.  ProbIoU >= thr needs bd <= bd* = -ln(1 + eps - (1 - thr)^2).
+// fp32: u = 2^-24, rho = L / s <= 128, so u rho^2 <= 2^-10.  sincosf and the roundings of A, B, C perturb each Sigma by at
+// most 16 u a in norm (a = L^2 / 12): its eigenvalues stay in [b (1 - 2^-6), a (1 + 16 u)], b = s^2 / 12, and it stays
+// positive definite, so the bounds above hold for the computed Gaussians.  Cancellation is bounded by the condition number
+// lmax / lmin <= 1.04 rho^2 of S: den = a12 b12 - c12^2 is within 8 u lmax^2 = 0.9 % of det S, each P within 0.7 %, and
+// t1 + t2 (positive t1 against t2 with |t2| <= lmax |d|^2 / (4 dene)) within 15 u lmax / lmin = 1.6 %.  So the computed
+//   t1 + t2 >= 0.976 * 3 |d|^2 / (L_i^2 + L_j^2)  and  t3 >= 1/2 ln(0.9919 / 1.0063) - 1 ulp >= -0.0073.
+// The computed iou is 1 - sqrt(1 - expf(-bd) + eps) with expf within 2 ulp and the rest correctly rounded; iou >= thr then
+// needs bd <= bd_lim = -ln(1 + eps - (1 - thr + 4u)^2 (1 + 2u) - 8u), or bd_lim = 100 where that argument is not positive
+// (bd is clamped to 100, where the computed iou is 0 < thr).  Hence a regular pair can only suppress when
+//   |d|^2 <= K (L_i^2 + L_j^2),   K = (bd_lim + 1/16) * 17 / 48          (>= (bd_lim + 0.008) / 2.928, the bound above)
+// -- at thr 0.3, |d| <= 0.72 max(L_i, L_j) (0.67 without the rounding margins).  The pair is examined by its member with the longer side (ties: the higher index),
+// within R = sqrt(2 K) L + 1 px of it (L of the partner <= L, 1 px covers the fp64 rounding of the scan window), over the cells
+// of a hashed uniform grid of kMnmsCell px; a box whose R would span more than kMnmsReach cells either side is not regular.
+// So one large box among millions of small ones widens its own scan only.
+//
+// Every other eligible record is IRREGULAR (zero-area, needle, huge, far or non-finite boxes: with eps = 1e-7 two zero-area
+// boxes of one class reach ProbIoU 0.9995 at any distance).  They sit in a compacted list, and each is tested against every
+// eligible record, the bound being used for none of them: O(D N) for D irregular records.
+constexpr double kMnmsCell = 64.0;        // px; a power of two, so X / cell is exact
+constexpr int kMnmsReach = 48;            // cells either side of a regular box's own cell
+constexpr float kMnmsAspect = 128.f;
+constexpr double kMnmsMaxCoord = 2147483648.0;
+
+struct MnmsGrid {
+    double2* xy;            // [N] merge-frame centre (eligible records)
+    float4* gs;             // [N] Gaussian A, B, C, P (eligible records)
+    float* len;             // [N] long side (regular records)
+    uint8_t* kind;          // [N] 0 not eligible, 1 regular (in the grid), 2 irregular (in the list)
+    int* next;              // [N] next point of the same cell
+    int* irr;               // [N] the irregular records, *irr_count of them, in no particular order
+    int* irr_count;
+    long long* cell_key;    // [cap_mask + 1]
+    int* cell_head;
+    unsigned cap_mask;
+};
+
+__global__ void __launch_bounds__(256) mosaic_nms_prep_kernel(const b2d_obb* __restrict__ dets, const int* __restrict__ counts,
+                                                              const double* __restrict__ params, int cap, int total, float conf_thr,
+                                                              float max_len, MnmsGrid g, uint8_t* __restrict__ keep) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= total) return;
+    const int r = k / cap, s = k - r * cap;
+    const b2d_obb d = dets[k];
+    const bool eligible = s < counts[r] && d.conf > conf_thr;
+    keep[k] = eligible ? 1 : 0;
+    if (!eligible) { g.kind[k] = 0; return; }
+    const double* P = params + (size_t)r * B2D_GEO_PARAMS;
+    const ObbUndo u = obb_affine_undo(d, P);
+    const double2 m = source_px(u.cx, u.cy, P);
+    const ObbGauss q = obb_gaussian(u.w, u.h, d.theta);
+    g.xy[k] = m;
+    g.gs[k] = make_float4(q.A, q.B, q.C, q.P);
+    const float sh = fminf(u.w, u.h), L = fmaxf(u.w, u.h);
+    const bool regular = fabs(m.x) < kMnmsMaxCoord && fabs(m.y) < kMnmsMaxCoord && isfinite(u.w) && isfinite(u.h) &&
+                         isfinite(d.theta) && sh >= 1.f && L <= __fmul_rn(kMnmsAspect, sh) && L <= max_len;
+    if (regular) {
+        g.len[k] = L;
+        const long long cx = (long long)floor(m.x * (1.0 / kMnmsCell)), cy = (long long)floor(m.y * (1.0 / kMnmsCell));
+        const unsigned slot = cell_claim(g.cell_key, g.cap_mask, pack_cell(cx, cy));
+        g.next[k] = atomicExch(&g.cell_head[slot], k);
+        g.kind[k] = 1;
+    } else {
+        g.irr[atomicAdd(g.irr_count, 1)] = k;
+        g.kind[k] = 2;
+    }
+}
+
+// Examine the pair (k, t) of one class: the higher-priority member as batch_probiou's obb1, dx = (float)(X_hi - X_lo)
+__device__ __forceinline__ void mnms_pair(const MnmsGrid& g, int k, double2 pk, float4 qk, float ck, int t, float ct, float thr,
+                                          uint8_t* keep) {
+    const bool k_first = ck > ct || (ck == ct && k < t);
+    const int lo = k_first ? t : k;
+    if (((volatile uint8_t*)keep)[lo] == 0) return;          // already suppressed: a keep byte never returns to 1
+    const double2 pt = g.xy[t];
+    const float4 qt = g.gs[t];
+    const double2 ph = k_first ? pk : pt, pl = k_first ? pt : pk;
+    const float4 qh = k_first ? qk : qt, ql = k_first ? qt : qk;
+    if (probiou_suppresses((float)__dsub_rn(ph.x, pl.x), (float)__dsub_rn(ph.y, pl.y), qh.x, qh.y, qh.z, qh.w, ql.x, ql.y, ql.z, ql.w, thr))
+        keep[lo] = 0;
+}
+
+__global__ void __launch_bounds__(256) mosaic_nms_grid_kernel(const b2d_obb* __restrict__ dets, int total, double reach_coef, float thr,
+                                                              MnmsGrid g, uint8_t* keep) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= total || g.kind[k] != 1) return;
+    const double2 p = g.xy[k];
+    const float4 q = g.gs[k];
+    const float L = g.len[k];
+    const int cls = dets[k].cls;
+    const float conf = dets[k].conf;
+    const double R = __dadd_rn(__dmul_rn(reach_coef, (double)L), 1.0);
+    const double ic = 1.0 / kMnmsCell;
+    const long long x0 = (long long)floor(__dsub_rn(p.x, R) * ic), x1 = (long long)floor(__dadd_rn(p.x, R) * ic);
+    const long long y0 = (long long)floor(__dsub_rn(p.y, R) * ic), y1 = (long long)floor(__dadd_rn(p.y, R) * ic);
+    for (long long cx = x0; cx <= x1; ++cx)
+        for (long long cy = y0; cy <= y1; ++cy)
+            for (int t = cell_first(g.cell_key, g.cell_head, g.cap_mask, pack_cell(cx, cy)); t >= 0; t = g.next[t]) {
+                const float Lt = g.len[t];
+                if (!(Lt < L || (Lt == L && t < k))) continue;      // the pair belongs to its member with the longer side
+                if (dets[t].cls != cls) continue;
+                mnms_pair(g, k, p, q, conf, t, dets[t].conf, thr, keep);
+            }
+}
+
+// Every eligible record against the irregular list; a pair of two irregular records is examined once, by the lower index
+__global__ void __launch_bounds__(256) mosaic_nms_irregular_kernel(const b2d_obb* __restrict__ dets, int total, float thr, MnmsGrid g,
+                                                                   uint8_t* keep) {
+    __shared__ int s_irr[256];
+    const int nd = *g.irr_count;
+    if (nd == 0) return;
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    const int kind = k < total ? g.kind[k] : 0;
+    double2 p = make_double2(0.0, 0.0);
+    float4 q = make_float4(0.f, 0.f, 0.f, 0.f);
+    int cls = 0;
+    float conf = 0.f;
+    if (kind) { p = g.xy[k]; q = g.gs[k]; cls = dets[k].cls; conf = dets[k].conf; }
+    for (int base = 0; base < nd; base += 256) {
+        __syncthreads();
+        if (base + (int)threadIdx.x < nd) s_irr[threadIdx.x] = g.irr[base + threadIdx.x];
+        __syncthreads();
+        if (!kind) continue;
+        const int m = min(256, nd - base);
+        for (int i = 0; i < m; ++i) {
+            const int t = s_irr[i];
+            if (t == k || (kind == 2 && t < k) || dets[t].cls != cls) continue;
+            mnms_pair(g, k, p, q, conf, t, dets[t].conf, thr, keep);
+        }
+    }
+}
+
+size_t mnms_table_cap(int total) {
+    size_t cap = 1024;
+    while (cap < 2 * (size_t)total) cap <<= 1;
+    return cap;
 }
 
 // Sorts each tile's candidates into keys (tile stride keys_stride(cand_cap)): by confidence, else in slot order
@@ -820,6 +1006,52 @@ int obb_georef_launch(const b2d_obb* dets, const int* counts, int n, int cap, in
     if (n <= 0 || cap <= 0) return 0;
     dim3 grid(ceil_div(cap, 256), n);
     obb_georef_kernel<<<grid, 256, 0, stream>>>(dets, counts, cap, mode, params, out);
+    B2D_LAUNCH_CHECK();
+    return 0;
+}
+
+// Scratch of the mosaic merge: per-record arrays, then the grid's cell table, each 256-byte aligned
+static size_t mnms_layout(int total, uint8_t* base, MnmsGrid* g) {
+    const size_t n = (size_t)total, cap = mnms_table_cap(total);
+    size_t off = 0;
+    auto take = [&](size_t bytes) { uint8_t* p = base ? base + off : nullptr; off += (bytes + 255) & ~(size_t)255; return p; };
+    MnmsGrid t;
+    t.xy = (double2*)take(n * sizeof(double2));
+    t.gs = (float4*)take(n * sizeof(float4));
+    t.len = (float*)take(n * sizeof(float));
+    t.kind = take(n);
+    t.next = (int*)take(n * sizeof(int));
+    t.irr = (int*)take(n * sizeof(int));
+    t.irr_count = (int*)take(sizeof(int));
+    t.cell_key = (long long*)take(cap * sizeof(long long));
+    t.cell_head = (int*)take(cap * sizeof(int));
+    t.cap_mask = (unsigned)(cap - 1);
+    if (g) *g = t;
+    return off;
+}
+
+size_t mosaic_nms_obb_scratch_bytes(int total) { return mnms_layout(total, nullptr, nullptr); }
+
+int mosaic_nms_obb_launch(const b2d_obb* dets, const int* counts, const double* params, int n, int cap, float conf_thr, float iou_thr,
+                          uint8_t* keep, void* scratch, size_t scratch_bytes, cudaStream_t stream) {
+    const int total = n * cap;                 // the caller has checked that n * cap fits an int
+    if (total <= 0) return 0;
+    B2D_CHECK(scratch_bytes >= mosaic_nms_obb_scratch_bytes(total), "mosaic_nms_obb: scratch too small");
+    MnmsGrid g;
+    const size_t cell_bytes = mnms_layout(total, (uint8_t*)scratch, &g) - (size_t)((uint8_t*)g.cell_key - (uint8_t*)scratch);
+    // the proof above mosaic_nms_prep_kernel: bd_lim, K and the scan radius sqrt(2 K) L of a regular box's long side L
+    const double u = 1.0 / 16777216.0, eps = (double)kProbEps;
+    const double hm = 1.0 - (double)iou_thr + 4.0 * u;
+    const double arg = 1.0 + eps - hm * hm * (1.0 + 2.0 * u) - 8.0 * u;
+    const double bd_lim = arg > exp(-100.0) ? fmin(-log(arg), 100.0) : 100.0;
+    const double reach_coef = sqrt(2.0 * (bd_lim + 1.0 / 16.0) * 17.0 / 48.0);
+    const float max_len = (float)((kMnmsReach * kMnmsCell - 1.0) / reach_coef);
+    B2D_CUDA(cudaMemsetAsync(g.cell_key, 0xFF, cell_bytes, stream));          // cell keys and heads: -1
+    B2D_CUDA(cudaMemsetAsync(g.irr_count, 0, sizeof(int), stream));
+    const int blocks = ceil_div(total, 256);
+    mosaic_nms_prep_kernel<<<blocks, 256, 0, stream>>>(dets, counts, params, cap, total, conf_thr, max_len, g, keep);
+    mosaic_nms_grid_kernel<<<blocks, 256, 0, stream>>>(dets, total, reach_coef, iou_thr, g, keep);
+    mosaic_nms_irregular_kernel<<<blocks, 256, 0, stream>>>(dets, total, iou_thr, g, keep);
     B2D_LAUNCH_CHECK();
     return 0;
 }

@@ -270,6 +270,20 @@ class Engine:
                                        self.stream), "georef")
         return out
 
+    def mosaic_nms_obb(self, dets: torch.Tensor, counts: torch.Tensor, params: torch.Tensor, conf_thr: float, iou_thr: float) -> torch.Tensor:
+        """Mosaic-wide ProbIoU fast NMS of an oriented-box engine's window records (``b2d_mosaic_nms_obb``): dets float32
+        [n, cap, 9] ``OBB_DTYPE`` records and counts int32 [n] as ``postprocess`` returns them, params float64 [n, 16] in the
+        "affine" form of each window.  Returns keep uint8 [n, cap]: 1 for a record with ``conf > conf_thr`` that no record of
+        its class with higher priority (confidence, then lower row, then lower slot) overlaps by ProbIoU >= ``iou_thr``."""
+        n, cap = dets.shape[0], dets.shape[1]
+        assert dets.dtype == torch.float32 and dets.is_cuda and dets.dim() == 3 and dets.shape[2] == OBB_WORDS
+        assert counts.dtype == torch.int32 and tuple(counts.shape) == (n,) and counts.is_cuda
+        assert params.dtype == torch.float64 and tuple(params.shape) == (n, GEO_PARAMS) and params.is_cuda
+        keep = torch.empty((n, cap), dtype=torch.uint8, device=self.device)
+        _lib.check(self.lib.b2d_mosaic_nms_obb(self.h, _ptr(dets.contiguous()), _ptr(counts.contiguous()), _ptr(params.contiguous()), n, cap,
+                                               float(conf_thr), float(iou_thr), _ptr(keep), self.stream), "mosaic_nms_obb")
+        return keep
+
     def dedup(self, x: torch.Tensor, y: torch.Tensor, conf: torch.Tensor, thr: float, inclusive: bool = True,
               tiebreak: Optional[torch.Tensor] = None) -> torch.Tensor:
         n = x.numel()

@@ -1,4 +1,5 @@
-"""Sliding-window detection over a large georeferenced mosaic, tile-sharded across GPUs.
+"""Sliding-window detection over a large georeferenced mosaic, tile-sharded across GPUs (``MosaicDetector``), and oriented-box
+detection over a whole mosaic on one GPU, merged by a mosaic-wide ProbIoU fast NMS (``ObbMosaicDetector``).
 
 Ancestor in the reference: the notebook loop at ``x_arch/02_analyze_images:1 (cell 6)`` --
 ``for y in range(0,h,stride): for x in range(0,w,stride): model(window)`` -> boxes with
@@ -136,6 +137,47 @@ def affine_params(windows: np.ndarray, geotransform: Sequence[float], win: int =
     return p
 
 
+def run_windows(eng, mosaic, windows: np.ndarray, y_offset: int, gt: Sequence[float], win: int, fill: int, nms_conf: float, iou: float,
+                max_det: int):
+    """Detection on every window (x0, y0, w0, h0) of ``windows`` (mosaic coordinates; ``mosaic`` is the uint8 CUDA tensor of pixel
+    rows [y_offset, ...)): cut (win = the model input) or resampled windows, network, per-window NMS and affine georef, batch
+    by batch with nothing read back.  Returns device tensors (geo records [n, cap, *], dets [n, cap, *], counts [n], affine params
+    [n, 16]) in window order -- records of ``eng``'s kind, axis-aligned or oriented -- or None for no windows."""
+    import torch
+    dev = eng.device
+    if not len(windows):
+        return None
+    # equal batches: 780 windows at max_batch 64 are 13 launches either way, but 13 x 60 keeps every step full
+    # where 12 x 64 + 12 ends a band on a step that is four fifths empty
+    nb = -(-len(windows) // eng.max_batch)
+    B = -(-len(windows) // nb)
+    local = windows.copy()
+    local[:, 1] -= y_offset
+    # every per-window table goes to the device once; the batch loop below queues kernels only (no host
+    # synchronisation: a boolean-mask gather per batch would stall the launch queue ~100 times per mosaic)
+    resample = win != eng.imgsz
+    if resample:
+        # windows of another size are resampled from the mosaic straight into the network input: checked once here,
+        # since the per-batch launches below leave the origins on the device
+        check_windows(local, win, mosaic.shape[0], mosaic.shape[1])
+    params_all = torch.from_numpy(affine_params(windows, gt, win, eng.imgsz if resample else None)).to(dev)
+    org_all = torch.from_numpy(local).to(dev)
+    outs = []
+    for s in range(0, len(windows), B):
+        e = min(s + B, len(windows))
+        n = e - s
+        if resample:
+            eng.resize_windows(mosaic, org_all[s:e], win, fill, checked=True)
+            eng.forward(n)
+            dets, counts = eng.postprocess(n, nms_conf, False, iou, 0, max_det)
+        else:
+            tiles = eng.cut_windows(mosaic, org_all[s:e], win, fill)
+            dets, counts = eng.infer(tiles, "identity", False, nms_conf, False, iou, 0, max_det)
+        geo = eng.georef(dets, counts, params_all[s:e], "affine")
+        outs.append((geo, dets, counts))
+    return (torch.cat([o[0] for o in outs]), torch.cat([o[1] for o in outs]), torch.cat([o[2] for o in outs]), params_all)
+
+
 # -------------------------------------------------------------------------------------------------
 # seam exchange: host-side protocol, independent of the device (tested on CPU with gloo)
 # -------------------------------------------------------------------------------------------------
@@ -209,42 +251,12 @@ class MosaicDetector:
         import torch
         eng = self.eng
         dev = eng.device
-        outs = []
-        # equal batches: 780 windows at max_batch 64 are 13 launches either way, but 13 x 60 keeps every step full
-        # where 12 x 64 + 12 ends a band on a step that is four fifths empty
-        nb = -(-len(windows) // eng.max_batch) if len(windows) else 1
-        B = -(-len(windows) // nb) if len(windows) else eng.max_batch
-        local = windows.copy()
-        local[:, 1] -= y_offset
-        # every per-window table goes to the device once; the batch loop below queues kernels only (no host
-        # synchronisation: a boolean-mask gather per batch would stall the launch queue ~100 times per mosaic)
-        resample = self.win != eng.imgsz
-        if resample:
-            # windows of another size are resampled from the mosaic straight into the network input: checked once here,
-            # since the per-batch launches below leave the origins on the device
-            check_windows(local, self.win, mosaic.shape[0], mosaic.shape[1])
-        params_all = torch.from_numpy(affine_params(windows, self.gt, self.win, eng.imgsz if resample else None)).to(dev)
-        org_all = torch.from_numpy(local).to(dev)
-        ids_all = torch.from_numpy(ids).to(dev)
-        for s in range(0, len(windows), B):
-            e = min(s + B, len(windows))
-            n = e - s
-            if resample:
-                eng.resize_windows(mosaic, org_all[s:e], self.win, self.fill, checked=True)
-                eng.forward(n)
-                dets, counts = eng.postprocess(n, self.nms_conf, False, self.iou, 0, self.max_det)
-            else:
-                tiles = eng.cut_windows(mosaic, org_all[s:e], self.win, self.fill)
-                dets, counts = eng.infer(tiles, "identity", False, self.nms_conf, False, self.iou, 0, self.max_det)
-            geo = eng.georef(dets, counts, params_all[s:e], "affine")
-            outs.append((geo, dets, counts, ids_all[s:e]))
-        if not outs:
+        out = run_windows(eng, mosaic, windows, y_offset, self.gt, self.win, self.fill, self.nms_conf, self.iou, self.max_det)
+        if out is None:
             z = torch.zeros(0, device=dev)
             return z.double(), z.double(), z.float(), z.int(), z.long(), z.int(), z.float()
-        geo = torch.cat([o[0] for o in outs])
-        dets = torch.cat([o[1] for o in outs])
-        counts = torch.cat([o[2] for o in outs])
-        wid_n = torch.cat([o[3] for o in outs])
+        geo, dets, counts, _ = out
+        wid_n = torch.from_numpy(ids).to(dev)
         n, cap = dets.shape[0], dets.shape[1]
         slot = torch.arange(cap, device=dev, dtype=torch.int32)[None, :].expand(n, cap)
         conf = dets[..., 4]
@@ -386,3 +398,57 @@ class MosaicDetector:
         x, y, conf, cls, wid, slot, py = self.detect_windows(mosaic, windows, ids, y_offset)
         self.last_raw = int(x.numel())
         return self.dedup(x, y, conf, cls, wid, slot, py, rank, world, covers, group)
+
+
+class ObbMosaicDetector:
+    """Oriented-box detection over a whole orthomosaic on one GPU: every window of the y-outer / x-inner grid through an
+    oriented-box engine (``Engine("yolov8m-obb")``), then ONE mosaic-wide merge on the device (``Engine.mosaic_nms_obb``):
+    Ultralytics' DOTA slice merge, ProbIoU fast NMS at ``merge_iou`` one class at a time over the records with
+    ``conf > conf``, in the mosaic's pixel frame, so an object seen by two to four overlapping windows is reported once.
+    Priority ties go to the earlier window, then the lower slot.  ``run`` returns the survivors' georeferenced footprints."""
+
+    # GEOOBB_DTYPE with the global window (int64) in place of the batch-local tile, and the slot inside the window; the device
+    # writes these 112-byte records and the host only re-labels them
+    OUT_DTYPE = np.dtype({"names": ["x", "y", "corners", "conf", "w", "h", "theta", "cls", "slot", "window"],
+                          "formats": ["<f8", "<f8", ("<f8", (4, 2)), "<f4", "<f4", "<f4", "<f4", "<i4", "<i4", "<i8"],
+                          "offsets": [0, 8, 16, 80, 84, 88, 92, 96, 100, 104], "itemsize": 112})
+
+    def __init__(self, engine, geotransform: Sequence[float], win: int = 640, stride: int = 512, conf: float = 0.4,
+                 nms_conf: float = 0.25, iou: float = 0.7, max_det: int = 300, merge_iou: float = 0.3, fill: int = 114):
+        if not getattr(engine, "is_obb", False):
+            raise ValueError(f"ObbMosaicDetector needs an oriented-box engine (e.g. Engine('yolov8m-obb')); {engine.arch!r} is "
+                             "axis-aligned: use MosaicDetector")
+        self.eng = engine
+        self.gt = tuple(float(v) for v in geotransform)
+        self.win, self.stride = win, stride
+        self.conf, self.nms_conf, self.iou, self.max_det = conf, nms_conf, iou, max_det
+        self.merge_iou = merge_iou
+        self.fill = fill
+        assert self.gt[2] == 0.0 and self.gt[4] == 0.0, "the merge frame is the mosaic's pixel grid: an axis-aligned geotransform"
+
+    def run(self, mosaic, height: int, width: int) -> np.ndarray:
+        """mosaic: uint8 CUDA tensor [height, width, 3].  Returns ``OUT_DTYPE`` records of the merge's survivors in ascending
+        (window, slot) order; ``last_raw`` is the number of records with ``conf > conf`` before the merge."""
+        import torch
+        eng = self.eng
+        windows = window_grid(height, width, self.win, self.stride)
+        out = run_windows(eng, mosaic, windows, 0, self.gt, self.win, self.fill, self.nms_conf, self.iou, self.max_det)
+        if out is None:
+            self.last_raw = 0
+            return np.zeros(0, self.OUT_DTYPE)
+        geo, dets, counts, params = out
+        keep = eng.mosaic_nms_obb(dets, counts, params, self.conf, self.merge_iou)
+        n, cap = keep.shape
+        slot = torch.arange(cap, device=eng.device, dtype=torch.int32)[None, :].expand(n, cap)
+        self.last_raw = int(((slot < counts[:, None]) & (dets[..., 5] > self.conf)).sum())
+        idx = keep.reshape(-1).nonzero().squeeze(1)                   # ascending record index = (window, slot) order
+        m = int(idx.numel())
+        words = geo.view(torch.int32).view(n * cap, -1)                 # 26 words: x, y, corners, conf, w, h, theta, cls, tile
+        rec = torch.empty((m, 28), dtype=torch.int32, device=eng.device)
+        rec[:, :25] = words[idx, :25]
+        rec[:, 25] = (idx % cap).int()
+        rec.view(torch.int64)[:, 13] = idx // cap
+        host = torch.empty((m, 28), dtype=torch.int32).pin_memory() if m else torch.empty((0, 28), dtype=torch.int32)
+        host.copy_(rec, non_blocking=True)
+        torch.cuda.current_stream(eng.device).synchronize()
+        return host.numpy().view(self.OUT_DTYPE).reshape(m).copy()

@@ -220,6 +220,24 @@ int b2d_postprocess_obb(b2d_engine* e, int n, float conf_thr, int inclusive, flo
 int b2d_georef_obb(b2d_engine* e, const b2d_obb* dets_dev, const int32_t* counts_dev, int n, int cap,
                    int mode, const double* params_dev, b2d_geoobb* out_dev, void* stream);
 
+/* Mosaic-wide merge of oriented boxes from overlapping windows: Ultralytics' DOTA slice merge (obb/val.py, nms_rotated
+ * ProbIoU "fast NMS" on boxes shifted into the full-image frame), over all windows at once.  dets_dev b2d_obb [n][cap] with
+ * counts_dev int32 [n] (b2d_postprocess_obb), params_dev double [n][B2D_GEO_PARAMS] in the B2D_GEO_AFFINE form of each window;
+ * record (r, s) is row r, slot s.  keep_dev uint8 [n][cap].  The rule:
+ *  1. frame: cx' = (cx - pad_x) / gain, cy' likewise, w' = w / gain, h' likewise, in fp32, theta unchanged;
+ *     X = (double)cx' + win_x, Y likewise, in fp64 -- b2d_georef_obb's B2D_GEO_AFFINE arithmetic, so merged boxes and
+ *     georeferenced footprints are in one frame;
+ *  2. eligible iff s < counts[r] and conf > conf_thr (strict); an ineligible record is never kept and suppresses nothing;
+ *  3. priority: confidence descending as floats compare (+0.0 == -0.0), ties to the lower row, then the lower slot;
+ *  4. record j is suppressed iff an eligible record i of higher priority and the same class (no class offset) has
+ *     ProbIoU(i, j) >= iou_thr, with i as batch_probiou's obb1, centre difference dx = (float)(X_i - X_j) (dy likewise)
+ *     and each box's Gaussian from (w', h', theta) as in b2d_postprocess_obb; a suppressed record still suppresses;
+ *  5. keep = eligible and not suppressed.
+ * The result equals the all-pairs evaluation of this rule, degenerate and non-finite boxes included (DESIGN.md section 6).
+ * iou_thr must lie in (0, 1) and n * cap must fit an int32.                                                           */
+int b2d_mosaic_nms_obb(b2d_engine* e, const b2d_obb* dets_dev, const int32_t* counts_dev, const double* params_dev, int n, int cap,
+                       float conf_thr, float iou_thr, uint8_t* keep_dev, void* stream);
+
 /* Greedy centre-distance dedup in a metric CRS.  Replaces SimpleDetector._remove_duplicates
  * (simple_detector.py:558-596, inclusive=1) and ResultsManager.remove_duplicates
  * (_script/utils.py:229-256, inclusive=0).  Priority = conf desc, then tiebreak_dev asc
